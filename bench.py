@@ -2,7 +2,7 @@
 """bench.py — DeformConv2d fwd+bwd images/sec on B200 (the metric of BASELINE.json).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload cfg2|cfg3|det2|det5]
-                    [--variant torch|jittor] [--impl ours|reference]
+                    [--variant torch|jittor] [--impl ours|reference] [--dump-outputs DIR]
     torchrun ... bench.py --gpus N ...            (N > 1, one rank per GPU, NCCL)
 
 A "step" is one pass of the hot path (engine forward + backward through the C ABI,
@@ -114,7 +114,34 @@ def parse_args():
                          "channels-last hand-over between every post-op and the next layer (SURVEY 8f.2)")
     ap.add_argument("--stock-bn", action="store_true",
                     help="detector workload: the framework's BatchNorm2d + ReLU instead of the engine's fused post-op")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="single-layer workloads: write what the last timed step computed on rank 0 (output and "
+                         "gradients) as DIR/<name>.npy in float32, at most 64 MB in all: a larger array as a fixed, seeded "
+                         "sample of its elements")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+DUMP_BUDGET_BYTES = 64 * 10**6
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes each tensor of `arrays` ({name: tensor}) as out_dir/<name>.npy in float32.  Every file gets an equal share
+    of DUMP_BUDGET_BYTES; an array larger than its share is stored as a fixed sample, the flattened array's elements at
+    sorted(numpy.random.default_rng(0).choice(numel, share, replace=False)), so that runs with the same arguments store
+    the same positions and two builds can be compared element for element."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    share = (DUMP_BUDGET_BYTES // len(arrays) - 256) // 4          # elements; 256 bytes per file for the .npy header
+    for name, t in arrays.items():
+        t = t.detach()
+        if t.numel() > share:
+            idx = np.sort(np.random.default_rng(0).choice(t.numel(), share, replace=False))
+            t = t.reshape(-1)[torch.as_tensor(idx, device=t.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), t.float().cpu().numpy())
 
 
 def peaks():
@@ -663,6 +690,8 @@ def measure_other_configs(args, dev, variant):
 def main():
     args = parse_args()
     claim_stdout()
+    if args.dump_outputs and (args.workload in ("stack", "detector") or args.impl == "reference"):
+        raise SystemExit("--dump-outputs supports the single-layer workloads of --impl ours")
     if args.workload == "stack":
         if args.impl == "reference":
             raise SystemExit("--impl reference supports the single-layer workloads")
@@ -738,15 +767,17 @@ def main():
         ws = layer_workspace(x, wt, k, s, p, variant, flags)
 
     def step():
+        """-> {name: tensor} of what the caller of the timed path receives"""
         if layer_scope:
             off_l, out = dcn_layer_forward(x, w_off, b_off, wt, bias, k, s, p, variant, flags, ws=ws)
             gx, gwo, gbo, gw, gb = dcn_layer_backward(x, off_l, w_off, wt, gout, True, True, k, s, p, variant, flags,
                                                       ws=ws, xt_staged=True)
-            goff = None
+            res = {"offset": off_l, "out": out, "grad_x": gx, "grad_offset_weight": gwo, "grad_offset_bias": gbo}
         else:
             out = dcn.dcn_forward(x, off, wt, bias, k, s, p, variant, operand=operand, flags=flags, ws=ws)
             gx, goff, gw, gb = dcn.dcn_backward(x, off, wt, gout, True, k, s, p, variant, operand=operand, flags=flags,
                                                 ws=ws, xt_staged=ws is not None)
+            res = {"out": out, "grad_x": gx, "grad_offset": goff}
         if comm is not None:
             bucket[:n_w].copy_(gw.view(-1))
             bucket[n_w:n_w + n_b].copy_(gb)
@@ -754,7 +785,8 @@ def main():
                 bucket[n_w + n_b:n_w + n_b + n_ow].copy_(gwo.view(-1))
                 bucket[n_w + n_b + n_ow:].copy_(gbo)
             comm.allreduce_mean_(bucket)
-        return out, gx, goff
+        res.update(grad_weight=gw, grad_bias=gb)
+        return res
 
     def barrier():
         if world > 1:
@@ -777,23 +809,30 @@ def main():
     flush_buf = torch.empty(512 << 20, dtype=torch.uint8, device=dev) if needs_flush else None
     ev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True))
           for _ in range(args.steps if needs_flush else 1)]
+    # the last step's results are kept for --dump-outputs; every step first drops its predecessor's, so that the
+    # allocator reuses the same buffers as in the warm-up steps
     barrier()
     if needs_flush:
         for a, b in ev:
+            outs = None
             flush_buf.fill_(1)
             a.record(stream)
-            step()
+            outs = step()
             b.record(stream)
     else:
         ev[0][0].record(stream)
         for _ in range(args.steps):
-            step()
+            outs = None
+            outs = step()
         ev[0][1].record(stream)
     barrier()
     elapsed_ms = sum(a.elapsed_time(b) for a, b in ev)
     launches = int(lib.dcn_launch_count())
     prof = _lib.profile_end()
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, outs)
+    del outs
     if world > 1:
         t = torch.tensor([elapsed_ms], device=dev)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)

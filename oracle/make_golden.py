@@ -33,6 +33,9 @@ import torch.nn as tnn
 from . import ref_loader, torch_chain
 
 OUT = os.path.join(os.path.dirname(os.path.abspath(__file__)), "..", "tests", "golden")
+# torch's CPU kernels split their sums by thread: the goldens in tests/golden/ were made with 8 threads, and
+# tests/test_oracle_golden.py runs its bitwise torch comparisons at that count to reproduce them on any host
+GOLDEN_CPU_THREADS = 8
 
 
 def _save(name, **arrays):
@@ -335,7 +338,7 @@ def make_dcnv1(rng):
 def main():
     assert ref_loader.available(), "needs /root/reference (build container only)"
     os.makedirs(OUT, exist_ok=True)
-    torch.set_num_threads(max(1, os.cpu_count() or 1))
+    torch.set_num_threads(GOLDEN_CPU_THREADS)
     if "--only-module-umma" in sys.argv:
         make_module_umma_goldens()
         return 0

@@ -62,8 +62,18 @@ def test_c_oracle_matches_reference_layer(name):
         assert rel_err(gb, g["gb"]) < 5e-6
 
 
+@pytest.fixture
+def golden_cpu_threads():
+    """torch's CPU convolution and GEMM kernels split their sums by thread, so a golden made by a multi-threaded CPU run
+    is reproduced bit for bit only at the thread count it was made with (oracle/make_golden.py: GOLDEN_CPU_THREADS)."""
+    n = torch.get_num_threads()
+    torch.set_num_threads(8)
+    yield
+    torch.set_num_threads(n)
+
+
 @pytest.mark.parametrize("name", golden_names("layer_") + golden_names("umma_") + golden_names("gemm_"))
-def test_torch_chain_is_bitwise_the_reference(name):
+def test_torch_chain_is_bitwise_the_reference(name, golden_cpu_threads):
     """Same torch ops in the same order => identical bits (forward and autograd)."""
     g = golden(name)
     B, C, O, H, W, kh, kw, sh, sw, ph, pw = (int(v) for v in g["cfg"])
@@ -128,7 +138,7 @@ def test_dcnv1_oracle_matches_torchvision(name):
     assert rel_err(gb, g["gb"]) < 5e-6
 
 
-def test_harness_detector_with_the_chain_port_reproduces_the_reference_training_step():
+def test_harness_detector_with_the_chain_port_reproduces_the_reference_training_step(golden_cpu_threads):
     """The harness detector topology (jittor_dcn_b200/detector.py) with its DCN layers replaced by the CPU port of
     the reference's op chain (oracle/torch_chain.py) and the framework's BatchNorm2d + ReLU is the reference
     detector restated: one training step (train mode, loss of train.py:242-248) must reproduce the golden made by
