@@ -2,7 +2,6 @@
 // dispatch to a kernel family.  No torch types, no allocation, no device synchronisation.
 #include <cstdarg>
 #include <cstdio>
-#include <cstdlib>
 #include <cstring>
 #include <atomic>
 #include <map>
@@ -30,38 +29,6 @@ void set_error(const char* fmt, ...) {
 int cuda_fail(cudaError_t e, const char* what) {
   set_error("CUDA error %d (%s) at %s", (int)e, cudaGetErrorString(e), what);
   return DCN_ERR_CUDA;
-}
-
-static int env_int(const char* name, int dflt) {
-  const char* e = getenv(name);
-  return e ? atoi(e) : dflt;
-}
-static int env_set(const char* name) { return getenv(name) != nullptr; }
-
-const Knobs& knobs() {
-  // C++11 magic static: initialised once, thread-safe
-  static const Knobs k = [] {
-    Knobs v;
-    v.fwd_no_tma_out = env_set("DCN_FWD_NO_TMA_OUT");
-    v.fwd_stages = env_int("DCN_FWD_STAGES", 3);
-    v.fwd_no_kperm = env_set("DCN_FWD_NO_KPERM");
-    v.fwd_no_split88 = env_set("DCN_FWD_NO_SPLIT88");
-    v.bwd_no_resident = env_set("DCN_BWD_NO_RESIDENT");
-    v.bwd_no_ring1 = env_set("DCN_BWD_NO_RING1");
-    v.bwd_slice_cb = env_int("DCN_BWD_SLICE_CB", 6);
-    v.bwd_no_fuse = env_int("DCN_BWD_NO_FUSE", 0);
-    v.bwd_gbuf1 = env_int("DCN_BWD_GBUF", 0) == 1;
-    v.bwd_data_simt = env_int("DCN_BWD_DATA_SIMT", 0);
-    v.conv_off = env_set("DCN_CONV_OFF");
-    v.gemm_off = env_set("DCN_GEMM_OFF");
-    v.gemm_sgemm = env_set("DCN_GEMM_SGEMM");
-    v.conv_small_c = env_set("DCN_CONV_SMALL_C");
-    v.conv_small_off = env_set("DCN_CONV_SMALL_OFF");
-    v.conv_debug = env_set("DCN_CONV_DEBUG");
-    v.conv_wstream = env_set("DCN_CONV_WSTREAM");
-    return v;
-  }();
-  return k;
 }
 
 void count_launch(int n) { g_launches.fetch_add((uint64_t)n, std::memory_order_relaxed); }

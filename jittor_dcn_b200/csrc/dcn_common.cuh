@@ -243,34 +243,6 @@ struct KernelScope {
 
 static inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
-// Tuning knobs for A/B measurements (INTEGRATION.md "Tuning knobs").  The environment is read ONCE, on the first
-// call into the library; afterwards the dispatch path touches no process-global state.  Defaults = production.
-struct Knobs {
-  int fwd_no_tma_out;   // DCN_FWD_NO_TMA_OUT   forward epilogue: direct stores instead of the staged tensor-map store
-  int fwd_stages;       // DCN_FWD_STAGES       forward pipeline depth wanted (2..4, default 3)
-  int fwd_no_kperm;     // DCN_FWD_NO_KPERM     pixel-row layouts: walk the K blocks tap-major
-  int bwd_no_resident;  // DCN_BWD_NO_RESIDENT  fused backward: always stream the Wm^T images through the ring
-  int bwd_no_ring1;     // DCN_BWD_NO_RING1     fused backward: never take the 1-stage ring plan
-  int bwd_slice_cb;     // DCN_BWD_SLICE_CB     fused backward (Torch layout): max column blocks per slice (1..6)
-  int fwd_no_split88;   // DCN_FWD_NO_SPLIT88   forward, Torch layout with 16 channels per sampling point: 4 plan + 16 gather warps
-                        //                      like every other shape instead of 8 + 8
-  int bwd_no_fuse;      // DCN_BWD_NO_FUSE      weight gradient as its own pass
-  int bwd_gbuf1;        // DCN_BWD_GBUF=1       one grad_out tile buffer
-  int bwd_data_simt;    // DCN_BWD_DATA_SIMT    fp32 data gradient on the generic kernels
-  int conv_wstream;     // DCN_CONV_WSTREAM     shifted-view conv: stream the weight tap images per K step even when they fit
-  int conv_debug;       // DCN_CONV_DEBUG       shifted-view conv: print per-role wait / work cycle counters of CTA 0
-  int conv_small_c;     // DCN_CONV_SMALL_C     shifted-view conv also for 16 / 32 input channels (slower; for A/B runs)
-  int conv_small_off;   // DCN_CONV_SMALL_OFF   companion offset conv of layers with < 64 input channels: plain mode of the
-                        //                      DCN kernels instead of the warp-MMA kernels (dcn_conv_small.cu)
-  int gemm_sgemm;       // DCN_GEMM_SGEMM       GEMM path, fp32 operands: true-fp32 cuBLAS GEMMs instead of three bf16 tensor-core
-                        //                      GEMMs over (hi, lo) splits
-  int gemm_off;         // DCN_GEMM_OFF         Torch layout with gcd(HoWo, C) % 16 != 0: generic kernels instead of the
-                        //                      materialised-sample + cuBLAS path (dcn_gemm_path.cu)
-  int conv_off;         // DCN_CONV_OFF         companion offset conv: the plain mode of the DCN kernels instead of the
-                        //                      shifted-view convolution kernels (dcn_conv.cu)
-};
-const Knobs& knobs();
-
 // ---- kernel families (each returns a DcnStatus) --------------------------------------
 // plan: Tap per (b, q); stored in q-order [b][p][n] (Torch) or tap-major [b][n][p] (Jittor)
 int launch_plan(const Geo& g, const float* off, Tap* plan, cudaStream_t st);

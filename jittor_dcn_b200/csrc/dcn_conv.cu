@@ -28,7 +28,6 @@
 // Warp roles (960 threads, 1 CTA / SM, persistent): warps 0-3 epilogue, 4 MMA issuer, 5 bulk loader (weight tap
 // images), 6-29 conversion (global -> bf16 hi/lo -> swizzled shared memory; all loads of a K step are issued before
 // the first conversion).  fp32 parity as in the DCN kernels: hi*hi + hi*lo + lo*hi, fp32 accumulation in TMEM.
-#include <cstdio>
 #include <cstring>
 
 #include "dcn_umma.h"
@@ -50,6 +49,7 @@ constexpr uint32_t kImgRows = 136;                 // 128 GEMM rows + shifted vi
 constexpr uint32_t kImg = kImgRows * 128;          // one bf16 image: 17408 B = 17 * 1024
 constexpr int kMaxItems = 3;                       // conversion items per thread and K step (x image)
 constexpr int kMaxStages = 3;
+constexpr int kSlab = 64;                          // channels of one K slab of the x image (FWD / WGRAD): one 128 B row
 
 struct Params {
   // the convolution: x[B, C, H, W] -> [B, O, Ho, Wo], kernel kh x kw, stride s, padding p (both axes)
@@ -62,9 +62,8 @@ struct Params {
   int ncolseg, nrowt;         // column segments per row, row tiles per image
   int nchunks_n;              // DGRAD: 64-channel chunks of C handled as separate tiles
   int num_tiles;
-  int Ks;                     // channels of one K slab of the x image: min(C, 64) (FWD / WGRAD)
-  int nslab;                  // FWD: C / Ks
-  int nk4;                    // K = 16 steps per image: Ks / 16 (FWD), ceil(O / 16) (DGRAD)
+  int nslab;                  // FWD: C / kSlab
+  int nk4;                    // K = 16 steps per image: kSlab / 16 (FWD), ceil(O / 16) (DGRAD)
   int Nn;                     // MMA N: o_pad (FWD, WGRAD), channels per chunk (DGRAD)
   int nph;                    // phase images per stage: s (FWD / WGRAD), 1 (DGRAD)
   int ncols_in;               // input columns one image row holds, all phases together
@@ -88,7 +87,6 @@ struct Params {
   int pitch;                  // elements per frame row
   // WGRAD: CTA = (slab, chunk of tiles)
   int w_nchunks;
-  long long* dbg;             // DCN_CONV_DEBUG: per-role wait / work cycle counters of CTA 0 (null = off)
 };
 
 struct TileInfo {
@@ -123,9 +121,6 @@ __device__ __forceinline__ int dgrad_acc(const Params& P, int ki, int kj) {
   return P.s == 1 ? 0 : ((ki == 1 ? 2 : 0) + (kj == 1 ? 1 : 0));
 }
 
-#define CV_T0() const long long _t0 = dbg_on ? clock64() : 0
-#define CV_T1(slot) do { if (dbg_on) dbg_acc[slot] += clock64() - _t0; } while (0)
-
 template <int MODE>
 __global__ void __launch_bounds__(kThreads, 1) conv_kernel(const __grid_constant__ Params P) {
   extern __shared__ __align__(1024) uint8_t smem_raw[];
@@ -147,9 +142,6 @@ __global__ void __launch_bounds__(kThreads, 1) conv_kernel(const __grid_constant
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(wfull + 1);
 
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  const bool dbg_on = P.dbg != nullptr && blockIdx.x == 0 && lane == 0;
-  long long dbg_acc[4] = {0, 0, 0, 0};
-  const long long dbg_start = dbg_on ? clock64() : 0;
   const bool wstream = MODE != MODE_WGRAD && !P.w_res;   // weight tap images arrive by bulk copy, once per K step
   if (tid == 0) {
     for (int s = 0; s < P.stages; ++s) {
@@ -206,7 +198,7 @@ __global__ void __launch_bounds__(kThreads, 1) conv_kernel(const __grid_constant
         const int r = ti.r0 + hr, c = ti.c0 + wl;
         const bool valid = r < P.GR && wl < P.Wt && c < P.GC;
         float* dst = P.out + (size_t)ti.b * P.O * P.Ho * P.Wo + (size_t)r * P.Wo + c;
-        { CV_T0(); mbar_wait_relaxed(&tfull[acc], acc_phase); CV_T1(0); }
+        mbar_wait_relaxed(&tfull[acc], acc_phase);
         tc_fence_after();
         const uint32_t taddr = tmem_base + ((uint32_t)(warp * 32) << 16) + (uint32_t)(acc * 2 * P.Nn);
         for (int c0 = 0; c0 < P.Nn; c0 += 16) {
@@ -280,7 +272,7 @@ __global__ void __launch_bounds__(kThreads, 1) conv_kernel(const __grid_constant
       // WGRAD: one-shot epilogue.  TMEM lane = staged channel of the slab, columns = (tap, o)
       mbar_wait_relaxed(&tfull[0], 0);
       tc_fence_after();
-      const int cs = slab0 * P.Ks + m;   // staged channel
+      const int cs = slab0 * kSlab + m;   // staged channel
       int c_real = cs;
       if (P.perm_G) c_real = (cs % P.perm_G) * P.perm_Cs + cs / P.perm_G;
       const int ntaps = P.kh * P.kw;
@@ -289,7 +281,7 @@ __global__ void __launch_bounds__(kThreads, 1) conv_kernel(const __grid_constant
         for (int c0 = 0; c0 < P.Nn; c0 += 16) {
           float v[16];
           tmem_ld16(taddr + c0, v);
-          if (m < P.Ks) {
+          if (m < kSlab) {
 #pragma unroll
             for (int i = 0; i < 16; ++i)
               if (c0 + i < P.O) atomicAdd(P.gw + ((size_t)(c0 + i) * P.C + c_real) * ntaps + t, v[i]);
@@ -324,12 +316,12 @@ __global__ void __launch_bounds__(kThreads, 1) conv_kernel(const __grid_constant
         }
         for (int tile = tile0; tile < P.num_tiles; tile += tile_step) {
           const int nch = MODE == MODE_DGRAD ? decode_tile(P, tile).nch : 0;
-          { CV_T0(); mbar_wait_relaxed(&tempty[acc], acc_phase ^ 1, 32); CV_T1(0); }
+          mbar_wait_relaxed(&tempty[acc], acc_phase ^ 1, 32);
           tc_fence_after();
           uint32_t started = 0;   // accumulators that already hold a partial sum
           for (int ks = 0; ks < ksteps; ++ks) {
             const int ki = MODE == MODE_FWD ? ks % P.kh : ks;
-            { CV_T0(); mbar_wait_relaxed(&full[s], phase, 20); CV_T1(1); }
+            mbar_wait_relaxed(&full[s], phase, 20);
             tc_fence_after();
             const uint64_t ad = desc0 + (uint64_t)((uint32_t)s * stage16);
             // streamed: the K step's kw tap images sit behind the phase images of the stage; resident: image
@@ -501,8 +493,7 @@ __global__ void __launch_bounds__(kThreads, 1) conv_kernel(const __grid_constant
     if constexpr (MODE != MODE_DGRAD) {
       // x image: items = (row hr, input column j, 4-channel quad); the decomposition does not depend on the tile.
       // packed item: bits 0..16 byte offset inside the stage, 17..24 column j, 25..27 row hr, 28 live
-      const int q4 = P.Ks >> 2;                               // quads per pixel: 4, 8 or 16 (power of two)
-      const int q4_sh = q4 == 16 ? 4 : (q4 == 8 ? 3 : 2);
+      constexpr int q4 = kSlab / 4, q4_sh = 4;                // 16 quads of 4 channels per pixel
       const int n_items = P.rpt * P.ncols_in * q4;
       uint32_t src_off[kMaxItems], item[kMaxItems];
 #pragma unroll
@@ -523,7 +514,7 @@ __global__ void __launch_bounds__(kThreads, 1) conv_kernel(const __grid_constant
       auto issue = [&](const Step& q, float4 (&v)[kMaxItems], uint32_t& ok) {
         const int slab = MODE == MODE_FWD ? q.ks / P.kh : slab0, ki = MODE == MODE_FWD ? q.ks % P.kh : q.ks;
         const int fy0 = q.ti.r0 * P.s + ki + 1 - P.p, fx0 = q.ti.c0 * P.s + 1 - P.p;
-        const float* base = P.xt + (size_t)q.ti.b * P.img_stride + ((size_t)fy0 * (P.W + 2) + fx0) * P.C + slab * P.Ks;
+        const float* base = P.xt + (size_t)q.ti.b * P.img_stride + ((size_t)fy0 * (P.W + 2) + fx0) * P.C + slab * kSlab;
         ok = 0;
 #pragma unroll
         for (int i = 0; i < kMaxItems; ++i) {
@@ -572,9 +563,8 @@ __global__ void __launch_bounds__(kThreads, 1) conv_kernel(const __grid_constant
             if (gb == 0) gphase ^= 1;
           }
         }
-        { CV_T0(); mbar_wait(&empty[s], phase ^ 1); CV_T1(0); }
+        mbar_wait(&empty[s], phase ^ 1);
         uint8_t* st = stage_base + (size_t)s * P.stage_bytes;
-        CV_T0();
 #pragma unroll
         for (int i = 0; i < kMaxItems; ++i) {
           if (!((ok >> i) & 1u)) continue;
@@ -585,8 +575,7 @@ __global__ void __launch_bounds__(kThreads, 1) conv_kernel(const __grid_constant
           *reinterpret_cast<uint2*>(d) = hi;
           *reinterpret_cast<uint2*>(d + kImg) = lo;
         }
-        CV_T1(1);
-        { CV_T0(); publish(); CV_T1(2); }
+        publish();
       };
       float4 va[kMaxItems], vb[kMaxItems];
       uint32_t oka = 0, okb = 0;
@@ -673,11 +662,6 @@ __global__ void __launch_bounds__(kThreads, 1) conv_kernel(const __grid_constant
     }
   }
 
-  if (dbg_on) {
-    long long* o = P.dbg + warp * 8;
-    o[0] = clock64() - dbg_start;
-    for (int i = 0; i < 4; ++i) o[1 + i] = dbg_acc[i];
-  }
   tc_fence_before();
   __syncthreads();
   if (warp == 0) {
@@ -694,19 +678,9 @@ __global__ void __launch_bounds__(256) conv_weight_tiles_kernel(Params P, int dg
   const int total = groups * ntaps * P.Nn * 64;
   for (int i = blockIdx.x * 256 + threadIdx.x; i < total; i += gridDim.x * 256) {
     const int k = i & 63, row = (i >> 6) % P.Nn, t = (i / (64 * P.Nn)) % ntaps, grp = i / (64 * P.Nn * ntaps);
-    int o, cs;
-    bool ok;
-    if (dgrad) {
-      cs = grp * 64 + row;
-      o = k;
-      ok = row < (P.C < 64 ? P.C : 64) && cs < P.C && o < P.O;
-    } else {
-      cs = grp * P.Ks + k;
-      o = row;
-      ok = k < P.Ks && o < P.O;
-    }
+    const int cs = grp * 64 + (dgrad ? row : k), o = dgrad ? k : row;
     float v = 0.f;
-    if (ok) {
+    if (o < P.O) {
       int c = cs;
       if (P.perm_G) c = (cs % P.perm_G) * P.perm_Cs + cs / P.perm_G;
       v = w[((size_t)o * P.C + c) * ntaps + t];
@@ -747,8 +721,7 @@ static bool conv_params(const Geo& g, int mode, cv::Params* Pp) {
   // 16-column steps x hi/lo terms) dominates and the plain mode of the DCN kernels, which packs (tap, channel) pairs
   // into its K blocks, is faster (measured on the detector's 16- and 32-channel layers: backward 6.6 vs 2.8 ms).  Those
   // layers run on the warp-MMA kernels of dcn_conv_small.cu instead (conv_offset_*_supported below).
-  if (g.C % 64 != 0 && !knobs().conv_small_c) return false;
-  if (!(g.C == 16 || g.C == 32 || g.C % 64 == 0)) return false;
+  if (g.C % 64 != 0) return false;
   const int O = 2 * g.N;
   if (O > 32) return false;
   // every read stays inside the framed copy
@@ -799,17 +772,15 @@ static bool conv_params(const Geo& g, int mode, cv::Params* Pp) {
   if (mode == cv::MODE_DGRAD) {
     P.ncols_in = P.Wt + extra;
     P.ne0 = P.ncols_in;
-    P.Ks = 64;
     P.nslab = 1;
     P.nk4 = (O + 15) / 16;
-    P.Nn = g.C < 64 ? g.C : 64;
-    P.nchunks_n = (g.C + 63) / 64;
+    P.Nn = 64;
+    P.nchunks_n = g.C / 64;
   } else {
     P.ncols_in = (P.Wt - 1) * P.s + P.kw;
     P.ne0 = (P.ncols_in + P.s - 1) / P.s;
-    P.Ks = g.C < 64 ? g.C : 64;
-    P.nslab = g.C / P.Ks;
-    P.nk4 = P.Ks / 16;
+    P.nslab = g.C / cv::kSlab;
+    P.nk4 = cv::kSlab / 16;
     P.Nn = (O + 15) / 16 * 16;
     P.nchunks_n = 1;
   }
@@ -827,7 +798,7 @@ static bool conv_params(const Geo& g, int mode, cv::Params* Pp) {
   const size_t all_w = (size_t)(mode == cv::MODE_DGRAD ? P.nchunks_n : P.nslab) * P.kh * P.kw * 2 * P.w_tile;
   P.w_res = 0;
   P.w_res_bytes = 0;
-  if (mode != cv::MODE_WGRAD && !knobs().conv_wstream && fixed + all_w + 2 * img_bytes <= 227 * 1024) {
+  if (mode != cv::MODE_WGRAD && fixed + all_w + 2 * img_bytes <= 227 * 1024) {
     P.w_res = 1;
     P.w_res_bytes = (uint32_t)all_w;
   }
@@ -838,8 +809,7 @@ static bool conv_params(const Geo& g, int mode, cv::Params* Pp) {
   if (stages < 2) return false;
   P.stages = stages;
   // conversion items per thread
-  const int per_px = mode == cv::MODE_DGRAD ? 0 : (P.Ks >> 2);
-  if (mode != cv::MODE_DGRAD && (P.rpt * P.ncols_in * per_px + cv::kConvThreads - 1) / cv::kConvThreads > cv::kMaxItems)
+  if (mode != cv::MODE_DGRAD && (P.rpt * P.ncols_in * (cv::kSlab / 4) + cv::kConvThreads - 1) / cv::kConvThreads > cv::kMaxItems)
     return false;
   if (mode == cv::MODE_DGRAD && (P.rpt * P.ncols_in * P.nk4 * 2 + cv::kConvThreads - 1) / cv::kConvThreads > 2) return false;
   if (P.ncols_in > 255 || P.rpt > 8) return false;   // packed item fields
@@ -873,11 +843,9 @@ static bool conv_bwd_shifted(const Geo& g) {
 }
 
 bool conv_offset_fwd_supported(const Geo& g) {
-  if (knobs().conv_off) return false;
   return conv_fwd_shifted(g) || conv_small_supported(g);
 }
 bool conv_offset_bwd_supported(const Geo& g) {
-  if (knobs().conv_off) return false;
   // measured on the detector's layers (batch 1024): the warp-MMA backward wins below 64 channels (conv2 1.4 vs 1.8 ms,
   // conv3 0.7 vs 0.7 ms); at 64 / 128 channels the plain mode of the fused DCN backward kernel is faster (0.23 vs 0.35 ms)
   return conv_bwd_shifted(g) || (g.C < 64 && conv_small_supported(g));
@@ -901,24 +869,6 @@ template <int MODE>
 static int conv_launch(const cv::Params& P, int grid, cudaStream_t st, const char* name) {
   const size_t smem = conv_smem(P, MODE);
   DCN_CUDA_TRY(cudaFuncSetAttribute(cv::conv_kernel<MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  if (knobs().conv_debug) {
-    cv::Params Q = P;
-    long long* d = nullptr;
-    cudaMalloc(&d, 32 * 8 * sizeof(long long));
-    cudaMemset(d, 0, 32 * 8 * sizeof(long long));
-    Q.dbg = d;
-    cv::conv_kernel<MODE><<<grid, cv::kThreads, smem, st>>>(Q);
-    cudaStreamSynchronize(st);
-    long long h[32 * 8];
-    cudaMemcpy(h, d, sizeof(h), cudaMemcpyDeviceToHost);
-    cudaFree(d);
-    fprintf(stderr, "[conv dbg] %s tiles %d stages %d w_res %d\n", name, P.num_tiles, P.stages, P.w_res);
-    for (int w = 0; w < cv::kThreads / 32; ++w)
-      if (w < 7 || w == cv::kThreads / 32 - 1)
-        fprintf(stderr, "[conv dbg]   warp %2d total %lld | %lld %lld %lld %lld\n", w, h[w * 8], h[w * 8 + 1], h[w * 8 + 2],
-                h[w * 8 + 3], h[w * 8 + 4]);
-    return DCN_OK;
-  }
   KernelScope scope(name, st);
   cv::conv_kernel<MODE><<<grid, cv::kThreads, smem, st>>>(P);
   DCN_KERNEL_CHECK(name);

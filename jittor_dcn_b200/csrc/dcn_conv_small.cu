@@ -418,7 +418,7 @@ static int small_sms() {
 
 bool conv_small_supported(const Geo& g) {
   cs::Params P;
-  return !knobs().conv_small_off && small_params(g, &P);
+  return small_params(g, &P);
 }
 
 // fragment scratch: the forward and the data-gradient pass run one after the other and share it

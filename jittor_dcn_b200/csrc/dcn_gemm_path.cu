@@ -12,8 +12,9 @@
 //   data gradient gS_b[HW, K]   = gout_b^T[HW, O] * Wm[O, K]   -> scatter kernel (bilinear col2im + coordinate gradient)
 //   weight grad   gW[O, K]      = goutT[O, B*HW] * A[B*HW, K]
 // Plain library GEMMs go to cuBLAS (dlopen'ed like NCCL: no link-time dependency; inside a PyTorch process this binds
-// to the libcublas.so.12 torch already loaded).  fp32 operands: CUBLAS_COMPUTE_32F on float data (no TF32); bf16
-// operands: bf16 x bf16 -> fp32 accumulate, S and gS stored in bf16 (one rounding of each sample, as the tensor path).
+// to the libcublas.so.12 torch already loaded).  Every GEMM is bf16 x bf16 -> fp32 accumulate.  fp32 operands: three
+// GEMMs over (hi, lo) bfloat16 splits (see gemm_path_forward); bf16 operands: one GEMM, S and gS stored in bf16 (one
+// rounding of each sample, as the tensor path).
 #include <cublas_v2.h>
 #include <cuda_bf16.h>
 #include <dlfcn.h>
@@ -109,12 +110,11 @@ __device__ __forceinline__ Corner corner_of(const Geo& g, const Tap& tp) {
 // S[b, c, q] = bilinear sample of channel c at sampling point q (deform_conv.py:47-52 / train.py:121-127).
 // Block = 32 points of one image; loop over 128-channel tiles: warps gather point by point (lane = channel: 128-byte
 // coalesced corner reads), the tile is transposed through shared memory and written with lane = point.
-// SPLIT (fp32 operands): S is written as TWO bfloat16 matrices, hi = bf16(v) and lo = bf16(v - hi), for the three-term
-// tensor-core GEMMs (see gemm_path_forward)
-template <typename T, bool SPLIT>
+// fp32 operands (T = float): S is written as TWO bfloat16 matrices, hi = bf16(v) into S and lo = bf16(v - hi) into S_lo,
+// for the three-term tensor-core GEMMs (see gemm_path_forward); bf16 operands: S only
+template <typename T>
 __global__ void __launch_bounds__(256) sample_kernel(Geo g, const T* __restrict__ xt, const Tap* __restrict__ plan,
-                                                     T* __restrict__ S, __nv_bfloat16* __restrict__ S_hi,
-                                                     __nv_bfloat16* __restrict__ S_lo) {
+                                                     __nv_bfloat16* __restrict__ S, __nv_bfloat16* __restrict__ S_lo) {
   __shared__ float tile[kQT][kCT + 1];
   const int b = blockIdx.y, q0 = blockIdx.x * kQT;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -151,10 +151,10 @@ __global__ void __launch_bounds__(256) sample_kernel(Geo g, const T* __restrict_
       const int cl = warp + 8 * j, c = c0 + cl;
       if (c < g.C && q < g.P) {
         const size_t idx = ((size_t)b * g.C + c) * g.P + q;
-        if (SPLIT) {
+        if constexpr (sizeof(T) == 4) {
           __nv_bfloat16 hi, lo;
           ptx::split_bf16(tile[lane][cl], hi, lo);
-          S_hi[idx] = hi;
+          S[idx] = hi;
           S_lo[idx] = lo;
         } else {
           S[idx] = (T)tile[lane][cl];
@@ -255,13 +255,13 @@ __global__ void __launch_bounds__(256) bias_fill_kernel(int B, int O, int Oimg, 
   }
 }
 
-// goutT[o, b*HW + p] = gout[b, o, p]: rows of HW elements re-ordered (o, b)
-template <typename T>
-__global__ void __launch_bounds__(256) gout_rows_kernel(int B, int O, int Oimg, int HW, const T* __restrict__ gout,
-                                                        T* __restrict__ goutT) {
+// goutT[o, b*HW + p] = gout[b, o, p]: rows of HW elements re-ordered (o, b)  (bf16 operands)
+__global__ void __launch_bounds__(256) gout_rows_kernel(int B, int O, int Oimg, int HW,
+                                                        const __nv_bfloat16* __restrict__ gout,
+                                                        __nv_bfloat16* __restrict__ goutT) {
   const int o = blockIdx.x, b = blockIdx.y;
-  const T* src = gout + ((size_t)b * Oimg + o) * HW;
-  T* dst = goutT + ((size_t)o * B + b) * HW;
+  const __nv_bfloat16* src = gout + ((size_t)b * Oimg + o) * HW;
+  __nv_bfloat16* dst = goutT + ((size_t)o * B + b) * HW;
   for (int p = threadIdx.x; p < HW; p += 256) dst[p] = src[p];
 }
 
@@ -303,7 +303,6 @@ static size_t gp_plan_bytes(const Geo& g) { return align_up(sizeof(Tap) * (size_
 static size_t gp_S_bytes(const Geo& g, int operand) { return align_up(gp_esz(operand) * (size_t)g.B * g.C * g.P, 1024); }
 
 bool gemm_path_supported(const Geo& g, int operand) {
-  if (knobs().gemm_off) return false;
   if (g.variant != DCN_VARIANT_TORCH || g.plain) return false;
   if (operand != DCN_OPERAND_FP32 && operand != DCN_OPERAND_BF16) return false;
   if (g.C % 4 || (operand == DCN_OPERAND_BF16 && g.C % 8)) return false;     // framed staging copy: 16-byte pixels
@@ -316,19 +315,20 @@ bool gemm_path_supported(const Geo& g, int operand) {
 // fp32 operands on tensor cores: every operand of the three GEMMs as a (hi, lo) bfloat16 pair, every product as
 // lo*hi + hi*lo + hi*hi with fp32 accumulation (the split of the tcgen05 kernels; relative error ~5e-6).  The true-fp32
 // cuBLAS GEMMs took 2.5 ms each for a C5 layer (47 TFLOP/s) against 0.5 ms for one bf16 GEMM.
-static bool gp_split(int operand) { return operand == DCN_OPERAND_FP32 && !knobs().gemm_sgemm; }
-static size_t gp_W_bytes(const Geo& g, int operand) { return gp_split(operand) ? align_up(4 * (size_t)g.O * g.K, 1024) : 0; }
+static size_t gp_W_bytes(const Geo& g, int operand) {
+  return operand == DCN_OPERAND_FP32 ? align_up(4 * (size_t)g.O * g.K, 1024) : 0;
+}
 static size_t gp_gout_bytes(const Geo& g, int operand) {
   return align_up(gp_esz(operand) * (size_t)g.B * g.O * g.HW, 1024);
 }
 
 // forward: [xt][plan][S][W hi|lo][cuBLAS workspace]; backward: [xt][plan][S][gS][gxt][goutT][gout hi|lo][W hi|lo][cuBLAS
-// workspace] — S and goutT hold (hi | lo) halves in split mode (same bytes as the fp32 matrix)
+// workspace] — S and goutT hold (hi | lo) halves for fp32 operands (same bytes as the fp32 matrix)
 size_t gemm_path_workspace(const Geo& g, int operand, int phase) {
   size_t b = umma_xt_bytes(g, operand) + gp_plan_bytes(g) + gp_S_bytes(g, operand) + gp_W_bytes(g, operand) + gp::kCublasWs;
   if (phase == DCN_PHASE_BACKWARD)
     b += gp_S_bytes(g, operand) + umma_xt_bytes(g, DCN_OPERAND_FP32) + gp_gout_bytes(g, operand) +
-         (gp_split(operand) ? gp_gout_bytes(g, operand) : 0);
+         (operand == DCN_OPERAND_FP32 ? gp_gout_bytes(g, operand) : 0);
   return b;
 }
 
@@ -360,13 +360,10 @@ static int gp_stage_and_sample(const Geo& g, int operand, const void* x, const f
   {
     KernelScope scope("gemm_sample_kernel", st);
     if (operand == DCN_OPERAND_BF16)
-      gp::sample_kernel<__nv_bfloat16, false><<<grid, 256, 0, st>>>(g, (const __nv_bfloat16*)xt, plan, (__nv_bfloat16*)S,
-                                                                    nullptr, nullptr);
-    else if (gp_split(operand))
-      gp::sample_kernel<float, true><<<grid, 256, 0, st>>>(g, (const float*)xt, plan, nullptr, (__nv_bfloat16*)S,
-                                                           (__nv_bfloat16*)S + (size_t)g.B * g.C * g.P);
+      gp::sample_kernel<__nv_bfloat16><<<grid, 256, 0, st>>>(g, (const __nv_bfloat16*)xt, plan, (__nv_bfloat16*)S, nullptr);
     else
-      gp::sample_kernel<float, false><<<grid, 256, 0, st>>>(g, (const float*)xt, plan, (float*)S, nullptr, nullptr);
+      gp::sample_kernel<float><<<grid, 256, 0, st>>>(g, (const float*)xt, plan, (__nv_bfloat16*)S,
+                                                     (__nv_bfloat16*)S + (size_t)g.B * g.C * g.P);
     DCN_KERNEL_CHECK("gemm_sample_kernel");
   }
   return DCN_OK;
@@ -384,7 +381,7 @@ int gemm_path_forward(const Geo& g, int operand, const void* x, const float* off
   if ((rc = gp_stage_and_sample(g, operand, x, off, ws, st, &xt, &plan, &S))) return rc;
   uint8_t* whl = (uint8_t*)S + gp_S_bytes(g, operand);
   uint8_t* cws = whl + gp_W_bytes(g, operand);
-  const bool split = gp_split(operand);
+  const bool split = operand == DCN_OPERAND_FP32;
   {
     KernelScope scope("gemm_bias_fill_kernel", st);
     gp::bias_fill_kernel<<<1024, 256, 0, st>>>(g.B, g.O, g.Oimg, g.HW, bias, out);
@@ -397,7 +394,6 @@ int gemm_path_forward(const Geo& g, int operand, const void* x, const float* off
     gp::split_flat_kernel<<<256, 256, 0, st>>>(nW, (const float*)wt, w_hi, w_lo);
     DCN_KERNEL_CHECK("gemm_split_kernel");
   }
-  const cudaDataType dt = operand == DCN_OPERAND_FP32 && !split ? CUDA_R_32F : CUDA_R_16BF;
   const float one = 1.f;
   cublasStatus_t cs;
   std::lock_guard<std::mutex> use(gp::g_use_mu);   // a cuBLAS handle must not be driven by two host threads at once
@@ -407,9 +403,9 @@ int gemm_path_forward(const Geo& g, int operand, const void* x, const float* off
   KernelScope scope("cublas_gemm_fwd", st);
   auto gemm = [&](const void* Sm, const void* Wm) {
     count_launch();
-    return gp::g_api.GemmStridedBatchedEx(h, CUBLAS_OP_T, CUBLAS_OP_N, g.HW, g.O, g.K, &one, Sm, dt, g.K, (long long)g.C * g.P,
-                                          Wm, dt, g.K, 0, &one, out, CUDA_R_32F, g.HW, (long long)g.Oimg * g.HW, g.B,
-                                          CUBLAS_COMPUTE_32F, CUBLAS_GEMM_DEFAULT);
+    return gp::g_api.GemmStridedBatchedEx(h, CUBLAS_OP_T, CUBLAS_OP_N, g.HW, g.O, g.K, &one, Sm, CUDA_R_16BF, g.K,
+                                          (long long)g.C * g.P, Wm, CUDA_R_16BF, g.K, 0, &one, out, CUDA_R_32F, g.HW,
+                                          (long long)g.Oimg * g.HW, g.B, CUBLAS_COMPUTE_32F, CUBLAS_GEMM_DEFAULT);
   };
   if (split) {
     const __nv_bfloat16 *s_hi = (const __nv_bfloat16*)S, *s_lo = s_hi + nS;
@@ -435,12 +431,11 @@ int gemm_path_backward(const Geo& g, int operand, int flags, const void* x, cons
   uint8_t* gS = (uint8_t*)S + gp_S_bytes(g, operand);
   float* gxt = (float*)(gS + gp_S_bytes(g, operand));
   uint8_t* goutT = (uint8_t*)gxt + umma_xt_bytes(g, DCN_OPERAND_FP32);
-  const bool split = gp_split(operand);
+  const bool split = operand == DCN_OPERAND_FP32;
   uint8_t* ghl = goutT + gp_gout_bytes(g, operand);                       // split mode: compact grad_out, hi | lo
   uint8_t* whl = ghl + (split ? gp_gout_bytes(g, operand) : 0);
   uint8_t* cws = whl + gp_W_bytes(g, operand);
   const bool want_gx = !(flags & DCN_FLAG_NO_GRAD_X) && gx != nullptr;
-  const cudaDataType dt = operand == DCN_OPERAND_FP32 && !split ? CUDA_R_32F : CUDA_R_16BF;
   const cudaDataType dt_gs = operand == DCN_OPERAND_BF16 ? CUDA_R_16BF : CUDA_R_32F;   // gS feeds the scatter kernel
   const float one = 1.f, zero = 0.f;
   const size_t nS = (size_t)g.B * g.C * g.P, nW = (size_t)g.O * g.K, nG = (size_t)g.B * g.O * g.HW;
@@ -465,9 +460,9 @@ int gemm_path_backward(const Geo& g, int operand, int flags, const void* x, cons
     KernelScope scope("cublas_gemm_bwd_data", st);
     auto gemm = [&](const void* Wm, const void* Gm, long long gstride, const float* beta) {
       count_launch();
-      return gp::g_api.GemmStridedBatchedEx(h, CUBLAS_OP_N, CUBLAS_OP_T, g.K, g.HW, g.O, &one, Wm, dt, g.K, 0, Gm, dt, g.HW,
-                                            gstride, beta, gS, dt_gs, g.K, (long long)g.C * g.P, g.B, CUBLAS_COMPUTE_32F,
-                                            CUBLAS_GEMM_DEFAULT);
+      return gp::g_api.GemmStridedBatchedEx(h, CUBLAS_OP_N, CUBLAS_OP_T, g.K, g.HW, g.O, &one, Wm, CUDA_R_16BF, g.K, 0, Gm,
+                                            CUDA_R_16BF, g.HW, gstride, beta, gS, dt_gs, g.K, (long long)g.C * g.P, g.B,
+                                            CUBLAS_COMPUTE_32F, CUBLAS_GEMM_DEFAULT);
     };
     if (split) {
       const long long gs = (long long)g.O * g.HW;
@@ -502,12 +497,9 @@ int gemm_path_backward(const Geo& g, int operand, int flags, const void* x, cons
   // weight gradient: row-major gW[O, K] = goutT[O, B*HW] * A[B*HW, K]  <=>  column-major C'[K, O] = A'[K, BHW] * G'[BHW, O]
   if (!split) {
     KernelScope scope("gemm_gout_rows_kernel", st);
-    const dim3 grid((unsigned)g.O, (unsigned)g.B);
-    if (operand == DCN_OPERAND_BF16)
-      gp::gout_rows_kernel<__nv_bfloat16><<<grid, 256, 0, st>>>(g.B, g.O, g.Oimg, g.HW, (const __nv_bfloat16*)gout,
-                                                                (__nv_bfloat16*)goutT);
-    else
-      gp::gout_rows_kernel<float><<<grid, 256, 0, st>>>(g.B, g.O, g.Oimg, g.HW, (const float*)gout, (float*)goutT);
+    gp::gout_rows_kernel<<<dim3((unsigned)g.O, (unsigned)g.B), 256, 0, st>>>(g.B, g.O, g.Oimg, g.HW,
+                                                                             (const __nv_bfloat16*)gout,
+                                                                             (__nv_bfloat16*)goutT);
     DCN_KERNEL_CHECK("gemm_gout_rows_kernel");
   }
   {
@@ -515,8 +507,8 @@ int gemm_path_backward(const Geo& g, int operand, int flags, const void* x, cons
     const int bhw = g.B * g.HW;
     auto gemm = [&](const void* Sm, const void* Gm, const float* beta) {
       count_launch();
-      return gp::g_api.GemmEx(h, CUBLAS_OP_N, CUBLAS_OP_N, g.K, g.O, bhw, &one, Sm, dt, g.K, Gm, dt, bhw, beta, gw, CUDA_R_32F,
-                              g.K, CUBLAS_COMPUTE_32F, CUBLAS_GEMM_DEFAULT);
+      return gp::g_api.GemmEx(h, CUBLAS_OP_N, CUBLAS_OP_N, g.K, g.O, bhw, &one, Sm, CUDA_R_16BF, g.K, Gm, CUDA_R_16BF, bhw,
+                              beta, gw, CUDA_R_32F, g.K, CUBLAS_COMPUTE_32F, CUBLAS_GEMM_DEFAULT);
     };
     if (split) {
       if ((cs = gemm(s_lo, gT_hi, &zero)) == CUBLAS_STATUS_SUCCESS && (cs = gemm(s_hi, gT_lo, &one)) == CUBLAS_STATUS_SUCCESS)

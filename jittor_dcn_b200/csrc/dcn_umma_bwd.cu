@@ -34,11 +34,6 @@ Geo o_group_geo(const Geo& g, int o0, int size);
 
 static size_t plan_bytes(const Geo& g) { return align_up(sizeof(Tap) * (size_t)g.B * g.P, 1024); }
 
-static bool use_umma_data(const Geo& g, int operand) {
-  if (knobs().bwd_data_simt) return false;
-  return umma_bwd_data_supported(g, operand);
-}
-
 bool umma_bwd_supported(const Geo& g, int operand) {
   if (!umma_wgrad_supported(g, operand)) return false;
   // the generic data-gradient kernel is fp32 only: bf16 needs the tensor-path one
@@ -66,7 +61,7 @@ bool umma_layer_bwd_supported(const Geo& g) {
   int gsize;
   if (!o_groups(g, &gsize)) return false;
   const Geo g0 = o_group_geo(g, 0, gsize);
-  return umma_bwd_supported(g0, DCN_OPERAND_FP32) && use_umma_data(g0, DCN_OPERAND_FP32) && plain_bwd_ok(g);
+  return umma_bwd_supported(g0, DCN_OPERAND_FP32) && umma_bwd_data_supported(g0, DCN_OPERAND_FP32) && plain_bwd_ok(g);
 }
 
 static size_t goff_bytes(const Geo& g) { return align_up(sizeof(float) * (size_t)g.B * 2 * g.N * g.HW, 1024); }
@@ -128,7 +123,7 @@ int umma_backward_any(const Geo& g, int operand, int flags, const void* xv, cons
   if (!(flags & DCN_FLAG_XT_STAGED) && (rc = launch_nchw_to_nhwc(g, t, x, xt, operand, st))) return rc;
   const bool want_gx = !(flags & DCN_FLAG_NO_GRAD_X) && gx != nullptr;
   bool all_fused = true;
-  if (operand != DCN_OPERAND_FP32 || use_umma_data(g0, operand)) {
+  if (operand != DCN_OPERAND_FP32 || umma_bwd_data_supported(g0, operand)) {
     // DCN_FLAG_GRAD_X_FRAMED: grad_x IS the framed channels-last accumulator (the producer-side post-op reads it in
     // that layout, dcn_bn_relu_backward_staged): scatter straight into the caller's buffer, no transposition at the end
     const bool gx_framed = (flags & DCN_FLAG_GRAD_X_FRAMED) != 0;
@@ -188,7 +183,7 @@ int umma_backward_any(const Geo& g, int operand, int flags, const void* xv, cons
   // pass of the remaining groups stages its grad_out tiles there
   for (int o0 = 0; o0 < g.O; o0 += gsize) {
     const Geo gc = o_group_geo(g, o0, gsize);
-    const bool data_on_umma = operand != DCN_OPERAND_FP32 || use_umma_data(g0, operand);
+    const bool data_on_umma = operand != DCN_OPERAND_FP32 || umma_bwd_data_supported(g0, operand);
     if (data_on_umma && umma_bwd_data_fuses_wgrad(gc, operand)) continue;
     if ((rc = umma_wgrad_any(gc, operand, xt, off, (const uint8_t*)goutv + (size_t)o0 * g.HW * esz,
                              gw + (size_t)o0 * g.K, rest, st)))

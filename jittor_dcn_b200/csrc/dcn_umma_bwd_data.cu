@@ -1056,7 +1056,6 @@ __global__ void __launch_bounds__(256) weight_tiles_bwd_kernel(Geo g, int ncols,
 //   buffers and the Wm^T stages
 static void choose_slices(bd::Params* P, int max_cb, size_t real, size_t zero, size_t other) {
   const size_t cap = 227 * 1024;
-  const bool allow_res = !knobs().bwd_no_resident;
   const int ns_min = (P->cblocks + max_cb - 1) / max_cb;
   double best = 1e30;
   for (int ns = ns_min; ns <= ns_min + 2 && ns <= P->cblocks; ++ns) {
@@ -1075,10 +1074,9 @@ static void choose_slices(bd::Params* P, int max_cb, size_t real, size_t zero, s
   // (the dynamic shared-memory window starts 1 KB-aligned in practice; the kernel traps if it would overrun).
   const int plans[5][3] = {{2, 1, 2}, {2, 0, 2}, {2, 0, 1}, {1, 1, 2}, {1, 0, 2}};
   for (const auto& pl : plans) {
-    if (pl[1] && !allow_res) continue;
     const size_t n_w = pl[1] ? n_res : (size_t)pl[2];
     const size_t need = pl[0] * real + zero + n_w * P->w_stage + other;
-    if (need <= cap || (pl[2] == 1 && need - 768 <= cap && !knobs().bwd_no_ring1)) {
+    if (need <= cap || (pl[2] == 1 && need - 768 <= cap)) {
       P->g_nbuf = pl[0];
       P->w_resident = pl[1] ? (int)n_res : 0;
       P->w_ring = pl[2];
@@ -1088,7 +1086,7 @@ static void choose_slices(bd::Params* P, int max_cb, size_t real, size_t zero, s
 }
 
 // ---------------------------------------------------------------------------- host side
-static bool bwd_data_tiling(const Geo& g, int operand, bd::Params* P, bool allow_fuse = true) {
+static bool bwd_data_tiling(const Geo& g, int operand, bd::Params* P) {
   const size_t nimg = operand == DCN_OPERAND_BF16 ? 1 : 2;
   if (!make_tiling(g, &P->t)) return false;
   P->fuse_w = 0;
@@ -1120,7 +1118,7 @@ static bool bwd_data_tiling(const Geo& g, int operand, bd::Params* P, bool allow
     P->divChunks = FastDiv::make(P->chunks);
     P->g_imgs = P->OB;
     // fused weight gradient: 64-column blocks, <= 6 blocks of gW accumulators next to the 2 gA buffers
-    if (allow_fuse && g.O <= 256) {
+    if (g.O <= 256) {
       const int ncols = 64;
       const int halves = g.O > 128 ? 2 : 1;  // the gW MMAs take 128 channels (two 64-o images) at a time
       const size_t plan = 2 * (size_t)P->Rt * ncols * sizeof(bd::ScatEntry);
@@ -1136,8 +1134,7 @@ static bool bwd_data_tiling(const Geo& g, int operand, bd::Params* P, bool allow
         P->g_img = bd::kGImg;
         P->w_stage = (uint32_t)nimg * ncols * 128;
         P->tmem_cols = 512;
-        const int cap_cb = 6 / halves;  // 512 TMEM columns - 2 gA buffers, one accumulator set per half
-        const int max_cb = knobs().bwd_slice_cb < 1 ? 1 : (knobs().bwd_slice_cb > cap_cb ? cap_cb : knobs().bwd_slice_cb);
+        const int max_cb = 6 / halves;  // 512 TMEM columns - 2 gA buffers, one accumulator set per half
         choose_slices(P, max_cb, real, zero, rest - 2 * (size_t)P->w_stage);
         return true;
       }
@@ -1166,7 +1163,7 @@ static bool bwd_data_tiling(const Geo& g, int operand, bd::Params* P, bool allow
   const int taps = g.C >= 128 ? 1 : 128 / g.C;
   P->o_cols = 0;
   // fused weight gradient: 64-pixel tiles, gW^T accumulator blocks of O columns next to the 2 gA buffers
-  if (allow_fuse && g.O <= 256) {
+  if (g.O <= 256) {
     const int ncols = 64, o_cols = (g.O + 15) / 16 * 16;
     const size_t plan = 2 * (size_t)taps * ncols * sizeof(bd::ScatEntry);
     const size_t real = (size_t)P->OB * nimg * (ncols * 128);
@@ -1208,28 +1205,24 @@ static bool bwd_data_tiling(const Geo& g, int operand, bd::Params* P, bool allow
   return false;
 }
 
-static bool fuse_allowed() {
-  return !knobs().bwd_no_fuse;
-}
-
 bool umma_bwd_data_supported(const Geo& g, int operand) {
   if (operand != DCN_OPERAND_FP32 && operand != DCN_OPERAND_BF16) return false;
   bd::Params P;
   P.g = g;
-  return bwd_data_tiling(g, operand, &P, fuse_allowed());
+  return bwd_data_tiling(g, operand, &P);
 }
 
 // does umma_bwd_data_any also produce grad_weight for this shape?
 bool umma_bwd_data_fuses_wgrad(const Geo& g, int operand) {
   bd::Params P;
   P.g = g;
-  return bwd_data_tiling(g, operand, &P, fuse_allowed()) && P.fuse_w;
+  return bwd_data_tiling(g, operand, &P) && P.fuse_w;
 }
 
 size_t umma_bwd_data_wtile_bytes(const Geo& g, int operand) {
   bd::Params P;
   P.g = g;
-  if (!bwd_data_tiling(g, operand, &P, fuse_allowed())) return 0;
+  if (!bwd_data_tiling(g, operand, &P)) return 0;
   return align_up((size_t)P.cblocks * P.OB * P.w_stage, 1024);
 }
 
@@ -1295,7 +1288,7 @@ int launch_gout_tiles_fwd_order(const Geo& g, int operand, const void* gout, uin
 size_t umma_bwd_data_gtile_bytes(const Geo& g, int operand) {
   bd::Params P;
   P.g = g;
-  if (!bwd_data_tiling(g, operand, &P, fuse_allowed())) return 0;
+  if (!bwd_data_tiling(g, operand, &P)) return 0;
   if (g.variant != DCN_VARIANT_TORCH) return gtile_pix_bytes(g, operand);
   return align_up((size_t)P.num_tiles * P.OB * (operand == DCN_OPERAND_BF16 ? 1 : 2) * bd::kGImg, 1024);
 }
@@ -1310,7 +1303,7 @@ int umma_bwd_data_any(const Geo& g, int operand, const void* xt, float* gxt, con
   P.g = g;
   const bool bf = operand == DCN_OPERAND_BF16;
   const size_t nimg = bf ? 1 : 2;
-  if (!bwd_data_tiling(g, operand, &P, fuse_allowed())) {
+  if (!bwd_data_tiling(g, operand, &P)) {
     set_error("umma bwd_data: shape not tileable");
     return DCN_ERR_UNSUPPORTED;
   }
@@ -1347,7 +1340,6 @@ int umma_bwd_data_any(const Geo& g, int operand, const void* xt, float* gxt, con
   // (autograd of train.py:111-113 -> GridSampler.h:27-36; dcn_simt.cu:offset_scale_kernel)
   P.scale_iy = g.variant == DCN_VARIANT_DCNV1 ? 1.f : g.sy * 2.0f / g.Dx;
   P.scale_ix = g.variant == DCN_VARIANT_DCNV1 ? 1.f : g.sx * 2.0f / g.Dy;
-  if (knobs().bwd_gbuf1) P.g_nbuf = 1;
   size_t smem = ((size_t)P.g_nbuf * P.OB + (P.g_imgs - P.OB)) * nimg * P.g_img +
                 (size_t)(P.w_resident ? P.w_resident : P.w_ring) * P.w_stage +
                 (P.fuse_w ? 2 * nimg * (size_t)(128 * 128) : 0) +

@@ -44,6 +44,9 @@ constexpr int kPlanMax = 512;                                    // plan entries
 constexpr uint32_t kATile = 128 * 64 * 2;                        // one bf16 A image (16 KB)
 constexpr uint32_t kAMnLbo = 1024, kAMnSbo = 2048;               // MN-major A: atom strides
 constexpr int kMaxStages = 4;
+// forward pipeline depth (fewer when shared memory runs out): a few stages are enough to overlap the (fast) MMAs with
+// the (slow) gather; every KB of shared memory not taken stays L1 for the gather's footprint (L1 + smem share 256 KB)
+constexpr int kFwdStages = 3;
 
 enum { MODE_FWD = 0, MODE_WGRAD = 1 };
 
@@ -1033,7 +1036,7 @@ static int launch_gemm(const Geo& g, int operand, const FwdParams& P, const CUte
   // layouts with 4 taps per K block): 8 plan + 8 gather warps
   const int n_ent = g.variant == DCN_VARIANT_TORCH ? P.t.Rt * 64 : 128 * P.t.taps_per_kb;
   // (measured at 256 and 128 chains per block — det3, c3, cfg2 — the 8 + 8 split is 18 - 43 % SLOWER: those are gather-bound)
-  if (n_ent > 256 && !knobs().fwd_no_split88) {
+  if (n_ent > 256) {
     constexpr int kThreads88 = (kFirstPlanWarp + 8 + 8) * 32;
 #define DCN_GEMM_CASE88(V, BFV)                                                                            \
   do {                                                                                                     \
@@ -1093,7 +1096,7 @@ int umma_forward_any(const Geo& g, int operand, const void* x, const float* off,
   memset(&tmap, 0, sizeof(tmap));
   // (Rt = 2 only: with Rt >= 4 the direct stores already write 16-byte runs, and the staged path
   // measured slower there)
-  if (g.variant == DCN_VARIANT_TORCH && P.t.Rt == 2 && !knobs().fwd_no_tma_out && !g.out_framed) {
+  if (g.variant == DCN_VARIANT_TORCH && P.t.Rt == 2 && !g.out_framed) {
     const int box_r = P.t.Rt < 4 ? 4 : P.t.Rt;
     const size_t bytes = sizeof(float) * (size_t)g.O * P.t.Gt * box_r;
     if (P.t.R % box_r == 0 && bytes <= 64 * 1024 && g.O <= 256 &&
@@ -1107,20 +1110,14 @@ int umma_forward_any(const Geo& g, int operand, const void* x, const float* off,
       fixed += (size_t)P.n_ost * P.stage_out_bytes;
     }
   }
-  int stages = (int)((227 * 1024 - fixed) / P.stage_bytes);
-  // A few stages are enough to overlap the (fast) MMAs with the (slow) gather; every KB of
-  // shared memory not taken stays L1 for the gather's footprint (L1 + smem share 256 KB).
-  int want = knobs().fwd_stages;
-  if (want < 2) want = 2;
-  if (want > kMaxStages) want = kMaxStages;
-  P.stages = stages > want ? want : stages;
+  const int stages = (int)((227 * 1024 - fixed) / P.stage_bytes);
+  P.stages = stages > kFwdStages ? kFwdStages : stages;
   if (P.stages < 2) {
     set_error("umma forward: not enough shared memory for 2 stages");
     return DCN_ERR_UNSUPPORTED;
   }
   P.tmem_cols = pow2_cols(2 * g.O);
-  if (g.variant != DCN_VARIANT_TORCH && g.C % 64 == 0 && g.C > 64 && P.t.KB == g.N * (g.C / 64) &&
-      !knobs().fwd_no_kperm)
+  if (g.variant != DCN_VARIANT_TORCH && g.C % 64 == 0 && g.C > 64 && P.t.KB == g.N * (g.C / 64))
     P.kperm_slabs = g.C / 64;
   const size_t smem = (size_t)P.stages * P.stage_bytes + fixed;
   const int sms = num_sms();

@@ -107,6 +107,14 @@ def test_product_never_imports_the_oracle():
                 assert "oracle" not in text.replace("no CPU fallback", ""), os.path.join(dirpath, f)
 
 
+def test_library_reads_no_environment():
+    """Which kernel and launch plan runs depends on the shape alone, never on the process environment."""
+    csrc = os.path.join(ROOT, "jittor_dcn_b200", "csrc")
+    for f in os.listdir(csrc):
+        if f.endswith((".cu", ".cuh", ".h", ".cpp")):
+            assert "getenv" not in open(os.path.join(csrc, f)).read(), f
+
+
 def test_detector_harness_keeps_reference_parameter_names():
     """state_dict keys/shapes of train.py:142-175 (435,862 parameters, SURVEY 2 #6)."""
     from jittor_dcn_b200.detector import EDNetDetection
