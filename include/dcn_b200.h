@@ -65,7 +65,8 @@ enum {
    * memory-reinterpreting reshape of the [B,C,Ho,Wo,N] sample tensor (:129-131). */
   DCN_VARIANT_TORCH = 1,
   /* Not in the reference (SURVEY.md 8f.3): standard deformable convolution v1 as in
-   * torchvision.ops.deform_conv2d / mmcv (one offset group, no mask, dilation 1): sampling point
+   * torchvision.ops.deform_conv2d / mmcv (one offset group, dilation 1; with a mask through
+   * dcn_forward_modulated / dcn_backward_modulated = DCNv2): sampling point
    * (h*s - p + ki + dy, w*s - p + kj + dx), offsets interleaved (dy, dx) per tap, columns ordered
    * (c, tap).  Same kernels, different coordinate generator; torchvision is its oracle. */
   DCN_VARIANT_DCNV1 = 2
@@ -171,6 +172,27 @@ DCN_API int dcn_forward(const DcnShape* s, const void* x, const void* offset, co
 DCN_API int dcn_backward(const DcnShape* s, const void* x, const void* offset, const void* weight,
                  const void* grad_out, void* grad_x, void* grad_offset, void* grad_weight,
                  void* grad_bias, void* workspace, size_t workspace_bytes, void* stream);
+
+/* ---- modulated deformable convolution (DCNv2: torchvision.ops.deform_conv2d(..., mask=), mmcv's
+ * ModulatedDeformConv2d) ------------------------------------------------------------------------------------------
+ * DCN_VARIANT_DCNV1 sampling, every sample scaled by a per-(tap, output pixel) mask value:
+ *   out[b,o,p]       = bias[o] + sum_{c,n} W[o,c,n] * m[b,n,p] * bil(x[b,c], sample(n,p))
+ *   grad_mask[b,n,p] = sum_c gA[b,c,n,p] * bil(x[b,c], sample(n,p))   (gA = W^T grad_out; the UNmasked sample)
+ * grad_x, grad_offset and grad_weight are those of dcn_backward with every sample (and its corner weights) scaled by m.
+ *   mask        [B,N,Ho,Wo]  float32 in both operand modes, channel n = ki*kw + kj (torchvision's tap order); any
+ *                            value is allowed (no range or sigmoid is applied)
+ *   grad_mask   [B,N,Ho,Wo]  float32, overwritten; a sample with no corner inside the image gets 0
+ * Both are required and 16-byte aligned.  Every other argument, flag, workspace size (dcn_workspace_bytes with
+ * DCN_PHASE_FORWARD / DCN_PHASE_BACKWARD) and kernel family (dcn_path_name) is exactly that of dcn_forward /
+ * dcn_backward: the mask needs no extra workspace and never moves a shape off the tensor path.
+ * variant != DCN_VARIANT_DCNV1: DCN_ERR_UNSUPPORTED. */
+DCN_API int dcn_forward_modulated(const DcnShape* s, const void* x, const void* offset, const void* mask,
+                                  const void* weight, const void* bias, void* out,
+                                  void* workspace, size_t workspace_bytes, void* stream);
+DCN_API int dcn_backward_modulated(const DcnShape* s, const void* x, const void* offset, const void* mask,
+                                   const void* weight, const void* grad_out, void* grad_x, void* grad_offset,
+                                   void* grad_mask, void* grad_weight, void* grad_bias,
+                                   void* workspace, size_t workspace_bytes, void* stream);
 
 /* ---- the whole layer: companion offset convolution + DCN span (SURVEY 8f.1) ------------------------------------
  * The offset conv (deform_conv.py:16-21,58 / train.py:80-85,98: C -> 2N channels, same kernel / stride / padding) runs

@@ -29,7 +29,7 @@ ROI_POOL, PSROI_POOL = 0, 1                        # dcn_roi_pool_* kind (deform
 EXPORTS = (
     "dcn_version", "dcn_last_error", "dcn_status_string", "dcn_output_hw", "dcn_workspace_bytes",
     "dcn_path_name", "dcn_launch_count", "dcn_launch_count_reset", "dcn_profile_begin",
-    "dcn_profile_end", "dcn_forward", "dcn_backward",
+    "dcn_profile_end", "dcn_forward", "dcn_backward", "dcn_forward_modulated", "dcn_backward_modulated",
     "dcn_debug_corners", "dcn_comm_unique_id", "dcn_comm_init", "dcn_allreduce_sum_f32",
     "dcn_comm_destroy", "dcn_bn_workspace_bytes", "dcn_bn_relu_forward", "dcn_bn_relu_backward",
     "dcn_offset_conv_forward", "dcn_layer_forward", "dcn_layer_backward",
@@ -80,6 +80,8 @@ def load():
     lib.dcn_profile_end.argtypes = [ctypes.c_char_p, sz]
     lib.dcn_forward.argtypes = [shp, vp, vp, vp, vp, vp, vp, sz, vp]
     lib.dcn_backward.argtypes = [shp, vp, vp, vp, vp, vp, vp, vp, vp, vp, sz, vp]
+    lib.dcn_forward_modulated.argtypes = [shp, vp, vp, vp, vp, vp, vp, vp, sz, vp]
+    lib.dcn_backward_modulated.argtypes = [shp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, sz, vp]
     lib.dcn_debug_corners.argtypes = [shp, vp, vp, vp, vp, vp]
     lib.dcn_offset_conv_forward.argtypes = [shp, vp, vp, vp, vp, vp, sz, vp]
     lib.dcn_layer_forward.argtypes = [shp, vp, vp, vp, vp, vp, vp, vp, vp, sz, vp]

@@ -149,6 +149,19 @@ static bool layer_ok(const DcnShape* s, const Geo& g, int phase) {
   return umma_layer_bwd_supported(g);
 }
 
+// mask: the modulated calls (dcn_forward_modulated / dcn_backward_modulated): DCNv1 only, float32 [B, N, Ho, Wo]
+static int check_modulated(const DcnShape* s, const void* mask, const char* mname, const void* gmask = nullptr,
+                           bool backward = false) {
+  int rc;
+  if ((rc = check_ptr(mask, mname)) || (backward && (rc = check_ptr(gmask, "grad_mask")))) return rc;
+  if (s->variant != DCN_VARIANT_DCNV1) {
+    set_error("a mask (modulated deformable convolution, DCNv2) exists for DCN_VARIANT_DCNV1 only, not variant %d: "
+              "the reference's two variants have no modulated form", s->variant);
+    return DCN_ERR_UNSUPPORTED;
+  }
+  return DCN_OK;
+}
+
 static size_t layer_workspace(const Geo& g, int operand, int phase) {
   const size_t f1 = umma_offset_conv_fwd_workspace(g), f2 = umma_workspace_bytes(g, operand, DCN_PHASE_FORWARD);
   const size_t f = f1 > f2 ? f1 : f2;
@@ -258,9 +271,13 @@ int dcn_profile_end(char* out, size_t cap) {
 uint64_t dcn_launch_count(void) { return g_launches.load(); }
 void dcn_launch_count_reset(void) { g_launches.store(0); }
 
-int dcn_forward(const DcnShape* s, const void* x, const void* offset, const void* weight,
-                const void* bias, void* out, void* workspace, size_t workspace_bytes,
-                void* stream) {
+}  // extern "C"
+
+namespace dcn {
+
+// dcn_forward and dcn_forward_modulated: mask == nullptr = unmodulated
+static int forward_impl(const DcnShape* s, const void* x, const void* offset, const float* mask, const void* weight,
+                        const void* bias, void* out, void* workspace, size_t workspace_bytes, void* stream) {
   Geo g;
   int rc = geo_or_error(s, &g);
   if (rc) return rc;
@@ -277,7 +294,7 @@ int dcn_forward(const DcnShape* s, const void* x, const void* offset, const void
   cudaStream_t st = (cudaStream_t)stream;
   if (use_umma(s, g, DCN_PHASE_FORWARD))
     return umma_forward(g, s->operand, s->flags, x, (const float*)offset, weight, (const float*)bias,
-                        out, workspace, st);
+                        out, workspace, st, mask);
   if (use_gemm(s, g, DCN_PHASE_FORWARD))
     return gemm_path_forward(g, s->operand, x, (const float*)offset, weight, (const float*)bias, (float*)out, workspace,
                              st);
@@ -290,14 +307,16 @@ int dcn_forward(const DcnShape* s, const void* x, const void* offset, const void
     x = xf;
     weight = wf;
   }
+  // (the plan of the DCNv1 layout is [b][n][p], the order of the mask: the sampling kernels index both alike)
   if ((rc = launch_plan(g, (const float*)offset, plan, st))) return rc;
   return simt_forward(g, (const float*)x, plan, (const float*)weight, (const float*)bias, (float*)out,
-                      st);
+                      st, mask);
 }
 
-int dcn_backward(const DcnShape* s, const void* x, const void* offset, const void* weight,
-                 const void* grad_out, void* grad_x, void* grad_offset, void* grad_weight,
-                 void* grad_bias, void* workspace, size_t workspace_bytes, void* stream) {
+// dcn_backward and dcn_backward_modulated: mask == nullptr = unmodulated (grad_mask unused)
+static int backward_impl(const DcnShape* s, const void* x, const void* offset, const float* mask, const void* weight,
+                         const void* grad_out, void* grad_x, void* grad_offset, float* grad_mask, void* grad_weight,
+                         void* grad_bias, void* workspace, size_t workspace_bytes, void* stream) {
   Geo g;
   int rc = geo_or_error(s, &g);
   if (rc) return rc;
@@ -317,7 +336,7 @@ int dcn_backward(const DcnShape* s, const void* x, const void* offset, const voi
   if (use_umma(s, g, DCN_PHASE_BACKWARD))
     return umma_backward(g, s->operand, s->flags, x, (const float*)offset, weight, grad_out,
                          (float*)grad_x, (float*)grad_offset, (float*)grad_weight,
-                         (float*)grad_bias, workspace, st);
+                         (float*)grad_bias, workspace, st, mask, grad_mask);
   if (use_gemm(s, g, DCN_PHASE_BACKWARD))
     return gemm_path_backward(g, s->operand, s->flags, x, (const float*)offset, weight, grad_out, (float*)grad_x,
                               (float*)grad_offset, (float*)grad_weight, (float*)grad_bias, workspace, st);
@@ -336,7 +355,44 @@ int dcn_backward(const DcnShape* s, const void* x, const void* offset, const voi
   if ((rc = launch_plan(g, (const float*)offset, plan, st))) return rc;
   return simt_backward(g, s->flags, (const float*)x, plan, (const float*)weight,
                        (const float*)grad_out, (float*)grad_x, (float*)grad_offset,
-                       (float*)grad_weight, (float*)grad_bias, st);
+                       (float*)grad_weight, (float*)grad_bias, st, SIMT_BWD_ALL, mask, grad_mask);
+}
+
+}  // namespace dcn
+
+extern "C" {
+
+int dcn_forward(const DcnShape* s, const void* x, const void* offset, const void* weight,
+                const void* bias, void* out, void* workspace, size_t workspace_bytes,
+                void* stream) {
+  return forward_impl(s, x, offset, nullptr, weight, bias, out, workspace, workspace_bytes, stream);
+}
+
+int dcn_backward(const DcnShape* s, const void* x, const void* offset, const void* weight,
+                 const void* grad_out, void* grad_x, void* grad_offset, void* grad_weight,
+                 void* grad_bias, void* workspace, size_t workspace_bytes, void* stream) {
+  return backward_impl(s, x, offset, nullptr, weight, grad_out, grad_x, grad_offset, nullptr, grad_weight, grad_bias,
+                       workspace, workspace_bytes, stream);
+}
+
+int dcn_forward_modulated(const DcnShape* s, const void* x, const void* offset, const void* mask,
+                          const void* weight, const void* bias, void* out,
+                          void* workspace, size_t workspace_bytes, void* stream) {
+  Geo g;
+  int rc = geo_or_error(s, &g);
+  if (rc || (rc = check_modulated(s, mask, "mask"))) return rc;
+  return forward_impl(s, x, offset, (const float*)mask, weight, bias, out, workspace, workspace_bytes, stream);
+}
+
+int dcn_backward_modulated(const DcnShape* s, const void* x, const void* offset, const void* mask,
+                           const void* weight, const void* grad_out, void* grad_x, void* grad_offset,
+                           void* grad_mask, void* grad_weight, void* grad_bias,
+                           void* workspace, size_t workspace_bytes, void* stream) {
+  Geo g;
+  int rc = geo_or_error(s, &g);
+  if (rc || (rc = check_modulated(s, mask, "mask", grad_mask, true))) return rc;
+  return backward_impl(s, x, offset, (const float*)mask, weight, grad_out, grad_x, grad_offset, (float*)grad_mask,
+                       grad_weight, grad_bias, workspace, workspace_bytes, stream);
 }
 
 int dcn_offset_conv_forward(const DcnShape* s, const void* x, const void* offset_weight, const void* offset_bias,

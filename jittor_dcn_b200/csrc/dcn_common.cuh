@@ -247,14 +247,15 @@ static inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; 
 // plan: Tap per (b, q); stored in q-order [b][p][n] (Torch) or tap-major [b][n][p] (Jittor)
 int launch_plan(const Geo& g, const float* off, Tap* plan, cudaStream_t st);
 int launch_corners(const Geo& g, const float* off, int32_t* y0, int32_t* x0, float* w4, cudaStream_t st);
+// mask / gmask [B, N, Ho, Wo] (DCNv1 only; nullptr = unmodulated): modulated sampling and its gradient
 int simt_forward(const Geo& g, const float* x, const Tap* plan, const float* wt, const float* bias,
-                 float* out, cudaStream_t st);
+                 float* out, cudaStream_t st, const float* mask = nullptr);
 int launch_offset_scale(const Geo& g, float* goff, cudaStream_t st);
 int launch_bias_grad(const Geo& g, const void* gout, int operand, float* gb, cudaStream_t st);
 int launch_widen_bf16(const void* src, float* dst, size_t n, cudaStream_t st);
 enum { SIMT_BWD_DATA = 1, SIMT_BWD_WEIGHT = 2, SIMT_BWD_BIAS = 4, SIMT_BWD_ALL = 7 };
 int simt_backward(const Geo& g, int flags, const float* x, const Tap* plan, const float* wt,
                   const float* gout, float* gx, float* goff, float* gw, float* gb, cudaStream_t st,
-                  int parts = SIMT_BWD_ALL);
+                  int parts = SIMT_BWD_ALL, const float* mask = nullptr, float* gmask = nullptr);
 
 }  // namespace dcn

@@ -12,6 +12,10 @@
 //                        coordinate-gradient reduction                (autograd, A.4)
 //   bwd_weight_kernel    gW = g^T * A with A re-sampled                (autograd, A.4)
 //   bias_grad / offset_scale kernels
+//
+// MOD instantiations (modulated DCNv1 = DCNv2, pixel-row column order): every sample is scaled by
+// mask[b, n, p] ([B, N, Ho, Wo], the same [b][n][p] order as the plan of that layout), and
+// bwd_data_kernel also writes grad_mask[b, n, p] = sum_c gA * (unmasked sample).
 #include <cuda_bf16.h>
 
 #include "dcn_common.cuh"
@@ -117,12 +121,14 @@ __device__ __forceinline__ float sample_a(const Geo& g, const float* __restrict_
 // tile 64 rows x 64 outputs, BK = 16, 256 threads, 4x4 micro-tile per thread.
 constexpr int TM = 64, TN = 64, TK = 16;
 
-template <int VARIANT>
+template <int VARIANT, bool MOD = false>
 __global__ void __launch_bounds__(256) fwd_kernel(Geo g, const float* __restrict__ x,
                                                   const Tap* __restrict__ plan,
                                                   const float* __restrict__ wt,
                                                   const float* __restrict__ bias,
-                                                  float* __restrict__ out) {
+                                                  float* __restrict__ out,
+                                                  const float* __restrict__ mask) {
+  static_assert(!MOD || VARIANT != DCN_VARIANT_TORCH, "modulation exists for the DCNv1 (pixel-row) order only");
   __shared__ float As[TK][TM + 4];
   __shared__ float Bs[TK][TN + 4];
   const int b = blockIdx.z, r0 = blockIdx.x * TM, o0 = blockIdx.y * TN;
@@ -143,7 +149,14 @@ __global__ void __launch_bounds__(256) fwd_kernel(Geo g, const float* __restrict
         kk = (tid >> 6) + 4 * i;
       }
       float v = 0.f;
-      if (r0 + rr < g.HW && k0 + kk < g.K) v = sample_a<VARIANT>(g, xb, planb, r0 + rr, k0 + kk);
+      if (r0 + rr < g.HW && k0 + kk < g.K) {
+        v = sample_a<VARIANT>(g, xb, planb, r0 + rr, k0 + kk);
+        if (MOD) {
+          const size_t mi = ((size_t)b * g.N + (k0 + kk) / g.C) * g.HW + r0 + rr;
+          DCN_DEV_ASSERT(mi < (size_t)g.B * g.N * g.HW);
+          v = __ldg(mask + mi) * v;
+        }
+      }
       As[kk][rr] = v;
     }
 // B tile: Wm[o0..o0+63, k0..k0+15]
@@ -193,13 +206,15 @@ __global__ void __launch_bounds__(256) fwd_kernel(Geo g, const float* __restrict
 }
 
 int simt_forward(const Geo& g, const float* x, const Tap* plan, const float* wt, const float* bias,
-                 float* out, cudaStream_t st) {
+                 float* out, cudaStream_t st, const float* mask) {
   dim3 grid((g.HW + TM - 1) / TM, (g.O + TN - 1) / TN, g.B);
   KernelScope scope("fwd_kernel", st);
-  if (g.variant == DCN_VARIANT_TORCH)
-    fwd_kernel<DCN_VARIANT_TORCH><<<grid, 256, 0, st>>>(g, x, plan, wt, bias, out);
+  if (mask)
+    fwd_kernel<DCN_VARIANT_JITTOR, true><<<grid, 256, 0, st>>>(g, x, plan, wt, bias, out, mask);
+  else if (g.variant == DCN_VARIANT_TORCH)
+    fwd_kernel<DCN_VARIANT_TORCH><<<grid, 256, 0, st>>>(g, x, plan, wt, bias, out, nullptr);
   else
-    fwd_kernel<DCN_VARIANT_JITTOR><<<grid, 256, 0, st>>>(g, x, plan, wt, bias, out);
+    fwd_kernel<DCN_VARIANT_JITTOR><<<grid, 256, 0, st>>>(g, x, plan, wt, bias, out, nullptr);
   DCN_KERNEL_CHECK("fwd_kernel");
   return DCN_OK;
 }
@@ -212,14 +227,17 @@ int simt_forward(const Geo& g, const float* x, const Tap* plan, const float* wt,
 // g_iy is accumulated raw into grad_offset channel n, g_ix into channel N+n (the "x"
 // offset moves the ROW because the reference hands grid_sample [norm_y, norm_x]);
 // offset_scale_kernel applies the chain-rule factors afterwards.
-template <int VARIANT>
+template <int VARIANT, bool MOD = false>
 __global__ void __launch_bounds__(256) bwd_data_kernel(Geo g, int want_gx,
                                                        const float* __restrict__ x,
                                                        const Tap* __restrict__ plan,
                                                        const float* __restrict__ wt,
                                                        const float* __restrict__ gout,
                                                        float* __restrict__ gx,
-                                                       float* __restrict__ goff) {
+                                                       float* __restrict__ goff,
+                                                       const float* __restrict__ mask,
+                                                       float* __restrict__ gmask) {
+  static_assert(!MOD || VARIANT != DCN_VARIANT_TORCH, "modulation exists for the DCNv1 (pixel-row) order only");
   __shared__ float Gs[TK][TM + 4];  // g[r, o]   (o along TK)
   __shared__ float Ws[TK][TN + 4];  // Wm[o, j]
   const int b = blockIdx.z, r0 = blockIdx.x * TM, j0 = blockIdx.y * TN;
@@ -266,6 +284,7 @@ __global__ void __launch_bounds__(256) bwd_data_kernel(Geo g, int want_gx,
   float* goffb = goff + (size_t)b * 2 * g.N * g.HW;
   int q_prev = -1;
   float six = 0.f, siy = 0.f;
+  float smk = 0.f;  // MOD: sum of gA * (unmasked sample) of sampling point q_prev
   auto flush = [&]() {
     if (q_prev >= 0 && (six != 0.f || siy != 0.f)) {
       const int p = q_prev / g.N, n = q_prev - p * g.N;
@@ -273,6 +292,22 @@ __global__ void __launch_bounds__(256) bwd_data_kernel(Geo g, int want_gx,
       atomicAdd(goffb + (size_t)off_col_ch(g, n) * g.HW + p, six);
     }
     six = siy = 0.f;
+    if constexpr (MOD) {
+      if (q_prev >= 0 && smk != 0.f) {
+        const int p = q_prev / g.N, n = q_prev - p * g.N;
+        const size_t mi = ((size_t)b * g.N + n) * g.HW + p;
+        DCN_DEV_ASSERT(mi < (size_t)g.B * g.N * g.HW);
+        atomicAdd(gmask + mi, smk);
+      }
+      smk = 0.f;
+    }
+  };
+  // MOD: gA of sampling point q scaled by its mask value
+  auto modulated = [&](float ga, int q) {
+    const int p = q / g.N, n = q - p * g.N;
+    const size_t mi = ((size_t)b * g.N + n) * g.HW + p;
+    DCN_DEV_ASSERT(mi < (size_t)g.B * g.N * g.HW);
+    return __ldg(mask + mi) * ga;
   };
 #pragma unroll
   for (int i = 0; i < 4; ++i) {
@@ -299,7 +334,7 @@ __global__ void __launch_bounds__(256) bwd_data_kernel(Geo g, int want_gx,
       if (!m) continue;
       float cw[4];
       corner_weights(t, cw);
-      const float gs = acc[i][jj];
+      const float gs = MOD ? modulated(acc[i][jj], q) : acc[i][jj];
       const ptrdiff_t base = (ptrdiff_t)c * g.H * g.W + (ptrdiff_t)t.y0 * g.W + t.x0;
       const float v0 = (m & 1u) ? __ldg(xb + base) : 0.f;
       const float v1 = (m & 2u) ? __ldg(xb + base + 1) : 0.f;
@@ -313,6 +348,7 @@ __global__ void __launch_bounds__(256) bwd_data_kernel(Geo g, int want_gx,
       }
       six += gs * ((v1 - v0) * (1.f - t.fy) + (v3 - v2) * t.fy);
       siy += gs * ((v2 - v0) * (1.f - t.fx) + (v3 - v1) * t.fx);
+      if constexpr (MOD) smk += acc[i][jj] * (v0 * cw[0] + v1 * cw[1] + v2 * cw[2] + v3 * cw[3]);
     }
   }
   flush();
@@ -334,12 +370,14 @@ __global__ void __launch_bounds__(256) offset_scale_kernel(Geo g, float* __restr
 // ------------------------------------------------------------------ backward: weight
 // gW[o, j] = sum_{b, r} g_b[r, o] * A_b[r, j]; the (b, r) range is split over gridDim.z
 // and partial tiles are reduced with red.global.add.f32 into a zeroed gW.
-template <int VARIANT>
+template <int VARIANT, bool MOD = false>
 __global__ void __launch_bounds__(256) bwd_weight_kernel(Geo g, int chunks_per_split,
                                                          const float* __restrict__ x,
                                                          const Tap* __restrict__ plan,
                                                          const float* __restrict__ gout,
-                                                         float* __restrict__ gw) {
+                                                         float* __restrict__ gw,
+                                                         const float* __restrict__ mask) {
+  static_assert(!MOD || VARIANT != DCN_VARIANT_TORCH, "modulation exists for the DCNv1 (pixel-row) order only");
   __shared__ float Gs[TK][TM + 4];  // g[r, o]  (r along TK)
   __shared__ float As[TK][TN + 4];  // A[r, j]
   const int o0 = blockIdx.x * TM, j0 = blockIdx.y * TN;
@@ -372,7 +410,14 @@ __global__ void __launch_bounds__(256) bwd_weight_kernel(Geo g, int chunks_per_s
         jj = (tid >> 4) + 16 * i;
       }
       float v = 0.f;
-      if (r0 + rr < g.HW && j0 + jj < g.K) v = sample_a<VARIANT>(g, xb, planb, r0 + rr, j0 + jj);
+      if (r0 + rr < g.HW && j0 + jj < g.K) {
+        v = sample_a<VARIANT>(g, xb, planb, r0 + rr, j0 + jj);
+        if (MOD) {
+          const size_t mi = ((size_t)b * g.N + (j0 + jj) / g.C) * g.HW + r0 + rr;
+          DCN_DEV_ASSERT(mi < (size_t)g.B * g.N * g.HW);
+          v = __ldg(mask + mi) * v;
+        }
+      }
       As[rr][jj] = v;
     }
     __syncthreads();
@@ -489,22 +534,28 @@ int launch_offset_scale(const Geo& g, float* goff, cudaStream_t st) {
 
 int simt_backward(const Geo& g, int flags, const float* x, const Tap* plan, const float* wt,
                   const float* gout, float* gx, float* goff, float* gw, float* gb,
-                  cudaStream_t st, int parts) {
+                  cudaStream_t st, int parts, const float* mask, float* gmask) {
   const bool want_gx = !(flags & DCN_FLAG_NO_GRAD_X) && gx != nullptr;
   if (parts & SIMT_BWD_DATA) {
     if (want_gx && !(flags & DCN_FLAG_ACCUM_GRAD_X))
       DCN_CUDA_TRY(cudaMemsetAsync(gx, 0, sizeof(float) * (size_t)g.B * g.C * g.H * g.W, st));
     DCN_CUDA_TRY(cudaMemsetAsync(goff, 0, sizeof(float) * (size_t)g.B * 2 * g.N * g.HW, st));
+    if (mask) DCN_CUDA_TRY(cudaMemsetAsync(gmask, 0, sizeof(float) * (size_t)g.B * g.N * g.HW, st));
   }
   if (parts & SIMT_BWD_WEIGHT) DCN_CUDA_TRY(cudaMemsetAsync(gw, 0, sizeof(float) * (size_t)g.O * g.K, st));
   if (parts & SIMT_BWD_DATA) {
     dim3 grid((g.HW + TM - 1) / TM, (g.K + TN - 1) / TN, g.B);
     {
       KernelScope scope("bwd_data_kernel", st);
-      if (g.variant == DCN_VARIANT_TORCH)
-          bwd_data_kernel<DCN_VARIANT_TORCH><<<grid, 256, 0, st>>>(g, want_gx, x, plan, wt, gout, gx, goff);
+      if (mask)
+        bwd_data_kernel<DCN_VARIANT_JITTOR, true><<<grid, 256, 0, st>>>(g, want_gx, x, plan, wt, gout, gx, goff,
+                                                                         mask, gmask);
+      else if (g.variant == DCN_VARIANT_TORCH)
+          bwd_data_kernel<DCN_VARIANT_TORCH><<<grid, 256, 0, st>>>(g, want_gx, x, plan, wt, gout, gx, goff, nullptr,
+                                                                   nullptr);
       else
-        bwd_data_kernel<DCN_VARIANT_JITTOR><<<grid, 256, 0, st>>>(g, want_gx, x, plan, wt, gout, gx, goff);
+        bwd_data_kernel<DCN_VARIANT_JITTOR><<<grid, 256, 0, st>>>(g, want_gx, x, plan, wt, gout, gx, goff, nullptr,
+                                                                  nullptr);
     }
     DCN_KERNEL_CHECK("bwd_data_kernel");
     int rc = launch_offset_scale(g, goff, st);
@@ -518,10 +569,12 @@ int simt_backward(const Geo& g, int flags, const float* x, const Tap* plan, cons
     splits = (chunks + cps - 1) / cps;
     dim3 grid((g.O + TM - 1) / TM, (g.K + TN - 1) / TN, splits);
     KernelScope scope("bwd_weight_kernel", st);
-    if (g.variant == DCN_VARIANT_TORCH)
-      bwd_weight_kernel<DCN_VARIANT_TORCH><<<grid, 256, 0, st>>>(g, cps, x, plan, gout, gw);
+    if (mask)
+      bwd_weight_kernel<DCN_VARIANT_JITTOR, true><<<grid, 256, 0, st>>>(g, cps, x, plan, gout, gw, mask);
+    else if (g.variant == DCN_VARIANT_TORCH)
+      bwd_weight_kernel<DCN_VARIANT_TORCH><<<grid, 256, 0, st>>>(g, cps, x, plan, gout, gw, nullptr);
     else
-      bwd_weight_kernel<DCN_VARIANT_JITTOR><<<grid, 256, 0, st>>>(g, cps, x, plan, gout, gw);
+      bwd_weight_kernel<DCN_VARIANT_JITTOR><<<grid, 256, 0, st>>>(g, cps, x, plan, gout, gw, nullptr);
     DCN_KERNEL_CHECK("bwd_weight_kernel");
   }
   if (gb && (parts & SIMT_BWD_BIAS)) {

@@ -9,11 +9,14 @@ namespace dcn {
 bool umma_supported(const Geo& g, int operand, int phase);
 size_t umma_workspace_bytes(const Geo& g, int operand, int phase);
 
+// mask [B, N, Ho, Wo] (DCNv1 only; nullptr = unmodulated) scales every sample; gmask [B, N, Ho, Wo] receives its
+// gradient (overwritten; required with a mask)
 int umma_forward(const Geo& g, int operand, int flags, const void* x, const float* off,
-                 const void* wt, const float* bias, void* out, void* workspace, cudaStream_t st);
+                 const void* wt, const float* bias, void* out, void* workspace, cudaStream_t st,
+                 const float* mask = nullptr);
 int umma_backward(const Geo& g, int operand, int flags, const void* x, const float* off,
                   const void* wt, const void* gout, float* gx, float* goff, float* gw, float* gb,
-                  void* workspace, cudaStream_t st);
+                  void* workspace, cudaStream_t st, const float* mask = nullptr, float* gmask = nullptr);
 
 // ---- whole layer (companion offset conv as a PLAIN problem + DCN span), fp32 operands
 bool umma_offset_conv_fwd_supported(const Geo& g);

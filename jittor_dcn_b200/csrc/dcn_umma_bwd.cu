@@ -20,14 +20,15 @@ namespace dcn {
 bool umma_wgrad_supported(const Geo& g, int operand);
 size_t umma_xt_bytes(const Geo& g, int operand);
 int umma_wgrad_any(const Geo& g, int operand, const void* xt, const float* off, const void* gout, float* gw,
-                   uint8_t* gtiles, cudaStream_t st);
+                   uint8_t* gtiles, cudaStream_t st, const float* mask = nullptr);
 size_t umma_wgrad_gtile_bytes(const Geo& g, int operand);
 bool umma_bwd_data_supported(const Geo& g, int operand);
 size_t umma_bwd_data_wtile_bytes(const Geo& g, int operand);
 bool umma_bwd_data_fuses_wgrad(const Geo& g, int operand);
 int umma_bwd_data_any(const Geo& g, int operand, const void* xt, float* gxt, const float* off, const void* wt,
                       const void* gout, float* goff, float* gw, uint8_t* wtiles, uint8_t* gtiles,
-                      cudaStream_t st, float* gb_fused = nullptr);
+                      cudaStream_t st, float* gb_fused = nullptr, const float* mask = nullptr,
+                      float* gmask = nullptr);
 size_t umma_bwd_data_gtile_bytes(const Geo& g, int operand);
 bool o_groups(const Geo& g, int* size);
 Geo o_group_geo(const Geo& g, int o0, int size);
@@ -99,9 +100,13 @@ size_t umma_bwd_workspace(const Geo& g, int operand) {
 // woff != nullptr: whole-layer backward — the companion offset convolution's backward runs as a PLAIN pass between the
 // DCN data gradient and the final transposition: grad_offset (goff) is its grad_out, its data gradient accumulates
 // into the SAME channels-last grad_x buffer, gwoff / gboff receive its parameter gradients.
+// mask != nullptr: modulated DCNv1 (DCNv2); gmask [B, N, Ho, Wo] is zeroed next to grad_offset and, like it, accumulates
+// over the output-channel groups.  Every branch below passes the mask on: fused data + weight gradient, tensor-path
+// data gradient + unfused weight gradient, generic data gradient + tensor-path weight gradient.
 int umma_backward_any(const Geo& g, int operand, int flags, const void* xv, const float* off, const void* wtv,
                       const void* goutv, float* gx, float* goff, float* gw, float* gb, void* workspace,
-                      cudaStream_t st, const float* woff, float* gwoff, float* gboff) {
+                      cudaStream_t st, const float* woff, float* gwoff, float* gboff, const float* mask,
+                      float* gmask) {
   int gsize;
   if (!o_groups(g, &gsize)) {
     set_error("umma backward: O = %d cannot be split into groups", g.O);
@@ -132,6 +137,7 @@ int umma_backward_any(const Geo& g, int operand, int flags, const void* xv, cons
     uint8_t* gtiles = wtiles + umma_bwd_data_wtile_bytes(g0, operand);
     if (want_gx) DCN_CUDA_TRY(cudaMemsetAsync(gxt, 0, sizeof(float) * (size_t)g.B * xt_image_stride(g), st));
     DCN_CUDA_TRY(cudaMemsetAsync(goff, 0, sizeof(float) * (size_t)g.B * 2 * g.N * g.HW, st));
+    if (mask) DCN_CUDA_TRY(cudaMemsetAsync(gmask, 0, sizeof(float) * (size_t)g.B * g.N * g.HW, st));
     // Torch layout: the staging pass of grad_out sums grad_bias on its way (every element passes through it once)
     const bool gb_rides = gb != nullptr && g.variant == DCN_VARIANT_TORCH;
     if (gb_rides) DCN_CUDA_TRY(cudaMemsetAsync(gb, 0, sizeof(float) * (size_t)g.O, st));
@@ -144,7 +150,7 @@ int umma_backward_any(const Geo& g, int operand, int flags, const void* xv, cons
       if ((rc = umma_bwd_data_any(gc, operand, xt, want_gx ? gxt : nullptr, off,
                                   (const uint8_t*)wtv + (size_t)o0 * g.K * esz,
                                   (const uint8_t*)goutv + (size_t)o0 * g.HW * esz, goff, gwc, wtiles, gtiles, st,
-                                  gb_rides ? gb + o0 : nullptr)))
+                                  gb_rides ? gb + o0 : nullptr, mask, gmask)))
         return rc;
     }
     if (woff && conv_offset_bwd_supported(g)) {
@@ -176,7 +182,7 @@ int umma_backward_any(const Geo& g, int operand, int flags, const void* xv, cons
     Tap* plan = (Tap*)rest;
     if ((rc = launch_plan(g, off, plan, st))) return rc;
     if ((rc = simt_backward(g, flags, (const float*)x, plan, (const float*)wtv, (const float*)goutv, gx, goff, gw,
-                            gb, st, SIMT_BWD_DATA | SIMT_BWD_BIAS)))
+                            gb, st, SIMT_BWD_DATA | SIMT_BWD_BIAS, mask, gmask)))
       return rc;
   }
   // everything that lived in `rest` (gxt, tiles, plan) is dead by now: the unfused weight-gradient
@@ -186,7 +192,7 @@ int umma_backward_any(const Geo& g, int operand, int flags, const void* xv, cons
     const bool data_on_umma = operand != DCN_OPERAND_FP32 || umma_bwd_data_supported(g0, operand);
     if (data_on_umma && umma_bwd_data_fuses_wgrad(gc, operand)) continue;
     if ((rc = umma_wgrad_any(gc, operand, xt, off, (const uint8_t*)goutv + (size_t)o0 * g.HW * esz,
-                             gw + (size_t)o0 * g.K, rest, st)))
+                             gw + (size_t)o0 * g.K, rest, st, mask)))
       return rc;
   }
   return DCN_OK;
@@ -202,7 +208,7 @@ int umma_layer_backward(const Geo& g, int flags, const void* x, const float* off
                         void* workspace, size_t workspace_bytes, cudaStream_t st) {
   float* goff = (float*)((uint8_t*)workspace + workspace_bytes - goff_bytes(g));
   return umma_backward_any(g, DCN_OPERAND_FP32, flags, x, off, wt, gout, gx, goff, gw, gb, workspace, st, woff, gwoff,
-                           gboff);
+                           gboff, nullptr, nullptr);
 }
 
 }  // namespace dcn

@@ -126,10 +126,12 @@ __device__ __forceinline__ RowInfo decode(const Params& P, int inst) {
 struct PlanWork {
   float ox, oy;
   int h, w, n, chan_base, gidx, valid;
+  float mk;  // MOD: the mask value, loaded on the same prefetch as the offsets
 };
 
-template <int VARIANT, bool PLAIN = false>
-__device__ __forceinline__ void plan_prepare(const Params& P, int tile, int cb, int e, PlanWork& pw) {
+template <int VARIANT, bool PLAIN = false, bool MOD = false>
+__device__ __forceinline__ void plan_prepare(const Params& P, int tile, int cb, int e, PlanWork& pw,
+                                             const float* __restrict__ mask = nullptr) {
   const Geo& g = P.g;
   pw.valid = 0;
   pw.ox = pw.oy = 0.f;
@@ -165,6 +167,11 @@ __device__ __forceinline__ void plan_prepare(const Params& P, int tile, int cb, 
     const float* ob = P.off + (size_t)b * 2 * g.N * g.HW;
     pw.ox = __ldg(ob + (size_t)off_row_ch(g, (int)n) * g.HW + p);
     pw.oy = __ldg(ob + (size_t)off_col_ch(g, (int)n) * g.HW + p);
+  }
+  if constexpr (MOD) {
+    static_assert(VARIANT != DCN_VARIANT_TORCH && !PLAIN, "modulation exists for the pixel-row DCNv1 layout only");
+    DCN_DEV_ASSERT(((size_t)b * g.N + n) * g.HW + p < (size_t)g.B * g.N * g.HW);
+    pw.mk = __ldg(mask + ((size_t)b * g.N + n) * g.HW + p);
   }
   pw.valid = 1;
 }
@@ -208,8 +215,16 @@ __device__ __forceinline__ ScatEntry plan_finish(const Geo& g, const PlanWork& p
 // PLAIN = backward of a regular convolution (the companion offset conv, Geo::plain): one exact pixel per column
 //         instead of four weighted corners — one red.global per column, the "sample" of the fused weight gradient
 //         is the pixel itself, no coordinate gradient
-template <int VARIANT, int RW, bool FUSE, bool BF, int PW, bool PLAIN = false>
-__global__ void __launch_bounds__(threads_of(PW), 1) bwd_data_kernel(const __grid_constant__ Params P) {
+// MOD = modulated DCNv1 (DCNv2; pixel-row layout): the plan ring carries one mask value per entry beside the scatter
+//       entries; per column the accumulator value gs is scaled by it once (grad_x and grad_offset then follow unchanged
+//       in form), a third per-column partial gs * bilinear sample is reduced over the lanes of the sampling point into
+//       ONE red.global per column of grad_mask, and the fused weight gradient's sample operand is m * sample.
+//       mask / gmask [B, N, Ho, Wo] (gmask zeroed) are trailing kernel arguments rather than Params fields: Params is
+//       also passed by value to gout_tiles_torch_kernel, whose following argument would move if Params grew.
+template <int VARIANT, int RW, bool FUSE, bool BF, int PW, bool PLAIN = false, bool MOD = false>
+__global__ void __launch_bounds__(threads_of(PW), 1) bwd_data_kernel(const __grid_constant__ Params P,
+                                                                     const float* __restrict__ mask,
+                                                                     float* __restrict__ gmask) {
   constexpr int NIMG = BF ? 1 : 2;
   typedef typename std::conditional<BF, __nv_bfloat16, float>::type XT;
   extern __shared__ __align__(1024) uint8_t smem_raw[];
@@ -226,7 +241,10 @@ __global__ void __launch_bounds__(threads_of(PW), 1) bwd_data_kernel(const __gri
   uint8_t* sbuf = wstage + (size_t)(P.w_resident ? P.w_resident : P.w_ring) * P.w_stage;
   const uint32_t s_img = 128u * 128u, s_buf = FUSE ? NIMG * s_img : 0u;
   ScatEntry* plan = reinterpret_cast<ScatEntry*>(sbuf + 2 * (size_t)s_buf);
-  uint64_t* bars = reinterpret_cast<uint64_t*>(plan + 2 * P.plan_cap);
+  // MOD: [2 x plan_cap] mask values, parallel to the plan ring
+  float* mplan = reinterpret_cast<float*>(plan + 2 * P.plan_cap);
+  uint64_t* bars = MOD ? reinterpret_cast<uint64_t*>(mplan + 2 * P.plan_cap)
+                       : reinterpret_cast<uint64_t*>(plan + 2 * P.plan_cap);
   uint64_t* wfull = bars;        // [2]
   uint64_t* wempty = bars + 2;   // [2]
   uint64_t* tfull = bars + 4;    // [2]
@@ -327,11 +345,13 @@ __global__ void __launch_bounds__(threads_of(PW), 1) bwd_data_kernel(const __gri
         bimg = tile / P.pix_blocks;
       }
       for (int cb = cb0; cb < cb1; ++cb) {
+        int mrow = 0;  // MOD: grad_mask index of this block's pixel column 0 for the lane's tap
         if (VARIANT != DCN_VARIANT_TORCH) {
           // Jittor: lane = column j = 128*cb + m = (tap j / C, channel j % C); slot = tap inside the block
           const int j = cb * 128 + m, n = j / g.C;
           chan = j - n * g.C;
           slot = n - (cb * 128) / g.C;
+          if (MOD) mrow = (bimg * g.N + n) * g.HW + (tile - bimg * P.pix_blocks) * ncols;
         }
         // byte-addressed image bases: address = base + zero-extended 32-bit offset (2 instructions)
         const char* ximg =
@@ -344,15 +364,41 @@ __global__ void __launch_bounds__(threads_of(PW), 1) bwd_data_kernel(const __gri
         // fused: this lane's row m of the sample operand (8-row groups of 1024 B, 128 B per row)
         uint8_t* s_row = sbuf + (size_t)sb * s_buf + (size_t)(m >> 3) * 1024 + (m & 7) * 128;
         const ScatEntry* pl = plan + pb * P.plan_cap + slot * ncols;
+        const float* mkp = mplan + pb * P.plan_cap + slot * ncols;  // MOD only
         const uint32_t taddr = tmem_base + ((uint32_t)(quarter * 32) << 16) + (uint32_t)(acc * ncols);
         // WIDE would reduce the coordinate gradient in batches of 16 columns (32 values over 32 lanes cost
         // the same 31 shuffles as 16 values do).  Measured SLOWER on B200 (cfg2: 13.2 vs 11.7 ms): one
         // long pass per block exposes more latency than the saved shuffles buy.  Kept for reference.
         constexpr bool WIDE = false;
         constexpr int NB = WIDE ? 2 : 1;  // 8-column sub-batches per reduction
+        static_assert(!MOD || !WIDE, "the grad_mask reduction assumes one 8-column batch");
+        // MOD: one grad_mask RED per column, after an 8-value reduce-scatter over the RW lanes of the sampling points
+        auto mask_red = [&](const int cc, float (&part_m)[8]) {
+          if (RW == 32) {
+#pragma unroll
+            for (int k = 0; k < 8; ++k) part_m[k] += __shfl_xor_sync(0xffffffffu, part_m[k], 16);
+          }
+#pragma unroll
+          for (int s = 8, n = 4; s >= 2; s >>= 1, n >>= 1) {
+            const bool up = (lane & s) != 0;
+#pragma unroll
+            for (int k = 0; k < n; ++k) {
+              const float send = up ? part_m[k] : part_m[k + n];
+              const float keep = up ? part_m[k + n] : part_m[k];
+              part_m[k] = keep + __shfl_xor_sync(grp_mask, send, s);
+            }
+          }
+          part_m[0] += __shfl_xor_sync(grp_mask, part_m[0], 1);
+          if ((gl & 1) == 0 && (RW == 16 || lane < 16)) {
+            const int col = cc + ((gl >> 1) & 7);
+            DCN_DEV_ASSERT(pl[col].gidx < 0 || (size_t)(mrow + col) < (size_t)g.B * g.N * g.HW);
+            if (pl[col].gidx >= 0 && part_m[0] != 0.f) atomicAdd(gmask + mrow + col, part_m[0]);
+          }
+        };
         // one pass = 8 * NB columns whose accumulator values are already in registers
         auto pass = [&](const int cc, const uint32_t* rawv) {
           float part_g[16 * NB];  // [0 .. 8*NB) g_ix of the batch's columns, [8*NB .. 16*NB) g_iy
+          float part_m[8];        // MOD: gA * sample of the batch's columns
 #pragma unroll
           for (int nb = 0; nb < NB; ++nb) {
           const int c0 = cc + 8 * nb;
@@ -360,7 +406,9 @@ __global__ void __launch_bounds__(threads_of(PW), 1) bwd_data_kernel(const __gri
           float smp8[8];     // fused: the 8 samples of this row
 #pragma unroll
           for (int u = 0; u < 8; ++u) {
-            const float gs = __uint_as_float(raw[u]);
+            const float ga = __uint_as_float(raw[u]);
+            const float mkv = MOD ? mkp[c0 + u] : 1.f;
+            const float gs = MOD ? ga * mkv : ga;
             const uint4 e4 = *reinterpret_cast<const uint4*>(pl + c0 + u);  // {base, fx, fy, gidx}
             const float fx = __uint_as_float(e4.y), fy = __uint_as_float(e4.z);
             // entry offsets are bytes of the float grad image; the bf16 x image is half as wide
@@ -391,7 +439,13 @@ __global__ void __launch_bounds__(threads_of(PW), 1) bwd_data_kernel(const __gri
             part_g[8 * nb + u] = gs * ((v1 - v0) * sy + (v3 - v2) * fy);
             part_g[8 * NB + 8 * nb + u] = gs * ((v2 - v0) * ex + (v3 - v1) * fx);
             // the sample itself (same blend order as the forward pass)
-            if (FUSE) smp8[u] = fmaf(v3, w3, fmaf(v2, w2, fmaf(v1, w1, v0 * w0)));
+            if (MOD) {
+              const float bil = fmaf(v3, w3, fmaf(v2, w2, fmaf(v1, w1, v0 * w0)));
+              part_m[u] = ga * bil;
+              if (FUSE) smp8[u] = mkv * bil;
+            } else if (FUSE) {
+              smp8[u] = fmaf(v3, w3, fmaf(v2, w2, fmaf(v1, w1, v0 * w0)));
+            }
           }
           if (FUSE) {
             // columns c0..c0+7 of row m: one 16-byte chunk of the MN-major operand, swizzled by m % 8
@@ -406,6 +460,7 @@ __global__ void __launch_bounds__(threads_of(PW), 1) bwd_data_kernel(const __gri
           }
           }  // sub-batch
           if (PLAIN) return;
+          if (MOD) mask_red(cc, part_m);
           // butterfly reduce-scatter over the RW lanes that share the sampling points:
           // afterwards lane gl (< 16*NB) holds the total of value index gl
           if (!WIDE && RW == 32) {
@@ -454,6 +509,9 @@ __global__ void __launch_bounds__(threads_of(PW), 1) bwd_data_kernel(const __gri
           char* gpair = gimg ? gimg - odd * 4 : nullptr;
           float part_g[8];  // [0..3] g_ix of this thread's 4 columns (both channels), [4..7] g_iy
           float sa[4], sb2[4];
+          float part_m[8];  // MOD: [0..3] gA * sample of this thread's 4 columns (both channels)
+          float4 mk4 = make_float4(1.f, 1.f, 1.f, 1.f);
+          if (MOD) mk4 = *reinterpret_cast<const float4*>(mkp + cu0);
 #pragma unroll
           for (int u = 0; u < 4; ++u) {
             const uint4 e4 = *reinterpret_cast<const uint4*>(pl + cu0 + u);  // {base, fx, fy, gidx}
@@ -496,6 +554,18 @@ __global__ void __launch_bounds__(threads_of(PW), 1) bwd_data_kernel(const __gri
             const float ex = __fsub_rn(1.0f, fx), sy = __fsub_rn(1.0f, fy);
             const float w0 = __fmul_rn(sy, ex), w1 = __fmul_rn(sy, fx), w2 = __fmul_rn(fy, ex),
                         w3 = __fmul_rn(fy, fx);
+            if (MOD) {
+              const float mkv = u == 0 ? mk4.x : (u == 1 ? mk4.y : (u == 2 ? mk4.z : mk4.w));
+              const float bila = fmaf(v3.x, w3, fmaf(v2.x, w2, fmaf(v1.x, w1, v0.x * w0)));
+              const float bilb = fmaf(v3.y, w3, fmaf(v2.y, w2, fmaf(v1.y, w1, v0.y * w0)));
+              part_m[u] = ga[u] * bila + gb[u] * bilb;
+              ga[u] *= mkv;
+              gb[u] *= mkv;
+              if (FUSE) {
+                sa[u] = mkv * bila;
+                sb2[u] = mkv * bilb;
+              }
+            }
             if (gpair && (int)e4.w >= 0) {
               char* gp = gpair + e4.x;
               atomicAdd(reinterpret_cast<float2*>(gp), make_float2(ga[u] * w0, gb[u] * w0));
@@ -507,7 +577,7 @@ __global__ void __launch_bounds__(threads_of(PW), 1) bwd_data_kernel(const __gri
                         gb[u] * ((v1.y - v0.y) * sy + (v3.y - v2.y) * fy);
             part_g[4 + u] = ga[u] * ((v2.x - v0.x) * ex + (v3.x - v1.x) * fx) +
                             gb[u] * ((v2.y - v0.y) * ex + (v3.y - v1.y) * fx);
-            if (FUSE) {
+            if (FUSE && !MOD) {
               sa[u] = fmaf(v3.x, w3, fmaf(v2.x, w2, fmaf(v1.x, w1, v0.x * w0)));
               sb2[u] = fmaf(v3.y, w3, fmaf(v2.y, w2, fmaf(v1.y, w1, v0.y * w0)));
             }
@@ -550,6 +620,28 @@ __global__ void __launch_bounds__(threads_of(PW), 1) bwd_data_kernel(const __gri
             if (gidx >= 0 && part_g[0] != 0.f)
               atomicAdd(P.goff + (size_t)gidx + (vi < 4 ? (size_t)P.ix_delta : 0),
                         part_g[0] * (vi < 4 ? P.scale_ix : P.scale_iy));
+          }
+          if (MOD) {
+            // grad_mask: the 4 values over the 16 lanes of equal parity, then one RED per column
+#pragma unroll
+            for (int k = 0; k < 4; ++k) part_m[k] += __shfl_xor_sync(0xffffffffu, part_m[k], 16);
+#pragma unroll
+            for (int s2 = 8, n = 2; s2 >= 4; s2 >>= 1, n >>= 1) {
+              const bool up = (lane & s2) != 0;
+#pragma unroll
+              for (int k = 0; k < n; ++k) {
+                const float send = up ? part_m[k] : part_m[k + n];
+                const float keep = up ? part_m[k + n] : part_m[k];
+                part_m[k] = keep + __shfl_xor_sync(0xffffffffu, send, s2);
+              }
+            }
+            part_m[0] += __shfl_xor_sync(0xffffffffu, part_m[0], 2);
+            if (lane < 16 && (lane & 2) == 0) {
+              // lane bits 3..2 -> column inside the thread's four
+              const int col = cu0 + ((lane >> 2) & 3);
+              DCN_DEV_ASSERT(pl[col].gidx < 0 || (size_t)(mrow + col) < (size_t)g.B * g.N * g.HW);
+              if (pl[col].gidx >= 0 && part_m[0] != 0.f) atomicAdd(gmask + mrow + col, part_m[0]);
+            }
           }
         };
         constexpr bool PAIR = RW == 32;
@@ -861,7 +953,7 @@ __global__ void __launch_bounds__(threads_of(PW), 1) bwd_data_kernel(const __gri
     if (tile0 < P.num_tiles) {
 #pragma unroll
       for (int u = 0; u < kPlanPerThread; ++u)
-        if (pt + u * kPlanThreads < n_ent) plan_prepare<VARIANT, PLAIN>(P, tile0, cb0, pt + u * kPlanThreads, pw[u]);
+        if (pt + u * kPlanThreads < n_ent) plan_prepare<VARIANT, PLAIN, MOD>(P, tile0, cb0, pt + u * kPlanThreads, pw[u], mask);
     }
     for (int tile = tile0; tile < P.num_tiles; tile += tile_step) {
       for (int cb = cb0; cb < cb1; ++cb) {
@@ -871,6 +963,13 @@ __global__ void __launch_bounds__(threads_of(PW), 1) bwd_data_kernel(const __gri
         for (int u = 0; u < kPlanPerThread; ++u)
           if (pt + u * kPlanThreads < n_ent)
             pl[pt + u * kPlanThreads] = PLAIN ? plan_finish_plain(g, pw[u]) : plan_finish(g, pw[u]);
+        if (MOD) {
+          // dead entries get 0: their sample is 0, and m * 0 must stay finite for the fused weight gradient
+          float* mpl = mplan + pb * P.plan_cap;
+#pragma unroll
+          for (int u = 0; u < kPlanPerThread; ++u)
+            if (pt + u * kPlanThreads < n_ent) mpl[pt + u * kPlanThreads] = pw[u].valid ? pw[u].mk : 0.f;
+        }
         __syncwarp();
         if (lane == 0) mbar_arrive(&pfull[pb]);
         int ntile = tile, ncb = cb + 1;
@@ -881,7 +980,7 @@ __global__ void __launch_bounds__(threads_of(PW), 1) bwd_data_kernel(const __gri
         if (ntile < P.num_tiles) {
 #pragma unroll
           for (int u = 0; u < kPlanPerThread; ++u)
-            if (pt + u * kPlanThreads < n_ent) plan_prepare<VARIANT, PLAIN>(P, ntile, ncb, pt + u * kPlanThreads, pw[u]);
+            if (pt + u * kPlanThreads < n_ent) plan_prepare<VARIANT, PLAIN, MOD>(P, ntile, ncb, pt + u * kPlanThreads, pw[u], mask);
         }
         pb ^= 1;
         if (pb == 0) pphase ^= 1;
@@ -1296,9 +1395,10 @@ size_t umma_bwd_data_gtile_bytes(const Geo& g, int operand) {
 // gxt (channels-last grad_x, may be null), goff and — when the shape fuses the weight gradient
 // (umma_bwd_data_fuses_wgrad) — gw must be zero on entry.
 // gb_fused (Torch layout only, may be null): grad_bias [g.O], zeroed by the caller, summed by the grad_out staging pass
+// mask / gmask (DCNv1 only, both or neither): modulated; gmask must be zero on entry like goff.
 int umma_bwd_data_any(const Geo& g, int operand, const void* xt, float* gxt, const float* off, const void* wt,
                       const void* gout, float* goff, float* gw, uint8_t* wtiles, uint8_t* gtiles,
-                      cudaStream_t st, float* gb_fused) {
+                      cudaStream_t st, float* gb_fused, const float* mask, float* gmask) {
   bd::Params P;
   P.g = g;
   const bool bf = operand == DCN_OPERAND_BF16;
@@ -1344,6 +1444,8 @@ int umma_bwd_data_any(const Geo& g, int operand, const void* xt, float* gxt, con
                 (size_t)(P.w_resident ? P.w_resident : P.w_ring) * P.w_stage +
                 (P.fuse_w ? 2 * nimg * (size_t)(128 * 128) : 0) +
                 2 * (size_t)P.plan_cap * sizeof(bd::ScatEntry) + 256 + 1024;
+  // modulated: the mask values beside the plan ring (float per entry; the kernel traps if the window is too small)
+  if (mask) smem += 2 * (size_t)P.plan_cap * sizeof(float);
   if (smem > 227 * 1024) smem = 227 * 1024;  // tight plan (choose_slices): less alignment slack, checked in the kernel
   int dev = 0, sms = 148;
   cudaGetDevice(&dev);
@@ -1362,11 +1464,11 @@ int umma_bwd_data_any(const Geo& g, int operand, const void* xt, float* gxt, con
     if (bf) {                                                                                             \
       DCN_CUDA_TRY(cudaFuncSetAttribute(bd::bwd_data_kernel<V, RW, F, true, PW>,                          \
                                         cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));         \
-      bd::bwd_data_kernel<V, RW, F, true, PW><<<grid, bd::threads_of(PW), smem, st>>>(P);              \
+      bd::bwd_data_kernel<V, RW, F, true, PW><<<grid, bd::threads_of(PW), smem, st>>>(P, mask, gmask);              \
     } else {                                                                                              \
       DCN_CUDA_TRY(cudaFuncSetAttribute(bd::bwd_data_kernel<V, RW, F, false, PW>,                         \
                                         cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));         \
-      bd::bwd_data_kernel<V, RW, F, false, PW><<<grid, bd::threads_of(PW), smem, st>>>(P);             \
+      bd::bwd_data_kernel<V, RW, F, false, PW><<<grid, bd::threads_of(PW), smem, st>>>(P, mask, gmask);             \
     }                                                                                                     \
   } while (0)
   // <= 128 plan entries per block (2 per plan thread): 2 plan warps are enough (20 warps, 96 registers for
@@ -1382,7 +1484,7 @@ int umma_bwd_data_any(const Geo& g, int operand, const void* xt, float* gxt, con
   do {                                                                                                        \
     DCN_CUDA_TRY(cudaFuncSetAttribute(bd::bwd_data_kernel<DCN_VARIANT_JITTOR, RW, true, false, PW, true>,     \
                                       cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));               \
-    bd::bwd_data_kernel<DCN_VARIANT_JITTOR, RW, true, false, PW, true><<<grid, bd::threads_of(PW), smem, st>>>(P); \
+    bd::bwd_data_kernel<DCN_VARIANT_JITTOR, RW, true, false, PW, true><<<grid, bd::threads_of(PW), smem, st>>>(P, mask, gmask); \
   } while (0)
     if (narrow) {
       if (slim) DCN_LAUNCH_PLAIN(16, 2);
@@ -1400,7 +1502,39 @@ int umma_bwd_data_any(const Geo& g, int operand, const void* xt, float* gxt, con
     if (slim) DCN_LAUNCH_BD(V, RW, F, 2);              \
     else DCN_LAUNCH_BD(V, RW, F, 4);                   \
   } while (0)
-  if (g.variant == DCN_VARIANT_TORCH) {
+  if (mask) {
+    // modulated DCNv1: the pixel-row instantiations with MOD
+    if (g.variant != DCN_VARIANT_DCNV1 || !gmask) {
+      set_error("umma bwd_data: a mask exists for the DCNv1 variant only, and needs grad_mask");
+      return DCN_ERR_UNSUPPORTED;
+    }
+#define DCN_LAUNCH_MOD(RW, F, PW)                                                                               \
+  do {                                                                                                          \
+    if (bf) {                                                                                                   \
+      DCN_CUDA_TRY(cudaFuncSetAttribute(bd::bwd_data_kernel<DCN_VARIANT_JITTOR, RW, F, true, PW, false, true>,  \
+                                        cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));               \
+      bd::bwd_data_kernel<DCN_VARIANT_JITTOR, RW, F, true, PW, false, true><<<grid, bd::threads_of(PW), smem, st>>>(P, mask, gmask); \
+    } else {                                                                                                    \
+      DCN_CUDA_TRY(cudaFuncSetAttribute(bd::bwd_data_kernel<DCN_VARIANT_JITTOR, RW, F, false, PW, false, true>, \
+                                        cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));               \
+      bd::bwd_data_kernel<DCN_VARIANT_JITTOR, RW, F, false, PW, false, true><<<grid, bd::threads_of(PW), smem, st>>>(P, mask, gmask); \
+    }                                                                                                           \
+  } while (0)
+#define DCN_LAUNCH_MOD2(RW, F)                         \
+  do {                                                 \
+    if (slim) DCN_LAUNCH_MOD(RW, F, 2);                \
+    else DCN_LAUNCH_MOD(RW, F, 4);                     \
+  } while (0)
+    if (P.fuse_w) {
+      if (narrow) DCN_LAUNCH_MOD2(16, true);
+      else DCN_LAUNCH_MOD2(32, true);
+    } else {
+      if (narrow) DCN_LAUNCH_MOD2(16, false);
+      else DCN_LAUNCH_MOD2(32, false);
+    }
+#undef DCN_LAUNCH_MOD2
+#undef DCN_LAUNCH_MOD
+  } else if (g.variant == DCN_VARIANT_TORCH) {
     if (P.fuse_w) {
       if (narrow) DCN_LAUNCH_BD(DCN_VARIANT_TORCH, 16, true, 4);
       else DCN_LAUNCH_BD2(DCN_VARIANT_TORCH, 32, true);

@@ -82,18 +82,25 @@ struct FwdParams {
   // steps then gather the same 64 channels around the same pixels (only the tap's offset differs), so the
   // corner lines of one step are L1 hits of the next.  The accumulation order over K is irrelevant.
   int kperm_slabs;
+  // modulated instantiations (MOD, DCNv1 only): mask [B, N, Ho, Wo] float32; every sample is scaled by
+  // mask[b, n, p], folded into the four corner weights of its plan entry (appended last: the fields above keep
+  // their parameter offsets)
+  const float* mask;
 };
 
 // One plan entry in the making: the index math is done and the two offset loads are in
 // flight (issued one K block ahead so that their latency hides behind the gather phase).
+// mk: the modulation scalar (MOD instantiations only; loaded on the same prefetch as the offsets).
 struct PlanWork {
   float ox, oy;
   int h, w, n, chan_base, valid;
+  float mk;
 };
 
-template <int VARIANT, bool PLAIN = false>
+template <int VARIANT, bool PLAIN = false, bool MOD = false>
 __device__ __forceinline__ void plan_prepare(const Geo& g, const Tiling& t, const float* __restrict__ off,
-                                             int tile, int kb, int e, PlanWork& pw) {
+                                             int tile, int kb, int e, PlanWork& pw,
+                                             const float* __restrict__ mask = nullptr) {
   pw.valid = 0;
   pw.ox = pw.oy = 0.f;
   pw.h = pw.w = pw.n = pw.chan_base = 0;
@@ -131,6 +138,11 @@ __device__ __forceinline__ void plan_prepare(const Geo& g, const Tiling& t, cons
     pw.ox = __ldg(ob + (size_t)off_row_ch(g, n) * g.HW + p);
     pw.oy = __ldg(ob + (size_t)off_col_ch(g, n) * g.HW + p);
   }
+  if constexpr (MOD) {
+    static_assert(VARIANT != DCN_VARIANT_TORCH && !PLAIN, "modulation exists for the pixel-row DCNv1 layout only");
+    DCN_DEV_ASSERT(((size_t)b * g.N + n) * g.HW + p < (size_t)g.B * g.N * g.HW);
+    pw.mk = __ldg(mask + ((size_t)b * g.N + n) * g.HW + p);
+  }
   pw.valid = 1;
 }
 
@@ -151,7 +163,9 @@ __device__ __forceinline__ PlanEntry plan_finish_plain(const Geo& g, const PlanW
 
 // coordinate chain (bit-exact, dcn_common.cuh:tap_of) -> branch-free gather entry: corners
 // outside the image fall on the zero frame of the staging copy, samples with no corner inside
-// (and padding rows / columns) on the frame-only block with zero weights
+// (and padding rows / columns) on the frame-only block with zero weights.
+// MOD: the corner weights carry the sample's mask (m * w_k; m == 1 leaves them bit-identical)
+template <bool MOD = false>
 __device__ __forceinline__ PlanEntry plan_finish(const Geo& g, const PlanWork& pw) {
   PlanEntry e;
   int base = xt_null_base(g);
@@ -162,6 +176,10 @@ __device__ __forceinline__ PlanEntry plan_finish(const Geo& g, const PlanWork& p
     bool inside;
     base = xt_corner_base(g, tp.y0, tp.x0, inside);
     if (inside) corner_weights(tp, e.w);
+    if constexpr (MOD) {
+#pragma unroll
+      for (int k = 0; k < 4; ++k) e.w[k] = __fmul_rn(e.w[k], pw.mk);
+    }
   }
   base += pw.chan_base;
   const int pitch = xt_row_pitch(g);
@@ -194,7 +212,9 @@ __device__ __forceinline__ void split4(const float4& v, uint2& hi, uint2& lo) {
 // PW / GW = plan / gather warps.  4 + 16 everywhere except the Torch layout with 16 channels per sampling point
 // (Rt = 8: 512 coordinate chains per K block for 2048 gather items — the 4 plan warps, one per scheduler, were the
 // critical path and the gather warps waited 40 % of the time, profiles/r1_ncu_det2.txt): 8 + 8 there.
-template <int VARIANT, int MODE, bool BF, bool PLAIN = false, int PW = 4, int GW = 16>
+// MOD = modulated deformable convolution (DCNv2, pixel-row layout): the plan warps scale each entry's corner weights
+// by its mask value, so the gather, MMA and epilogue roles are the unmodulated ones.
+template <int VARIANT, int MODE, bool BF, bool PLAIN = false, int PW = 4, int GW = 16, bool MOD = false>
 __global__ void __launch_bounds__((kFirstPlanWarp + PW + GW) * 32, 1)
     umma_gemm_kernel(const __grid_constant__ FwdParams P, const __grid_constant__ CUtensorMap tmap_out) {
   // role layout of this instantiation (shadows the file-scope defaults)
@@ -601,7 +621,7 @@ __global__ void __launch_bounds__((kFirstPlanWarp + PW + GW) * 32, 1)
 #pragma unroll
       for (int u = 0; u < kPlanPerThread; ++u)
         if (pt + u * kPlanThreads < n_ent)
-          plan_prepare<VARIANT, PLAIN>(g, t, P.off, tile0, kb_of(kb0), pt + u * kPlanThreads, pw[u]);
+          plan_prepare<VARIANT, PLAIN, MOD>(g, t, P.off, tile0, kb_of(kb0), pt + u * kPlanThreads, pw[u], P.mask);
     }
     for (int tile = tile0; tile < t.num_tiles; tile = next_tile(tile)) {
       for (int kb = kb0; kb < kb1; ++kb) {
@@ -611,7 +631,7 @@ __global__ void __launch_bounds__((kFirstPlanWarp + PW + GW) * 32, 1)
 #pragma unroll
         for (int u = 0; u < kPlanPerThread; ++u)
           if (pt + u * kPlanThreads < n_ent)
-            pl[pt + u * kPlanThreads] = PLAIN ? plan_finish_plain(g, pw[u]) : plan_finish(g, pw[u]);
+            pl[pt + u * kPlanThreads] = PLAIN ? plan_finish_plain(g, pw[u]) : plan_finish<MOD>(g, pw[u]);
         __syncwarp();
         if (lane == 0) mbar_arrive(&pfull[pbuf]);
         // ... and start the next block's
@@ -624,7 +644,7 @@ __global__ void __launch_bounds__((kFirstPlanWarp + PW + GW) * 32, 1)
 #pragma unroll
           for (int u = 0; u < kPlanPerThread; ++u)
             if (pt + u * kPlanThreads < n_ent)
-              plan_prepare<VARIANT, PLAIN>(g, t, P.off, ntile, kb_of(nkb), pt + u * kPlanThreads, pw[u]);
+              plan_prepare<VARIANT, PLAIN, MOD>(g, t, P.off, ntile, kb_of(nkb), pt + u * kPlanThreads, pw[u], P.mask);
         }
         pbuf ^= 1;
         if (pbuf == 0) pphase ^= 1;
@@ -1009,6 +1029,7 @@ static void common_params(const Geo& g, FwdParams& P) {
   P.box_r = 0;
   P.stage_out_bytes = 0;
   P.kperm_slabs = 0;
+  P.mask = nullptr;
 }
 
 template <int MODE>
@@ -1032,6 +1053,30 @@ static int launch_gemm(const Geo& g, int operand, const FwdParams& P, const CUte
     umma_gemm_kernel<V, MODE, BFV><<<grid, kFwdThreads, smem, st>>>(P, tmap);                              \
   } while (0)
   const bool bf = operand == DCN_OPERAND_BF16;
+  if (P.mask) {
+    // modulated (DCNv1 only): the pixel-row instantiations with the mask folded into the plan entries
+    if (g.variant != DCN_VARIANT_DCNV1) {
+      set_error("umma: a mask exists for the DCNv1 variant only");
+      return DCN_ERR_UNSUPPORTED;
+    }
+    const int n_ent = 128 * P.t.taps_per_kb;
+#define DCN_GEMM_MOD(BFV, PWV, GWV)                                                                         \
+  do {                                                                                                     \
+    DCN_CUDA_TRY(cudaFuncSetAttribute(umma_gemm_kernel<DCN_VARIANT_JITTOR, MODE, BFV, false, PWV, GWV, true>, \
+                                      cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));            \
+    umma_gemm_kernel<DCN_VARIANT_JITTOR, MODE, BFV, false, PWV, GWV, true>                                 \
+        <<<grid, (kFirstPlanWarp + PWV + GWV) * 32, smem, st>>>(P, tmap);                                   \
+  } while (0)
+    if (n_ent > 256) {
+      if (bf) DCN_GEMM_MOD(true, 8, 8);
+      else DCN_GEMM_MOD(false, 8, 8);
+    } else {
+      if (bf) DCN_GEMM_MOD(true, 4, 16);
+      else DCN_GEMM_MOD(false, 4, 16);
+    }
+#undef DCN_GEMM_MOD
+    return DCN_OK;
+  }
   // more than 256 coordinate chains per K block (16 channels per sampling point: Torch layout with Rt = 8, pixel-row
   // layouts with 4 taps per K block): 8 plan + 8 gather warps
   const int n_ent = g.variant == DCN_VARIANT_TORCH ? P.t.Rt * 64 : 128 * P.t.taps_per_kb;
@@ -1068,7 +1113,8 @@ static int launch_gemm(const Geo& g, int operand, const FwdParams& P, const CUte
 // stage_x = false: the head of the workspace already holds the staged copy of x (an earlier
 // output-channel group of the same call wrote it)
 int umma_forward_any(const Geo& g, int operand, const void* x, const float* off, const void* wt,
-                     const float* bias, float* out, void* workspace, cudaStream_t st, bool stage_x) {
+                     const float* bias, float* out, void* workspace, cudaStream_t st, bool stage_x,
+                     const float* mask) {
   FwdParams P;
   P.g = g;
   if (!make_tiling(g, &P.t)) {
@@ -1087,6 +1133,7 @@ int umma_forward_any(const Geo& g, int operand, const void* x, const float* off,
   P.wtiles = wtiles;
   P.bias = bias;
   P.out = out;
+  P.mask = mask;
   P.b_tile = (uint32_t)g.O * 128;
   P.stage_bytes = nimg * (kATile + P.b_tile);
   size_t fixed = 2 * (size_t)P.plan_cap * sizeof(PlanEntry) + 256 + 1024;  // plan ring, barriers, align slack
@@ -1167,17 +1214,18 @@ int umma_offset_conv_forward(const Geo& g, const void* x, const float* woff, con
     return conv_offset_forward(g, (const float*)workspace, woff, boff, offset_out,
                                (uint8_t*)workspace + umma_xt_bytes(g, DCN_OPERAND_FP32), st);
   const Geo gp = plain_geo(g, t, true);
-  return umma_forward_any(gp, DCN_OPERAND_FP32, x, nullptr, woff, boff, offset_out, workspace, st, false);
+  return umma_forward_any(gp, DCN_OPERAND_FP32, x, nullptr, woff, boff, offset_out, workspace, st, false, nullptr);
 }
 
 // grad_weight[O, K] (zeroed here) = sum over all rows of gout^T * S, S re-sampled by the same
-// plan / gather warps as the forward pass.  xt = channels-last staging copy (already built).
+// plan / gather warps as the forward pass (mask != null: S = m * bilinear sample, as in the modulated forward).
+// xt = channels-last staging copy (already built).
 size_t umma_wgrad_gtile_bytes(const Geo& g, int operand);
 int launch_gout_tiles_fwd_order(const Geo& g, int operand, const void* gout, uint8_t* gtiles, cudaStream_t st);
 
 // gtiles: scratch of umma_wgrad_gtile_bytes() for the staged grad_out tile images (Torch layout; unused otherwise)
 int umma_wgrad_any(const Geo& g, int operand, const void* xt, const float* off, const void* gout, float* gw,
-                   uint8_t* gtiles, cudaStream_t st) {
+                   uint8_t* gtiles, cudaStream_t st, const float* mask) {
   FwdParams P;
   P.g = g;
   if (!make_tiling(g, &P.t)) {
@@ -1195,6 +1243,7 @@ int umma_wgrad_any(const Geo& g, int operand, const void* xt, const float* off, 
   P.gout = gout;
   P.gw = gw;
   P.gtiles = gtiles;
+  P.mask = mask;
   P.g_OB = (g.O + 63) / 64;
   {
     int rc = launch_gout_tiles_fwd_order(g, operand, gout, gtiles, st);

@@ -15,12 +15,14 @@ namespace dcn {
 bool umma_fwd_supported(const Geo& g, int operand);
 size_t umma_fwd_workspace(const Geo& g, int operand);
 int umma_forward_any(const Geo& g, int operand, const void* x, const float* off, const void* wt,
-                     const float* bias, float* out, void* workspace, cudaStream_t st, bool stage_x);
+                     const float* bias, float* out, void* workspace, cudaStream_t st, bool stage_x,
+                     const float* mask);
 bool umma_bwd_supported(const Geo& g, int operand);
 size_t umma_bwd_workspace(const Geo& g, int operand);
 int umma_backward_any(const Geo& g, int operand, int flags, const void* x, const float* off, const void* wt,
                       const void* gout, float* gx, float* goff, float* gw, float* gb, void* workspace,
-                      cudaStream_t st, const float* woff, float* gwoff, float* gboff);
+                      cudaStream_t st, const float* woff, float* gwoff, float* gboff, const float* mask,
+                      float* gmask);
 
 bool o_groups(const Geo& g, int* size) {
   if (g.O <= 256) {
@@ -58,7 +60,7 @@ size_t umma_workspace_bytes(const Geo& g, int operand, int phase) {
 }
 
 int umma_forward(const Geo& g, int operand, int flags, const void* x, const float* off, const void* wt,
-                 const float* bias, void* out, void* workspace, cudaStream_t st) {
+                 const float* bias, void* out, void* workspace, cudaStream_t st, const float* mask) {
   int size;
   if (!o_groups(g, &size)) {
     set_error("umma forward: O = %d cannot be split into groups", g.O);
@@ -69,7 +71,7 @@ int umma_forward(const Geo& g, int operand, int flags, const void* x, const floa
     const Geo gc = o_group_geo(g, o0, size);
     const int rc = umma_forward_any(gc, operand, x, off, (const uint8_t*)wt + (size_t)o0 * g.K * esz,
                                     bias ? bias + o0 : nullptr, (float*)out + (size_t)o0 * g.HW, workspace, st,
-                                    o0 == 0 && !(flags & DCN_FLAG_XT_STAGED));
+                                    o0 == 0 && !(flags & DCN_FLAG_XT_STAGED), mask);
     if (rc) return rc;
   }
   return DCN_OK;
@@ -77,9 +79,9 @@ int umma_forward(const Geo& g, int operand, int flags, const void* x, const floa
 
 int umma_backward(const Geo& g, int operand, int flags, const void* x, const float* off, const void* wt,
                   const void* gout, float* gx, float* goff, float* gw, float* gb, void* workspace,
-                  cudaStream_t st) {
+                  cudaStream_t st, const float* mask, float* gmask) {
   return umma_backward_any(g, operand, flags, x, off, wt, gout, gx, goff, gw, gb, workspace, st, nullptr, nullptr,
-                           nullptr);
+                           nullptr, mask, gmask);
 }
 
 }  // namespace dcn

@@ -172,6 +172,84 @@ def dcn_backward(x, offset, weight, grad_out, has_bias, kernel_size=3, stride=1,
     return gx, goff, gw, gb
 
 
+# ---- modulated deformable convolution (DCNv2): DCNv1 sampling, every sample scaled by mask[b, n, p] ----------------
+def _check_mask(mask, shp, Ho, Wo):
+    N = shp.kh * shp.kw
+    if tuple(mask.shape) != (shp.B, N, Ho, Wo):
+        raise ValueError(f"mask shape {tuple(mask.shape)} != {(shp.B, N, Ho, Wo)} ([B, kh*kw, H_out, W_out])")
+
+
+def dcn_forward_modulated(x, offset, mask, weight, bias, kernel_size=3, stride=1, padding=1, operand=OPERAND_FP32,
+                          flags=0, ws=None):
+    """out[B,O,Ho,Wo] = modulated DCNv1 forward on CUDA tensors (no autograd); mask [B, kh*kw, Ho, Wo] float32
+    (torchvision's tap order, any values).  Arguments otherwise as dcn_forward with variant = VARIANT_DCNV1."""
+    lib = _lib.load()
+    shp = _shape_of(x, weight, kernel_size, stride, padding, VARIANT_DCNV1, operand, flags)
+    Ho, Wo = _lib.output_hw(shp)
+    N = shp.kh * shp.kw
+    if tuple(offset.shape) != (shp.B, 2 * N, Ho, Wo):
+        raise ValueError(f"offset shape {tuple(offset.shape)} != {(shp.B, 2 * N, Ho, Wo)}")
+    if tuple(weight.shape) != (shp.O, shp.C, shp.kh, shp.kw):
+        raise ValueError(f"weight shape {tuple(weight.shape)} != {(shp.O, shp.C, shp.kh, shp.kw)}")
+    _check_mask(mask, shp, Ho, Wo)
+    act = torch.bfloat16 if operand == OPERAND_BF16 else torch.float32
+    x, weight = _dev_ready(x, act), _dev_ready(weight, act)
+    offset, mask, bias = _dev_ready(offset), _dev_ready(mask), _dev_ready(bias)
+    out = torch.empty((shp.B, shp.O, Ho, Wo), dtype=torch.float32, device=x.device)
+    with torch.cuda.device(x.device):
+        stream = torch.cuda.current_stream(x.device)
+        need = lib.dcn_workspace_bytes(ctypes.byref(shp), PHASE_FORWARD)
+        if ws is None:
+            ws = _workspace(x.device, stream.cuda_stream, need)
+        rc = lib.dcn_forward_modulated(ctypes.byref(shp), _ptr(x), _ptr(offset), _ptr(mask), _ptr(weight), _ptr(bias),
+                                       _ptr(out), _ptr(ws), ws.numel(), ctypes.c_void_p(stream.cuda_stream))
+    _lib.check(rc, "dcn_forward_modulated")
+    return out
+
+
+def dcn_backward_modulated(x, offset, mask, weight, grad_out, has_bias, kernel_size=3, stride=1, padding=1,
+                           operand=OPERAND_FP32, flags=0, need_grad_x=True, ws=None, xt_staged=False, grad_x=None):
+    """-> grad_x (or None), grad_offset, grad_mask, grad_weight, grad_bias (or None); all float32.
+    Arguments as dcn_backward with variant = VARIANT_DCNV1, plus the forward's mask."""
+    lib = _lib.load()
+    if grad_x is not None:
+        if not need_grad_x:
+            raise ValueError("grad_x given but need_grad_x is False")
+        if grad_x.dtype != torch.float32 or tuple(grad_x.shape) != tuple(x.shape) or not grad_x.is_contiguous() \
+                or grad_x.data_ptr() % 16:
+            raise ValueError("grad_x must be a dense, 16-byte aligned float32 tensor of x's shape")
+        flags |= FLAG_ACCUM_GRAD_X
+    elif flags & FLAG_ACCUM_GRAD_X:
+        raise ValueError("FLAG_ACCUM_GRAD_X needs the tensor to accumulate into: pass grad_x=")
+    if not need_grad_x:
+        flags |= FLAG_NO_GRAD_X
+    if xt_staged and ws is not None:
+        flags |= FLAG_XT_STAGED
+    shp = _shape_of(x, weight, kernel_size, stride, padding, VARIANT_DCNV1, operand, flags)
+    Ho, Wo = _lib.output_hw(shp)
+    N = shp.kh * shp.kw
+    _check_mask(mask, shp, Ho, Wo)
+    act = torch.bfloat16 if operand == OPERAND_BF16 else torch.float32
+    x, weight, grad_out = _dev_ready(x, act), _dev_ready(weight, act), _dev_ready(grad_out, act)
+    offset, mask = _dev_ready(offset), _dev_ready(mask)
+    dev = x.device
+    gx = grad_x if grad_x is not None else (torch.empty(x.shape, dtype=torch.float32, device=dev) if need_grad_x else None)
+    goff = torch.empty((shp.B, 2 * N, Ho, Wo), dtype=torch.float32, device=dev)
+    gmask = torch.empty((shp.B, N, Ho, Wo), dtype=torch.float32, device=dev)
+    gw = torch.empty(weight.shape, dtype=torch.float32, device=dev)
+    gb = torch.empty((shp.O,), dtype=torch.float32, device=dev) if has_bias else None
+    with torch.cuda.device(dev):
+        stream = torch.cuda.current_stream(dev)
+        need = lib.dcn_workspace_bytes(ctypes.byref(shp), PHASE_BACKWARD)
+        if ws is None:
+            ws = _workspace(dev, stream.cuda_stream, need)
+        rc = lib.dcn_backward_modulated(ctypes.byref(shp), _ptr(x), _ptr(offset), _ptr(mask), _ptr(weight),
+                                        _ptr(grad_out), _ptr(gx), _ptr(goff), _ptr(gmask), _ptr(gw), _ptr(gb),
+                                        _ptr(ws), ws.numel(), ctypes.c_void_p(stream.cuda_stream))
+    _lib.check(rc, "dcn_backward_modulated")
+    return gx, goff, gmask, gw, gb
+
+
 # ---- whole layer: companion offset conv + DCN span on the engine (SURVEY 8f.1) -----------------------------------
 def layer_supported(x_shape, out_channels, kernel_size=3, stride=1, padding=1, variant=VARIANT_TORCH,
                     operand=OPERAND_FP32, flags=0):
@@ -390,13 +468,79 @@ def deform_conv2d(x, offset, weight, bias=None, kernel_size=3, stride=1, padding
     return DeformConvFunction.apply(x, offset, weight, bias, cfg)
 
 
-def deform_conv2d_v1(input, offset, weight, bias=None, stride=1, padding=0):
-    """Standard deformable convolution v1 with the call signature (and semantics) of
-    ``torchvision.ops.deform_conv2d(input, offset, weight, bias, stride, padding)`` for one offset
-    group, no mask, dilation 1 — the same kernels as the reference's operators with the textbook
-    coordinate generator (SURVEY.md 8f.3).  Differentiable in input, offset, weight and bias."""
+class ModulatedDeformConvFunction(torch.autograd.Function):
+    """autograd node of the modulated DCNv1 operator (DCNv2): differentiable in x, offset, mask, weight and bias.
+    Host tensors are accepted and answered on their device, as DeformConvFunction does."""
+
+    @staticmethod
+    def forward(ctx, x, offset, mask, weight, bias, cfg):
+        kernel_size, stride, padding, operand, flags = cfg
+        home = x.device
+        dev = _compute_device(x)
+        xd, od, md, wd = (_to_device(t, dev) for t in (x, offset, mask, weight))
+        bd = _to_device(bias, dev)
+        out = dcn_forward_modulated(xd, od, md, wd, bd, kernel_size, stride, padding, operand, flags)
+        ctx.save_for_backward(xd, od, md, wd)
+        ctx.cfg, ctx.home, ctx.has_bias = cfg, home, bias is not None
+        ctx.dtypes = (x.dtype, offset.dtype, mask.dtype, weight.dtype)
+        return out if home == dev else out.to(home)
+
+    @staticmethod
+    def backward(ctx, grad_out):
+        xd, od, md, wd = ctx.saved_tensors
+        kernel_size, stride, padding, operand, flags = ctx.cfg
+        flags &= ~(FLAG_ACCUM_GRAD_X | FLAG_RELU_OUT)
+        dev = xd.device
+        grad_out = _to_device(grad_out, dev)
+        gx, goff, gmask, gw, gb = dcn_backward_modulated(xd, od, md, wd, grad_out, ctx.has_bias, kernel_size, stride,
+                                                         padding, operand, flags,
+                                                         need_grad_x=ctx.needs_input_grad[0])
+        home = ctx.home
+
+        def back(t, dtype):
+            if t is None:
+                return None
+            t = t.to(dtype) if t.dtype != dtype else t
+            return t if home == dev else t.to(home)
+
+        return (back(gx, ctx.dtypes[0]), back(goff, ctx.dtypes[1]), back(gmask, ctx.dtypes[2]),
+                back(gw, ctx.dtypes[3]), back(gb, torch.float32), None)
+
+
+def deform_conv2d_modulated(x, offset, mask, weight, bias=None, kernel_size=3, stride=1, padding=1,
+                            operand=OPERAND_FP32, flags=0):
+    """Differentiable modulated DCNv1 (DCNv2) core: mask [B, kh*kw, Ho, Wo] scales every sample."""
+    cfg = (_lib._pair(kernel_size), _lib._pair(stride), _lib._pair(padding), operand, flags & ~FLAG_RELU_OUT)
+    return ModulatedDeformConvFunction.apply(x, offset, mask, weight, bias, cfg)
+
+
+def _out_hw(H, W, kernel_size, stride, padding):
+    (kh, kw), (sh, sw), (ph, pw) = kernel_size, stride, padding
+    return (H + 2 * ph - kh) // sh + 1, (W + 2 * pw - kw) // sw + 1
+
+
+def deform_conv2d_v1(input, offset, weight, bias=None, stride=1, padding=0, dilation=1, mask=None):
+    """Standard deformable convolution with the call signature (and semantics) of
+    ``torchvision.ops.deform_conv2d(input, offset, weight, bias, stride, padding, dilation, mask)`` for one offset
+    group and dilation 1 — the same kernels as the reference's operators with the textbook coordinate generator
+    (SURVEY.md 8f.3).  mask=None: DCNv1, differentiable in input, offset, weight and bias.  mask [B, kh*kw, Ho, Wo]:
+    modulated (DCNv2), every sample scaled by its mask value (no range or sigmoid applied), differentiable in the mask
+    as well."""
+    if _lib._pair(dilation) != (1, 1):
+        raise ValueError(f"deform_conv2d_v1: dilation {dilation} is not supported (only 1)")
     kernel_size = (int(weight.shape[2]), int(weight.shape[3]))
-    return deform_conv2d(input, offset, weight, bias, kernel_size, stride, padding, variant=VARIANT_DCNV1)
+    B, _, H, W = (int(v) for v in input.shape)
+    Ho, Wo = _out_hw(H, W, kernel_size, _lib._pair(stride), _lib._pair(padding))
+    N = kernel_size[0] * kernel_size[1]
+    if tuple(offset.shape) != (B, 2 * N, Ho, Wo):
+        raise ValueError(f"deform_conv2d_v1: offset shape {tuple(offset.shape)} != {(B, 2 * N, Ho, Wo)} "
+                         "(one offset group: [B, 2*kh*kw, H_out, W_out])")
+    if mask is None:
+        return deform_conv2d(input, offset, weight, bias, kernel_size, stride, padding, variant=VARIANT_DCNV1)
+    if tuple(mask.shape) != (B, N, Ho, Wo):
+        raise ValueError(f"deform_conv2d_v1: mask shape {tuple(mask.shape)} != {(B, N, Ho, Wo)} "
+                         "([B, kh*kw, H_out, W_out])")
+    return deform_conv2d_modulated(input, offset, mask, weight, bias, kernel_size, stride, padding)
 
 
 # ---- post-op: BatchNorm2d + ReLU (SURVEY 8f.2; train.py:167-170) -------------------------------------

@@ -12,8 +12,8 @@ import torch
 import torch.nn as nn
 
 from . import _lib
-from .functional import (batch_norm_relu, batch_norm_relu_staged, deform_conv2d, deform_layer, deform_layer_framed,
-                         layer_supported, stem_conv, stem_conv_supported)
+from .functional import (batch_norm_relu, batch_norm_relu_staged, deform_conv2d, deform_conv2d_v1, deform_layer,
+                         deform_layer_framed, layer_supported, stem_conv, stem_conv_supported)
 
 
 class TorchDeformConv2d(nn.Module):
@@ -161,3 +161,56 @@ class StemConv2d(nn.Conv2d):
                 and self.padding_mode == "zeros" and stem_conv_supported(x, self.weight)):
             return stem_conv(x, self.weight, self.bias)
         return super().forward(x)
+
+
+class TorchvisionDeformConv2d(nn.Module):
+    """Drop-in for ``torchvision.ops.DeformConv2d``: the same constructor, attributes, parameters (``weight``,
+    ``bias``: state dicts load unchanged), initialisation (``reset_parameters``) and ``forward(input, offset,
+    mask=None)``.  ``mask=None`` is deformable convolution v1, a mask [B, kh*kw, H_out, W_out] makes it the
+    modulated form (DCNv2); both run on the engine (``deform_conv2d_v1``).  One offset group; ``dilation`` and
+    ``groups`` other than 1 are refused at construction."""
+
+    def __init__(self, in_channels, out_channels, kernel_size, stride=1, padding=0, dilation=1, groups=1, bias=True):
+        super().__init__()
+        if in_channels % groups != 0:
+            raise ValueError("in_channels must be divisible by groups")
+        if out_channels % groups != 0:
+            raise ValueError("out_channels must be divisible by groups")
+        if groups != 1:
+            raise ValueError(f"TorchvisionDeformConv2d: groups={groups} is not supported (only 1)")
+        if _lib._pair(dilation) != (1, 1):
+            raise ValueError(f"TorchvisionDeformConv2d: dilation={dilation} is not supported (only 1)")
+        self.in_channels = in_channels
+        self.out_channels = out_channels
+        self.kernel_size = _lib._pair(kernel_size)
+        self.stride = _lib._pair(stride)
+        self.padding = _lib._pair(padding)
+        self.dilation = _lib._pair(dilation)
+        self.groups = groups
+        self.weight = nn.Parameter(torch.empty(out_channels, in_channels // groups, self.kernel_size[0],
+                                               self.kernel_size[1]))
+        if bias:
+            self.bias = nn.Parameter(torch.empty(out_channels))
+        else:
+            self.register_parameter("bias", None)
+        self.reset_parameters()
+
+    def reset_parameters(self):
+        # the same draws, in the same order, as torchvision.ops.DeformConv2d.reset_parameters
+        nn.init.kaiming_uniform_(self.weight, a=math.sqrt(5))
+        if self.bias is not None:
+            fan_in, _ = nn.init._calculate_fan_in_and_fan_out(self.weight)
+            bound = 1 / math.sqrt(fan_in)
+            nn.init.uniform_(self.bias, -bound, bound)
+
+    def forward(self, input, offset, mask=None):
+        return deform_conv2d_v1(input, offset, self.weight, self.bias, stride=self.stride, padding=self.padding,
+                                dilation=self.dilation, mask=mask)
+
+    def extra_repr(self):
+        s = f"{self.in_channels}, {self.out_channels}, kernel_size={self.kernel_size}, stride={self.stride}"
+        s += f", padding={self.padding}" if self.padding != (0, 0) else ""
+        s += f", dilation={self.dilation}" if self.dilation != (1, 1) else ""
+        s += f", groups={self.groups}" if self.groups != 1 else ""
+        s += ", bias=False" if self.bias is None else ""
+        return s
