@@ -128,7 +128,10 @@ enum {
   /* whole layer = companion offset convolution + DCN span (dcn_layer_forward / dcn_layer_backward); dcn_path_name
    * answers "umma" when the layer calls are available for the shape, "unsupported" otherwise (the caller then keeps
    * the offset conv on its framework and uses dcn_forward / dcn_backward) */
-  DCN_PHASE_LAYER_FORWARD = 3, DCN_PHASE_LAYER_BACKWARD = 4
+  DCN_PHASE_LAYER_FORWARD = 3, DCN_PHASE_LAYER_BACKWARD = 4,
+  /* whole MODULATED layer (dcn_*_modulated layer calls below: 3N-channel offset-and-mask conv + DCNv2 span); "umma"
+   * or "unsupported" as for the two phases above */
+  DCN_PHASE_LAYER_FORWARD_MODULATED = 5, DCN_PHASE_LAYER_BACKWARD_MODULATED = 6
 };
 
 /* ---- introspection ---------------------------------------------------------------- */
@@ -215,6 +218,33 @@ DCN_API int dcn_layer_backward(const DcnShape* s, const void* x, const void* off
                        const void* weight, const void* grad_out, void* grad_x, void* grad_offset_weight,
                        void* grad_offset_bias, void* grad_weight, void* grad_bias, void* workspace,
                        size_t workspace_bytes, void* stream);
+
+/* ---- the whole modulated layer (DCNv2): mmcv's ModulatedDeformConv2dPack / mmdet's DCNv2 backbone layers --------
+ * That layer owns a conv_offset with 3N outputs (same kernel / stride / padding, bias): channels [0, 2N) are the
+ * offsets (torchvision's interleaved (dy, dx) per tap, as dcn_forward_modulated reads them), channels [2N, 3N) one
+ * mask logit per tap, and mask = sigmoid(logit).  Here that conv runs on the engine's own convolution kernels, its
+ * epilogue writes `offset` and `mask` directly (no [B, 3N, Ho, Wo] tensor), and the modulated DCN span follows on the
+ * same staged copy of x.  The backward pass packs the conv's output gradient [grad_offset ; grad_mask * m * (1 - m)]
+ * inside the workspace, runs the conv's data gradient into the same channels-last grad_x accumulator as the DCN data
+ * gradient (one transposition at the end) and returns the conv's parameter gradients.
+ * DCN_VARIANT_DCNV1 and fp32 operands only (anything else: DCN_ERR_UNSUPPORTED); shapes: dcn_path_name(s,
+ * DCN_PHASE_LAYER_*_MODULATED) == "umma", workspace: dcn_workspace_bytes with the same phases.  DCN_FLAG_NO_GRAD_X and
+ * DCN_FLAG_XT_STAGED behave as in dcn_layer_*: one buffer of the larger phase size passed to both calls stages x once.
+ *   offset_weight [3N,C,kh,kw]   offset_bias [3N] or NULL
+ *   offset [B,2N,Ho,Wo] = conv channels [0,2N)   mask [B,N,Ho,Wo] = sigmoid(conv channels [2N,3N)) (bias added first)
+ * offset and mask are written by the forward pass and handed back to the backward pass (the saved activations).
+ *   grad_offset_weight [3N,C,kh,kw]   grad_offset_bias [3N] or NULL   grad_x may be NULL with DCN_FLAG_NO_GRAD_X */
+DCN_API int dcn_offset_conv_forward_modulated(const DcnShape* s, const void* x, const void* offset_weight,
+                                              const void* offset_bias, void* offset, void* mask, void* workspace,
+                                              size_t workspace_bytes, void* stream);
+DCN_API int dcn_layer_forward_modulated(const DcnShape* s, const void* x, const void* offset_weight,
+                                        const void* offset_bias, const void* weight, const void* bias, void* offset,
+                                        void* mask, void* out, void* workspace, size_t workspace_bytes, void* stream);
+DCN_API int dcn_layer_backward_modulated(const DcnShape* s, const void* x, const void* offset, const void* mask,
+                                         const void* offset_weight, const void* weight, const void* grad_out,
+                                         void* grad_x, void* grad_offset_weight, void* grad_offset_bias,
+                                         void* grad_weight, void* grad_bias, void* workspace, size_t workspace_bytes,
+                                         void* stream);
 
 /* ---- chained inference: channels-last activations between consecutive engine layers (SURVEY 8f.2) ----------------
  * dcn_layer_forward_chained is dcn_layer_forward whose epilogue writes the output DIRECTLY as the staged input of the

@@ -8,12 +8,13 @@ from ._lib import (DcnError, DcnShape, FLAG_ACCUM_GRAD_X, FLAG_FORCE_SIMT, FLAG_
 from .deform_conv import DeformConv2d
 from .functional import (batch_norm_relu, clear_workspaces, dcn_backward, dcn_backward_modulated, dcn_corners,
                          dcn_forward, dcn_forward_modulated, dcn_layer_backward, dcn_layer_forward,
-                         dcn_offset_conv_forward, deform_conv2d, deform_conv2d_modulated, deform_conv2d_v1,
-                         deform_layer, layer_supported)
+                         dcn_layer_backward_modulated, dcn_layer_forward_modulated, dcn_offset_conv_forward,
+                         dcn_offset_conv_forward_modulated, deform_conv2d, deform_conv2d_modulated, deform_conv2d_v1,
+                         deform_layer, layer_supported, modulated_deform_layer, modulated_layer_supported)
 from .chain import ChainedDeformStages
 from .roi_pool import DeformPSRoIPool, DeformRoIPool
-from .torch_module import (BatchNormReLU2d, StemConv2d, TorchDeformConv2d, TorchDeformConv2dJittorSemantics,
-                           TorchvisionDeformConv2d, fuse_eval_bn_relu)
+from .torch_module import (BatchNormReLU2d, ModulatedDeformConv2dPack, StemConv2d, TorchDeformConv2d,
+                           TorchDeformConv2dJittorSemantics, TorchvisionDeformConv2d, fuse_eval_bn_relu)
 
 __all__ = [
     "DeformConv2d", "TorchDeformConv2d", "BatchNormReLU2d", "batch_norm_relu", "TorchDeformConv2dJittorSemantics", "deform_conv2d",
@@ -22,4 +23,6 @@ __all__ = [
     "FLAG_FORCE_SIMT", "FLAG_NO_GRAD_X", "FLAG_RELU_OUT", "clear_workspaces", "dcn_offset_conv_forward", "dcn_layer_forward", "dcn_layer_backward", "deform_layer",
     "layer_supported", "fuse_eval_bn_relu", "DeformRoIPool", "DeformPSRoIPool", "ChainedDeformStages", "StemConv2d",
     "dcn_forward_modulated", "dcn_backward_modulated", "deform_conv2d_modulated", "TorchvisionDeformConv2d",
+    "dcn_offset_conv_forward_modulated", "dcn_layer_forward_modulated", "dcn_layer_backward_modulated",
+    "modulated_deform_layer", "modulated_layer_supported", "ModulatedDeformConv2dPack",
 ]

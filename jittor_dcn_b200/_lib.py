@@ -23,6 +23,8 @@ FLAG_XT_STAGED = 1 << 4
 FLAG_GRAD_X_FRAMED = 1 << 6   # grad_x = the framed channels-last accumulator itself (training hand-over, SURVEY 8f.2)
 PHASE_FORWARD, PHASE_BACKWARD, PHASE_CORNERS = 0, 1, 2
 PHASE_LAYER_FORWARD, PHASE_LAYER_BACKWARD = 3, 4   # offset conv + DCN span (dcn_layer_*)
+# offset-and-mask conv + modulated DCN span (dcn_layer_*_modulated)
+PHASE_LAYER_FORWARD_MODULATED, PHASE_LAYER_BACKWARD_MODULATED = 5, 6
 ROI_POOL, PSROI_POOL = 0, 1                        # dcn_roi_pool_* kind (deform_conv.py:83 / :160)
 
 # every symbol include/dcn_b200.h declares (tests/test_abi.py checks the two lists agree)
@@ -37,6 +39,7 @@ EXPORTS = (
     "dcn_p2p_allreduce_sum_f32", "dcn_p2p_destroy", "dcn_roi_pool_forward", "dcn_roi_pool_backward",
     "dcn_staged_input_bytes", "dcn_staged_input_clear", "dcn_layer_forward_chained",
     "dcn_bn_relu_forward_staged", "dcn_bn_relu_backward_staged", "dcn_stem_conv_forward", "dcn_stem_conv_backward",
+    "dcn_offset_conv_forward_modulated", "dcn_layer_forward_modulated", "dcn_layer_backward_modulated",
 )
 
 
@@ -86,6 +89,9 @@ def load():
     lib.dcn_offset_conv_forward.argtypes = [shp, vp, vp, vp, vp, vp, sz, vp]
     lib.dcn_layer_forward.argtypes = [shp, vp, vp, vp, vp, vp, vp, vp, vp, sz, vp]
     lib.dcn_layer_backward.argtypes = [shp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, sz, vp]
+    lib.dcn_offset_conv_forward_modulated.argtypes = [shp, vp, vp, vp, vp, vp, vp, sz, vp]
+    lib.dcn_layer_forward_modulated.argtypes = [shp, vp, vp, vp, vp, vp, vp, vp, vp, vp, sz, vp]
+    lib.dcn_layer_backward_modulated.argtypes = [shp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, sz, vp]
     lib.dcn_comm_unique_id.argtypes = [vp]
     lib.dcn_comm_init.argtypes = [ctypes.c_int, ctypes.c_int, vp, ctypes.POINTER(vp)]
     lib.dcn_allreduce_sum_f32.argtypes = [vp, vp, sz, ctypes.c_float, vp]

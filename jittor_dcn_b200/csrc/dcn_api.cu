@@ -169,6 +169,34 @@ static size_t layer_workspace(const Geo& g, int operand, int phase) {
   return umma_layer_bwd_workspace(g);
 }
 
+// whole modulated layer (3N-channel offset-and-mask conv + modulated DCN span): DCNv1, fp32, tensor path only
+static bool modulated_layer_ok(const DcnShape* s, const Geo& g, int phase) {
+  if ((s->flags & DCN_FLAG_FORCE_SIMT) || s->operand != DCN_OPERAND_FP32 || s->variant != DCN_VARIANT_DCNV1) return false;
+  if (!umma_supported(g, DCN_OPERAND_FP32, DCN_PHASE_FORWARD) || !umma_offset_mask_conv_fwd_supported(g)) return false;
+  if (phase == DCN_PHASE_LAYER_FORWARD_MODULATED) return true;
+  return umma_layer_bwd_modulated_supported(g);
+}
+
+static size_t modulated_layer_workspace(const Geo& g, int phase) {
+  if (phase == DCN_PHASE_LAYER_BACKWARD_MODULATED) return umma_layer_bwd_modulated_workspace(g);
+  const size_t f1 = umma_offset_mask_conv_fwd_workspace(g), f2 = umma_workspace_bytes(g, DCN_OPERAND_FP32, DCN_PHASE_FORWARD);
+  return f1 > f2 ? f1 : f2;
+}
+
+// refusal of a modulated layer call: variant, operand, then shape / flags, each with its own message
+static int modulated_layer_refusal(const DcnShape* s, const Geo& g, int phase, const char* what) {
+  if (modulated_layer_ok(s, g, phase)) return DCN_OK;
+  if (s->variant != DCN_VARIANT_DCNV1)
+    set_error("%s: a mask (modulated deformable convolution, DCNv2) exists for DCN_VARIANT_DCNV1 only, not variant %d",
+              what, s->variant);
+  else if (s->operand != DCN_OPERAND_FP32)
+    set_error("%s: fp32 operands only (operand %d)", what, s->operand);
+  else
+    set_error("%s: shape / flags not supported (dcn_path_name(s, DCN_PHASE_LAYER_%s_MODULATED))", what,
+              phase == DCN_PHASE_LAYER_FORWARD_MODULATED ? "FORWARD" : "BACKWARD");
+  return DCN_ERR_UNSUPPORTED;
+}
+
 }  // namespace dcn
 
 using namespace dcn;
@@ -208,6 +236,8 @@ size_t dcn_workspace_bytes(const DcnShape* s, int phase) {
   if (phase == DCN_PHASE_CORNERS) return 0;
   if (phase == DCN_PHASE_LAYER_FORWARD || phase == DCN_PHASE_LAYER_BACKWARD)
     return layer_ok(s, g, phase) ? layer_workspace(g, s->operand, phase) : 0;
+  if (phase == DCN_PHASE_LAYER_FORWARD_MODULATED || phase == DCN_PHASE_LAYER_BACKWARD_MODULATED)
+    return modulated_layer_ok(s, g, phase) ? modulated_layer_workspace(g, phase) : 0;
   if (use_umma(s, g, phase)) return umma_workspace_bytes(g, s->operand, phase);
   if (use_gemm(s, g, phase)) return gemm_path_workspace(g, s->operand, phase);
   return simt_workspace(g, s->operand, phase);
@@ -218,6 +248,8 @@ const char* dcn_path_name(const DcnShape* s, int phase) {
   if (geo_or_error(s, &g)) return "invalid";
   if (phase == DCN_PHASE_LAYER_FORWARD || phase == DCN_PHASE_LAYER_BACKWARD)
     return layer_ok(s, g, phase) ? "umma" : "unsupported";
+  if (phase == DCN_PHASE_LAYER_FORWARD_MODULATED || phase == DCN_PHASE_LAYER_BACKWARD_MODULATED)
+    return modulated_layer_ok(s, g, phase) ? "umma" : "unsupported";
   return use_umma(s, g, phase) ? "umma" : (use_gemm(s, g, phase) ? "gemm" : "simt");
 }
 
@@ -585,6 +617,78 @@ int dcn_layer_backward(const DcnShape* s, const void* x, const void* offset, con
   return umma_layer_backward(g, s->flags, x, (const float*)offset, (const float*)offset_weight, weight, grad_out,
                              (float*)grad_x, (float*)grad_offset_weight, (float*)grad_offset_bias,
                              (float*)grad_weight, (float*)grad_bias, workspace, need, (cudaStream_t)stream);
+}
+
+// ---- whole modulated layer (mmcv's ModulatedDeformConv2dPack) -----------------------------------------------------
+int dcn_offset_conv_forward_modulated(const DcnShape* s, const void* x, const void* offset_weight,
+                                      const void* offset_bias, void* offset, void* mask, void* workspace,
+                                      size_t workspace_bytes, void* stream) {
+  Geo g;
+  int rc = geo_or_error(s, &g);
+  if (rc) return rc;
+  if ((rc = check_ptr(x, "x")) || (rc = check_ptr(offset_weight, "offset_weight")) ||
+      (rc = check_ptr(offset_bias, "offset_bias", false)) || (rc = check_ptr(offset, "offset")) ||
+      (rc = check_ptr(mask, "mask")) || (rc = check_ptr(workspace, "workspace")))
+    return rc;
+  if ((rc = modulated_layer_refusal(s, g, DCN_PHASE_LAYER_FORWARD_MODULATED, "offset-and-mask conv"))) return rc;
+  const size_t need = umma_offset_mask_conv_fwd_workspace(g);
+  if (workspace_bytes < need) {
+    set_error("offset-and-mask conv workspace: have %zu bytes, need %zu", workspace_bytes, need);
+    return DCN_ERR_WORKSPACE;
+  }
+  return umma_offset_conv_forward(g, x, (const float*)offset_weight, (const float*)offset_bias, (float*)offset,
+                                  workspace, (cudaStream_t)stream, !(s->flags & DCN_FLAG_XT_STAGED), (float*)mask);
+}
+
+int dcn_layer_forward_modulated(const DcnShape* s, const void* x, const void* offset_weight, const void* offset_bias,
+                                const void* weight, const void* bias, void* offset, void* mask, void* out,
+                                void* workspace, size_t workspace_bytes, void* stream) {
+  Geo g;
+  int rc = geo_or_error(s, &g);
+  if (rc) return rc;
+  if ((rc = check_ptr(x, "x")) || (rc = check_ptr(offset_weight, "offset_weight")) ||
+      (rc = check_ptr(offset_bias, "offset_bias", false)) || (rc = check_ptr(weight, "weight")) ||
+      (rc = check_ptr(bias, "bias", false)) || (rc = check_ptr(offset, "offset")) || (rc = check_ptr(mask, "mask")) ||
+      (rc = check_ptr(out, "out")) || (rc = check_ptr(workspace, "workspace")))
+    return rc;
+  if ((rc = modulated_layer_refusal(s, g, DCN_PHASE_LAYER_FORWARD_MODULATED, "modulated layer forward"))) return rc;
+  const size_t need = modulated_layer_workspace(g, DCN_PHASE_LAYER_FORWARD_MODULATED);
+  if (workspace_bytes < need) {
+    set_error("modulated layer forward workspace: have %zu bytes, need %zu", workspace_bytes, need);
+    return DCN_ERR_WORKSPACE;
+  }
+  if ((rc = dcn_offset_conv_forward_modulated(s, x, offset_weight, offset_bias, offset, mask, workspace,
+                                              workspace_bytes, stream)))
+    return rc;
+  return umma_forward(g, DCN_OPERAND_FP32, s->flags | DCN_FLAG_XT_STAGED, x, (const float*)offset, weight,
+                      (const float*)bias, out, workspace, (cudaStream_t)stream, (const float*)mask);
+}
+
+int dcn_layer_backward_modulated(const DcnShape* s, const void* x, const void* offset, const void* mask,
+                                 const void* offset_weight, const void* weight, const void* grad_out, void* grad_x,
+                                 void* grad_offset_weight, void* grad_offset_bias, void* grad_weight, void* grad_bias,
+                                 void* workspace, size_t workspace_bytes, void* stream) {
+  Geo g;
+  int rc = geo_or_error(s, &g);
+  if (rc) return rc;
+  const bool want_gx = !(s->flags & DCN_FLAG_NO_GRAD_X);
+  if ((rc = check_ptr(x, "x")) || (rc = check_ptr(offset, "offset")) || (rc = check_ptr(mask, "mask")) ||
+      (rc = check_ptr(offset_weight, "offset_weight")) || (rc = check_ptr(weight, "weight")) ||
+      (rc = check_ptr(grad_out, "grad_out")) || (rc = check_ptr(grad_x, "grad_x", want_gx)) ||
+      (rc = check_ptr(grad_offset_weight, "grad_offset_weight")) ||
+      (rc = check_ptr(grad_offset_bias, "grad_offset_bias", false)) || (rc = check_ptr(grad_weight, "grad_weight")) ||
+      (rc = check_ptr(grad_bias, "grad_bias", false)) || (rc = check_ptr(workspace, "workspace")))
+    return rc;
+  if ((rc = modulated_layer_refusal(s, g, DCN_PHASE_LAYER_BACKWARD_MODULATED, "modulated layer backward"))) return rc;
+  const size_t need = modulated_layer_workspace(g, DCN_PHASE_LAYER_BACKWARD_MODULATED);
+  if (workspace_bytes < need) {
+    set_error("modulated layer backward workspace: have %zu bytes, need %zu", workspace_bytes, need);
+    return DCN_ERR_WORKSPACE;
+  }
+  return umma_layer_backward_modulated(g, s->flags, x, (const float*)offset, (const float*)mask,
+                                       (const float*)offset_weight, weight, grad_out, (float*)grad_x,
+                                       (float*)grad_offset_weight, (float*)grad_offset_bias, (float*)grad_weight,
+                                       (float*)grad_bias, workspace, need, (cudaStream_t)stream);
 }
 
 int dcn_debug_corners(const DcnShape* s, const void* offset, int32_t* y0, int32_t* x0, float* w4,

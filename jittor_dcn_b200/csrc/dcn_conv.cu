@@ -121,8 +121,11 @@ __device__ __forceinline__ int dgrad_acc(const Params& P, int ki, int kj) {
   return P.s == 1 ? 0 : ((ki == 1 ? 2 : 0) + (kj == 1 ? 1 : 0));
 }
 
-template <int MODE>
-__global__ void __launch_bounds__(kThreads, 1) conv_kernel(const __grid_constant__ Params P) {
+// MASK (MODE_FWD only): the modulated layer's 3N-channel conv (mmcv's ModulatedDeformConv2dPack.conv_offset): channels
+// [0, 2N) go to out [B, 2N, Ho, Wo], channels [2N, 3N) to mask [B, N, Ho, Wo] as sigmoid(acc + bias).  The pointer is a
+// trailing argument so that the parameter layout of the unmodulated instantiations does not move.
+template <int MODE, bool MASK = false>
+__global__ void __launch_bounds__(kThreads, 1) conv_kernel(const __grid_constant__ Params P, float* mask = nullptr) {
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
   // carve-up: [stages x (phase images hi|lo, weight tap images)] [WGRAD: 2 grad tiles (2 K blocks x hi|lo x 4 KB)]
@@ -190,7 +193,44 @@ __global__ void __launch_bounds__(kThreads, 1) conv_kernel(const __grid_constant
     // ================================================================ epilogue
     const int m = warp * 32 + lane;
     const int hr = m / P.Wseg, wl = m - hr * P.Wseg;
-    if constexpr (MODE == MODE_FWD) {
+    if constexpr (MODE == MODE_FWD && MASK) {
+      const int n_off = P.O / 3 * 2;   // offset channels; the remaining P.O / 3 are mask logits
+      const size_t plane = (size_t)P.Ho * P.Wo;
+      int acc = 0;
+      uint32_t acc_phase = 0;
+      for (int tile = tile0; tile < P.num_tiles; tile += tile_step) {
+        const TileInfo ti = decode_tile(P, tile);
+        const int r = ti.r0 + hr, c = ti.c0 + wl;
+        const bool valid = r < P.GR && wl < P.Wt && c < P.GC;
+        float* dst = P.out + (size_t)ti.b * n_off * plane + (size_t)r * P.Wo + c;
+        float* mdst = mask + (size_t)ti.b * (P.O - n_off) * plane + (size_t)r * P.Wo + c;
+        mbar_wait_relaxed(&tfull[acc], acc_phase);
+        tc_fence_after();
+        const uint32_t taddr = tmem_base + ((uint32_t)(warp * 32) << 16) + (uint32_t)(acc * 2 * P.Nn);
+        for (int c0 = 0; c0 < P.Nn; c0 += 16) {
+          float v[16], w[16];
+          tmem_ld16(taddr + c0, v);
+          tmem_ld16(taddr + P.Nn + c0, w);   // the hi*lo half
+#pragma unroll
+          for (int i = 0; i < 16; ++i) v[i] += w[i];
+          if (valid) {
+#pragma unroll
+            for (int i = 0; i < 16; ++i) {
+              const int o = c0 + i;
+              if (o >= P.O) break;
+              const float z = v[i] + (P.bias ? __ldg(P.bias + o) : 0.f);
+              if (o < n_off) dst[(size_t)o * plane] = z;
+              else mdst[(size_t)(o - n_off) * plane] = 1.f / (1.f + expf(-z));
+            }
+          }
+        }
+        tc_fence_before();
+        __syncwarp();
+        if (lane == 0) mbar_arrive(&tempty[acc]);
+        acc ^= 1;
+        if (acc == 0) acc_phase ^= 1;
+      }
+    } else if constexpr (MODE == MODE_FWD) {
       int acc = 0;
       uint32_t acc_phase = 0;
       for (int tile = tile0; tile < P.num_tiles; tile += tile_step) {
@@ -709,8 +749,9 @@ static uint32_t conv_pow2_cols(int cols) {
   return c;
 }
 
-// g = the DCN layer (its companion conv: same input, kernel, stride, padding; 2N outputs)
-static bool conv_params(const Geo& g, int mode, cv::Params* Pp) {
+// g = the DCN layer (its companion conv: same input, kernel, stride, padding; O outputs: 2N, or 3N for the modulated
+// layer's offset-and-mask conv)
+static bool conv_params(const Geo& g, int mode, cv::Params* Pp, int O) {
   cv::Params& P = *Pp;
   memset(&P, 0, sizeof(P));
   const int kh = g.N / g.kw;
@@ -722,7 +763,6 @@ static bool conv_params(const Geo& g, int mode, cv::Params* Pp) {
   // into its K blocks, is faster (measured on the detector's 16- and 32-channel layers: backward 6.6 vs 2.8 ms).  Those
   // layers run on the warp-MMA kernels of dcn_conv_small.cu instead (conv_offset_*_supported below).
   if (g.C % 64 != 0) return false;
-  const int O = 2 * g.N;
   if (O > 32) return false;
   // every read stays inside the framed copy
   if ((g.Ho - 1) * g.sh + kh - g.ph > g.H + 2 || (g.Wo - 1) * g.sw + g.kw - g.pw > g.W + 1) return false;
@@ -826,51 +866,52 @@ static size_t conv_smem(const cv::Params& P, int mode) {
 }
 
 // warp-MMA kernels (dcn_conv_small.cu): narrow layers and whatever else the shifted-view kernels refuse
-bool conv_small_supported(const Geo& g);
-size_t conv_small_wfrag_bytes(const Geo& g);
-int conv_small_forward(const Geo& g, const float* xt, const float* woff, const float* boff, float* offset_out,
-                       uint8_t* wfrag, cudaStream_t st);
-int conv_small_backward(const Geo& g, const float* xt, float* gxt, const float* goff, const float* woff, float* gwoff,
-                        uint8_t* wfrag, cudaStream_t st);
+bool conv_small_supported(const Geo& g, int O);
+size_t conv_small_wfrag_bytes(const Geo& g, int O);
+int conv_small_forward(const Geo& g, int O, const float* xt, const float* woff, const float* boff, float* offset_out,
+                       uint8_t* wfrag, cudaStream_t st, float* mask_out);
+int conv_small_backward(const Geo& g, int O, const float* xt, float* gxt, const float* goff, const float* woff,
+                        float* gwoff, uint8_t* wfrag, cudaStream_t st);
 
-static bool conv_fwd_shifted(const Geo& g) {
+static bool conv_fwd_shifted(const Geo& g, int O) {
   cv::Params P;
-  return conv_params(g, cv::MODE_FWD, &P);
+  return conv_params(g, cv::MODE_FWD, &P, O);
 }
-static bool conv_bwd_shifted(const Geo& g) {
+static bool conv_bwd_shifted(const Geo& g, int O) {
   cv::Params P;
-  return conv_params(g, cv::MODE_DGRAD, &P) && conv_params(g, cv::MODE_WGRAD, &P);
+  return conv_params(g, cv::MODE_DGRAD, &P, O) && conv_params(g, cv::MODE_WGRAD, &P, O);
 }
 
-bool conv_offset_fwd_supported(const Geo& g) {
-  return conv_fwd_shifted(g) || conv_small_supported(g);
+// O = the conv's output channels: 2N (offsets) or 3N (offsets and mask logits of the modulated layer)
+bool conv_offset_fwd_supported(const Geo& g, int O) {
+  return conv_fwd_shifted(g, O) || conv_small_supported(g, O);
 }
-bool conv_offset_bwd_supported(const Geo& g) {
+bool conv_offset_bwd_supported(const Geo& g, int O) {
   // measured on the detector's layers (batch 1024): the warp-MMA backward wins below 64 channels (conv2 1.4 vs 1.8 ms,
   // conv3 0.7 vs 0.7 ms); at 64 / 128 channels the plain mode of the fused DCN backward kernel is faster (0.23 vs 0.35 ms)
-  return conv_bwd_shifted(g) || (g.C < 64 && conv_small_supported(g));
+  return conv_bwd_shifted(g, O) || (g.C < 64 && conv_small_supported(g, O));
 }
 
 // bytes of weight tap images one pass needs (the backward passes run one after the other and share the region)
-size_t conv_offset_wtile_bytes(const Geo& g) {
+size_t conv_offset_wtile_bytes(const Geo& g, int O) {
   cv::Params P;
   size_t need = 0;
-  if (conv_params(g, cv::MODE_FWD, &P)) need = (size_t)P.nslab * P.kh * P.kw * 2 * P.w_tile;
-  if (conv_params(g, cv::MODE_DGRAD, &P)) {
+  if (conv_params(g, cv::MODE_FWD, &P, O)) need = (size_t)P.nslab * P.kh * P.kw * 2 * P.w_tile;
+  if (conv_params(g, cv::MODE_DGRAD, &P, O)) {
     const size_t d = (size_t)P.nchunks_n * P.kh * P.kw * 2 * P.w_tile;
     need = d > need ? d : need;
   }
-  const size_t sm = conv_small_wfrag_bytes(g);
+  const size_t sm = conv_small_wfrag_bytes(g, O);
   need = sm > need ? sm : need;
   return align_up(need, 1024);
 }
 
-template <int MODE>
-static int conv_launch(const cv::Params& P, int grid, cudaStream_t st, const char* name) {
+template <int MODE, bool MASK = false>
+static int conv_launch(const cv::Params& P, int grid, cudaStream_t st, const char* name, float* mask = nullptr) {
   const size_t smem = conv_smem(P, MODE);
-  DCN_CUDA_TRY(cudaFuncSetAttribute(cv::conv_kernel<MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  DCN_CUDA_TRY(cudaFuncSetAttribute(cv::conv_kernel<MODE, MASK>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   KernelScope scope(name, st);
-  cv::conv_kernel<MODE><<<grid, cv::kThreads, smem, st>>>(P);
+  cv::conv_kernel<MODE, MASK><<<grid, cv::kThreads, smem, st>>>(P, mask);
   DCN_KERNEL_CHECK(name);
   return DCN_OK;
 }
@@ -884,12 +925,15 @@ static int conv_weight_tiles(const cv::Params& P, int dgrad, const float* w, uin
 }
 
 // offset[B, 2N, Ho, Wo] = conv(x) + bias; xt = the layer's framed channels-last copy of x; wtiles = scratch of
-// conv_offset_wtile_bytes()
+// conv_offset_wtile_bytes().  mask_out != nullptr: the modulated layer's conv, woff / boff have 3N output channels and
+// channels [2N, 3N) are written to mask_out [B, N, Ho, Wo] through the sigmoid (same pass, same kernels).
 int conv_offset_forward(const Geo& g, const float* xt, const float* woff, const float* boff, float* offset_out,
-                        uint8_t* wtiles, cudaStream_t st) {
+                        uint8_t* wtiles, cudaStream_t st, float* mask_out) {
   cv::Params P;
-  if (!conv_fwd_shifted(g) && conv_small_supported(g)) return conv_small_forward(g, xt, woff, boff, offset_out, wtiles, st);
-  if (!conv_params(g, cv::MODE_FWD, &P)) {
+  const int O = (mask_out ? 3 : 2) * g.N;
+  if (!conv_fwd_shifted(g, O) && conv_small_supported(g, O))
+    return conv_small_forward(g, O, xt, woff, boff, offset_out, wtiles, st, mask_out);
+  if (!conv_params(g, cv::MODE_FWD, &P, O)) {
     set_error("offset conv (shifted-view kernel): shape not supported");
     return DCN_ERR_UNSUPPORTED;
   }
@@ -900,19 +944,23 @@ int conv_offset_forward(const Geo& g, const float* xt, const float* woff, const 
   P.out = offset_out;
   P.wtiles = wtiles;
   const int sms = conv_sms();
+  if (mask_out)
+    return conv_launch<cv::MODE_FWD, true>(P, P.num_tiles < sms ? P.num_tiles : sms, st, "conv_offset_mask_fwd_kernel",
+                                           mask_out);
   return conv_launch<cv::MODE_FWD>(P, P.num_tiles < sms ? P.num_tiles : sms, st, "conv_offset_fwd_kernel");
 }
 
-// backward of the offset conv: gxt += dgrad (may be null), gwoff = wgrad (zeroed here).  goff = grad_offset.
-int conv_offset_backward(const Geo& g, const float* xt, float* gxt, const float* goff, const float* woff, float* gwoff,
-                         uint8_t* wtiles, cudaStream_t st) {
+// backward of the offset conv: gxt += dgrad (may be null), gwoff = wgrad (zeroed here).  goff = the gradient of the
+// conv's O output channels [B, O, Ho, Wo] (grad_offset, or the modulated layer's 3N-channel gradient).
+int conv_offset_backward(const Geo& g, int O, const float* xt, float* gxt, const float* goff, const float* woff,
+                         float* gwoff, uint8_t* wtiles, cudaStream_t st) {
   cv::Params P;
   int rc;
-  if (!conv_bwd_shifted(g) && g.C < 64 && conv_small_supported(g))
-    return conv_small_backward(g, xt, gxt, goff, woff, gwoff, wtiles, st);
+  if (!conv_bwd_shifted(g, O) && g.C < 64 && conv_small_supported(g, O))
+    return conv_small_backward(g, O, xt, gxt, goff, woff, gwoff, wtiles, st);
   const int sms = conv_sms();
   if (gxt) {
-    if (!conv_params(g, cv::MODE_DGRAD, &P)) {
+    if (!conv_params(g, cv::MODE_DGRAD, &P, O)) {
       set_error("offset conv backward (shifted-view kernel): shape not supported");
       return DCN_ERR_UNSUPPORTED;
     }
@@ -923,7 +971,7 @@ int conv_offset_backward(const Geo& g, const float* xt, float* gxt, const float*
     if ((rc = conv_launch<cv::MODE_DGRAD>(P, P.num_tiles < sms ? P.num_tiles : sms, st, "conv_offset_dgrad_kernel")))
       return rc;
   }
-  if (!conv_params(g, cv::MODE_WGRAD, &P)) {
+  if (!conv_params(g, cv::MODE_WGRAD, &P, O)) {
     set_error("offset conv weight gradient (shifted-view kernel): shape not supported");
     return DCN_ERR_UNSUPPORTED;
   }

@@ -109,8 +109,10 @@ __global__ void __launch_bounds__(256) wfrag_kernel(Params P, int dgrad, int NT,
 }
 
 // ---- forward --------------------------------------------------------------------------------------------------------
-template <int NT>
-__global__ void __launch_bounds__(kThreads) fwd_kernel(Params P) {
+// MASK: the modulated layer's 3N-channel conv: outputs [0, 2N) go to out [B, 2N, Ho*Wo], outputs [2N, 3N) to
+// mask [B, N, Ho*Wo] as sigmoid(acc + bias); a trailing argument, the unmodulated parameter layout does not move
+template <int NT, bool MASK = false>
+__global__ void __launch_bounds__(kThreads) fwd_kernel(Params P, float* mask = nullptr) {
   const int lane = threadIdx.x & 31, g = lane >> 2, t = lane & 3;
   const int warps = gridDim.x * (kThreads / 32);
   const int units = P.B * P.chunks;
@@ -162,6 +164,31 @@ __global__ void __launch_bounds__(kThreads) fwd_kernel(Params P) {
       }
     }
     // offsets [B, O, Ho*Wo]: thread holds pixels g / g + 8, outputs nt * 8 + 2t (+1)
+    if constexpr (MASK) {
+      const int n_off = P.O / 3 * 2;
+      float* ob = P.out + (size_t)b * n_off * P.HoWo;
+      float* mb = mask + (size_t)b * (P.O - n_off) * P.HoWo;
+#pragma unroll
+      for (int nt = 0; nt < NT; ++nt) {
+#pragma unroll
+        for (int j = 0; j < 2; ++j) {
+          const int o = nt * 8 + 2 * t + j;
+          if (o >= P.O) continue;
+          const float bv = P.bias ? P.bias[o] : 0.f;
+#pragma unroll
+          for (int mt = 0; mt < 2; ++mt)
+#pragma unroll
+            for (int h = 0; h < 2; ++h) {
+              const int q = q0 + mt * 16 + h * 8 + g;
+              if (q >= P.HoWo) continue;
+              const float z = acc[mt][nt][h * 2 + j] + bv;
+              if (o < n_off) ob[(size_t)o * P.HoWo + q] = z;
+              else mb[(size_t)(o - n_off) * P.HoWo + q] = 1.f / (1.f + expf(-z));
+            }
+        }
+      }
+      continue;
+    }
     float* ob = P.out + (size_t)b * P.O * P.HoWo;
 #pragma unroll
     for (int nt = 0; nt < NT; ++nt) {
@@ -383,10 +410,10 @@ __global__ void __launch_bounds__(kWgradThreads) wgrad_kernel(Params P) {
 }  // namespace cs
 
 // ---------------------------------------------------------------------------- host side
-static bool small_params(const Geo& g, cs::Params* Pp) {
+// O = output channels of the conv: 2N (offsets) or 3N (offsets and mask logits of the modulated layer)
+static bool small_params(const Geo& g, cs::Params* Pp, int O) {
   cs::Params& P = *Pp;
   memset(&P, 0, sizeof(P));
-  const int O = 2 * g.N;
   if (g.N != 9 || g.kw != 3 || g.sh != g.sw || g.ph != 1 || g.pw != 1) return false;
   if (g.sh != 1 && g.sh != 2) return false;
   if (g.C % 16 != 0 || g.C > 512 || O > 32) return false;
@@ -416,15 +443,15 @@ static int small_sms() {
   return sms;
 }
 
-bool conv_small_supported(const Geo& g) {
+bool conv_small_supported(const Geo& g, int O) {
   cs::Params P;
-  return small_params(g, &P);
+  return small_params(g, &P, O);
 }
 
 // fragment scratch: the forward and the data-gradient pass run one after the other and share it
-size_t conv_small_wfrag_bytes(const Geo& g) {
+size_t conv_small_wfrag_bytes(const Geo& g, int O) {
   cs::Params P;
-  if (!small_params(g, &P)) return 0;
+  if (!small_params(g, &P, O)) return 0;
   const int NT = (P.O + 7) / 8;
   const size_t f = (size_t)9 * P.KS * NT, d = (size_t)9 * (P.C / 8) * P.KO;
   return align_up((f > d ? f : d) * 64 * sizeof(uint2), 1024);
@@ -438,10 +465,11 @@ static int small_wfrag(const cs::Params& P, int dgrad, int NT, const float* w, u
   return DCN_OK;
 }
 
-int conv_small_forward(const Geo& g, const float* xt, const float* woff, const float* boff, float* offset_out,
-                       uint8_t* wfrag, cudaStream_t st) {
+// mask_out != nullptr: O = 3N, outputs [2N, 3N) go to mask_out through the sigmoid
+int conv_small_forward(const Geo& g, int O, const float* xt, const float* woff, const float* boff, float* offset_out,
+                       uint8_t* wfrag, cudaStream_t st, float* mask_out) {
   cs::Params P;
-  if (!small_params(g, &P)) {
+  if (!small_params(g, &P, O)) {
     set_error("offset conv (warp-MMA kernel): shape not supported");
     return DCN_ERR_UNSUPPORTED;
   }
@@ -456,6 +484,15 @@ int conv_small_forward(const Geo& g, const float* xt, const float* woff, const f
   P.div_chunks = FastDiv::make(P.chunks);
   const long long units = (long long)P.B * P.chunks;
   const int grid = (int)std::min<long long>((units + 7) / 8, (long long)small_sms() * 8);
+  if (mask_out) {
+    KernelScope scope("conv_small_mask_fwd_kernel", st);
+    if (NT == 4) cs::fwd_kernel<4, true><<<grid, cs::kThreads, 0, st>>>(P, mask_out);
+    else if (NT == 3) cs::fwd_kernel<3, true><<<grid, cs::kThreads, 0, st>>>(P, mask_out);
+    else if (NT == 2) cs::fwd_kernel<2, true><<<grid, cs::kThreads, 0, st>>>(P, mask_out);
+    else cs::fwd_kernel<1, true><<<grid, cs::kThreads, 0, st>>>(P, mask_out);
+    DCN_KERNEL_CHECK("conv_small_mask_fwd_kernel");
+    return DCN_OK;
+  }
   KernelScope scope("conv_small_fwd_kernel", st);
   switch (NT) {
     case 1: cs::fwd_kernel<1><<<grid, cs::kThreads, 0, st>>>(P); break;
@@ -468,10 +505,10 @@ int conv_small_forward(const Geo& g, const float* xt, const float* woff, const f
 }
 
 // gxt += data gradient (gxt may be null), gwoff = weight gradient (zeroed here)
-int conv_small_backward(const Geo& g, const float* xt, float* gxt, const float* goff, const float* woff, float* gwoff,
-                        uint8_t* wfrag, cudaStream_t st) {
+int conv_small_backward(const Geo& g, int O, const float* xt, float* gxt, const float* goff, const float* woff,
+                        float* gwoff, uint8_t* wfrag, cudaStream_t st) {
   cs::Params P;
-  if (!small_params(g, &P)) {
+  if (!small_params(g, &P, O)) {
     set_error("offset conv backward (warp-MMA kernel): shape not supported");
     return DCN_ERR_UNSUPPORTED;
   }

@@ -11,6 +11,7 @@
 //                 S re-sampled by the forward's plan / gather warps; nothing is materialised.
 //   grad_bias     column sums of gout (dcn_simt.cu:bias_grad_kernel).
 #include <cstdlib>
+#include <type_traits>
 
 #include "dcn_umma.h"
 #include "dcn_umma_common.cuh"
@@ -42,17 +43,18 @@ bool umma_bwd_supported(const Geo& g, int operand) {
 }
 
 // shifted-view convolution kernels (dcn_conv.cu): preferred when they cover the shape
-bool conv_offset_bwd_supported(const Geo& g);
-size_t conv_offset_wtile_bytes(const Geo& g);
-int conv_offset_backward(const Geo& g, const float* xt, float* gxt, const float* goff, const float* woff, float* gwoff,
-                         uint8_t* wtiles, cudaStream_t st);
+bool conv_offset_bwd_supported(const Geo& g, int O);
+size_t conv_offset_wtile_bytes(const Geo& g, int O);
+int conv_offset_backward(const Geo& g, int O, const float* xt, float* gxt, const float* goff, const float* woff,
+                         float* gwoff, uint8_t* wtiles, cudaStream_t st);
 
 // ---- companion offset convolution (PLAIN problem) inside the layer's backward pass ---------------------------------
-static bool plain_bwd_ok(const Geo& g) {
+// n_out = the conv's output channels (2N; 3N for the modulated layer's offset-and-mask conv)
+static bool plain_bwd_ok(const Geo& g, int n_out = 0) {
   Tiling t;
   if (!make_tiling(g, &t)) return false;
-  if (conv_offset_bwd_supported(g)) return true;
-  const Geo gp = plain_geo(g, t, false);
+  if (conv_offset_bwd_supported(g, n_out ? n_out : 2 * g.N)) return true;
+  const Geo gp = plain_geo(g, t, false, n_out);
   return umma_bwd_data_supported(gp, DCN_OPERAND_FP32) && umma_bwd_data_fuses_wgrad(gp, DCN_OPERAND_FP32);
 }
 
@@ -65,7 +67,48 @@ bool umma_layer_bwd_supported(const Geo& g) {
   return umma_bwd_supported(g0, DCN_OPERAND_FP32) && umma_bwd_data_supported(g0, DCN_OPERAND_FP32) && plain_bwd_ok(g);
 }
 
+// The modulated layer's conv output gradient, per image b: g3[b] = [goff[b] (2N planes) ; gmask[b] * m * (1 - m)
+// (N planes)], m = mask[b] = sigmoid(logit): the derivative of the sigmoid the forward epilogue applied.  Units of 4
+// floats when a plane is a multiple of 4 long (then every segment boundary is too), else single floats.
+template <int V>
+__global__ void __launch_bounds__(256) pack_offset_mask_grad_kernel(size_t per_b, size_t n_off, size_t total,
+                                                                    const float* __restrict__ goff,
+                                                                    const float* __restrict__ gmask,
+                                                                    const float* __restrict__ mask,
+                                                                    float* __restrict__ g3) {
+  using T = typename std::conditional<V == 4, float4, float>::type;
+  for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
+    const size_t b = i / per_b, r = i - b * per_b;
+    T v;
+    if (r < n_off) {
+      v = __ldg(reinterpret_cast<const T*>(goff) + b * n_off + r);
+    } else {
+      const size_t k = b * (per_b - n_off) + (r - n_off);
+      const T gm = __ldg(reinterpret_cast<const T*>(gmask) + k), m = __ldg(reinterpret_cast<const T*>(mask) + k);
+      if constexpr (V == 4)
+        v = make_float4(gm.x * (m.x * (1.f - m.x)), gm.y * (m.y * (1.f - m.y)), gm.z * (m.z * (1.f - m.z)),
+                        gm.w * (m.w * (1.f - m.w)));
+      else
+        v = gm * (m * (1.f - m));
+    }
+    reinterpret_cast<T*>(g3)[i] = v;
+  }
+}
+
+static int launch_pack_offset_mask_grad(const Geo& g, const float* goff, const float* gmask, const float* mask,
+                                        float* g3, cudaStream_t st) {
+  const int v = g.HW % 4 == 0 ? 4 : 1;
+  const size_t per_b = (size_t)3 * g.N * g.HW / v, n_off = (size_t)2 * g.N * g.HW / v, total = per_b * g.B;
+  const int grid = (int)(total / 256 + 1 < 148 * 16 ? total / 256 + 1 : 148 * 16);
+  KernelScope scope("pack_offset_mask_grad_kernel", st);
+  if (v == 4) pack_offset_mask_grad_kernel<4><<<grid, 256, 0, st>>>(per_b, n_off, total, goff, gmask, mask, g3);
+  else pack_offset_mask_grad_kernel<1><<<grid, 256, 0, st>>>(per_b, n_off, total, goff, gmask, mask, g3);
+  DCN_KERNEL_CHECK("pack_offset_mask_grad_kernel");
+  return DCN_OK;
+}
+
 static size_t goff_bytes(const Geo& g) { return align_up(sizeof(float) * (size_t)g.B * 2 * g.N * g.HW, 1024); }
+static size_t planes_bytes(const Geo& g, int ch) { return align_up(sizeof(float) * (size_t)g.B * ch * g.HW, 1024); }
 
 // [xt][rest as umma_bwd_workspace, its tile regions sized for the larger of the two passes][grad_offset]
 size_t umma_layer_bwd_workspace(const Geo& g) {
@@ -77,7 +120,7 @@ size_t umma_layer_bwd_workspace(const Geo& g) {
   const Geo gp = plain_geo(g, t, false);
   const size_t tiles_dcn = umma_bwd_data_wtile_bytes(g0, DCN_OPERAND_FP32) + umma_bwd_data_gtile_bytes(g0, DCN_OPERAND_FP32);
   size_t tiles_pln = umma_bwd_data_wtile_bytes(gp, DCN_OPERAND_FP32) + umma_bwd_data_gtile_bytes(gp, DCN_OPERAND_FP32);
-  if (conv_offset_bwd_supported(g)) tiles_pln = conv_offset_wtile_bytes(g);
+  if (conv_offset_bwd_supported(g, 2 * g.N)) tiles_pln = conv_offset_wtile_bytes(g, 2 * g.N);
   const size_t a = umma_xt_bytes(g, DCN_OPERAND_FP32) + (tiles_dcn > tiles_pln ? tiles_dcn : tiles_pln);
   const size_t c = umma_wgrad_gtile_bytes(g0, DCN_OPERAND_FP32);
   return umma_xt_bytes(g, DCN_OPERAND_FP32) + (a > c ? a : c) + goff_bytes(g);
@@ -103,10 +146,13 @@ size_t umma_bwd_workspace(const Geo& g, int operand) {
 // mask != nullptr: modulated DCNv1 (DCNv2); gmask [B, N, Ho, Wo] is zeroed next to grad_offset and, like it, accumulates
 // over the output-channel groups.  Every branch below passes the mask on: fused data + weight gradient, tensor-path
 // data gradient + unfused weight gradient, generic data gradient + tensor-path weight gradient.
+// woff and g3 != nullptr: the modulated whole layer, whose conv has 3N outputs (offsets, then mask logits).  Its output
+// gradient g3 [B, 3N, Ho, Wo] = [grad_offset ; grad_mask * m * (1 - m)] is packed after the DCN data gradient and
+// drives the conv's backward (shifted-view or warp-MMA kernels).
 int umma_backward_any(const Geo& g, int operand, int flags, const void* xv, const float* off, const void* wtv,
                       const void* goutv, float* gx, float* goff, float* gw, float* gb, void* workspace,
                       cudaStream_t st, const float* woff, float* gwoff, float* gboff, const float* mask,
-                      float* gmask) {
+                      float* gmask, float* g3) {
   int gsize;
   if (!o_groups(g, &gsize)) {
     set_error("umma backward: O = %d cannot be split into groups", g.O);
@@ -153,10 +199,33 @@ int umma_backward_any(const Geo& g, int operand, int flags, const void* xv, cons
                                   gb_rides ? gb + o0 : nullptr, mask, gmask)))
         return rc;
     }
-    if (woff && conv_offset_bwd_supported(g)) {
+    if (woff && g3) {
+      if (!mask || !plain_bwd_ok(g, 3 * g.N)) {
+        set_error("modulated layer backward: the offset-and-mask conv of this shape has no backward kernel");
+        return DCN_ERR_UNSUPPORTED;
+      }
+      const Geo gp = plain_geo(g, t, false, 3 * g.N);
+      uint8_t* wtiles2 = rest + umma_xt_bytes(g, DCN_OPERAND_FP32);
+      if ((rc = launch_pack_offset_mask_grad(g, goff, gmask, mask, g3, st))) return rc;
+      if (conv_offset_bwd_supported(g, 3 * g.N)) {
+        if ((rc = conv_offset_backward(g, 3 * g.N, (const float*)xt, want_gx ? gxt : nullptr, g3, woff, gwoff, wtiles2,
+                                       st)))
+          return rc;
+      } else {
+        // plain mode of the fused data-gradient kernel (stride 2 at 64+ channels: the shifted-view data gradient
+        // would need four parity accumulators of 64 columns, more than TMEM holds double-buffered)
+        uint8_t* gtiles2 = wtiles2 + umma_bwd_data_wtile_bytes(gp, DCN_OPERAND_FP32);
+        DCN_CUDA_TRY(cudaMemsetAsync(gwoff, 0, sizeof(float) * (size_t)gp.O * g.K, st));
+        if ((rc = umma_bwd_data_any(gp, DCN_OPERAND_FP32, xt, want_gx ? gxt : nullptr, nullptr, woff, g3, nullptr,
+                                    gwoff, wtiles2, gtiles2, st)))
+          return rc;
+      }
+      if ((rc = launch_bias_grad(gp, g3, DCN_OPERAND_FP32, gboff, st))) return rc;
+    } else if (woff && conv_offset_bwd_supported(g, 2 * g.N)) {
       const Geo gp = plain_geo(g, t, false);
       uint8_t* wtiles2 = rest + umma_xt_bytes(g, DCN_OPERAND_FP32);
-      if ((rc = conv_offset_backward(g, (const float*)xt, want_gx ? gxt : nullptr, goff, woff, gwoff, wtiles2, st)))
+      if ((rc = conv_offset_backward(g, 2 * g.N, (const float*)xt, want_gx ? gxt : nullptr, goff, woff, gwoff, wtiles2,
+                                     st)))
         return rc;
       if ((rc = launch_bias_grad(gp, goff, DCN_OPERAND_FP32, gboff, st))) return rc;
     } else if (woff) {
@@ -208,7 +277,47 @@ int umma_layer_backward(const Geo& g, int flags, const void* x, const float* off
                         void* workspace, size_t workspace_bytes, cudaStream_t st) {
   float* goff = (float*)((uint8_t*)workspace + workspace_bytes - goff_bytes(g));
   return umma_backward_any(g, DCN_OPERAND_FP32, flags, x, off, wt, gout, gx, goff, gw, gb, workspace, st, woff, gwoff,
-                           gboff, nullptr, nullptr);
+                           gboff, nullptr, nullptr, nullptr);
+}
+
+// ---- whole modulated layer -----------------------------------------------------------------------------------------
+bool umma_layer_bwd_modulated_supported(const Geo& g) {
+  int gsize;
+  if (!o_groups(g, &gsize)) return false;
+  const Geo g0 = o_group_geo(g, 0, gsize);
+  Tiling t;
+  return make_tiling(g, &t) && umma_bwd_supported(g0, DCN_OPERAND_FP32) &&
+         umma_bwd_data_supported(g0, DCN_OPERAND_FP32) && plain_bwd_ok(g, 3 * g.N);
+}
+
+// [xt][rest as umma_layer_bwd_workspace, conv tiles sized for 3N outputs][grad_offset][grad_mask][g3]
+size_t umma_layer_bwd_modulated_workspace(const Geo& g) {
+  int gsize;
+  if (!o_groups(g, &gsize)) return 0;
+  const Geo g0 = o_group_geo(g, 0, gsize);
+  Tiling t;
+  if (!make_tiling(g, &t)) return 0;
+  const Geo gp = plain_geo(g, t, false, 3 * g.N);
+  const size_t tiles_dcn = umma_bwd_data_wtile_bytes(g0, DCN_OPERAND_FP32) + umma_bwd_data_gtile_bytes(g0, DCN_OPERAND_FP32);
+  const size_t tiles_conv = conv_offset_bwd_supported(g, 3 * g.N) ? conv_offset_wtile_bytes(g, 3 * g.N) :
+      umma_bwd_data_wtile_bytes(gp, DCN_OPERAND_FP32) + umma_bwd_data_gtile_bytes(gp, DCN_OPERAND_FP32);
+  const size_t a = umma_xt_bytes(g, DCN_OPERAND_FP32) + (tiles_dcn > tiles_conv ? tiles_dcn : tiles_conv);
+  const size_t c = umma_wgrad_gtile_bytes(g0, DCN_OPERAND_FP32);
+  return umma_xt_bytes(g, DCN_OPERAND_FP32) + (a > c ? a : c) + goff_bytes(g) + planes_bytes(g, g.N) +
+         planes_bytes(g, 3 * g.N);
+}
+
+// grad_offset, grad_mask and the packed 3N-channel conv gradient sit at the tail of the workspace
+int umma_layer_backward_modulated(const Geo& g, int flags, const void* x, const float* off, const float* mask,
+                                  const float* woff, const void* wt, const void* gout, float* gx, float* gwoff,
+                                  float* gboff, float* gw, float* gb, void* workspace, size_t workspace_bytes,
+                                  cudaStream_t st) {
+  uint8_t* tail = (uint8_t*)workspace + workspace_bytes;
+  float* g3 = (float*)(tail - planes_bytes(g, 3 * g.N));
+  float* gmask = (float*)((uint8_t*)g3 - planes_bytes(g, g.N));
+  float* goff = (float*)((uint8_t*)gmask - goff_bytes(g));
+  return umma_backward_any(g, DCN_OPERAND_FP32, flags, x, off, wt, gout, gx, goff, gw, gb, workspace, st, woff, gwoff,
+                           gboff, mask, gmask, g3);
 }
 
 }  // namespace dcn

@@ -154,15 +154,17 @@ __device__ __forceinline__ int plain_base(const Geo& g, int h, int w, int n, boo
 // kernel, stride and padding, 2N output channels, columns ordered (tap, staged channel) like the DCNv1 layout, weight
 // element (o, c, ki, kj) with c un-permuted when the staged copy follows the Torch layout's channel permutation.
 // pad_o: round O up to 16 accumulator columns (forward kernel); the real count stays in o_valid / Oimg.
-__host__ inline Geo plain_geo(const Geo& g, const Tiling& layer_tiling, bool pad_o) {
+// n_out: output channels, 0 = 2N (the modulated layer's offset-and-mask conv has 3N)
+__host__ inline Geo plain_geo(const Geo& g, const Tiling& layer_tiling, bool pad_o, int n_out = 0) {
+  const int O = n_out ? n_out : 2 * g.N;
   Geo p = g;
   p.variant = DCN_VARIANT_DCNV1;
   p.plain = 1;
   p.relu_out = 0;
   p.out_framed = p.out_G = p.out_Cs = 0;
-  p.o_valid = 2 * g.N;
-  p.Oimg = 2 * g.N;
-  p.O = pad_o ? (2 * g.N + 15) / 16 * 16 : 2 * g.N;
+  p.o_valid = O;
+  p.Oimg = O;
+  p.O = pad_o ? (O + 15) / 16 * 16 : O;
   p.perm_G = p.perm_Cs = 0;
   if (g.variant == DCN_VARIANT_TORCH) {
     p.perm_G = layer_tiling.G;

@@ -1180,15 +1180,15 @@ int umma_forward_any(const Geo& g, int operand, const void* x, const float* off,
 // g is the DCN layer; the staged copy of x at the head of the workspace is the layer's (channel-permuted for the
 // Torch layout), so offset conv, dcn_forward and dcn_backward share ONE staging pass.
 // shifted-view convolution kernels (dcn_conv.cu): preferred when they cover the shape
-bool conv_offset_fwd_supported(const Geo& g);
-size_t conv_offset_wtile_bytes(const Geo& g);
+bool conv_offset_fwd_supported(const Geo& g, int O);
+size_t conv_offset_wtile_bytes(const Geo& g, int O);
 int conv_offset_forward(const Geo& g, const float* xt, const float* woff, const float* boff, float* offset_out,
-                        uint8_t* wtiles, cudaStream_t st);
+                        uint8_t* wtiles, cudaStream_t st, float* mask_out);
 
 bool umma_offset_conv_fwd_supported(const Geo& g) {
   Tiling t;
   if (!make_tiling(g, &t)) return false;          // the layer's own staging layout
-  if (conv_offset_fwd_supported(g)) return true;
+  if (conv_offset_fwd_supported(g, 2 * g.N)) return true;
   const Geo gp = plain_geo(g, t, true);
   return umma_fwd_supported(gp, DCN_OPERAND_FP32);
 }
@@ -1197,22 +1197,37 @@ size_t umma_offset_conv_fwd_workspace(const Geo& g) {
   Tiling t;
   if (!make_tiling(g, &t)) return 0;
   const size_t a = umma_fwd_workspace(plain_geo(g, t, true), DCN_OPERAND_FP32);
-  const size_t b = umma_xt_bytes(g, DCN_OPERAND_FP32) + conv_offset_wtile_bytes(g);
+  const size_t b = umma_xt_bytes(g, DCN_OPERAND_FP32) + conv_offset_wtile_bytes(g, 2 * g.N);
   return a > b ? a : b;
 }
 
+// The modulated layer's offset-and-mask conv (3N outputs): shifted-view or warp-MMA kernels only (the plain mode's
+// epilogue has no mask output)
+bool umma_offset_mask_conv_fwd_supported(const Geo& g) {
+  Tiling t;
+  return make_tiling(g, &t) && conv_offset_fwd_supported(g, 3 * g.N);
+}
+
+size_t umma_offset_mask_conv_fwd_workspace(const Geo& g) {
+  return umma_xt_bytes(g, DCN_OPERAND_FP32) + conv_offset_wtile_bytes(g, 3 * g.N);
+}
+
 int umma_offset_conv_forward(const Geo& g, const void* x, const float* woff, const float* boff, float* offset_out,
-                             void* workspace, cudaStream_t st, bool stage_x) {
+                             void* workspace, cudaStream_t st, bool stage_x, float* mask_out) {
   Tiling t;
   if (!make_tiling(g, &t)) {
     set_error("offset conv: layer shape not tileable");
     return DCN_ERR_UNSUPPORTED;
   }
+  if (mask_out && !conv_offset_fwd_supported(g, 3 * g.N)) {
+    set_error("offset-and-mask conv: shape not supported by the shifted-view or warp-MMA kernels");
+    return DCN_ERR_UNSUPPORTED;
+  }
   int rc;
   if (stage_x && (rc = launch_nchw_to_nhwc(g, t, x, workspace, DCN_OPERAND_FP32, st))) return rc;
-  if (conv_offset_fwd_supported(g))
+  if (mask_out || conv_offset_fwd_supported(g, 2 * g.N))
     return conv_offset_forward(g, (const float*)workspace, woff, boff, offset_out,
-                               (uint8_t*)workspace + umma_xt_bytes(g, DCN_OPERAND_FP32), st);
+                               (uint8_t*)workspace + umma_xt_bytes(g, DCN_OPERAND_FP32), st, mask_out);
   const Geo gp = plain_geo(g, t, true);
   return umma_forward_any(gp, DCN_OPERAND_FP32, x, nullptr, woff, boff, offset_out, workspace, st, false, nullptr);
 }

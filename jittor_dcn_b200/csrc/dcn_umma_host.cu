@@ -22,7 +22,7 @@ size_t umma_bwd_workspace(const Geo& g, int operand);
 int umma_backward_any(const Geo& g, int operand, int flags, const void* x, const float* off, const void* wt,
                       const void* gout, float* gx, float* goff, float* gw, float* gb, void* workspace,
                       cudaStream_t st, const float* woff, float* gwoff, float* gboff, const float* mask,
-                      float* gmask);
+                      float* gmask, float* g3);
 
 bool o_groups(const Geo& g, int* size) {
   if (g.O <= 256) {
@@ -81,7 +81,7 @@ int umma_backward(const Geo& g, int operand, int flags, const void* x, const flo
                   const void* gout, float* gx, float* goff, float* gw, float* gb, void* workspace,
                   cudaStream_t st, const float* mask, float* gmask) {
   return umma_backward_any(g, operand, flags, x, off, wt, gout, gx, goff, gw, gb, workspace, st, nullptr, nullptr,
-                           nullptr, mask, gmask);
+                           nullptr, mask, gmask, nullptr);
 }
 
 }  // namespace dcn

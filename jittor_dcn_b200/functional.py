@@ -9,8 +9,8 @@ import torch
 
 from . import _lib
 from ._lib import (FLAG_ACCUM_GRAD_X, FLAG_FORCE_SIMT, FLAG_NO_GRAD_X, FLAG_RELU_OUT, FLAG_XT_STAGED, OPERAND_BF16, OPERAND_FP32,
-                   PHASE_BACKWARD, PHASE_FORWARD, PHASE_LAYER_BACKWARD, PHASE_LAYER_FORWARD, VARIANT_DCNV1,
-                   VARIANT_JITTOR, VARIANT_TORCH)
+                   PHASE_BACKWARD, PHASE_FORWARD, PHASE_LAYER_BACKWARD, PHASE_LAYER_BACKWARD_MODULATED,
+                   PHASE_LAYER_FORWARD, PHASE_LAYER_FORWARD_MODULATED, VARIANT_DCNV1, VARIANT_JITTOR, VARIANT_TORCH)
 
 _workspaces = {}
 _captured = []   # scratch buffers whose addresses are baked into CUDA graphs: alive until clear_workspaces()
@@ -386,6 +386,156 @@ def deform_layer(x, offset_weight, offset_bias, weight, bias=None, kernel_size=3
     """Differentiable whole layer on the engine (CUDA float32 tensors; check layer_supported() first)."""
     cfg = (_lib._pair(kernel_size), _lib._pair(stride), _lib._pair(padding), variant, flags, bool(keep_staged))
     return DeformLayerFunction.apply(x, offset_weight, offset_bias, weight, bias, cfg)
+
+
+# ---- whole modulated layer: mmcv's ModulatedDeformConv2dPack (3N-channel offset-and-mask conv + DCNv2 span) --------
+_MOD_PHASES = (PHASE_LAYER_FORWARD_MODULATED, PHASE_LAYER_BACKWARD_MODULATED)
+
+
+def modulated_layer_supported(x_shape, out_channels, kernel_size, stride, padding, flags=0):
+    """True when dcn_layer_forward_modulated / dcn_layer_backward_modulated cover the shape (fp32, tensor path)."""
+    B, C, H, W = (int(v) for v in x_shape)
+    shp = _lib.make_shape(B, C, int(out_channels), H, W, kernel_size, stride, padding, VARIANT_DCNV1, OPERAND_FP32,
+                          flags)
+    return all(_lib.path_name(shp, ph) == "umma" for ph in _MOD_PHASES)
+
+
+def modulated_layer_workspace(x, weight, kernel_size, stride, padding, flags=0):
+    """One scratch buffer for both modulated layer calls: the backward pass reuses the staged copy of x."""
+    lib = _lib.load()
+    shp = _shape_of(x, weight, kernel_size, stride, padding, VARIANT_DCNV1, OPERAND_FP32, flags)
+    need = max(lib.dcn_workspace_bytes(ctypes.byref(shp), ph) for ph in _MOD_PHASES)
+    return torch.empty(need, dtype=torch.uint8, device=x.device)
+
+
+def _check_offset_mask_weight(offset_weight, shp):
+    N = shp.kh * shp.kw
+    if tuple(offset_weight.shape) != (3 * N, shp.C, shp.kh, shp.kw):
+        raise ValueError(f"offset_weight shape {tuple(offset_weight.shape)} != {(3 * N, shp.C, shp.kh, shp.kw)} "
+                         "(3N outputs: offsets, then one mask logit per tap)")
+
+
+def dcn_offset_conv_forward_modulated(x, offset_weight, offset_bias, out_channels, kernel_size=3, stride=1, padding=1,
+                                      flags=0, ws=None, xt_staged=False):
+    """-> (offset [B,2N,Ho,Wo], mask [B,N,Ho,Wo]): the modulated layer's 3N-channel conv on the engine, channels
+    [0, 2N) as offsets and sigmoid(channels [2N, 3N)) as the mask (no autograd)."""
+    lib = _lib.load()
+    B, C, H, W = x.shape
+    if xt_staged and ws is not None:
+        flags |= FLAG_XT_STAGED
+    shp = _lib.make_shape(B, C, int(out_channels), H, W, kernel_size, stride, padding, VARIANT_DCNV1, OPERAND_FP32,
+                          flags)
+    Ho, Wo = _lib.output_hw(shp)
+    N = shp.kh * shp.kw
+    _check_offset_mask_weight(offset_weight, shp)
+    x, offset_weight, offset_bias = _dev_ready(x), _dev_ready(offset_weight), _dev_ready(offset_bias)
+    offset = torch.empty((B, 2 * N, Ho, Wo), dtype=torch.float32, device=x.device)
+    mask = torch.empty((B, N, Ho, Wo), dtype=torch.float32, device=x.device)
+    with torch.cuda.device(x.device):
+        stream = torch.cuda.current_stream(x.device)
+        need = lib.dcn_workspace_bytes(ctypes.byref(shp), PHASE_LAYER_FORWARD_MODULATED)
+        if ws is None:
+            ws = _workspace(x.device, stream.cuda_stream, need)
+        rc = lib.dcn_offset_conv_forward_modulated(ctypes.byref(shp), _ptr(x), _ptr(offset_weight), _ptr(offset_bias),
+                                                   _ptr(offset), _ptr(mask), _ptr(ws), ws.numel(),
+                                                   ctypes.c_void_p(stream.cuda_stream))
+    _lib.check(rc, "dcn_offset_conv_forward_modulated")
+    return offset, mask
+
+
+def dcn_layer_forward_modulated(x, offset_weight, offset_bias, weight, bias, kernel_size=3, stride=1, padding=1,
+                                flags=0, ws=None):
+    """-> (offset, mask, out): offset-and-mask conv + modulated DCN forward, x staged once (no autograd)."""
+    lib = _lib.load()
+    shp = _shape_of(x, weight, kernel_size, stride, padding, VARIANT_DCNV1, OPERAND_FP32, flags)
+    Ho, Wo = _lib.output_hw(shp)
+    N = shp.kh * shp.kw
+    _check_offset_mask_weight(offset_weight, shp)
+    x, weight, bias = _dev_ready(x), _dev_ready(weight), _dev_ready(bias)
+    offset_weight, offset_bias = _dev_ready(offset_weight), _dev_ready(offset_bias)
+    offset = torch.empty((shp.B, 2 * N, Ho, Wo), dtype=torch.float32, device=x.device)
+    mask = torch.empty((shp.B, N, Ho, Wo), dtype=torch.float32, device=x.device)
+    out = torch.empty((shp.B, shp.O, Ho, Wo), dtype=torch.float32, device=x.device)
+    with torch.cuda.device(x.device):
+        stream = torch.cuda.current_stream(x.device)
+        need = lib.dcn_workspace_bytes(ctypes.byref(shp), PHASE_LAYER_FORWARD_MODULATED)
+        if ws is None:
+            ws = _workspace(x.device, stream.cuda_stream, need)
+        rc = lib.dcn_layer_forward_modulated(ctypes.byref(shp), _ptr(x), _ptr(offset_weight), _ptr(offset_bias),
+                                             _ptr(weight), _ptr(bias), _ptr(offset), _ptr(mask), _ptr(out), _ptr(ws),
+                                             ws.numel(), ctypes.c_void_p(stream.cuda_stream))
+    _lib.check(rc, "dcn_layer_forward_modulated")
+    return offset, mask, out
+
+
+def dcn_layer_backward_modulated(x, offset, mask, offset_weight, weight, grad_out, has_offset_bias=True, has_bias=True,
+                                 kernel_size=3, stride=1, padding=1, flags=0, need_grad_x=True, ws=None,
+                                 xt_staged=False):
+    """-> grad_x (or None), grad_offset_weight, grad_offset_bias (or None), grad_weight, grad_bias (or None).
+    offset / mask: what dcn_layer_forward_modulated returned.  The gradients of offset and mask stay in the workspace."""
+    lib = _lib.load()
+    if not need_grad_x:
+        flags |= FLAG_NO_GRAD_X
+    if xt_staged and ws is not None:
+        flags |= FLAG_XT_STAGED
+    shp = _shape_of(x, weight, kernel_size, stride, padding, VARIANT_DCNV1, OPERAND_FP32, flags)
+    _check_offset_mask_weight(offset_weight, shp)
+    x, weight, grad_out = _dev_ready(x), _dev_ready(weight), _dev_ready(grad_out)
+    offset, mask, offset_weight = _dev_ready(offset), _dev_ready(mask), _dev_ready(offset_weight)
+    dev = x.device
+    gx = torch.empty(x.shape, dtype=torch.float32, device=dev) if need_grad_x else None
+    gwoff = torch.empty(offset_weight.shape, dtype=torch.float32, device=dev)
+    gboff = torch.empty((offset_weight.shape[0],), dtype=torch.float32, device=dev) if has_offset_bias else None
+    gw = torch.empty(weight.shape, dtype=torch.float32, device=dev)
+    gb = torch.empty((shp.O,), dtype=torch.float32, device=dev) if has_bias else None
+    with torch.cuda.device(dev):
+        stream = torch.cuda.current_stream(dev)
+        need = lib.dcn_workspace_bytes(ctypes.byref(shp), PHASE_LAYER_BACKWARD_MODULATED)
+        if ws is None:
+            ws = _workspace(dev, stream.cuda_stream, need)
+        rc = lib.dcn_layer_backward_modulated(ctypes.byref(shp), _ptr(x), _ptr(offset), _ptr(mask), _ptr(offset_weight),
+                                              _ptr(weight), _ptr(grad_out), _ptr(gx), _ptr(gwoff), _ptr(gboff), _ptr(gw),
+                                              _ptr(gb), _ptr(ws), ws.numel(), ctypes.c_void_p(stream.cuda_stream))
+    _lib.check(rc, "dcn_layer_backward_modulated")
+    return gx, gwoff, gboff, gw, gb
+
+
+class ModulatedDeformLayerFunction(torch.autograd.Function):
+    """mmcv's ModulatedDeformConv2dPack.forward (conv_offset, chunk / cat, sigmoid, modulated_deform_conv2d) and its
+    autograd as ONE node on the engine: x is staged once per step, neither the [B, 3N, Ho, Wo] conv output nor the
+    gradients of offset and mask reach HBM as framework tensors, and both grad_x terms are summed before the single
+    transposition back to NCHW."""
+
+    @staticmethod
+    def forward(ctx, x, offset_weight, offset_bias, weight, bias, cfg):
+        kernel_size, stride, padding, flags, keep_staged = cfg
+        ctx.ws = modulated_layer_workspace(x, weight, kernel_size, stride, padding, flags) if keep_staged else None
+        offset, mask, out = dcn_layer_forward_modulated(x, offset_weight, offset_bias, weight, bias, kernel_size, stride,
+                                                        padding, flags, ws=ctx.ws)
+        ctx.save_for_backward(x, offset, mask, offset_weight, weight)
+        ctx.cfg = cfg
+        ctx.has = (offset_bias is not None, bias is not None)
+        return out
+
+    @staticmethod
+    def backward(ctx, grad_out):
+        x, offset, mask, offset_weight, weight = ctx.saved_tensors
+        kernel_size, stride, padding, flags, _ = ctx.cfg
+        gx, gwoff, gboff, gw, gb = dcn_layer_backward_modulated(
+            x, offset, mask, offset_weight, weight, grad_out, ctx.has[0], ctx.has[1], kernel_size, stride, padding,
+            flags & ~(FLAG_ACCUM_GRAD_X | FLAG_RELU_OUT), need_grad_x=ctx.needs_input_grad[0], ws=ctx.ws,
+            xt_staged=ctx.ws is not None)
+        ctx.ws = None
+        return gx, gwoff, gboff, gw, gb, None
+
+
+def modulated_deform_layer(x, offset_weight, offset_bias, weight, bias=None, kernel_size=3, stride=1, padding=1,
+                           flags=0, keep_staged=False):
+    """Differentiable whole modulated layer on the engine (CUDA float32 tensors; check modulated_layer_supported()
+    first).  offset_weight [3N, C, kh, kw]: offsets, then one mask logit per tap (mmcv's conv_offset)."""
+    cfg = (_lib._pair(kernel_size), _lib._pair(stride), _lib._pair(padding), flags & ~FLAG_RELU_OUT,
+           bool(keep_staged))
+    return ModulatedDeformLayerFunction.apply(x, offset_weight, offset_bias, weight, bias, cfg)
 
 
 def dcn_corners(offset, in_hw, kernel_size=3, stride=1, padding=1, variant=VARIANT_TORCH):

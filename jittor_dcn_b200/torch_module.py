@@ -13,7 +13,8 @@ import torch.nn as nn
 
 from . import _lib
 from .functional import (batch_norm_relu, batch_norm_relu_staged, deform_conv2d, deform_conv2d_v1, deform_layer,
-                         deform_layer_framed, layer_supported, stem_conv, stem_conv_supported)
+                         deform_layer_framed, layer_supported, modulated_deform_layer, modulated_layer_supported,
+                         stem_conv, stem_conv_supported)
 
 
 class TorchDeformConv2d(nn.Module):
@@ -212,5 +213,94 @@ class TorchvisionDeformConv2d(nn.Module):
         s += f", padding={self.padding}" if self.padding != (0, 0) else ""
         s += f", dilation={self.dilation}" if self.dilation != (1, 1) else ""
         s += f", groups={self.groups}" if self.groups != 1 else ""
+        s += ", bias=False" if self.bias is None else ""
+        return s
+
+
+class ModulatedDeformConv2dPack(nn.Module):
+    """Drop-in for mmcv's ``ModulatedDeformConv2dPack`` (the ``DCNv2`` layer of mmdet's ResNet backbones): the same
+    constructor, parameters (``weight``, ``bias``, ``conv_offset.weight``, ``conv_offset.bias``: mmcv checkpoints load
+    unchanged) and initialisation (mmcv's ``init_weights``).  ``conv_offset`` has 3N = 3 * kh * kw outputs; channels
+    [0, 2N) are the offsets and channels [2N, 3N) one mask logit per tap, mask = sigmoid(logit).
+
+    ``forward`` runs the whole layer (that conv, the sigmoid and the modulated span) as ONE autograd node on the
+    engine when the input is a float32 CUDA tensor and ``modulated_layer_supported`` covers the shape; otherwise, or
+    with ``engine_offset_conv = False``, it computes mmcv's composition: ``conv_offset`` as a framework convolution,
+    chunk / cat / sigmoid, and ``deform_conv2d_v1(..., mask=)`` as the span.  One offset group; ``dilation``,
+    ``groups`` and ``deform_groups`` other than 1 are refused at construction."""
+
+    def __init__(self, in_channels, out_channels, kernel_size, stride=1, padding=0, dilation=1, groups=1,
+                 deform_groups=1, bias=True):
+        super().__init__()
+        if _lib._pair(dilation) != (1, 1):
+            raise ValueError(f"ModulatedDeformConv2dPack: dilation={dilation} is not supported (only 1)")
+        if groups != 1:
+            raise ValueError(f"ModulatedDeformConv2dPack: groups={groups} is not supported (only 1)")
+        if deform_groups != 1:
+            raise ValueError(f"ModulatedDeformConv2dPack: deform_groups={deform_groups} is not supported (only 1)")
+        self.in_channels = in_channels
+        self.out_channels = out_channels
+        self.kernel_size = _lib._pair(kernel_size)
+        self.stride = _lib._pair(stride)
+        self.padding = _lib._pair(padding)
+        self.dilation = _lib._pair(dilation)
+        self.groups = groups
+        self.deform_groups = deform_groups
+        self.engine_flags = 0
+        # True (default): the whole layer is one autograd node on the engine when the shape allows it; False: the
+        # framework convolution + chunk / cat / sigmoid + the engine's modulated span, as mmcv composes it
+        self.engine_offset_conv = True
+        # True: a private scratch buffer lives from forward to backward so that the backward pass reuses the staged
+        # channels-last copy of x (one pass over x saved, device memory held in between)
+        self.keep_staged_input = False
+        self.weight = nn.Parameter(torch.empty(out_channels, in_channels // groups, *self.kernel_size))
+        if bias:
+            self.bias = nn.Parameter(torch.empty(out_channels))
+        else:
+            self.register_parameter("bias", None)
+        # the same draws, in the same order, as mmcv: init_weights() in the base constructor, the framework's default
+        # initialisation of conv_offset, then init_weights() again (which also zeroes conv_offset)
+        self._init_main()
+        self.conv_offset = nn.Conv2d(in_channels, deform_groups * 3 * self.kernel_size[0] * self.kernel_size[1],
+                                     kernel_size=self.kernel_size, stride=self.stride, padding=self.padding,
+                                     dilation=self.dilation, bias=True)
+        self.init_weights()
+
+    def _init_main(self):
+        n = self.in_channels * self.kernel_size[0] * self.kernel_size[1]
+        stdv = 1.0 / math.sqrt(n)
+        with torch.no_grad():
+            self.weight.uniform_(-stdv, stdv)
+            if self.bias is not None:
+                self.bias.zero_()
+
+    def init_weights(self):
+        self._init_main()
+        with torch.no_grad():
+            self.conv_offset.weight.zero_()
+            self.conv_offset.bias.zero_()
+
+    def _whole_layer_on_engine(self, x):
+        return (self.engine_offset_conv and x.is_cuda and x.dtype == torch.float32 and x.dim() == 4
+                and self.weight.is_cuda and self.weight.dtype == torch.float32
+                and self.conv_offset.weight.dtype == torch.float32
+                and modulated_layer_supported(x.shape, self.out_channels, self.kernel_size, self.stride, self.padding,
+                                              self.engine_flags))
+
+    def forward(self, x):
+        if self._whole_layer_on_engine(x):
+            return modulated_deform_layer(x, self.conv_offset.weight, self.conv_offset.bias, self.weight, self.bias,
+                                          self.kernel_size, self.stride, self.padding, self.engine_flags,
+                                          keep_staged=self.keep_staged_input and torch.is_grad_enabled())
+        out = self.conv_offset(x)
+        o1, o2, mask = torch.chunk(out, 3, dim=1)
+        offset = torch.cat((o1, o2), dim=1)
+        mask = torch.sigmoid(mask)
+        return deform_conv2d_v1(x, offset, self.weight, self.bias, stride=self.stride, padding=self.padding,
+                                dilation=self.dilation, mask=mask)
+
+    def extra_repr(self):
+        s = f"{self.in_channels}, {self.out_channels}, kernel_size={self.kernel_size}, stride={self.stride}"
+        s += f", padding={self.padding}" if self.padding != (0, 0) else ""
         s += ", bias=False" if self.bias is None else ""
         return s
