@@ -12,6 +12,9 @@
  *                                       train.py:249 (loss.backward) / train.py:414
  *                                       (optimizer.backward)
  *
+ * Beside it: multi-scale deformable attention (Deformable DETR's MSDeformAttn core), dcn_msda_forward /
+ * dcn_msda_backward below.
+ *
  * The companion offset convolution (deform_conv.py:16-21,58 / train.py:80-85,98) stays a
  * framework convolution: its output is the `offset` argument here and `grad_offset` is
  * handed back to it.
@@ -304,6 +307,34 @@ DCN_API int dcn_roi_pool_forward(int kind, int B, int C, int H, int W, int R, co
 DCN_API int dcn_roi_pool_backward(int kind, int B, int C, int H, int W, int R, const void* features, const void* rois,
                                   const void* offsets, float spatial_scale, float trans_std, int no_trans,
                                   const void* grad_out, void* grad_features, void* grad_offsets, void* stream);
+
+/* ---- multi-scale deformable attention (Deformable DETR's MSDeformAttn core; mmcv's MultiScaleDeformableAttnFunction) ----
+ *   out[b, q, m*D + d] = sum_{l,p} a[b,q,m,l,p] * bilinear(value_l[b, :, :, m, d], x*W_l - 0.5, y*H_l - 0.5)
+ * with (x, y) = sampling_locations[b,q,m,l,p] normalised to [0, 1] (any value allowed) and corners outside level l
+ * reading 0: F.grid_sample(bilinear, zeros, align_corners=False) on 2*loc - 1.  Tokens of `value` are level-major,
+ * row-major inside a level (S = sum_l H_l*W_l).  The softmax of the weights happens outside; any value is allowed.
+ *   value [B,S,M,D] f32   spatial_shapes [L,2] int64 = (H_l, W_l)   level_start_index [L] int64
+ *   sampling_locations [B,Q,M,L,P,2] f32   attention_weights [B,Q,M,L,P] f32   out [B,Q,M*D] f32
+ * spatial_shapes and level_start_index are DEVICE pointers and are read by the kernels only (no host synchronisation:
+ * the calls can be captured in a CUDA graph); a level that does not fit [0, S) reads as empty and no corner outside
+ * [0, S) is ever addressed.  Every pointer is 16-byte aligned.  No workspace.
+ * Limits (anything else: DCN_ERR_UNSUPPORTED, or DCN_ERR_BAD_SHAPE for non-positive extents and index spaces):
+ *   D in {16, 32, 64, 128, 256};  1 <= L <= 16;  1 <= P <= 32;  B*Q*M <= 2^31 - 1;  flags == 0.
+ * Backward: grad_value [B,S,M,D] is zeroed and accumulated with atomics (its summation order is not deterministic);
+ * grad_sampling_locations and grad_attention_weights are each written by one plain store per element, bit-identical
+ * across runs.  Each of the three may be NULL (not computed); spatial_shapes / level_start_index get no gradient. */
+typedef struct DcnMsdaShape {
+  int32_t B, S, Q, M, D, L, P; /* batch, value tokens, queries, heads, channels per head, levels, points */
+  int32_t flags;               /* must be 0 (reserved) */
+} DcnMsdaShape;
+
+DCN_API int dcn_msda_forward(const DcnMsdaShape* s, const void* value, const int64_t* spatial_shapes,
+                             const int64_t* level_start_index, const void* sampling_locations,
+                             const void* attention_weights, void* out, void* stream);
+DCN_API int dcn_msda_backward(const DcnMsdaShape* s, const void* value, const int64_t* spatial_shapes,
+                              const int64_t* level_start_index, const void* sampling_locations,
+                              const void* attention_weights, const void* grad_out, void* grad_value,
+                              void* grad_sampling_locations, void* grad_attention_weights, void* stream);
 
 /* ---- producer of the first DCN layer's input (train.py:145,166 / 307,328: conv1 = Conv2d(1, 16, 3, 1, 1)) ------------
  * A 3 x 3, stride 1, padding 1 convolution with Cin <= 4 input channels and O in {16, 32} outputs, float32 NCHW,

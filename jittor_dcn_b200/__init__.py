@@ -3,14 +3,16 @@
 Only what the hot path needs: the C-ABI library (csrc/ -> libdcn_b200.so), its ctypes
 binding and the two module classes that mirror the reference's operator interface.
 """
-from ._lib import (DcnError, DcnShape, FLAG_ACCUM_GRAD_X, FLAG_FORCE_SIMT, FLAG_NO_GRAD_X, FLAG_RELU_OUT,
+from ._lib import (DcnError, DcnMsdaShape, DcnShape, FLAG_ACCUM_GRAD_X, FLAG_FORCE_SIMT, FLAG_NO_GRAD_X, FLAG_RELU_OUT,
                    OPERAND_BF16, OPERAND_FP32, VARIANT_DCNV1, VARIANT_JITTOR, VARIANT_TORCH, load, make_shape)
 from .deform_conv import DeformConv2d
 from .functional import (batch_norm_relu, clear_workspaces, dcn_backward, dcn_backward_modulated, dcn_corners,
                          dcn_forward, dcn_forward_modulated, dcn_layer_backward, dcn_layer_forward,
                          dcn_layer_backward_modulated, dcn_layer_forward_modulated, dcn_offset_conv_forward,
                          dcn_offset_conv_forward_modulated, deform_conv2d, deform_conv2d_modulated, deform_conv2d_v1,
-                         deform_layer, layer_supported, modulated_deform_layer, modulated_layer_supported)
+                         deform_layer, layer_supported, modulated_deform_layer, modulated_layer_supported,
+                         MSDeformAttnFunction, dcn_msda_backward, dcn_msda_forward, ms_deform_attn)
+from .msda import MSDeformAttn
 from .chain import ChainedDeformStages
 from .roi_pool import DeformPSRoIPool, DeformRoIPool
 from .torch_module import (BatchNormReLU2d, ModulatedDeformConv2dPack, StemConv2d, TorchDeformConv2d,
@@ -25,4 +27,5 @@ __all__ = [
     "dcn_forward_modulated", "dcn_backward_modulated", "deform_conv2d_modulated", "TorchvisionDeformConv2d",
     "dcn_offset_conv_forward_modulated", "dcn_layer_forward_modulated", "dcn_layer_backward_modulated",
     "modulated_deform_layer", "modulated_layer_supported", "ModulatedDeformConv2dPack",
+    "DcnMsdaShape", "dcn_msda_forward", "dcn_msda_backward", "MSDeformAttnFunction", "ms_deform_attn", "MSDeformAttn",
 ]

@@ -40,6 +40,7 @@ EXPORTS = (
     "dcn_staged_input_bytes", "dcn_staged_input_clear", "dcn_layer_forward_chained",
     "dcn_bn_relu_forward_staged", "dcn_bn_relu_backward_staged", "dcn_stem_conv_forward", "dcn_stem_conv_backward",
     "dcn_offset_conv_forward_modulated", "dcn_layer_forward_modulated", "dcn_layer_backward_modulated",
+    "dcn_msda_forward", "dcn_msda_backward",
 )
 
 
@@ -48,6 +49,11 @@ class DcnShape(ctypes.Structure):
     _fields_ = [(n, ctypes.c_int32) for n in
                 ("B", "C", "O", "H", "W", "kh", "kw", "sh", "sw", "ph", "pw",
                  "variant", "operand", "flags")]
+
+
+class DcnMsdaShape(ctypes.Structure):
+    """Mirror of include/dcn_b200.h:DcnMsdaShape (multi-scale deformable attention)."""
+    _fields_ = [(n, ctypes.c_int32) for n in ("B", "S", "Q", "M", "D", "L", "P", "flags")]
 
 
 class DcnError(RuntimeError):
@@ -92,6 +98,9 @@ def load():
     lib.dcn_offset_conv_forward_modulated.argtypes = [shp, vp, vp, vp, vp, vp, vp, sz, vp]
     lib.dcn_layer_forward_modulated.argtypes = [shp, vp, vp, vp, vp, vp, vp, vp, vp, vp, sz, vp]
     lib.dcn_layer_backward_modulated.argtypes = [shp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, sz, vp]
+    msp = ctypes.POINTER(DcnMsdaShape)
+    lib.dcn_msda_forward.argtypes = [msp, vp, vp, vp, vp, vp, vp, vp]
+    lib.dcn_msda_backward.argtypes = [msp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp]
     lib.dcn_comm_unique_id.argtypes = [vp]
     lib.dcn_comm_init.argtypes = [ctypes.c_int, ctypes.c_int, vp, ctypes.POINTER(vp)]
     lib.dcn_allreduce_sum_f32.argtypes = [vp, vp, sz, ctypes.c_float, vp]

@@ -197,6 +197,45 @@ static int modulated_layer_refusal(const DcnShape* s, const Geo& g, int phase, c
   return DCN_ERR_UNSUPPORTED;
 }
 
+// multi-scale deformable attention (dcn_msda.cu)
+int msda_forward(const DcnMsdaShape& s, const float* value, const int64_t* shapes, const int64_t* starts,
+                 const float* loc, const float* attn, float* out, cudaStream_t st);
+int msda_backward(const DcnMsdaShape& s, const float* value, const int64_t* shapes, const int64_t* starts,
+                  const float* loc, const float* attn, const float* gout, float* gvalue, float* gloc, float* gattn,
+                  cudaStream_t st);
+
+static int msda_shape_ok(const DcnMsdaShape* s, const char* what) {
+  if (!s) {
+    set_error("%s: DcnMsdaShape is NULL", what);
+    return DCN_ERR_NULL_POINTER;
+  }
+  if (s->B <= 0 || s->S <= 0 || s->Q <= 0 || s->M <= 0 || s->D <= 0 || s->L <= 0 || s->P <= 0) {
+    set_error("%s: bad shape B=%d S=%d Q=%d M=%d D=%d L=%d P=%d", what, s->B, s->S, s->Q, s->M, s->D, s->L, s->P);
+    return DCN_ERR_BAD_SHAPE;
+  }
+  if ((long long)s->B * s->Q * s->M > 0x7fffffffLL) {
+    set_error("%s: B*Q*M = %lld exceeds the limit 2^31 - 1", what, (long long)s->B * s->Q * s->M);
+    return DCN_ERR_BAD_SHAPE;
+  }
+  if (s->flags != 0) {
+    set_error("%s: flags must be 0 (reserved), got %d", what, s->flags);
+    return DCN_ERR_UNSUPPORTED;
+  }
+  if (s->D != 16 && s->D != 32 && s->D != 64 && s->D != 128 && s->D != 256) {
+    set_error("%s: D = %d channels per head is not supported (D in {16, 32, 64, 128, 256})", what, s->D);
+    return DCN_ERR_UNSUPPORTED;
+  }
+  if (s->L > 16) {
+    set_error("%s: L = %d levels exceeds the limit L <= 16", what, s->L);
+    return DCN_ERR_UNSUPPORTED;
+  }
+  if (s->P > 32) {
+    set_error("%s: P = %d points exceeds the limit P <= 32", what, s->P);
+    return DCN_ERR_UNSUPPORTED;
+  }
+  return DCN_OK;
+}
+
 }  // namespace dcn
 
 using namespace dcn;
@@ -700,6 +739,37 @@ int dcn_debug_corners(const DcnShape* s, const void* offset, int32_t* y0, int32_
       (rc = check_ptr(x0, "x0")) || (rc = check_ptr(w4, "w4")))
     return rc;
   return launch_corners(g, (const float*)offset, y0, x0, w4, (cudaStream_t)stream);
+}
+
+int dcn_msda_forward(const DcnMsdaShape* s, const void* value, const int64_t* spatial_shapes,
+                     const int64_t* level_start_index, const void* sampling_locations, const void* attention_weights,
+                     void* out, void* stream) {
+  int rc;
+  if ((rc = msda_shape_ok(s, "dcn_msda_forward")) || (rc = check_ptr(value, "value")) ||
+      (rc = check_ptr(spatial_shapes, "spatial_shapes")) || (rc = check_ptr(level_start_index, "level_start_index")) ||
+      (rc = check_ptr(sampling_locations, "sampling_locations")) ||
+      (rc = check_ptr(attention_weights, "attention_weights")) || (rc = check_ptr(out, "out")))
+    return rc;
+  return msda_forward(*s, (const float*)value, spatial_shapes, level_start_index, (const float*)sampling_locations,
+                      (const float*)attention_weights, (float*)out, (cudaStream_t)stream);
+}
+
+int dcn_msda_backward(const DcnMsdaShape* s, const void* value, const int64_t* spatial_shapes,
+                      const int64_t* level_start_index, const void* sampling_locations, const void* attention_weights,
+                      const void* grad_out, void* grad_value, void* grad_sampling_locations,
+                      void* grad_attention_weights, void* stream) {
+  int rc;
+  if ((rc = msda_shape_ok(s, "dcn_msda_backward")) || (rc = check_ptr(value, "value")) ||
+      (rc = check_ptr(spatial_shapes, "spatial_shapes")) || (rc = check_ptr(level_start_index, "level_start_index")) ||
+      (rc = check_ptr(sampling_locations, "sampling_locations")) ||
+      (rc = check_ptr(attention_weights, "attention_weights")) || (rc = check_ptr(grad_out, "grad_out")) ||
+      (rc = check_ptr(grad_value, "grad_value", false)) ||
+      (rc = check_ptr(grad_sampling_locations, "grad_sampling_locations", false)) ||
+      (rc = check_ptr(grad_attention_weights, "grad_attention_weights", false)))
+    return rc;
+  return msda_backward(*s, (const float*)value, spatial_shapes, level_start_index, (const float*)sampling_locations,
+                       (const float*)attention_weights, (const float*)grad_out, (float*)grad_value,
+                       (float*)grad_sampling_locations, (float*)grad_attention_weights, (cudaStream_t)stream);
 }
 
 size_t dcn_bn_workspace_bytes(int32_t C) { return C > 0 ? bn_workspace_bytes(C) : 0; }

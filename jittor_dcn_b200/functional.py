@@ -953,3 +953,119 @@ def deform_layer_framed(xt, in_chw, offset_weight, offset_bias, weight, bias=Non
     """Whole layer on a staged input (see batch_norm_relu_staged); in_chw = (C, H, W) of the layer's logical input."""
     cfg = (tuple(int(v) for v in in_chw), _lib._pair(kernel_size), _lib._pair(stride), _lib._pair(padding), variant, flags)
     return DeformLayerFramedFunction.apply(xt, offset_weight, offset_bias, weight, bias, cfg)
+
+
+# ---- multi-scale deformable attention (Deformable DETR's MSDeformAttn core; csrc/dcn_msda.cu) --------------------
+def _msda_inputs(value, spatial_shapes, level_start_index, sampling_locations, attention_weights):
+    """Checks shapes, dtypes and devices from tensor metadata only (no host synchronisation, so the call can be
+    captured in a CUDA graph) -> (DcnMsdaShape, dense 16-byte aligned device tensors)."""
+    floats = (("value", value), ("sampling_locations", sampling_locations), ("attention_weights", attention_weights))
+    for name, t in floats:
+        if not isinstance(t, torch.Tensor) or t.dtype != torch.float32:
+            raise ValueError(f"ms_deform_attn: {name} must be a float32 tensor, got "
+                             f"{getattr(t, 'dtype', type(t).__name__)} (the kernels are float32 only)")
+    for name, t in floats:
+        if not t.is_cuda:
+            raise ValueError(f"ms_deform_attn: {name} must be a CUDA tensor: there is no CPU path")
+    dev = value.device
+    for name, t in (("sampling_locations", sampling_locations), ("attention_weights", attention_weights)):
+        if t.device != dev:
+            raise ValueError(f"ms_deform_attn: {name} is on {t.device}, value on {dev}")
+    for name, t in (("spatial_shapes", spatial_shapes), ("level_start_index", level_start_index)):
+        if not isinstance(t, torch.Tensor) or t.is_floating_point() or t.is_complex() or t.dtype == torch.bool:
+            raise ValueError(f"ms_deform_attn: {name} must be an integer tensor, got "
+                             f"{getattr(t, 'dtype', type(t).__name__)}")
+    if value.dim() != 4:
+        raise ValueError(f"ms_deform_attn: value must be [B, S, M, D], got shape {tuple(value.shape)}")
+    B, S, M, D = (int(v) for v in value.shape)
+    if spatial_shapes.dim() != 2 or spatial_shapes.shape[1] != 2:
+        raise ValueError(f"ms_deform_attn: spatial_shapes must be [L, 2], got shape {tuple(spatial_shapes.shape)}")
+    L = int(spatial_shapes.shape[0])
+    if tuple(level_start_index.shape) != (L,):
+        raise ValueError(f"ms_deform_attn: level_start_index shape {tuple(level_start_index.shape)} != {(L,)}")
+    if sampling_locations.dim() != 6:
+        raise ValueError("ms_deform_attn: sampling_locations must be [B, Q, M, L, P, 2], got shape "
+                         f"{tuple(sampling_locations.shape)}")
+    Q, P = int(sampling_locations.shape[1]), int(sampling_locations.shape[4])
+    if tuple(sampling_locations.shape) != (B, Q, M, L, P, 2):
+        raise ValueError(f"ms_deform_attn: sampling_locations shape {tuple(sampling_locations.shape)} != "
+                         f"{(B, Q, M, L, P, 2)} (value [B, S, M, D] = {(B, S, M, D)}, spatial_shapes [L, 2])")
+    if tuple(attention_weights.shape) != (B, Q, M, L, P):
+        raise ValueError(f"ms_deform_attn: attention_weights shape {tuple(attention_weights.shape)} != "
+                         f"{(B, Q, M, L, P)}")
+    if max(B, S, Q, M, D, L, P) > 0x7fffffff:
+        raise ValueError(f"ms_deform_attn: an extent of {(B, S, Q, M, D, L, P)} exceeds 2^31 - 1")
+    shp = _lib.DcnMsdaShape(B, S, Q, M, D, L, P, 0)
+    idx = tuple(_dev_ready(_to_device(t, dev), torch.int64) for t in (spatial_shapes, level_start_index))
+    return (shp, _dev_ready(value)) + idx + (_dev_ready(sampling_locations), _dev_ready(attention_weights))
+
+
+def dcn_msda_forward(value, spatial_shapes, level_start_index, sampling_locations, attention_weights):
+    """out [B, Q, M*D] of multi-scale deformable attention on CUDA tensors (no autograd)."""
+    lib = _lib.load()
+    shp, v, ss, ls, loc, aw = _msda_inputs(value, spatial_shapes, level_start_index, sampling_locations,
+                                           attention_weights)
+    out = torch.empty((shp.B, shp.Q, shp.M * shp.D), dtype=torch.float32, device=v.device)
+    with torch.cuda.device(v.device):
+        stream = torch.cuda.current_stream(v.device)
+        rc = lib.dcn_msda_forward(ctypes.byref(shp), _ptr(v), _ptr(ss), _ptr(ls), _ptr(loc), _ptr(aw), _ptr(out),
+                                  ctypes.c_void_p(stream.cuda_stream))
+    _lib.check(rc, "dcn_msda_forward")
+    return out
+
+
+def dcn_msda_backward(value, spatial_shapes, level_start_index, sampling_locations, attention_weights, grad_out,
+                      need=(True, True, True)):
+    """(grad_value, grad_sampling_locations, grad_attention_weights); need[i] False -> None, not computed."""
+    lib = _lib.load()
+    shp, v, ss, ls, loc, aw = _msda_inputs(value, spatial_shapes, level_start_index, sampling_locations,
+                                           attention_weights)
+    if tuple(grad_out.shape) != (shp.B, shp.Q, shp.M * shp.D):
+        raise ValueError(f"ms_deform_attn: grad_out shape {tuple(grad_out.shape)} != {(shp.B, shp.Q, shp.M * shp.D)}")
+    go = _dev_ready(_to_device(grad_out, v.device))
+    gv, gl, ga = (torch.empty_like(t) if n else None for t, n in zip((v, loc, aw), need))
+    if gv is None and gl is None and ga is None:
+        return None, None, None
+    with torch.cuda.device(v.device):
+        stream = torch.cuda.current_stream(v.device)
+        rc = lib.dcn_msda_backward(ctypes.byref(shp), _ptr(v), _ptr(ss), _ptr(ls), _ptr(loc), _ptr(aw), _ptr(go),
+                                   _ptr(gv), _ptr(gl), _ptr(ga), ctypes.c_void_p(stream.cuda_stream))
+    _lib.check(rc, "dcn_msda_backward")
+    return gv, gl, ga
+
+
+class MSDeformAttnFunction(torch.autograd.Function):
+    """Multi-scale deformable attention core as one autograd node, with the positional interface of Deformable DETR's
+    ``MSDeformAttnFunction`` and mmcv's ``MultiScaleDeformableAttnFunction``:
+
+        MSDeformAttnFunction.apply(value, value_spatial_shapes, value_level_start_index,
+                                   sampling_locations, attention_weights, im2col_step) -> [B, Q, M*D]
+
+    value [B, S, M, D] f32, spatial_shapes [L, 2] and level_start_index [L] integer tensors (kept on the device: the
+    node never synchronises with the host and can be captured in a CUDA graph), sampling_locations [B, Q, M, L, P, 2]
+    and attention_weights [B, Q, M, L, P] f32, all on one CUDA device.  ``im2col_step`` is accepted and ignored: it
+    exists only so that calls written for those implementations run unchanged.  Differentiable in value,
+    sampling_locations and attention_weights; only the gradients autograd asks for are computed."""
+
+    @staticmethod
+    def forward(ctx, value, value_spatial_shapes, value_level_start_index, sampling_locations, attention_weights,
+                im2col_step=64):
+        out = dcn_msda_forward(value, value_spatial_shapes, value_level_start_index, sampling_locations,
+                               attention_weights)
+        ctx.save_for_backward(value, value_spatial_shapes, value_level_start_index, sampling_locations,
+                              attention_weights)
+        return out
+
+    @staticmethod
+    @torch.autograd.function.once_differentiable
+    def backward(ctx, grad_output):
+        need = (ctx.needs_input_grad[0], ctx.needs_input_grad[3], ctx.needs_input_grad[4])
+        gv, gl, ga = dcn_msda_backward(*ctx.saved_tensors, grad_output, need=need)
+        return gv, None, None, gl, ga, None
+
+
+def ms_deform_attn(value, spatial_shapes, level_start_index, sampling_locations, attention_weights):
+    """Differentiable multi-scale deformable attention core (see MSDeformAttnFunction):
+    out[b, q, m*D + d] = sum_{l,p} a[b,q,m,l,p] * bilinear(value_l[b, :, :, m, d], x*W_l - 0.5, y*H_l - 0.5)."""
+    return MSDeformAttnFunction.apply(value, spatial_shapes, level_start_index, sampling_locations, attention_weights,
+                                      64)
