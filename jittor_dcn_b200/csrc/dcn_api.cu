@@ -141,14 +141,6 @@ static bool use_gemm(const DcnShape* s, const Geo& g, int phase) {
   return !umma_supported(g, s->operand, phase) && gemm_path_supported(g, s->operand);
 }
 
-// whole-layer calls (offset conv + DCN span): fp32 operands on the tensor path only
-static bool layer_ok(const DcnShape* s, const Geo& g, int phase) {
-  if ((s->flags & DCN_FLAG_FORCE_SIMT) || s->operand != DCN_OPERAND_FP32) return false;
-  if (!umma_supported(g, DCN_OPERAND_FP32, DCN_PHASE_FORWARD) || !umma_offset_conv_fwd_supported(g)) return false;
-  if (phase == DCN_PHASE_LAYER_FORWARD) return true;
-  return umma_layer_bwd_supported(g);
-}
-
 // mask: the modulated calls (dcn_forward_modulated / dcn_backward_modulated): DCNv1 only, float32 [B, N, Ho, Wo]
 static int check_modulated(const DcnShape* s, const void* mask, const char* mname, const void* gmask = nullptr,
                            bool backward = false) {
@@ -162,39 +154,54 @@ static int check_modulated(const DcnShape* s, const void* mask, const char* mnam
   return DCN_OK;
 }
 
-static size_t layer_workspace(const Geo& g, int operand, int phase) {
-  const size_t f1 = umma_offset_conv_fwd_workspace(g), f2 = umma_workspace_bytes(g, operand, DCN_PHASE_FORWARD);
-  const size_t f = f1 > f2 ? f1 : f2;
-  if (phase == DCN_PHASE_LAYER_FORWARD) return f;
-  return umma_layer_bwd_workspace(g);
+// ---- whole-layer calls (offset conv + DCN span), phases DCN_PHASE_LAYER_*: fp32 operands on the tensor path only.
+// The modulated layer (phases *_MODULATED; mmcv's ModulatedDeformConv2dPack) is DCNv1 only and its conv has 3N
+// outputs (offsets, then one mask logit per tap) instead of 2N.
+static bool is_layer_phase(int phase) {
+  return phase >= DCN_PHASE_LAYER_FORWARD && phase <= DCN_PHASE_LAYER_BACKWARD_MODULATED;
+}
+static bool modulated_phase(int phase) {
+  return phase == DCN_PHASE_LAYER_FORWARD_MODULATED || phase == DCN_PHASE_LAYER_BACKWARD_MODULATED;
+}
+static bool backward_phase(int phase) {
+  return phase == DCN_PHASE_LAYER_BACKWARD || phase == DCN_PHASE_LAYER_BACKWARD_MODULATED;
+}
+static int conv_outputs(const Geo& g, int phase) { return (modulated_phase(phase) ? 3 : 2) * g.N; }
+
+static bool layer_ok(const DcnShape* s, const Geo& g, int phase) {
+  if ((s->flags & DCN_FLAG_FORCE_SIMT) || s->operand != DCN_OPERAND_FP32) return false;
+  if (modulated_phase(phase) && s->variant != DCN_VARIANT_DCNV1) return false;
+  const int n_out = conv_outputs(g, phase);
+  if (!umma_supported(g, DCN_OPERAND_FP32, DCN_PHASE_FORWARD) || !umma_offset_conv_fwd_supported(g, n_out)) return false;
+  return !backward_phase(phase) || umma_layer_bwd_supported(g, n_out);
 }
 
-// whole modulated layer (3N-channel offset-and-mask conv + modulated DCN span): DCNv1, fp32, tensor path only
-static bool modulated_layer_ok(const DcnShape* s, const Geo& g, int phase) {
-  if ((s->flags & DCN_FLAG_FORCE_SIMT) || s->operand != DCN_OPERAND_FP32 || s->variant != DCN_VARIANT_DCNV1) return false;
-  if (!umma_supported(g, DCN_OPERAND_FP32, DCN_PHASE_FORWARD) || !umma_offset_mask_conv_fwd_supported(g)) return false;
-  if (phase == DCN_PHASE_LAYER_FORWARD_MODULATED) return true;
-  return umma_layer_bwd_modulated_supported(g);
-}
-
-static size_t modulated_layer_workspace(const Geo& g, int phase) {
-  if (phase == DCN_PHASE_LAYER_BACKWARD_MODULATED) return umma_layer_bwd_modulated_workspace(g);
-  const size_t f1 = umma_offset_mask_conv_fwd_workspace(g), f2 = umma_workspace_bytes(g, DCN_OPERAND_FP32, DCN_PHASE_FORWARD);
+static size_t layer_workspace(const Geo& g, int phase) {
+  const int n_out = conv_outputs(g, phase);
+  if (backward_phase(phase)) return umma_layer_bwd_workspace(g, n_out);
+  const size_t f1 = umma_offset_conv_fwd_workspace(g, n_out), f2 = umma_workspace_bytes(g, DCN_OPERAND_FP32, DCN_PHASE_FORWARD);
   return f1 > f2 ? f1 : f2;
 }
 
-// refusal of a modulated layer call: variant, operand, then shape / flags, each with its own message
-static int modulated_layer_refusal(const DcnShape* s, const Geo& g, int phase, const char* what) {
-  if (modulated_layer_ok(s, g, phase)) return DCN_OK;
-  if (s->variant != DCN_VARIANT_DCNV1)
+// the refusal of a whole-layer call `what` that layer_ok turns down, with its reason: variant, operand, shape / flags
+static int layer_refusal(const DcnShape* s, const Geo& g, int phase, const char* what) {
+  if (layer_ok(s, g, phase)) return DCN_OK;
+  static const char* const names[] = {"DCN_PHASE_LAYER_FORWARD", "DCN_PHASE_LAYER_BACKWARD",
+                                      "DCN_PHASE_LAYER_FORWARD_MODULATED", "DCN_PHASE_LAYER_BACKWARD_MODULATED"};
+  if (modulated_phase(phase) && s->variant != DCN_VARIANT_DCNV1)
     set_error("%s: a mask (modulated deformable convolution, DCNv2) exists for DCN_VARIANT_DCNV1 only, not variant %d",
               what, s->variant);
   else if (s->operand != DCN_OPERAND_FP32)
     set_error("%s: fp32 operands only (operand %d)", what, s->operand);
   else
-    set_error("%s: shape / flags not supported (dcn_path_name(s, DCN_PHASE_LAYER_%s_MODULATED))", what,
-              phase == DCN_PHASE_LAYER_FORWARD_MODULATED ? "FORWARD" : "BACKWARD");
+    set_error("%s: shape / flags not supported (dcn_path_name(s, %s))", what, names[phase - DCN_PHASE_LAYER_FORWARD]);
   return DCN_ERR_UNSUPPORTED;
+}
+
+static int check_workspace(size_t have, size_t need, const char* what) {
+  if (have >= need) return DCN_OK;
+  set_error("%s workspace: have %zu bytes, need %zu", what, have, need);
+  return DCN_ERR_WORKSPACE;
 }
 
 // multi-scale deformable attention (dcn_msda.cu)
@@ -273,10 +280,7 @@ size_t dcn_workspace_bytes(const DcnShape* s, int phase) {
   Geo g;
   if (geo_or_error(s, &g)) return 0;
   if (phase == DCN_PHASE_CORNERS) return 0;
-  if (phase == DCN_PHASE_LAYER_FORWARD || phase == DCN_PHASE_LAYER_BACKWARD)
-    return layer_ok(s, g, phase) ? layer_workspace(g, s->operand, phase) : 0;
-  if (phase == DCN_PHASE_LAYER_FORWARD_MODULATED || phase == DCN_PHASE_LAYER_BACKWARD_MODULATED)
-    return modulated_layer_ok(s, g, phase) ? modulated_layer_workspace(g, phase) : 0;
+  if (is_layer_phase(phase)) return layer_ok(s, g, phase) ? layer_workspace(g, phase) : 0;
   if (use_umma(s, g, phase)) return umma_workspace_bytes(g, s->operand, phase);
   if (use_gemm(s, g, phase)) return gemm_path_workspace(g, s->operand, phase);
   return simt_workspace(g, s->operand, phase);
@@ -285,10 +289,7 @@ size_t dcn_workspace_bytes(const DcnShape* s, int phase) {
 const char* dcn_path_name(const DcnShape* s, int phase) {
   Geo g;
   if (geo_or_error(s, &g)) return "invalid";
-  if (phase == DCN_PHASE_LAYER_FORWARD || phase == DCN_PHASE_LAYER_BACKWARD)
-    return layer_ok(s, g, phase) ? "umma" : "unsupported";
-  if (phase == DCN_PHASE_LAYER_FORWARD_MODULATED || phase == DCN_PHASE_LAYER_BACKWARD_MODULATED)
-    return modulated_layer_ok(s, g, phase) ? "umma" : "unsupported";
+  if (is_layer_phase(phase)) return layer_ok(s, g, phase) ? "umma" : "unsupported";
   return use_umma(s, g, phase) ? "umma" : (use_gemm(s, g, phase) ? "gemm" : "simt");
 }
 
@@ -358,10 +359,7 @@ static int forward_impl(const DcnShape* s, const void* x, const void* offset, co
     return rc;
   const size_t need = dcn_workspace_bytes(s, DCN_PHASE_FORWARD);
   if (need && (rc = check_ptr(workspace, "workspace"))) return rc;
-  if (workspace_bytes < need) {
-    set_error("forward workspace: have %zu bytes, need %zu", workspace_bytes, need);
-    return DCN_ERR_WORKSPACE;
-  }
+  if ((rc = check_workspace(workspace_bytes, need, "forward"))) return rc;
   cudaStream_t st = (cudaStream_t)stream;
   if (use_umma(s, g, DCN_PHASE_FORWARD))
     return umma_forward(g, s->operand, s->flags, x, (const float*)offset, weight, (const float*)bias,
@@ -399,10 +397,7 @@ static int backward_impl(const DcnShape* s, const void* x, const void* offset, c
     return rc;
   const size_t need = dcn_workspace_bytes(s, DCN_PHASE_BACKWARD);
   if (need && (rc = check_ptr(workspace, "workspace"))) return rc;
-  if (workspace_bytes < need) {
-    set_error("backward workspace: have %zu bytes, need %zu", workspace_bytes, need);
-    return DCN_ERR_WORKSPACE;
-  }
+  if ((rc = check_workspace(workspace_bytes, need, "backward"))) return rc;
   cudaStream_t st = (cudaStream_t)stream;
   if (use_umma(s, g, DCN_PHASE_BACKWARD))
     return umma_backward(g, s->operand, s->flags, x, (const float*)offset, weight, grad_out,
@@ -427,6 +422,99 @@ static int backward_impl(const DcnShape* s, const void* x, const void* offset, c
   return simt_backward(g, s->flags, (const float*)x, plan, (const float*)weight,
                        (const float*)grad_out, (float*)grad_x, (float*)grad_offset,
                        (float*)grad_weight, (float*)grad_bias, st, SIMT_BWD_ALL, mask, grad_mask);
+}
+
+// ---- whole-layer calls: phase DCN_PHASE_LAYER_FORWARD / _BACKWARD, or the *_MODULATED one with a mask; every call
+// checks shape, pointers, support, workspace, in that order, then launches
+
+// dcn_offset_conv_forward and dcn_offset_conv_forward_modulated
+static int offset_conv_impl(const DcnShape* s, int phase, const char* what, const void* x, const void* offset_weight,
+                            const void* offset_bias, void* offset, void* mask, void* workspace, size_t workspace_bytes,
+                            void* stream) {
+  Geo g;
+  int rc;
+  if ((rc = geo_or_error(s, &g)) || (rc = check_ptr(x, "x")) || (rc = check_ptr(offset_weight, "offset_weight")) ||
+      (rc = check_ptr(offset_bias, "offset_bias", false)) || (rc = check_ptr(offset, "offset")) ||
+      (rc = check_ptr(mask, "mask", modulated_phase(phase))) || (rc = check_ptr(workspace, "workspace")) ||
+      (rc = layer_refusal(s, g, phase, what)) ||
+      (rc = check_workspace(workspace_bytes, umma_offset_conv_fwd_workspace(g, conv_outputs(g, phase)), what)))
+    return rc;
+  return umma_offset_conv_forward(g, x, (const float*)offset_weight, (const float*)offset_bias, (float*)offset,
+                                  workspace, (cudaStream_t)stream, !(s->flags & DCN_FLAG_XT_STAGED), (float*)mask);
+}
+
+// chained inference (SURVEY 8f.2): the producer's epilogue writes the consumer's staged input.
+// Geo of the producer with out_framed set from the consumer's staging layout, or an error.
+static int chained_geo(const DcnShape* s, const DcnShape* consumer, Geo* g) {
+  int rc = geo_or_error(s, g);
+  if (rc) return rc;
+  Geo gc;
+  if ((rc = geo_or_error(consumer, &gc))) return rc;
+  if (s->operand != DCN_OPERAND_FP32 || consumer->operand != DCN_OPERAND_FP32 || g->O > 256 ||
+      gc.B != g->B || gc.C != g->O || gc.H != g->Ho || gc.W != g->Wo) {
+    set_error("chained forward: consumer must take this layer's output (B=%d C=%d H=%d W=%d, fp32, O <= 256); got "
+              "B=%d C=%d H=%d W=%d", g->B, g->O, g->Ho, g->Wo, gc.B, gc.C, gc.H, gc.W);
+    return DCN_ERR_BAD_SHAPE;
+  }
+  if (!use_umma(s, *g, DCN_PHASE_FORWARD) || !use_umma(consumer, gc, DCN_PHASE_FORWARD)) {
+    set_error("chained forward: both layers must run on the tensor path (dcn_path_name == \"umma\")");
+    return DCN_ERR_UNSUPPORTED;
+  }
+  Tiling tc;
+  if (!make_tiling(gc, &tc)) return DCN_ERR_UNSUPPORTED;
+  g->out_framed = 1;
+  g->out_G = gc.variant == DCN_VARIANT_TORCH ? tc.G : 0;
+  g->out_Cs = gc.variant == DCN_VARIANT_TORCH ? tc.Cs : 0;
+  return DCN_OK;
+}
+
+// dcn_layer_forward, dcn_layer_forward_chained (consumer != nullptr: out is the consumer's workspace) and
+// dcn_layer_forward_modulated.  The offset conv and the span share one staging pass of x.
+static int layer_forward_impl(const DcnShape* s, const DcnShape* consumer, int phase, const char* what, const void* x,
+                              const void* offset_weight, const void* offset_bias, const void* weight, const void* bias,
+                              void* offset, void* mask, void* out, void* workspace, size_t workspace_bytes,
+                              void* stream) {
+  Geo g;
+  int rc;
+  if ((rc = consumer ? chained_geo(s, consumer, &g) : geo_or_error(s, &g)) || (rc = check_ptr(x, "x")) ||
+      (rc = check_ptr(offset_weight, "offset_weight")) || (rc = check_ptr(offset_bias, "offset_bias", false)) ||
+      (rc = check_ptr(weight, "weight")) || (rc = check_ptr(bias, "bias", false)) ||
+      (rc = check_ptr(offset, "offset")) || (rc = check_ptr(mask, "mask", modulated_phase(phase))) ||
+      (rc = check_ptr(out, consumer ? "consumer_workspace" : "out")) || (rc = check_ptr(workspace, "workspace")) ||
+      (rc = layer_refusal(s, g, phase, what)) ||
+      (rc = check_workspace(workspace_bytes, layer_workspace(g, phase), what)))
+    return rc;
+  // (out_framed of a chained Geo only concerns the span's epilogue: the offset conv ignores it)
+  cudaStream_t st = (cudaStream_t)stream;
+  if ((rc = umma_offset_conv_forward(g, x, (const float*)offset_weight, (const float*)offset_bias, (float*)offset,
+                                     workspace, st, !(s->flags & DCN_FLAG_XT_STAGED), (float*)mask)))
+    return rc;
+  return umma_forward(g, DCN_OPERAND_FP32, s->flags | DCN_FLAG_XT_STAGED, x, (const float*)offset, weight,
+                      (const float*)bias, out, workspace, st, (const float*)mask);
+}
+
+// dcn_layer_backward and dcn_layer_backward_modulated
+static int layer_backward_impl(const DcnShape* s, int phase, const char* what, const void* x, const void* offset,
+                               const void* mask, const void* offset_weight, const void* weight, const void* grad_out,
+                               void* grad_x, void* grad_offset_weight, void* grad_offset_bias, void* grad_weight,
+                               void* grad_bias, void* workspace, size_t workspace_bytes, void* stream) {
+  Geo g;
+  int rc = geo_or_error(s, &g);
+  if (rc) return rc;
+  const bool want_gx = !(s->flags & DCN_FLAG_NO_GRAD_X);
+  if ((rc = check_ptr(x, "x")) || (rc = check_ptr(offset, "offset")) ||
+      (rc = check_ptr(mask, "mask", modulated_phase(phase))) || (rc = check_ptr(offset_weight, "offset_weight")) ||
+      (rc = check_ptr(weight, "weight")) || (rc = check_ptr(grad_out, "grad_out")) ||
+      (rc = check_ptr(grad_x, "grad_x", want_gx)) || (rc = check_ptr(grad_offset_weight, "grad_offset_weight")) ||
+      (rc = check_ptr(grad_offset_bias, "grad_offset_bias", false)) || (rc = check_ptr(grad_weight, "grad_weight")) ||
+      (rc = check_ptr(grad_bias, "grad_bias", false)) || (rc = check_ptr(workspace, "workspace")) ||
+      (rc = layer_refusal(s, g, phase, what)))
+    return rc;
+  const size_t need = layer_workspace(g, phase);
+  if ((rc = check_workspace(workspace_bytes, need, what))) return rc;
+  return umma_layer_backward(g, s->flags, x, (const float*)offset, (const float*)mask, (const float*)offset_weight,
+                             weight, grad_out, (float*)grad_x, (float*)grad_offset_weight, (float*)grad_offset_bias,
+                             (float*)grad_weight, (float*)grad_bias, workspace, need, (cudaStream_t)stream);
 }
 
 }  // namespace dcn
@@ -468,72 +556,15 @@ int dcn_backward_modulated(const DcnShape* s, const void* x, const void* offset,
 
 int dcn_offset_conv_forward(const DcnShape* s, const void* x, const void* offset_weight, const void* offset_bias,
                             void* offset, void* workspace, size_t workspace_bytes, void* stream) {
-  Geo g;
-  int rc = geo_or_error(s, &g);
-  if (rc) return rc;
-  if ((rc = check_ptr(x, "x")) || (rc = check_ptr(offset_weight, "offset_weight")) ||
-      (rc = check_ptr(offset_bias, "offset_bias", false)) || (rc = check_ptr(offset, "offset")) ||
-      (rc = check_ptr(workspace, "workspace")))
-    return rc;
-  if (!layer_ok(s, g, DCN_PHASE_LAYER_FORWARD)) {
-    set_error("offset conv on the engine: shape / operand / flags not supported (dcn_path_name(s, DCN_PHASE_LAYER_FORWARD))");
-    return DCN_ERR_UNSUPPORTED;
-  }
-  const size_t need = umma_offset_conv_fwd_workspace(g);
-  if (workspace_bytes < need) {
-    set_error("offset conv workspace: have %zu bytes, need %zu", workspace_bytes, need);
-    return DCN_ERR_WORKSPACE;
-  }
-  return umma_offset_conv_forward(g, x, (const float*)offset_weight, (const float*)offset_bias, (float*)offset,
-                                  workspace, (cudaStream_t)stream, !(s->flags & DCN_FLAG_XT_STAGED));
+  return offset_conv_impl(s, DCN_PHASE_LAYER_FORWARD, "offset conv", x, offset_weight, offset_bias, offset, nullptr,
+                          workspace, workspace_bytes, stream);
 }
 
 int dcn_layer_forward(const DcnShape* s, const void* x, const void* offset_weight, const void* offset_bias,
                       const void* weight, const void* bias, void* offset, void* out, void* workspace,
                       size_t workspace_bytes, void* stream) {
-  Geo g;
-  int rc = geo_or_error(s, &g);
-  if (rc) return rc;
-  if ((rc = check_ptr(weight, "weight")) || (rc = check_ptr(bias, "bias", false)) || (rc = check_ptr(out, "out")))
-    return rc;
-  if (!layer_ok(s, g, DCN_PHASE_LAYER_FORWARD)) {
-    set_error("layer forward: shape / operand / flags not supported (dcn_path_name(s, DCN_PHASE_LAYER_FORWARD))");
-    return DCN_ERR_UNSUPPORTED;
-  }
-  const size_t need = layer_workspace(g, s->operand, DCN_PHASE_LAYER_FORWARD);
-  if (workspace_bytes < need) {
-    set_error("layer forward workspace: have %zu bytes, need %zu", workspace_bytes, need);
-    return DCN_ERR_WORKSPACE;
-  }
-  if ((rc = dcn_offset_conv_forward(s, x, offset_weight, offset_bias, offset, workspace, workspace_bytes, stream)))
-    return rc;
-  return umma_forward(g, s->operand, s->flags | DCN_FLAG_XT_STAGED, x, (const float*)offset, weight,
-                      (const float*)bias, out, workspace, (cudaStream_t)stream);
-}
-
-// ---- chained inference (SURVEY 8f.2): the producer's epilogue writes the consumer's staged input --------------------
-// Geo of the producer with out_framed set from the consumer's staging layout, or an error.
-static int chained_geo(const DcnShape* s, const DcnShape* consumer, Geo* g) {
-  int rc = geo_or_error(s, g);
-  if (rc) return rc;
-  Geo gc;
-  if ((rc = geo_or_error(consumer, &gc))) return rc;
-  if (s->operand != DCN_OPERAND_FP32 || consumer->operand != DCN_OPERAND_FP32 || g->O > 256 ||
-      gc.B != g->B || gc.C != g->O || gc.H != g->Ho || gc.W != g->Wo) {
-    set_error("chained forward: consumer must take this layer's output (B=%d C=%d H=%d W=%d, fp32, O <= 256); got "
-              "B=%d C=%d H=%d W=%d", g->B, g->O, g->Ho, g->Wo, gc.B, gc.C, gc.H, gc.W);
-    return DCN_ERR_BAD_SHAPE;
-  }
-  if (!use_umma(s, *g, DCN_PHASE_FORWARD) || !use_umma(consumer, gc, DCN_PHASE_FORWARD)) {
-    set_error("chained forward: both layers must run on the tensor path (dcn_path_name == \"umma\")");
-    return DCN_ERR_UNSUPPORTED;
-  }
-  Tiling tc;
-  if (!make_tiling(gc, &tc)) return DCN_ERR_UNSUPPORTED;
-  g->out_framed = 1;
-  g->out_G = gc.variant == DCN_VARIANT_TORCH ? tc.G : 0;
-  g->out_Cs = gc.variant == DCN_VARIANT_TORCH ? tc.Cs : 0;
-  return DCN_OK;
+  return layer_forward_impl(s, nullptr, DCN_PHASE_LAYER_FORWARD, "layer forward", x, offset_weight, offset_bias, weight,
+                            bias, offset, nullptr, out, workspace, workspace_bytes, stream);
 }
 
 size_t dcn_staged_input_bytes(const DcnShape* s) {
@@ -554,27 +585,9 @@ int dcn_staged_input_clear(const DcnShape* s, void* workspace, void* stream) {
 int dcn_layer_forward_chained(const DcnShape* s, const DcnShape* consumer, const void* x, const void* offset_weight,
                               const void* offset_bias, const void* weight, const void* bias, void* offset,
                               void* consumer_workspace, void* workspace, size_t workspace_bytes, void* stream) {
-  Geo g;
-  int rc = chained_geo(s, consumer, &g);
-  if (rc) return rc;
-  if ((rc = check_ptr(x, "x")) || (rc = check_ptr(offset_weight, "offset_weight")) ||
-      (rc = check_ptr(offset_bias, "offset_bias", false)) || (rc = check_ptr(weight, "weight")) ||
-      (rc = check_ptr(bias, "bias", false)) || (rc = check_ptr(offset, "offset")) ||
-      (rc = check_ptr(consumer_workspace, "consumer_workspace")) || (rc = check_ptr(workspace, "workspace")))
-    return rc;
-  if (!layer_ok(s, g, DCN_PHASE_LAYER_FORWARD)) {
-    set_error("chained layer forward: shape / operand / flags not supported (dcn_path_name(s, DCN_PHASE_LAYER_FORWARD))");
-    return DCN_ERR_UNSUPPORTED;
-  }
-  const size_t need = layer_workspace(g, s->operand, DCN_PHASE_LAYER_FORWARD);
-  if (workspace_bytes < need) {
-    set_error("chained layer forward workspace: have %zu bytes, need %zu", workspace_bytes, need);
-    return DCN_ERR_WORKSPACE;
-  }
-  if ((rc = dcn_offset_conv_forward(s, x, offset_weight, offset_bias, offset, workspace, workspace_bytes, stream)))
-    return rc;
-  return umma_forward(g, s->operand, s->flags | DCN_FLAG_XT_STAGED, x, (const float*)offset, weight,
-                      (const float*)bias, consumer_workspace, workspace, (cudaStream_t)stream);
+  return layer_forward_impl(s, consumer, DCN_PHASE_LAYER_FORWARD, "chained layer forward", x, offset_weight,
+                            offset_bias, weight, bias, offset, nullptr, consumer_workspace, workspace, workspace_bytes,
+                            stream);
 }
 
 static int staged_consumer(const DcnShape* consumer, Geo* g, Tiling* t) {
@@ -633,101 +646,33 @@ int dcn_layer_backward(const DcnShape* s, const void* x, const void* offset, con
                        const void* weight, const void* grad_out, void* grad_x, void* grad_offset_weight,
                        void* grad_offset_bias, void* grad_weight, void* grad_bias, void* workspace,
                        size_t workspace_bytes, void* stream) {
-  Geo g;
-  int rc = geo_or_error(s, &g);
-  if (rc) return rc;
-  const bool want_gx = !(s->flags & DCN_FLAG_NO_GRAD_X);
-  if ((rc = check_ptr(x, "x")) || (rc = check_ptr(offset, "offset")) ||
-      (rc = check_ptr(offset_weight, "offset_weight")) || (rc = check_ptr(weight, "weight")) ||
-      (rc = check_ptr(grad_out, "grad_out")) || (rc = check_ptr(grad_x, "grad_x", want_gx)) ||
-      (rc = check_ptr(grad_offset_weight, "grad_offset_weight")) ||
-      (rc = check_ptr(grad_offset_bias, "grad_offset_bias", false)) || (rc = check_ptr(grad_weight, "grad_weight")) ||
-      (rc = check_ptr(grad_bias, "grad_bias", false)) || (rc = check_ptr(workspace, "workspace")))
-    return rc;
-  if (!layer_ok(s, g, DCN_PHASE_LAYER_BACKWARD)) {
-    set_error("layer backward: shape / operand / flags not supported (dcn_path_name(s, DCN_PHASE_LAYER_BACKWARD))");
-    return DCN_ERR_UNSUPPORTED;
-  }
-  const size_t need = layer_workspace(g, s->operand, DCN_PHASE_LAYER_BACKWARD);
-  if (workspace_bytes < need) {
-    set_error("layer backward workspace: have %zu bytes, need %zu", workspace_bytes, need);
-    return DCN_ERR_WORKSPACE;
-  }
-  return umma_layer_backward(g, s->flags, x, (const float*)offset, (const float*)offset_weight, weight, grad_out,
-                             (float*)grad_x, (float*)grad_offset_weight, (float*)grad_offset_bias,
-                             (float*)grad_weight, (float*)grad_bias, workspace, need, (cudaStream_t)stream);
+  return layer_backward_impl(s, DCN_PHASE_LAYER_BACKWARD, "layer backward", x, offset, nullptr, offset_weight, weight,
+                             grad_out, grad_x, grad_offset_weight, grad_offset_bias, grad_weight, grad_bias, workspace,
+                             workspace_bytes, stream);
 }
 
 // ---- whole modulated layer (mmcv's ModulatedDeformConv2dPack) -----------------------------------------------------
 int dcn_offset_conv_forward_modulated(const DcnShape* s, const void* x, const void* offset_weight,
                                       const void* offset_bias, void* offset, void* mask, void* workspace,
                                       size_t workspace_bytes, void* stream) {
-  Geo g;
-  int rc = geo_or_error(s, &g);
-  if (rc) return rc;
-  if ((rc = check_ptr(x, "x")) || (rc = check_ptr(offset_weight, "offset_weight")) ||
-      (rc = check_ptr(offset_bias, "offset_bias", false)) || (rc = check_ptr(offset, "offset")) ||
-      (rc = check_ptr(mask, "mask")) || (rc = check_ptr(workspace, "workspace")))
-    return rc;
-  if ((rc = modulated_layer_refusal(s, g, DCN_PHASE_LAYER_FORWARD_MODULATED, "offset-and-mask conv"))) return rc;
-  const size_t need = umma_offset_mask_conv_fwd_workspace(g);
-  if (workspace_bytes < need) {
-    set_error("offset-and-mask conv workspace: have %zu bytes, need %zu", workspace_bytes, need);
-    return DCN_ERR_WORKSPACE;
-  }
-  return umma_offset_conv_forward(g, x, (const float*)offset_weight, (const float*)offset_bias, (float*)offset,
-                                  workspace, (cudaStream_t)stream, !(s->flags & DCN_FLAG_XT_STAGED), (float*)mask);
+  return offset_conv_impl(s, DCN_PHASE_LAYER_FORWARD_MODULATED, "offset-and-mask conv", x, offset_weight, offset_bias,
+                          offset, mask, workspace, workspace_bytes, stream);
 }
 
 int dcn_layer_forward_modulated(const DcnShape* s, const void* x, const void* offset_weight, const void* offset_bias,
                                 const void* weight, const void* bias, void* offset, void* mask, void* out,
                                 void* workspace, size_t workspace_bytes, void* stream) {
-  Geo g;
-  int rc = geo_or_error(s, &g);
-  if (rc) return rc;
-  if ((rc = check_ptr(x, "x")) || (rc = check_ptr(offset_weight, "offset_weight")) ||
-      (rc = check_ptr(offset_bias, "offset_bias", false)) || (rc = check_ptr(weight, "weight")) ||
-      (rc = check_ptr(bias, "bias", false)) || (rc = check_ptr(offset, "offset")) || (rc = check_ptr(mask, "mask")) ||
-      (rc = check_ptr(out, "out")) || (rc = check_ptr(workspace, "workspace")))
-    return rc;
-  if ((rc = modulated_layer_refusal(s, g, DCN_PHASE_LAYER_FORWARD_MODULATED, "modulated layer forward"))) return rc;
-  const size_t need = modulated_layer_workspace(g, DCN_PHASE_LAYER_FORWARD_MODULATED);
-  if (workspace_bytes < need) {
-    set_error("modulated layer forward workspace: have %zu bytes, need %zu", workspace_bytes, need);
-    return DCN_ERR_WORKSPACE;
-  }
-  if ((rc = dcn_offset_conv_forward_modulated(s, x, offset_weight, offset_bias, offset, mask, workspace,
-                                              workspace_bytes, stream)))
-    return rc;
-  return umma_forward(g, DCN_OPERAND_FP32, s->flags | DCN_FLAG_XT_STAGED, x, (const float*)offset, weight,
-                      (const float*)bias, out, workspace, (cudaStream_t)stream, (const float*)mask);
+  return layer_forward_impl(s, nullptr, DCN_PHASE_LAYER_FORWARD_MODULATED, "modulated layer forward", x, offset_weight,
+                            offset_bias, weight, bias, offset, mask, out, workspace, workspace_bytes, stream);
 }
 
 int dcn_layer_backward_modulated(const DcnShape* s, const void* x, const void* offset, const void* mask,
                                  const void* offset_weight, const void* weight, const void* grad_out, void* grad_x,
                                  void* grad_offset_weight, void* grad_offset_bias, void* grad_weight, void* grad_bias,
                                  void* workspace, size_t workspace_bytes, void* stream) {
-  Geo g;
-  int rc = geo_or_error(s, &g);
-  if (rc) return rc;
-  const bool want_gx = !(s->flags & DCN_FLAG_NO_GRAD_X);
-  if ((rc = check_ptr(x, "x")) || (rc = check_ptr(offset, "offset")) || (rc = check_ptr(mask, "mask")) ||
-      (rc = check_ptr(offset_weight, "offset_weight")) || (rc = check_ptr(weight, "weight")) ||
-      (rc = check_ptr(grad_out, "grad_out")) || (rc = check_ptr(grad_x, "grad_x", want_gx)) ||
-      (rc = check_ptr(grad_offset_weight, "grad_offset_weight")) ||
-      (rc = check_ptr(grad_offset_bias, "grad_offset_bias", false)) || (rc = check_ptr(grad_weight, "grad_weight")) ||
-      (rc = check_ptr(grad_bias, "grad_bias", false)) || (rc = check_ptr(workspace, "workspace")))
-    return rc;
-  if ((rc = modulated_layer_refusal(s, g, DCN_PHASE_LAYER_BACKWARD_MODULATED, "modulated layer backward"))) return rc;
-  const size_t need = modulated_layer_workspace(g, DCN_PHASE_LAYER_BACKWARD_MODULATED);
-  if (workspace_bytes < need) {
-    set_error("modulated layer backward workspace: have %zu bytes, need %zu", workspace_bytes, need);
-    return DCN_ERR_WORKSPACE;
-  }
-  return umma_layer_backward_modulated(g, s->flags, x, (const float*)offset, (const float*)mask,
-                                       (const float*)offset_weight, weight, grad_out, (float*)grad_x,
-                                       (float*)grad_offset_weight, (float*)grad_offset_bias, (float*)grad_weight,
-                                       (float*)grad_bias, workspace, need, (cudaStream_t)stream);
+  return layer_backward_impl(s, DCN_PHASE_LAYER_BACKWARD_MODULATED, "modulated layer backward", x, offset, mask,
+                             offset_weight, weight, grad_out, grad_x, grad_offset_weight, grad_offset_bias,
+                             grad_weight, grad_bias, workspace, workspace_bytes, stream);
 }
 
 int dcn_debug_corners(const DcnShape* s, const void* offset, int32_t* y0, int32_t* x0, float* w4,

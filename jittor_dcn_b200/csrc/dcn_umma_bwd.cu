@@ -50,21 +50,22 @@ int conv_offset_backward(const Geo& g, int O, const float* xt, float* gxt, const
 
 // ---- companion offset convolution (PLAIN problem) inside the layer's backward pass ---------------------------------
 // n_out = the conv's output channels (2N; 3N for the modulated layer's offset-and-mask conv)
-static bool plain_bwd_ok(const Geo& g, int n_out = 0) {
+static bool plain_bwd_ok(const Geo& g, int n_out) {
   Tiling t;
   if (!make_tiling(g, &t)) return false;
-  if (conv_offset_bwd_supported(g, n_out ? n_out : 2 * g.N)) return true;
+  if (conv_offset_bwd_supported(g, n_out)) return true;
   const Geo gp = plain_geo(g, t, false, n_out);
   return umma_bwd_data_supported(gp, DCN_OPERAND_FP32) && umma_bwd_data_fuses_wgrad(gp, DCN_OPERAND_FP32);
 }
 
 // Whole-layer backward (DCN span + offset conv) on the tensor path: fp32 operands, one output-channel group or more,
 // data gradient on the tcgen05 kernel (so that the channels-last grad_x accumulator exists for both passes).
-bool umma_layer_bwd_supported(const Geo& g) {
+bool umma_layer_bwd_supported(const Geo& g, int n_out) {
   int gsize;
   if (!o_groups(g, &gsize)) return false;
   const Geo g0 = o_group_geo(g, 0, gsize);
-  return umma_bwd_supported(g0, DCN_OPERAND_FP32) && umma_bwd_data_supported(g0, DCN_OPERAND_FP32) && plain_bwd_ok(g);
+  return umma_bwd_supported(g0, DCN_OPERAND_FP32) && umma_bwd_data_supported(g0, DCN_OPERAND_FP32) &&
+         plain_bwd_ok(g, n_out);
 }
 
 // The modulated layer's conv output gradient, per image b: g3[b] = [goff[b] (2N planes) ; gmask[b] * m * (1 - m)
@@ -110,20 +111,22 @@ static int launch_pack_offset_mask_grad(const Geo& g, const float* goff, const f
 static size_t goff_bytes(const Geo& g) { return align_up(sizeof(float) * (size_t)g.B * 2 * g.N * g.HW, 1024); }
 static size_t planes_bytes(const Geo& g, int ch) { return align_up(sizeof(float) * (size_t)g.B * ch * g.HW, 1024); }
 
-// [xt][rest as umma_bwd_workspace, its tile regions sized for the larger of the two passes][grad_offset]
-size_t umma_layer_bwd_workspace(const Geo& g) {
+// [xt][rest as umma_bwd_workspace, its tile regions sized for the larger of the two passes][grad_offset], and for the
+// modulated layer (n_out = 3N) then [grad_mask][g3]
+size_t umma_layer_bwd_workspace(const Geo& g, int n_out) {
   int gsize;
   if (!o_groups(g, &gsize)) return 0;
   const Geo g0 = o_group_geo(g, 0, gsize);
   Tiling t;
   if (!make_tiling(g, &t)) return 0;
-  const Geo gp = plain_geo(g, t, false);
+  const Geo gp = plain_geo(g, t, false, n_out);
   const size_t tiles_dcn = umma_bwd_data_wtile_bytes(g0, DCN_OPERAND_FP32) + umma_bwd_data_gtile_bytes(g0, DCN_OPERAND_FP32);
-  size_t tiles_pln = umma_bwd_data_wtile_bytes(gp, DCN_OPERAND_FP32) + umma_bwd_data_gtile_bytes(gp, DCN_OPERAND_FP32);
-  if (conv_offset_bwd_supported(g, 2 * g.N)) tiles_pln = conv_offset_wtile_bytes(g, 2 * g.N);
-  const size_t a = umma_xt_bytes(g, DCN_OPERAND_FP32) + (tiles_dcn > tiles_pln ? tiles_dcn : tiles_pln);
+  const size_t tiles_conv = conv_offset_bwd_supported(g, n_out) ? conv_offset_wtile_bytes(g, n_out) :
+      umma_bwd_data_wtile_bytes(gp, DCN_OPERAND_FP32) + umma_bwd_data_gtile_bytes(gp, DCN_OPERAND_FP32);
+  const size_t a = umma_xt_bytes(g, DCN_OPERAND_FP32) + (tiles_dcn > tiles_conv ? tiles_dcn : tiles_conv);
   const size_t c = umma_wgrad_gtile_bytes(g0, DCN_OPERAND_FP32);
-  return umma_xt_bytes(g, DCN_OPERAND_FP32) + (a > c ? a : c) + goff_bytes(g);
+  const size_t tail = goff_bytes(g) + (n_out == 2 * g.N ? 0 : planes_bytes(g, g.N) + planes_bytes(g, n_out));
+  return umma_xt_bytes(g, DCN_OPERAND_FP32) + (a > c ? a : c) + tail;
 }
 
 size_t umma_bwd_workspace(const Geo& g, int operand) {
@@ -199,16 +202,22 @@ int umma_backward_any(const Geo& g, int operand, int flags, const void* xv, cons
                                   gb_rides ? gb + o0 : nullptr, mask, gmask)))
         return rc;
     }
-    if (woff && g3) {
-      if (!mask || !plain_bwd_ok(g, 3 * g.N)) {
-        set_error("modulated layer backward: the offset-and-mask conv of this shape has no backward kernel");
-        return DCN_ERR_UNSUPPORTED;
+    if (woff) {
+      // the conv's output count and output gradient: 2N and goff, or 3N and g3 = [goff ; gmask * m * (1 - m)]
+      const int n_out = g3 ? 3 * g.N : 2 * g.N;
+      const float* gconv = goff;
+      if (g3) {
+        if (!mask || !plain_bwd_ok(g, n_out)) {
+          set_error("modulated layer backward: the offset-and-mask conv of this shape has no backward kernel");
+          return DCN_ERR_UNSUPPORTED;
+        }
+        if ((rc = launch_pack_offset_mask_grad(g, goff, gmask, mask, g3, st))) return rc;
+        gconv = g3;
       }
-      const Geo gp = plain_geo(g, t, false, 3 * g.N);
+      const Geo gp = plain_geo(g, t, false, n_out);
       uint8_t* wtiles2 = rest + umma_xt_bytes(g, DCN_OPERAND_FP32);
-      if ((rc = launch_pack_offset_mask_grad(g, goff, gmask, mask, g3, st))) return rc;
-      if (conv_offset_bwd_supported(g, 3 * g.N)) {
-        if ((rc = conv_offset_backward(g, 3 * g.N, (const float*)xt, want_gx ? gxt : nullptr, g3, woff, gwoff, wtiles2,
+      if (conv_offset_bwd_supported(g, n_out)) {
+        if ((rc = conv_offset_backward(g, n_out, (const float*)xt, want_gx ? gxt : nullptr, gconv, woff, gwoff, wtiles2,
                                        st)))
           return rc;
       } else {
@@ -216,27 +225,11 @@ int umma_backward_any(const Geo& g, int operand, int flags, const void* xv, cons
         // would need four parity accumulators of 64 columns, more than TMEM holds double-buffered)
         uint8_t* gtiles2 = wtiles2 + umma_bwd_data_wtile_bytes(gp, DCN_OPERAND_FP32);
         DCN_CUDA_TRY(cudaMemsetAsync(gwoff, 0, sizeof(float) * (size_t)gp.O * g.K, st));
-        if ((rc = umma_bwd_data_any(gp, DCN_OPERAND_FP32, xt, want_gx ? gxt : nullptr, nullptr, woff, g3, nullptr,
+        if ((rc = umma_bwd_data_any(gp, DCN_OPERAND_FP32, xt, want_gx ? gxt : nullptr, nullptr, woff, gconv, nullptr,
                                     gwoff, wtiles2, gtiles2, st)))
           return rc;
       }
-      if ((rc = launch_bias_grad(gp, g3, DCN_OPERAND_FP32, gboff, st))) return rc;
-    } else if (woff && conv_offset_bwd_supported(g, 2 * g.N)) {
-      const Geo gp = plain_geo(g, t, false);
-      uint8_t* wtiles2 = rest + umma_xt_bytes(g, DCN_OPERAND_FP32);
-      if ((rc = conv_offset_backward(g, 2 * g.N, (const float*)xt, want_gx ? gxt : nullptr, goff, woff, gwoff, wtiles2,
-                                     st)))
-        return rc;
-      if ((rc = launch_bias_grad(gp, goff, DCN_OPERAND_FP32, gboff, st))) return rc;
-    } else if (woff) {
-      const Geo gp = plain_geo(g, t, false);
-      uint8_t* wtiles2 = rest + umma_xt_bytes(g, DCN_OPERAND_FP32);
-      uint8_t* gtiles2 = wtiles2 + umma_bwd_data_wtile_bytes(gp, DCN_OPERAND_FP32);
-      DCN_CUDA_TRY(cudaMemsetAsync(gwoff, 0, sizeof(float) * (size_t)gp.O * g.K, st));
-      if ((rc = umma_bwd_data_any(gp, DCN_OPERAND_FP32, xt, want_gx ? gxt : nullptr, nullptr, woff, goff, nullptr, gwoff,
-                                  wtiles2, gtiles2, st)))
-        return rc;
-      if ((rc = launch_bias_grad(gp, goff, DCN_OPERAND_FP32, gboff, st))) return rc;
+      if ((rc = launch_bias_grad(gp, gconv, DCN_OPERAND_FP32, gboff, st))) return rc;
     }
     if (want_gx && !gx_framed && (rc = launch_nhwc_to_nchw_add(g, t, gxt, gx, (flags & DCN_FLAG_ACCUM_GRAD_X) ? 1 : 0, st)))
       return rc;
@@ -271,51 +264,18 @@ int umma_backward_any(const Geo& g, int operand, int flags, const void* xv, cons
 
 namespace dcn {
 
-// Whole-layer backward: see umma_backward_any.  The internal grad_offset buffer sits at the tail of the workspace.
-int umma_layer_backward(const Geo& g, int flags, const void* x, const float* off, const float* woff, const void* wt,
-                        const void* gout, float* gx, float* gwoff, float* gboff, float* gw, float* gb,
+// Whole-layer backward: see umma_backward_any.  The internal grad_offset buffer, and with a mask the grad_mask and
+// packed 3N-channel conv gradient buffers after it, sit at the tail of the workspace (umma_layer_bwd_workspace).
+int umma_layer_backward(const Geo& g, int flags, const void* x, const float* off, const float* mask, const float* woff,
+                        const void* wt, const void* gout, float* gx, float* gwoff, float* gboff, float* gw, float* gb,
                         void* workspace, size_t workspace_bytes, cudaStream_t st) {
-  float* goff = (float*)((uint8_t*)workspace + workspace_bytes - goff_bytes(g));
-  return umma_backward_any(g, DCN_OPERAND_FP32, flags, x, off, wt, gout, gx, goff, gw, gb, workspace, st, woff, gwoff,
-                           gboff, nullptr, nullptr, nullptr);
-}
-
-// ---- whole modulated layer -----------------------------------------------------------------------------------------
-bool umma_layer_bwd_modulated_supported(const Geo& g) {
-  int gsize;
-  if (!o_groups(g, &gsize)) return false;
-  const Geo g0 = o_group_geo(g, 0, gsize);
-  Tiling t;
-  return make_tiling(g, &t) && umma_bwd_supported(g0, DCN_OPERAND_FP32) &&
-         umma_bwd_data_supported(g0, DCN_OPERAND_FP32) && plain_bwd_ok(g, 3 * g.N);
-}
-
-// [xt][rest as umma_layer_bwd_workspace, conv tiles sized for 3N outputs][grad_offset][grad_mask][g3]
-size_t umma_layer_bwd_modulated_workspace(const Geo& g) {
-  int gsize;
-  if (!o_groups(g, &gsize)) return 0;
-  const Geo g0 = o_group_geo(g, 0, gsize);
-  Tiling t;
-  if (!make_tiling(g, &t)) return 0;
-  const Geo gp = plain_geo(g, t, false, 3 * g.N);
-  const size_t tiles_dcn = umma_bwd_data_wtile_bytes(g0, DCN_OPERAND_FP32) + umma_bwd_data_gtile_bytes(g0, DCN_OPERAND_FP32);
-  const size_t tiles_conv = conv_offset_bwd_supported(g, 3 * g.N) ? conv_offset_wtile_bytes(g, 3 * g.N) :
-      umma_bwd_data_wtile_bytes(gp, DCN_OPERAND_FP32) + umma_bwd_data_gtile_bytes(gp, DCN_OPERAND_FP32);
-  const size_t a = umma_xt_bytes(g, DCN_OPERAND_FP32) + (tiles_dcn > tiles_conv ? tiles_dcn : tiles_conv);
-  const size_t c = umma_wgrad_gtile_bytes(g0, DCN_OPERAND_FP32);
-  return umma_xt_bytes(g, DCN_OPERAND_FP32) + (a > c ? a : c) + goff_bytes(g) + planes_bytes(g, g.N) +
-         planes_bytes(g, 3 * g.N);
-}
-
-// grad_offset, grad_mask and the packed 3N-channel conv gradient sit at the tail of the workspace
-int umma_layer_backward_modulated(const Geo& g, int flags, const void* x, const float* off, const float* mask,
-                                  const float* woff, const void* wt, const void* gout, float* gx, float* gwoff,
-                                  float* gboff, float* gw, float* gb, void* workspace, size_t workspace_bytes,
-                                  cudaStream_t st) {
   uint8_t* tail = (uint8_t*)workspace + workspace_bytes;
-  float* g3 = (float*)(tail - planes_bytes(g, 3 * g.N));
-  float* gmask = (float*)((uint8_t*)g3 - planes_bytes(g, g.N));
-  float* goff = (float*)((uint8_t*)gmask - goff_bytes(g));
+  float *g3 = nullptr, *gmask = nullptr;
+  if (mask) {
+    g3 = (float*)(tail -= planes_bytes(g, 3 * g.N));
+    gmask = (float*)(tail -= planes_bytes(g, g.N));
+  }
+  float* goff = (float*)(tail - goff_bytes(g));
   return umma_backward_any(g, DCN_OPERAND_FP32, flags, x, off, wt, gout, gx, goff, gw, gb, workspace, st, woff, gwoff,
                            gboff, mask, gmask, g3);
 }

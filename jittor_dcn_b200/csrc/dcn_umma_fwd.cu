@@ -1185,31 +1185,22 @@ size_t conv_offset_wtile_bytes(const Geo& g, int O);
 int conv_offset_forward(const Geo& g, const float* xt, const float* woff, const float* boff, float* offset_out,
                         uint8_t* wtiles, cudaStream_t st, float* mask_out);
 
-bool umma_offset_conv_fwd_supported(const Geo& g) {
+// n_out = 3N (the modulated layer's offset-and-mask conv): shifted-view or warp-MMA kernels only (the plain mode's
+// epilogue has no mask output)
+bool umma_offset_conv_fwd_supported(const Geo& g, int n_out) {
   Tiling t;
   if (!make_tiling(g, &t)) return false;          // the layer's own staging layout
-  if (conv_offset_fwd_supported(g, 2 * g.N)) return true;
-  const Geo gp = plain_geo(g, t, true);
-  return umma_fwd_supported(gp, DCN_OPERAND_FP32);
+  if (conv_offset_fwd_supported(g, n_out)) return true;
+  return n_out == 2 * g.N && umma_fwd_supported(plain_geo(g, t, true), DCN_OPERAND_FP32);
 }
 
-size_t umma_offset_conv_fwd_workspace(const Geo& g) {
+size_t umma_offset_conv_fwd_workspace(const Geo& g, int n_out) {
+  const size_t b = umma_xt_bytes(g, DCN_OPERAND_FP32) + conv_offset_wtile_bytes(g, n_out);
+  if (n_out != 2 * g.N) return b;
   Tiling t;
   if (!make_tiling(g, &t)) return 0;
   const size_t a = umma_fwd_workspace(plain_geo(g, t, true), DCN_OPERAND_FP32);
-  const size_t b = umma_xt_bytes(g, DCN_OPERAND_FP32) + conv_offset_wtile_bytes(g, 2 * g.N);
   return a > b ? a : b;
-}
-
-// The modulated layer's offset-and-mask conv (3N outputs): shifted-view or warp-MMA kernels only (the plain mode's
-// epilogue has no mask output)
-bool umma_offset_mask_conv_fwd_supported(const Geo& g) {
-  Tiling t;
-  return make_tiling(g, &t) && conv_offset_fwd_supported(g, 3 * g.N);
-}
-
-size_t umma_offset_mask_conv_fwd_workspace(const Geo& g) {
-  return umma_xt_bytes(g, DCN_OPERAND_FP32) + conv_offset_wtile_bytes(g, 3 * g.N);
 }
 
 int umma_offset_conv_forward(const Geo& g, const void* x, const float* woff, const float* boff, float* offset_out,

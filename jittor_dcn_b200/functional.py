@@ -101,30 +101,25 @@ def staged_workspace(x, weight, kernel_size=3, stride=1, padding=1, variant=VARI
     return torch.empty(need, dtype=torch.uint8, device=x.device)
 
 
+def _run(entry, dev, shp, tensors, phase=None, ws=None):
+    """lib.<entry>(shape, *tensors[, workspace, workspace_bytes], stream) on the current stream of `dev`, then its status
+    checked.  phase: the call takes a workspace, `ws` or else the cached scratch buffer sized for that phase."""
+    lib = _lib.load()
+    args = tuple(_ptr(t) for t in tensors)
+    with torch.cuda.device(dev):
+        stream = torch.cuda.current_stream(dev)
+        if phase is not None:
+            if ws is None:
+                ws = _workspace(dev, stream.cuda_stream, lib.dcn_workspace_bytes(ctypes.byref(shp), phase))
+            args += (_ptr(ws), ws.numel())
+        rc = getattr(lib, entry)(ctypes.byref(shp), *args, ctypes.c_void_p(stream.cuda_stream))
+    _lib.check(rc, entry)
+
+
 def dcn_forward(x, offset, weight, bias, kernel_size=3, stride=1, padding=1, variant=VARIANT_TORCH,
                 operand=OPERAND_FP32, flags=0, ws=None):
     """out[B,O,Ho,Wo] = engine forward on CUDA tensors (no autograd)."""
-    lib = _lib.load()
-    shp = _shape_of(x, weight, kernel_size, stride, padding, variant, operand, flags)
-    Ho, Wo = _lib.output_hw(shp)
-    N = shp.kh * shp.kw
-    if tuple(offset.shape) != (shp.B, 2 * N, Ho, Wo):
-        raise ValueError(f"offset shape {tuple(offset.shape)} != {(shp.B, 2 * N, Ho, Wo)}")
-    if tuple(weight.shape) != (shp.O, shp.C, shp.kh, shp.kw):
-        raise ValueError(f"weight shape {tuple(weight.shape)} != {(shp.O, shp.C, shp.kh, shp.kw)}")
-    act = torch.bfloat16 if operand == OPERAND_BF16 else torch.float32
-    x, weight = _dev_ready(x, act), _dev_ready(weight, act)
-    offset, bias = _dev_ready(offset), _dev_ready(bias)
-    out = torch.empty((shp.B, shp.O, Ho, Wo), dtype=torch.float32, device=x.device)
-    with torch.cuda.device(x.device):
-        stream = torch.cuda.current_stream(x.device)
-        need = lib.dcn_workspace_bytes(ctypes.byref(shp), PHASE_FORWARD)
-        if ws is None:
-            ws = _workspace(x.device, stream.cuda_stream, need)
-        rc = lib.dcn_forward(ctypes.byref(shp), _ptr(x), _ptr(offset), _ptr(weight), _ptr(bias),
-                             _ptr(out), _ptr(ws), ws.numel(), ctypes.c_void_p(stream.cuda_stream))
-    _lib.check(rc, "dcn_forward")
-    return out
+    return _span_forward(x, offset, None, weight, bias, kernel_size, stride, padding, variant, operand, flags, ws)
 
 
 def dcn_backward(x, offset, weight, grad_out, has_bias, kernel_size=3, stride=1, padding=1,
@@ -135,7 +130,58 @@ def dcn_backward(x, offset, weight, grad_out, has_bias, kernel_size=3, stride=1,
     grad_x: an existing float32 gradient of x's shape to ACCUMULATE into (DCN_FLAG_ACCUM_GRAD_X; e.g. the
     term the companion offset conv contributes); without it the flag is refused — the library would add into
     whatever the freshly allocated output buffer happens to hold."""
-    lib = _lib.load()
+    gx, goff, _, gw, gb = _span_backward(x, offset, None, weight, grad_out, has_bias, kernel_size, stride, padding,
+                                         variant, operand, flags, need_grad_x, ws, xt_staged, grad_x)
+    return gx, goff, gw, gb
+
+
+# ---- modulated deformable convolution (DCNv2): DCNv1 sampling, every sample scaled by mask[b, n, p] ----------------
+def dcn_forward_modulated(x, offset, mask, weight, bias, kernel_size=3, stride=1, padding=1, operand=OPERAND_FP32,
+                          flags=0, ws=None):
+    """out[B,O,Ho,Wo] = modulated DCNv1 forward on CUDA tensors (no autograd); mask [B, kh*kw, Ho, Wo] float32
+    (torchvision's tap order, any values).  Arguments otherwise as dcn_forward with variant = VARIANT_DCNV1."""
+    return _span_forward(x, offset, mask, weight, bias, kernel_size, stride, padding, VARIANT_DCNV1, operand, flags, ws)
+
+
+def dcn_backward_modulated(x, offset, mask, weight, grad_out, has_bias, kernel_size=3, stride=1, padding=1,
+                           operand=OPERAND_FP32, flags=0, need_grad_x=True, ws=None, xt_staged=False, grad_x=None):
+    """-> grad_x (or None), grad_offset, grad_mask, grad_weight, grad_bias (or None); all float32.
+    Arguments as dcn_backward with variant = VARIANT_DCNV1, plus the forward's mask."""
+    return _span_backward(x, offset, mask, weight, grad_out, has_bias, kernel_size, stride, padding, VARIANT_DCNV1,
+                          operand, flags, need_grad_x, ws, xt_staged, grad_x)
+
+
+def _check_mask(mask, shp, Ho, Wo):
+    N = shp.kh * shp.kw
+    if tuple(mask.shape) != (shp.B, N, Ho, Wo):
+        raise ValueError(f"mask shape {tuple(mask.shape)} != {(shp.B, N, Ho, Wo)} ([B, kh*kw, H_out, W_out])")
+
+
+# the span calls: mask None = unmodulated (dcn_forward / dcn_backward), else DCN_VARIANT_DCNV1 modulated
+def _span_forward(x, offset, mask, weight, bias, kernel_size, stride, padding, variant, operand, flags, ws):
+    shp = _shape_of(x, weight, kernel_size, stride, padding, variant, operand, flags)
+    Ho, Wo = _lib.output_hw(shp)
+    N = shp.kh * shp.kw
+    if tuple(offset.shape) != (shp.B, 2 * N, Ho, Wo):
+        raise ValueError(f"offset shape {tuple(offset.shape)} != {(shp.B, 2 * N, Ho, Wo)}")
+    if tuple(weight.shape) != (shp.O, shp.C, shp.kh, shp.kw):
+        raise ValueError(f"weight shape {tuple(weight.shape)} != {(shp.O, shp.C, shp.kh, shp.kw)}")
+    if mask is not None:
+        _check_mask(mask, shp, Ho, Wo)
+    act = torch.bfloat16 if operand == OPERAND_BF16 else torch.float32
+    x, weight = _dev_ready(x, act), _dev_ready(weight, act)
+    offset, mask, bias = _dev_ready(offset), _dev_ready(mask), _dev_ready(bias)
+    out = torch.empty((shp.B, shp.O, Ho, Wo), dtype=torch.float32, device=x.device)
+    if mask is None:
+        _run("dcn_forward", x.device, shp, (x, offset, weight, bias, out), PHASE_FORWARD, ws)
+    else:
+        _run("dcn_forward_modulated", x.device, shp, (x, offset, mask, weight, bias, out), PHASE_FORWARD, ws)
+    return out
+
+
+def _span_backward(x, offset, mask, weight, grad_out, has_bias, kernel_size, stride, padding, variant, operand, flags,
+                   need_grad_x, ws, xt_staged, grad_x):
+    """-> grad_x, grad_offset, grad_mask (None without a mask), grad_weight, grad_bias."""
     if grad_x is not None:
         if not need_grad_x:
             raise ValueError("grad_x given but need_grad_x is False")
@@ -152,121 +198,43 @@ def dcn_backward(x, offset, weight, grad_out, has_bias, kernel_size=3, stride=1,
     shp = _shape_of(x, weight, kernel_size, stride, padding, variant, operand, flags)
     Ho, Wo = _lib.output_hw(shp)
     N = shp.kh * shp.kw
-    act = torch.bfloat16 if operand == OPERAND_BF16 else torch.float32
-    x, weight, grad_out = _dev_ready(x, act), _dev_ready(weight, act), _dev_ready(grad_out, act)
-    offset = _dev_ready(offset)
-    dev = x.device
-    gx = grad_x if grad_x is not None else (torch.empty(x.shape, dtype=torch.float32, device=dev) if need_grad_x else None)
-    goff = torch.empty((shp.B, 2 * N, Ho, Wo), dtype=torch.float32, device=dev)
-    gw = torch.empty(weight.shape, dtype=torch.float32, device=dev)
-    gb = torch.empty((shp.O,), dtype=torch.float32, device=dev) if has_bias else None
-    with torch.cuda.device(dev):
-        stream = torch.cuda.current_stream(dev)
-        need = lib.dcn_workspace_bytes(ctypes.byref(shp), PHASE_BACKWARD)
-        if ws is None:
-            ws = _workspace(dev, stream.cuda_stream, need)
-        rc = lib.dcn_backward(ctypes.byref(shp), _ptr(x), _ptr(offset), _ptr(weight), _ptr(grad_out),
-                              _ptr(gx), _ptr(goff), _ptr(gw), _ptr(gb), _ptr(ws), ws.numel(),
-                              ctypes.c_void_p(stream.cuda_stream))
-    _lib.check(rc, "dcn_backward")
-    return gx, goff, gw, gb
-
-
-# ---- modulated deformable convolution (DCNv2): DCNv1 sampling, every sample scaled by mask[b, n, p] ----------------
-def _check_mask(mask, shp, Ho, Wo):
-    N = shp.kh * shp.kw
-    if tuple(mask.shape) != (shp.B, N, Ho, Wo):
-        raise ValueError(f"mask shape {tuple(mask.shape)} != {(shp.B, N, Ho, Wo)} ([B, kh*kw, H_out, W_out])")
-
-
-def dcn_forward_modulated(x, offset, mask, weight, bias, kernel_size=3, stride=1, padding=1, operand=OPERAND_FP32,
-                          flags=0, ws=None):
-    """out[B,O,Ho,Wo] = modulated DCNv1 forward on CUDA tensors (no autograd); mask [B, kh*kw, Ho, Wo] float32
-    (torchvision's tap order, any values).  Arguments otherwise as dcn_forward with variant = VARIANT_DCNV1."""
-    lib = _lib.load()
-    shp = _shape_of(x, weight, kernel_size, stride, padding, VARIANT_DCNV1, operand, flags)
-    Ho, Wo = _lib.output_hw(shp)
-    N = shp.kh * shp.kw
-    if tuple(offset.shape) != (shp.B, 2 * N, Ho, Wo):
-        raise ValueError(f"offset shape {tuple(offset.shape)} != {(shp.B, 2 * N, Ho, Wo)}")
-    if tuple(weight.shape) != (shp.O, shp.C, shp.kh, shp.kw):
-        raise ValueError(f"weight shape {tuple(weight.shape)} != {(shp.O, shp.C, shp.kh, shp.kw)}")
-    _check_mask(mask, shp, Ho, Wo)
-    act = torch.bfloat16 if operand == OPERAND_BF16 else torch.float32
-    x, weight = _dev_ready(x, act), _dev_ready(weight, act)
-    offset, mask, bias = _dev_ready(offset), _dev_ready(mask), _dev_ready(bias)
-    out = torch.empty((shp.B, shp.O, Ho, Wo), dtype=torch.float32, device=x.device)
-    with torch.cuda.device(x.device):
-        stream = torch.cuda.current_stream(x.device)
-        need = lib.dcn_workspace_bytes(ctypes.byref(shp), PHASE_FORWARD)
-        if ws is None:
-            ws = _workspace(x.device, stream.cuda_stream, need)
-        rc = lib.dcn_forward_modulated(ctypes.byref(shp), _ptr(x), _ptr(offset), _ptr(mask), _ptr(weight), _ptr(bias),
-                                       _ptr(out), _ptr(ws), ws.numel(), ctypes.c_void_p(stream.cuda_stream))
-    _lib.check(rc, "dcn_forward_modulated")
-    return out
-
-
-def dcn_backward_modulated(x, offset, mask, weight, grad_out, has_bias, kernel_size=3, stride=1, padding=1,
-                           operand=OPERAND_FP32, flags=0, need_grad_x=True, ws=None, xt_staged=False, grad_x=None):
-    """-> grad_x (or None), grad_offset, grad_mask, grad_weight, grad_bias (or None); all float32.
-    Arguments as dcn_backward with variant = VARIANT_DCNV1, plus the forward's mask."""
-    lib = _lib.load()
-    if grad_x is not None:
-        if not need_grad_x:
-            raise ValueError("grad_x given but need_grad_x is False")
-        if grad_x.dtype != torch.float32 or tuple(grad_x.shape) != tuple(x.shape) or not grad_x.is_contiguous() \
-                or grad_x.data_ptr() % 16:
-            raise ValueError("grad_x must be a dense, 16-byte aligned float32 tensor of x's shape")
-        flags |= FLAG_ACCUM_GRAD_X
-    elif flags & FLAG_ACCUM_GRAD_X:
-        raise ValueError("FLAG_ACCUM_GRAD_X needs the tensor to accumulate into: pass grad_x=")
-    if not need_grad_x:
-        flags |= FLAG_NO_GRAD_X
-    if xt_staged and ws is not None:
-        flags |= FLAG_XT_STAGED
-    shp = _shape_of(x, weight, kernel_size, stride, padding, VARIANT_DCNV1, operand, flags)
-    Ho, Wo = _lib.output_hw(shp)
-    N = shp.kh * shp.kw
-    _check_mask(mask, shp, Ho, Wo)
+    if mask is not None:
+        _check_mask(mask, shp, Ho, Wo)
     act = torch.bfloat16 if operand == OPERAND_BF16 else torch.float32
     x, weight, grad_out = _dev_ready(x, act), _dev_ready(weight, act), _dev_ready(grad_out, act)
     offset, mask = _dev_ready(offset), _dev_ready(mask)
     dev = x.device
     gx = grad_x if grad_x is not None else (torch.empty(x.shape, dtype=torch.float32, device=dev) if need_grad_x else None)
     goff = torch.empty((shp.B, 2 * N, Ho, Wo), dtype=torch.float32, device=dev)
-    gmask = torch.empty((shp.B, N, Ho, Wo), dtype=torch.float32, device=dev)
     gw = torch.empty(weight.shape, dtype=torch.float32, device=dev)
     gb = torch.empty((shp.O,), dtype=torch.float32, device=dev) if has_bias else None
-    with torch.cuda.device(dev):
-        stream = torch.cuda.current_stream(dev)
-        need = lib.dcn_workspace_bytes(ctypes.byref(shp), PHASE_BACKWARD)
-        if ws is None:
-            ws = _workspace(dev, stream.cuda_stream, need)
-        rc = lib.dcn_backward_modulated(ctypes.byref(shp), _ptr(x), _ptr(offset), _ptr(mask), _ptr(weight),
-                                        _ptr(grad_out), _ptr(gx), _ptr(goff), _ptr(gmask), _ptr(gw), _ptr(gb),
-                                        _ptr(ws), ws.numel(), ctypes.c_void_p(stream.cuda_stream))
-    _lib.check(rc, "dcn_backward_modulated")
+    if mask is None:
+        gmask = None
+        _run("dcn_backward", dev, shp, (x, offset, weight, grad_out, gx, goff, gw, gb), PHASE_BACKWARD, ws)
+    else:
+        gmask = torch.empty((shp.B, N, Ho, Wo), dtype=torch.float32, device=dev)
+        _run("dcn_backward_modulated", dev, shp, (x, offset, mask, weight, grad_out, gx, goff, gmask, gw, gb),
+             PHASE_BACKWARD, ws)
     return gx, goff, gmask, gw, gb
 
 
 # ---- whole layer: companion offset conv + DCN span on the engine (SURVEY 8f.1) -----------------------------------
+# The modulated layer (mmcv's ModulatedDeformConv2dPack) shares every body below: its conv has 3N outputs (offsets,
+# then one mask logit per tap, the mask being their sigmoid), DCNv1 sampling, and phases of its own.
+_PHASES = {False: (PHASE_LAYER_FORWARD, PHASE_LAYER_BACKWARD),
+           True: (PHASE_LAYER_FORWARD_MODULATED, PHASE_LAYER_BACKWARD_MODULATED)}
+
+
 def layer_supported(x_shape, out_channels, kernel_size=3, stride=1, padding=1, variant=VARIANT_TORCH,
                     operand=OPERAND_FP32, flags=0):
     """True when dcn_layer_forward / dcn_layer_backward cover the shape (both phases on the tensor path)."""
-    B, C, H, W = (int(v) for v in x_shape)
-    shp = _lib.make_shape(B, C, int(out_channels), H, W, kernel_size, stride, padding, variant, operand, flags)
-    return all(_lib.path_name(shp, ph) == "umma" for ph in (PHASE_LAYER_FORWARD, PHASE_LAYER_BACKWARD))
+    return _layer_supported(x_shape, out_channels, kernel_size, stride, padding, variant, operand, flags, False)
 
 
 def layer_workspace(x, weight, kernel_size=3, stride=1, padding=1, variant=VARIANT_TORCH, flags=0):
     """One scratch buffer big enough for dcn_layer_forward AND dcn_layer_backward of this layer: handing the same
     buffer to both lets the backward pass reuse the staged copy of x (DCN_FLAG_XT_STAGED)."""
-    lib = _lib.load()
-    shp = _shape_of(x, weight, kernel_size, stride, padding, variant, OPERAND_FP32, flags)
-    need = max(lib.dcn_workspace_bytes(ctypes.byref(shp), PHASE_LAYER_FORWARD),
-               lib.dcn_workspace_bytes(ctypes.byref(shp), PHASE_LAYER_BACKWARD))
-    return torch.empty(need, dtype=torch.uint8, device=x.device)
+    return _layer_workspace(x, weight, kernel_size, stride, padding, variant, flags, False)
 
 
 def dcn_offset_conv_forward(x, offset_weight, offset_bias, out_channels, kernel_size=3, stride=1, padding=1,
@@ -274,48 +242,15 @@ def dcn_offset_conv_forward(x, offset_weight, offset_bias, out_channels, kernel_
     """offset[B,2N,Ho,Wo] = the companion offset convolution on the engine (a plain mode of the tcgen05 forward
     kernel).  `variant` / out_channels describe the DCN layer the offsets are for: the staged copy of x is laid out
     for it, so a following dcn_forward(..., ws=ws, xt_staged=True) reuses it."""
-    lib = _lib.load()
-    B, C, H, W = x.shape
-    if xt_staged and ws is not None:
-        flags |= FLAG_XT_STAGED
-    shp = _lib.make_shape(B, C, int(out_channels), H, W, kernel_size, stride, padding, variant, OPERAND_FP32, flags)
-    Ho, Wo = _lib.output_hw(shp)
-    N = shp.kh * shp.kw
-    x, offset_weight, offset_bias = _dev_ready(x), _dev_ready(offset_weight), _dev_ready(offset_bias)
-    if tuple(offset_weight.shape) != (2 * N, C, shp.kh, shp.kw):
-        raise ValueError(f"offset_weight shape {tuple(offset_weight.shape)} != {(2 * N, C, shp.kh, shp.kw)}")
-    offset = torch.empty((B, 2 * N, Ho, Wo), dtype=torch.float32, device=x.device)
-    with torch.cuda.device(x.device):
-        stream = torch.cuda.current_stream(x.device)
-        need = lib.dcn_workspace_bytes(ctypes.byref(shp), PHASE_LAYER_FORWARD)
-        if ws is None:
-            ws = _workspace(x.device, stream.cuda_stream, need)
-        rc = lib.dcn_offset_conv_forward(ctypes.byref(shp), _ptr(x), _ptr(offset_weight), _ptr(offset_bias), _ptr(offset),
-                                         _ptr(ws), ws.numel(), ctypes.c_void_p(stream.cuda_stream))
-    _lib.check(rc, "dcn_offset_conv_forward")
-    return offset
+    return _offset_conv_forward(x, offset_weight, offset_bias, out_channels, kernel_size, stride, padding, variant,
+                                flags, ws, xt_staged, False)[0]
 
 
 def dcn_layer_forward(x, offset_weight, offset_bias, weight, bias, kernel_size=3, stride=1, padding=1,
                       variant=VARIANT_TORCH, flags=0, ws=None):
     """-> (offset, out): offset conv + DCN forward, x staged once (no autograd)."""
-    lib = _lib.load()
-    shp = _shape_of(x, weight, kernel_size, stride, padding, variant, OPERAND_FP32, flags)
-    Ho, Wo = _lib.output_hw(shp)
-    N = shp.kh * shp.kw
-    x, weight, bias = _dev_ready(x), _dev_ready(weight), _dev_ready(bias)
-    offset_weight, offset_bias = _dev_ready(offset_weight), _dev_ready(offset_bias)
-    offset = torch.empty((shp.B, 2 * N, Ho, Wo), dtype=torch.float32, device=x.device)
-    out = torch.empty((shp.B, shp.O, Ho, Wo), dtype=torch.float32, device=x.device)
-    with torch.cuda.device(x.device):
-        stream = torch.cuda.current_stream(x.device)
-        need = lib.dcn_workspace_bytes(ctypes.byref(shp), PHASE_LAYER_FORWARD)
-        if ws is None:
-            ws = _workspace(x.device, stream.cuda_stream, need)
-        rc = lib.dcn_layer_forward(ctypes.byref(shp), _ptr(x), _ptr(offset_weight), _ptr(offset_bias), _ptr(weight),
-                                   _ptr(bias), _ptr(offset), _ptr(out), _ptr(ws), ws.numel(),
-                                   ctypes.c_void_p(stream.cuda_stream))
-    _lib.check(rc, "dcn_layer_forward")
+    offset, _, out = _layer_forward(x, offset_weight, offset_bias, weight, bias, kernel_size, stride, padding, variant,
+                                    flags, ws, False)
     return offset, out
 
 
@@ -323,149 +258,42 @@ def dcn_layer_backward(x, offset, offset_weight, weight, grad_out, has_offset_bi
                        stride=1, padding=1, variant=VARIANT_TORCH, flags=0, need_grad_x=True, ws=None, xt_staged=False):
     """-> grad_x (or None), grad_offset_weight, grad_offset_bias (or None), grad_weight, grad_bias (or None).
     grad_offset stays inside the workspace; the offset conv's data gradient is accumulated on chip-side buffers."""
-    lib = _lib.load()
-    if not need_grad_x:
-        flags |= FLAG_NO_GRAD_X
-    if xt_staged and ws is not None:
-        flags |= FLAG_XT_STAGED
-    shp = _shape_of(x, weight, kernel_size, stride, padding, variant, OPERAND_FP32, flags)
-    x, weight, grad_out = _dev_ready(x), _dev_ready(weight), _dev_ready(grad_out)
-    offset, offset_weight = _dev_ready(offset), _dev_ready(offset_weight)
-    dev = x.device
-    gx = torch.empty(x.shape, dtype=torch.float32, device=dev) if need_grad_x else None
-    gwoff = torch.empty(offset_weight.shape, dtype=torch.float32, device=dev)
-    gboff = torch.empty((offset_weight.shape[0],), dtype=torch.float32, device=dev) if has_offset_bias else None
-    gw = torch.empty(weight.shape, dtype=torch.float32, device=dev)
-    gb = torch.empty((shp.O,), dtype=torch.float32, device=dev) if has_bias else None
-    with torch.cuda.device(dev):
-        stream = torch.cuda.current_stream(dev)
-        need = lib.dcn_workspace_bytes(ctypes.byref(shp), PHASE_LAYER_BACKWARD)
-        if ws is None:
-            ws = _workspace(dev, stream.cuda_stream, need)
-        rc = lib.dcn_layer_backward(ctypes.byref(shp), _ptr(x), _ptr(offset), _ptr(offset_weight), _ptr(weight),
-                                    _ptr(grad_out), _ptr(gx), _ptr(gwoff), _ptr(gboff), _ptr(gw), _ptr(gb), _ptr(ws),
-                                    ws.numel(), ctypes.c_void_p(stream.cuda_stream))
-    _lib.check(rc, "dcn_layer_backward")
-    return gx, gwoff, gboff, gw, gb
-
-
-class DeformLayerFunction(torch.autograd.Function):
-    """The whole reference module forward (offset conv + sampling + GEMM, deform_conv.py:56-81 / train.py:95-140)
-    and its autograd as ONE node on the engine: x is staged once per step, grad_offset never reaches HBM as a
-    framework tensor, and the two data-gradient terms are summed before the single transposition back to NCHW."""
-
-    @staticmethod
-    def forward(ctx, x, offset_weight, offset_bias, weight, bias, cfg):
-        kernel_size, stride, padding, variant, flags, keep_staged = cfg
-        ctx.ws = layer_workspace(x, weight, kernel_size, stride, padding, variant, flags) if keep_staged else None
-        offset, out = dcn_layer_forward(x, offset_weight, offset_bias, weight, bias, kernel_size, stride, padding,
-                                        variant, flags, ws=ctx.ws)
-        # DCN_FLAG_RELU_OUT: the epilogue applied the ReLU; the backward entry points want the gradient of the
-        # pre-activation sum, i.e. grad_out masked with out > 0
-        ctx.relu = bool(flags & FLAG_RELU_OUT)
-        ctx.save_for_backward(x, offset, offset_weight, weight, *((out,) if ctx.relu else ()))
-        ctx.cfg = cfg
-        ctx.has = (offset_bias is not None, bias is not None)
-        return out
-
-    @staticmethod
-    def backward(ctx, grad_out):
-        x, offset, offset_weight, weight = ctx.saved_tensors[:4]
-        if ctx.relu:
-            grad_out = grad_out * (ctx.saved_tensors[4] > 0)
-        kernel_size, stride, padding, variant, flags, _ = ctx.cfg
-        gx, gwoff, gboff, gw, gb = dcn_layer_backward(
-            x, offset, offset_weight, weight, grad_out, ctx.has[0], ctx.has[1], kernel_size, stride, padding, variant,
-            flags & ~FLAG_ACCUM_GRAD_X, need_grad_x=ctx.needs_input_grad[0], ws=ctx.ws, xt_staged=ctx.ws is not None)
-        ctx.ws = None
-        return gx, gwoff, gboff, gw, gb, None
+    return _layer_backward(x, offset, None, offset_weight, weight, grad_out, has_offset_bias, has_bias, kernel_size,
+                           stride, padding, variant, flags, need_grad_x, ws, xt_staged)
 
 
 def deform_layer(x, offset_weight, offset_bias, weight, bias=None, kernel_size=3, stride=1, padding=1,
                  variant=VARIANT_TORCH, flags=0, keep_staged=False):
     """Differentiable whole layer on the engine (CUDA float32 tensors; check layer_supported() first)."""
-    cfg = (_lib._pair(kernel_size), _lib._pair(stride), _lib._pair(padding), variant, flags, bool(keep_staged))
+    cfg = (_lib._pair(kernel_size), _lib._pair(stride), _lib._pair(padding), variant, flags, bool(keep_staged), False)
     return DeformLayerFunction.apply(x, offset_weight, offset_bias, weight, bias, cfg)
 
 
 # ---- whole modulated layer: mmcv's ModulatedDeformConv2dPack (3N-channel offset-and-mask conv + DCNv2 span) --------
-_MOD_PHASES = (PHASE_LAYER_FORWARD_MODULATED, PHASE_LAYER_BACKWARD_MODULATED)
-
-
 def modulated_layer_supported(x_shape, out_channels, kernel_size, stride, padding, flags=0):
     """True when dcn_layer_forward_modulated / dcn_layer_backward_modulated cover the shape (fp32, tensor path)."""
-    B, C, H, W = (int(v) for v in x_shape)
-    shp = _lib.make_shape(B, C, int(out_channels), H, W, kernel_size, stride, padding, VARIANT_DCNV1, OPERAND_FP32,
-                          flags)
-    return all(_lib.path_name(shp, ph) == "umma" for ph in _MOD_PHASES)
+    return _layer_supported(x_shape, out_channels, kernel_size, stride, padding, VARIANT_DCNV1, OPERAND_FP32, flags,
+                            True)
 
 
 def modulated_layer_workspace(x, weight, kernel_size, stride, padding, flags=0):
     """One scratch buffer for both modulated layer calls: the backward pass reuses the staged copy of x."""
-    lib = _lib.load()
-    shp = _shape_of(x, weight, kernel_size, stride, padding, VARIANT_DCNV1, OPERAND_FP32, flags)
-    need = max(lib.dcn_workspace_bytes(ctypes.byref(shp), ph) for ph in _MOD_PHASES)
-    return torch.empty(need, dtype=torch.uint8, device=x.device)
-
-
-def _check_offset_mask_weight(offset_weight, shp):
-    N = shp.kh * shp.kw
-    if tuple(offset_weight.shape) != (3 * N, shp.C, shp.kh, shp.kw):
-        raise ValueError(f"offset_weight shape {tuple(offset_weight.shape)} != {(3 * N, shp.C, shp.kh, shp.kw)} "
-                         "(3N outputs: offsets, then one mask logit per tap)")
+    return _layer_workspace(x, weight, kernel_size, stride, padding, VARIANT_DCNV1, flags, True)
 
 
 def dcn_offset_conv_forward_modulated(x, offset_weight, offset_bias, out_channels, kernel_size=3, stride=1, padding=1,
                                       flags=0, ws=None, xt_staged=False):
     """-> (offset [B,2N,Ho,Wo], mask [B,N,Ho,Wo]): the modulated layer's 3N-channel conv on the engine, channels
     [0, 2N) as offsets and sigmoid(channels [2N, 3N)) as the mask (no autograd)."""
-    lib = _lib.load()
-    B, C, H, W = x.shape
-    if xt_staged and ws is not None:
-        flags |= FLAG_XT_STAGED
-    shp = _lib.make_shape(B, C, int(out_channels), H, W, kernel_size, stride, padding, VARIANT_DCNV1, OPERAND_FP32,
-                          flags)
-    Ho, Wo = _lib.output_hw(shp)
-    N = shp.kh * shp.kw
-    _check_offset_mask_weight(offset_weight, shp)
-    x, offset_weight, offset_bias = _dev_ready(x), _dev_ready(offset_weight), _dev_ready(offset_bias)
-    offset = torch.empty((B, 2 * N, Ho, Wo), dtype=torch.float32, device=x.device)
-    mask = torch.empty((B, N, Ho, Wo), dtype=torch.float32, device=x.device)
-    with torch.cuda.device(x.device):
-        stream = torch.cuda.current_stream(x.device)
-        need = lib.dcn_workspace_bytes(ctypes.byref(shp), PHASE_LAYER_FORWARD_MODULATED)
-        if ws is None:
-            ws = _workspace(x.device, stream.cuda_stream, need)
-        rc = lib.dcn_offset_conv_forward_modulated(ctypes.byref(shp), _ptr(x), _ptr(offset_weight), _ptr(offset_bias),
-                                                   _ptr(offset), _ptr(mask), _ptr(ws), ws.numel(),
-                                                   ctypes.c_void_p(stream.cuda_stream))
-    _lib.check(rc, "dcn_offset_conv_forward_modulated")
-    return offset, mask
+    return _offset_conv_forward(x, offset_weight, offset_bias, out_channels, kernel_size, stride, padding,
+                                VARIANT_DCNV1, flags, ws, xt_staged, True)
 
 
 def dcn_layer_forward_modulated(x, offset_weight, offset_bias, weight, bias, kernel_size=3, stride=1, padding=1,
                                 flags=0, ws=None):
     """-> (offset, mask, out): offset-and-mask conv + modulated DCN forward, x staged once (no autograd)."""
-    lib = _lib.load()
-    shp = _shape_of(x, weight, kernel_size, stride, padding, VARIANT_DCNV1, OPERAND_FP32, flags)
-    Ho, Wo = _lib.output_hw(shp)
-    N = shp.kh * shp.kw
-    _check_offset_mask_weight(offset_weight, shp)
-    x, weight, bias = _dev_ready(x), _dev_ready(weight), _dev_ready(bias)
-    offset_weight, offset_bias = _dev_ready(offset_weight), _dev_ready(offset_bias)
-    offset = torch.empty((shp.B, 2 * N, Ho, Wo), dtype=torch.float32, device=x.device)
-    mask = torch.empty((shp.B, N, Ho, Wo), dtype=torch.float32, device=x.device)
-    out = torch.empty((shp.B, shp.O, Ho, Wo), dtype=torch.float32, device=x.device)
-    with torch.cuda.device(x.device):
-        stream = torch.cuda.current_stream(x.device)
-        need = lib.dcn_workspace_bytes(ctypes.byref(shp), PHASE_LAYER_FORWARD_MODULATED)
-        if ws is None:
-            ws = _workspace(x.device, stream.cuda_stream, need)
-        rc = lib.dcn_layer_forward_modulated(ctypes.byref(shp), _ptr(x), _ptr(offset_weight), _ptr(offset_bias),
-                                             _ptr(weight), _ptr(bias), _ptr(offset), _ptr(mask), _ptr(out), _ptr(ws),
-                                             ws.numel(), ctypes.c_void_p(stream.cuda_stream))
-    _lib.check(rc, "dcn_layer_forward_modulated")
-    return offset, mask, out
+    return _layer_forward(x, offset_weight, offset_bias, weight, bias, kernel_size, stride, padding, VARIANT_DCNV1,
+                          flags, ws, True)
 
 
 def dcn_layer_backward_modulated(x, offset, mask, offset_weight, weight, grad_out, has_offset_bias=True, has_bias=True,
@@ -473,13 +301,92 @@ def dcn_layer_backward_modulated(x, offset, mask, offset_weight, weight, grad_ou
                                  xt_staged=False):
     """-> grad_x (or None), grad_offset_weight, grad_offset_bias (or None), grad_weight, grad_bias (or None).
     offset / mask: what dcn_layer_forward_modulated returned.  The gradients of offset and mask stay in the workspace."""
+    return _layer_backward(x, offset, mask, offset_weight, weight, grad_out, has_offset_bias, has_bias, kernel_size,
+                           stride, padding, VARIANT_DCNV1, flags, need_grad_x, ws, xt_staged)
+
+
+def modulated_deform_layer(x, offset_weight, offset_bias, weight, bias=None, kernel_size=3, stride=1, padding=1,
+                           flags=0, keep_staged=False):
+    """Differentiable whole modulated layer on the engine (CUDA float32 tensors; check modulated_layer_supported()
+    first).  offset_weight [3N, C, kh, kw]: offsets, then one mask logit per tap (mmcv's conv_offset)."""
+    cfg = (_lib._pair(kernel_size), _lib._pair(stride), _lib._pair(padding), VARIANT_DCNV1, flags & ~FLAG_RELU_OUT,
+           bool(keep_staged), True)
+    return DeformLayerFunction.apply(x, offset_weight, offset_bias, weight, bias, cfg)
+
+
+# the layer bodies: modulated False = dcn_layer_* (2N-channel offset conv), True = dcn_layer_*_modulated
+def _layer_supported(x_shape, out_channels, kernel_size, stride, padding, variant, operand, flags, modulated):
+    B, C, H, W = (int(v) for v in x_shape)
+    shp = _lib.make_shape(B, C, int(out_channels), H, W, kernel_size, stride, padding, variant, operand, flags)
+    return all(_lib.path_name(shp, ph) == "umma" for ph in _PHASES[modulated])
+
+
+def _layer_workspace(x, weight, kernel_size, stride, padding, variant, flags, modulated):
     lib = _lib.load()
+    shp = _shape_of(x, weight, kernel_size, stride, padding, variant, OPERAND_FP32, flags)
+    need = max(lib.dcn_workspace_bytes(ctypes.byref(shp), ph) for ph in _PHASES[modulated])
+    return torch.empty(need, dtype=torch.uint8, device=x.device)
+
+
+def _check_offset_weight(offset_weight, shp, modulated):
+    n = 3 if modulated else 2
+    want = (n * shp.kh * shp.kw, shp.C, shp.kh, shp.kw)
+    if tuple(offset_weight.shape) != want:
+        raise ValueError(f"offset_weight shape {tuple(offset_weight.shape)} != {want}" +
+                         (" (3N outputs: offsets, then one mask logit per tap)" if modulated else ""))
+
+
+def _offset_conv_forward(x, offset_weight, offset_bias, out_channels, kernel_size, stride, padding, variant, flags, ws,
+                         xt_staged, modulated):
+    """-> (offset, mask or None)"""
+    B, C, H, W = x.shape
+    if xt_staged and ws is not None:
+        flags |= FLAG_XT_STAGED
+    shp = _lib.make_shape(B, C, int(out_channels), H, W, kernel_size, stride, padding, variant, OPERAND_FP32, flags)
+    Ho, Wo = _lib.output_hw(shp)
+    N = shp.kh * shp.kw
+    _check_offset_weight(offset_weight, shp, modulated)
+    x, offset_weight, offset_bias = _dev_ready(x), _dev_ready(offset_weight), _dev_ready(offset_bias)
+    offset = torch.empty((B, 2 * N, Ho, Wo), dtype=torch.float32, device=x.device)
+    if not modulated:
+        _run("dcn_offset_conv_forward", x.device, shp, (x, offset_weight, offset_bias, offset), PHASE_LAYER_FORWARD, ws)
+        return offset, None
+    mask = torch.empty((B, N, Ho, Wo), dtype=torch.float32, device=x.device)
+    _run("dcn_offset_conv_forward_modulated", x.device, shp, (x, offset_weight, offset_bias, offset, mask),
+         PHASE_LAYER_FORWARD_MODULATED, ws)
+    return offset, mask
+
+
+def _layer_forward(x, offset_weight, offset_bias, weight, bias, kernel_size, stride, padding, variant, flags, ws,
+                   modulated):
+    """-> (offset, mask or None, out)"""
+    shp = _shape_of(x, weight, kernel_size, stride, padding, variant, OPERAND_FP32, flags)
+    Ho, Wo = _lib.output_hw(shp)
+    N = shp.kh * shp.kw
+    _check_offset_weight(offset_weight, shp, modulated)
+    x, weight, bias = _dev_ready(x), _dev_ready(weight), _dev_ready(bias)
+    offset_weight, offset_bias = _dev_ready(offset_weight), _dev_ready(offset_bias)
+    offset = torch.empty((shp.B, 2 * N, Ho, Wo), dtype=torch.float32, device=x.device)
+    out = torch.empty((shp.B, shp.O, Ho, Wo), dtype=torch.float32, device=x.device)
+    if not modulated:
+        _run("dcn_layer_forward", x.device, shp, (x, offset_weight, offset_bias, weight, bias, offset, out),
+             PHASE_LAYER_FORWARD, ws)
+        return offset, None, out
+    mask = torch.empty((shp.B, N, Ho, Wo), dtype=torch.float32, device=x.device)
+    _run("dcn_layer_forward_modulated", x.device, shp, (x, offset_weight, offset_bias, weight, bias, offset, mask, out),
+         PHASE_LAYER_FORWARD_MODULATED, ws)
+    return offset, mask, out
+
+
+def _layer_backward(x, offset, mask, offset_weight, weight, grad_out, has_offset_bias, has_bias, kernel_size, stride,
+                    padding, variant, flags, need_grad_x, ws, xt_staged):
+    """mask None: dcn_layer_backward, else dcn_layer_backward_modulated"""
     if not need_grad_x:
         flags |= FLAG_NO_GRAD_X
     if xt_staged and ws is not None:
         flags |= FLAG_XT_STAGED
-    shp = _shape_of(x, weight, kernel_size, stride, padding, VARIANT_DCNV1, OPERAND_FP32, flags)
-    _check_offset_mask_weight(offset_weight, shp)
+    shp = _shape_of(x, weight, kernel_size, stride, padding, variant, OPERAND_FP32, flags)
+    _check_offset_weight(offset_weight, shp, mask is not None)
     x, weight, grad_out = _dev_ready(x), _dev_ready(weight), _dev_ready(grad_out)
     offset, mask, offset_weight = _dev_ready(offset), _dev_ready(mask), _dev_ready(offset_weight)
     dev = x.device
@@ -488,59 +395,54 @@ def dcn_layer_backward_modulated(x, offset, mask, offset_weight, weight, grad_ou
     gboff = torch.empty((offset_weight.shape[0],), dtype=torch.float32, device=dev) if has_offset_bias else None
     gw = torch.empty(weight.shape, dtype=torch.float32, device=dev)
     gb = torch.empty((shp.O,), dtype=torch.float32, device=dev) if has_bias else None
-    with torch.cuda.device(dev):
-        stream = torch.cuda.current_stream(dev)
-        need = lib.dcn_workspace_bytes(ctypes.byref(shp), PHASE_LAYER_BACKWARD_MODULATED)
-        if ws is None:
-            ws = _workspace(dev, stream.cuda_stream, need)
-        rc = lib.dcn_layer_backward_modulated(ctypes.byref(shp), _ptr(x), _ptr(offset), _ptr(mask), _ptr(offset_weight),
-                                              _ptr(weight), _ptr(grad_out), _ptr(gx), _ptr(gwoff), _ptr(gboff), _ptr(gw),
-                                              _ptr(gb), _ptr(ws), ws.numel(), ctypes.c_void_p(stream.cuda_stream))
-    _lib.check(rc, "dcn_layer_backward_modulated")
+    if mask is None:
+        _run("dcn_layer_backward", dev, shp, (x, offset, offset_weight, weight, grad_out, gx, gwoff, gboff, gw, gb),
+             PHASE_LAYER_BACKWARD, ws)
+    else:
+        _run("dcn_layer_backward_modulated", dev, shp,
+             (x, offset, mask, offset_weight, weight, grad_out, gx, gwoff, gboff, gw, gb), PHASE_LAYER_BACKWARD_MODULATED,
+             ws)
     return gx, gwoff, gboff, gw, gb
 
 
-class ModulatedDeformLayerFunction(torch.autograd.Function):
-    """mmcv's ModulatedDeformConv2dPack.forward (conv_offset, chunk / cat, sigmoid, modulated_deform_conv2d) and its
-    autograd as ONE node on the engine: x is staged once per step, neither the [B, 3N, Ho, Wo] conv output nor the
-    gradients of offset and mask reach HBM as framework tensors, and both grad_x terms are summed before the single
-    transposition back to NCHW."""
+class DeformLayerFunction(torch.autograd.Function):
+    """The whole reference module forward (offset conv + sampling + GEMM, deform_conv.py:56-81 / train.py:95-140)
+    and its autograd as ONE node on the engine: x is staged once per step, grad_offset never reaches HBM as a
+    framework tensor, and the two data-gradient terms are summed before the single transposition back to NCHW.
+    cfg[-1] (modulated): mmcv's ModulatedDeformConv2dPack.forward (conv_offset, chunk / cat, sigmoid,
+    modulated_deform_conv2d) instead, where neither the [B, 3N, Ho, Wo] conv output nor the gradients of offset and
+    mask reach HBM as framework tensors."""
 
     @staticmethod
     def forward(ctx, x, offset_weight, offset_bias, weight, bias, cfg):
-        kernel_size, stride, padding, flags, keep_staged = cfg
-        ctx.ws = modulated_layer_workspace(x, weight, kernel_size, stride, padding, flags) if keep_staged else None
-        offset, mask, out = dcn_layer_forward_modulated(x, offset_weight, offset_bias, weight, bias, kernel_size, stride,
-                                                        padding, flags, ws=ctx.ws)
-        ctx.save_for_backward(x, offset, mask, offset_weight, weight)
+        kernel_size, stride, padding, variant, flags, keep_staged, modulated = cfg
+        ctx.ws = _layer_workspace(x, weight, kernel_size, stride, padding, variant, flags, modulated) \
+            if keep_staged else None
+        offset, mask, out = _layer_forward(x, offset_weight, offset_bias, weight, bias, kernel_size, stride, padding,
+                                           variant, flags, ctx.ws, modulated)
+        # DCN_FLAG_RELU_OUT: the epilogue applied the ReLU; the backward entry points want the gradient of the
+        # pre-activation sum, i.e. grad_out masked with out > 0
+        ctx.relu = bool(flags & FLAG_RELU_OUT)
+        ctx.save_for_backward(x, offset, mask, offset_weight, weight, *((out,) if ctx.relu else ()))
         ctx.cfg = cfg
         ctx.has = (offset_bias is not None, bias is not None)
         return out
 
     @staticmethod
     def backward(ctx, grad_out):
-        x, offset, mask, offset_weight, weight = ctx.saved_tensors
-        kernel_size, stride, padding, flags, _ = ctx.cfg
-        gx, gwoff, gboff, gw, gb = dcn_layer_backward_modulated(
+        x, offset, mask, offset_weight, weight = ctx.saved_tensors[:5]
+        if ctx.relu:
+            grad_out = grad_out * (ctx.saved_tensors[5] > 0)
+        kernel_size, stride, padding, variant, flags = ctx.cfg[:5]
+        gx, gwoff, gboff, gw, gb = _layer_backward(
             x, offset, mask, offset_weight, weight, grad_out, ctx.has[0], ctx.has[1], kernel_size, stride, padding,
-            flags & ~(FLAG_ACCUM_GRAD_X | FLAG_RELU_OUT), need_grad_x=ctx.needs_input_grad[0], ws=ctx.ws,
-            xt_staged=ctx.ws is not None)
+            variant, flags & ~FLAG_ACCUM_GRAD_X, ctx.needs_input_grad[0], ctx.ws, ctx.ws is not None)
         ctx.ws = None
         return gx, gwoff, gboff, gw, gb, None
 
 
-def modulated_deform_layer(x, offset_weight, offset_bias, weight, bias=None, kernel_size=3, stride=1, padding=1,
-                           flags=0, keep_staged=False):
-    """Differentiable whole modulated layer on the engine (CUDA float32 tensors; check modulated_layer_supported()
-    first).  offset_weight [3N, C, kh, kw]: offsets, then one mask logit per tap (mmcv's conv_offset)."""
-    cfg = (_lib._pair(kernel_size), _lib._pair(stride), _lib._pair(padding), flags & ~FLAG_RELU_OUT,
-           bool(keep_staged))
-    return ModulatedDeformLayerFunction.apply(x, offset_weight, offset_bias, weight, bias, cfg)
-
-
 def dcn_corners(offset, in_hw, kernel_size=3, stride=1, padding=1, variant=VARIANT_TORCH):
     """Sampling geometry only: y0, x0 [B,N,Ho,Wo] int32 and w4 [B,N,Ho,Wo,4] float32."""
-    lib = _lib.load()
     B = offset.shape[0]
     shp = _lib.make_shape(B, 1, 1, in_hw[0], in_hw[1], kernel_size, stride, padding, variant)
     Ho, Wo = _lib.output_hw(shp)
@@ -550,51 +452,46 @@ def dcn_corners(offset, in_hw, kernel_size=3, stride=1, padding=1, variant=VARIA
     y0 = torch.empty((B, N, Ho, Wo), dtype=torch.int32, device=dev)
     x0 = torch.empty_like(y0)
     w4 = torch.empty((B, N, Ho, Wo, 4), dtype=torch.float32, device=dev)
-    with torch.cuda.device(dev):
-        stream = torch.cuda.current_stream(dev)
-        rc = lib.dcn_debug_corners(ctypes.byref(shp), _ptr(offset), _ptr(y0), _ptr(x0), _ptr(w4),
-                                   ctypes.c_void_p(stream.cuda_stream))
-    _lib.check(rc, "dcn_debug_corners")
+    _run("dcn_debug_corners", dev, shp, (offset, y0, x0, w4))
     return y0, x0, w4
 
 
 class DeformConvFunction(torch.autograd.Function):
     """autograd node standing where the reference has grid_sample + matmul + their autograd
-    (train.py:102-140 forward, train.py:249 backward)."""
+    (train.py:102-140 forward, train.py:249 backward).  With a mask (the last input): the modulated DCNv1 operator
+    (DCNv2), differentiable in the mask as well.  Host tensors are answered on their device."""
 
     @staticmethod
-    def forward(ctx, x, offset, weight, bias, cfg):
-        kernel_size, stride, padding, variant, operand, flags = cfg[:6]
-        keep_staged = len(cfg) > 6 and cfg[6]
+    def forward(ctx, x, offset, weight, bias, cfg, mask=None):
+        kernel_size, stride, padding, variant, operand, flags, keep_staged = cfg
         home = x.device
         dev = _compute_device(x)
-        xd, od, wd = _to_device(x, dev), _to_device(offset, dev), _to_device(weight, dev)
+        xd, od, md, wd = (_to_device(t, dev) for t in (x, offset, mask, weight))
         bd = _to_device(bias, dev)
         act = torch.bfloat16 if operand == OPERAND_BF16 else torch.float32
         ctx.ws = None
         if keep_staged and xd.dtype == act and xd.is_contiguous():
             # private scratch that lives until backward: its head keeps the staged copy of x
             ctx.ws = staged_workspace(xd, wd, kernel_size, stride, padding, variant, operand, flags)
-        out = dcn_forward(xd, od, wd, bd, kernel_size, stride, padding, variant, operand, flags, ws=ctx.ws)
+        out = _span_forward(xd, od, md, wd, bd, kernel_size, stride, padding, variant, operand, flags, ctx.ws)
         ctx.relu = bool(flags & FLAG_RELU_OUT)    # see DeformLayerFunction
-        ctx.save_for_backward(xd, od, wd, *((out,) if ctx.relu else ()))
+        ctx.save_for_backward(xd, od, md, wd, *((out,) if ctx.relu else ()))
         ctx.cfg, ctx.home, ctx.has_bias = cfg, home, bias is not None
-        ctx.dtypes = (x.dtype, offset.dtype, weight.dtype)
+        ctx.dtypes = (x.dtype, offset.dtype, weight.dtype, None if mask is None else mask.dtype)
         return out if home == dev else out.to(home)
 
     @staticmethod
     def backward(ctx, grad_out):
-        xd, od, wd = ctx.saved_tensors[:3]
+        xd, od, md, wd = ctx.saved_tensors[:4]
         kernel_size, stride, padding, variant, operand, flags = ctx.cfg[:6]
         flags &= ~FLAG_ACCUM_GRAD_X     # autograd sums gradient terms itself; the output buffer here is fresh
         dev = xd.device
         grad_out = _to_device(grad_out, dev)
         if ctx.relu:
-            grad_out = grad_out * (ctx.saved_tensors[3] > 0)
-        gx, goff, gw, gb = dcn_backward(xd, od, wd, grad_out, ctx.has_bias,
-                                        kernel_size, stride, padding, variant, operand, flags,
-                                        need_grad_x=ctx.needs_input_grad[0], ws=ctx.ws,
-                                        xt_staged=ctx.ws is not None)
+            grad_out = grad_out * (ctx.saved_tensors[4] > 0)
+        gx, goff, gmask, gw, gb = _span_backward(xd, od, md, wd, grad_out, ctx.has_bias, kernel_size, stride, padding,
+                                                 variant, operand, flags, ctx.needs_input_grad[0], ctx.ws,
+                                                 ctx.ws is not None, None)
         ctx.ws = None
         home = ctx.home
 
@@ -605,7 +502,7 @@ class DeformConvFunction(torch.autograd.Function):
             return t if home == dev else t.to(home)
 
         return (back(gx, ctx.dtypes[0]), back(goff, ctx.dtypes[1]), back(gw, ctx.dtypes[2]),
-                back(gb, torch.float32), None)
+                back(gb, torch.float32), None, back(gmask, ctx.dtypes[3]))
 
 
 def deform_conv2d(x, offset, weight, bias=None, kernel_size=3, stride=1, padding=1,
@@ -618,50 +515,12 @@ def deform_conv2d(x, offset, weight, bias=None, kernel_size=3, stride=1, padding
     return DeformConvFunction.apply(x, offset, weight, bias, cfg)
 
 
-class ModulatedDeformConvFunction(torch.autograd.Function):
-    """autograd node of the modulated DCNv1 operator (DCNv2): differentiable in x, offset, mask, weight and bias.
-    Host tensors are accepted and answered on their device, as DeformConvFunction does."""
-
-    @staticmethod
-    def forward(ctx, x, offset, mask, weight, bias, cfg):
-        kernel_size, stride, padding, operand, flags = cfg
-        home = x.device
-        dev = _compute_device(x)
-        xd, od, md, wd = (_to_device(t, dev) for t in (x, offset, mask, weight))
-        bd = _to_device(bias, dev)
-        out = dcn_forward_modulated(xd, od, md, wd, bd, kernel_size, stride, padding, operand, flags)
-        ctx.save_for_backward(xd, od, md, wd)
-        ctx.cfg, ctx.home, ctx.has_bias = cfg, home, bias is not None
-        ctx.dtypes = (x.dtype, offset.dtype, mask.dtype, weight.dtype)
-        return out if home == dev else out.to(home)
-
-    @staticmethod
-    def backward(ctx, grad_out):
-        xd, od, md, wd = ctx.saved_tensors
-        kernel_size, stride, padding, operand, flags = ctx.cfg
-        flags &= ~(FLAG_ACCUM_GRAD_X | FLAG_RELU_OUT)
-        dev = xd.device
-        grad_out = _to_device(grad_out, dev)
-        gx, goff, gmask, gw, gb = dcn_backward_modulated(xd, od, md, wd, grad_out, ctx.has_bias, kernel_size, stride,
-                                                         padding, operand, flags,
-                                                         need_grad_x=ctx.needs_input_grad[0])
-        home = ctx.home
-
-        def back(t, dtype):
-            if t is None:
-                return None
-            t = t.to(dtype) if t.dtype != dtype else t
-            return t if home == dev else t.to(home)
-
-        return (back(gx, ctx.dtypes[0]), back(goff, ctx.dtypes[1]), back(gmask, ctx.dtypes[2]),
-                back(gw, ctx.dtypes[3]), back(gb, torch.float32), None)
-
-
 def deform_conv2d_modulated(x, offset, mask, weight, bias=None, kernel_size=3, stride=1, padding=1,
                             operand=OPERAND_FP32, flags=0):
     """Differentiable modulated DCNv1 (DCNv2) core: mask [B, kh*kw, Ho, Wo] scales every sample."""
-    cfg = (_lib._pair(kernel_size), _lib._pair(stride), _lib._pair(padding), operand, flags & ~FLAG_RELU_OUT)
-    return ModulatedDeformConvFunction.apply(x, offset, mask, weight, bias, cfg)
+    cfg = (_lib._pair(kernel_size), _lib._pair(stride), _lib._pair(padding), VARIANT_DCNV1, operand,
+           flags & ~FLAG_RELU_OUT, False)
+    return DeformConvFunction.apply(x, offset, weight, bias, cfg, mask)
 
 
 def _out_hw(H, W, kernel_size, stride, padding):
@@ -908,12 +767,8 @@ class DeformLayerFramedFunction(torch.autograd.Function):
         offset_weight, offset_bias = _dev_ready(offset_weight), _dev_ready(offset_bias)
         offset = torch.empty((B, 2 * N, Ho, Wo), dtype=torch.float32, device=dev)
         out = torch.empty((B, shp.O, Ho, Wo), dtype=torch.float32, device=dev)
-        with torch.cuda.device(dev):
-            stream = torch.cuda.current_stream(dev)
-            rc = lib.dcn_layer_forward(ctypes.byref(shp), _ptr(ws), _ptr(offset_weight), _ptr(offset_bias), _ptr(weight),
-                                       _ptr(bias), _ptr(offset), _ptr(out), _ptr(ws), ws.numel(),
-                                       ctypes.c_void_p(stream.cuda_stream))
-        _lib.check(rc, "dcn_layer_forward")
+        _run("dcn_layer_forward", dev, shp, (ws, offset_weight, offset_bias, weight, bias, offset, out),
+             PHASE_LAYER_FORWARD, ws)
         ctx.relu = bool(flags & FLAG_RELU_OUT)
         ctx.save_for_backward(xt, offset, offset_weight, weight, *((out,) if ctx.relu else ()))
         ctx.cfg = cfg
@@ -922,7 +777,6 @@ class DeformLayerFramedFunction(torch.autograd.Function):
 
     @staticmethod
     def backward(ctx, grad_out):
-        lib = _lib.load()
         xt, offset, offset_weight, weight = ctx.saved_tensors[:4]
         if ctx.relu:
             grad_out = grad_out * (ctx.saved_tensors[4] > 0)
@@ -939,12 +793,8 @@ class DeformLayerFramedFunction(torch.autograd.Function):
         gboff = torch.empty((offset_weight.shape[0],), dtype=torch.float32, device=dev) if ctx.has[0] else None
         gw = torch.empty(weight.shape, dtype=torch.float32, device=dev)
         gb = torch.empty((shp.O,), dtype=torch.float32, device=dev) if ctx.has[1] else None
-        with torch.cuda.device(dev):
-            stream = torch.cuda.current_stream(dev)
-            rc = lib.dcn_layer_backward(ctypes.byref(shp), _ptr(ws), _ptr(offset), _ptr(offset_weight), _ptr(weight),
-                                        _ptr(grad_out), _ptr(gxt), _ptr(gwoff), _ptr(gboff), _ptr(gw), _ptr(gb), _ptr(ws),
-                                        ws.numel(), ctypes.c_void_p(stream.cuda_stream))
-        _lib.check(rc, "dcn_layer_backward")
+        _run("dcn_layer_backward", dev, shp, (ws, offset, offset_weight, weight, grad_out, gxt, gwoff, gboff, gw, gb),
+             PHASE_LAYER_BACKWARD, ws)
         return gxt, gwoff, gboff, gw, gb, None
 
 

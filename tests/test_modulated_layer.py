@@ -1,5 +1,6 @@
-"""The whole modulated layer (mmcv's ModulatedDeformConv2dPack) without a GPU: argument checks of the three C calls,
-the shapes the layer path covers, and the module's interface and initialisation."""
+"""The whole modulated layer (mmcv's ModulatedDeformConv2dPack) without a GPU: argument checks of the three C calls
+(and of the three unmodulated layer calls that share their implementation), the shapes the layer path covers, and the
+module's interface and initialisation."""
 import ctypes
 import math
 
@@ -10,6 +11,7 @@ import jittor_dcn_b200 as dcn
 from jittor_dcn_b200 import _lib
 
 FWD, BWD = _lib.PHASE_LAYER_FORWARD_MODULATED, _lib.PHASE_LAYER_BACKWARD_MODULATED
+FLAVOURS = (True, False)   # modulated: dcn_*_modulated; False: dcn_offset_conv_forward / dcn_layer_forward / _backward
 
 
 def _buffers():
@@ -22,26 +24,33 @@ def _shape(variant=dcn.VARIANT_DCNV1, operand=dcn.OPERAND_FP32, flags=0):
     return dcn.make_shape(2, 64, 64, 12, 12, 3, 1, 1, variant, operand, flags)
 
 
-def _calls(lib, s, x=None, offset=None, mask=None, gwoff=None, ws_bytes=1 << 15, ok=None):
-    """(name, rc) of the three calls with every pointer valid except those given."""
+def _calls(lib, s, x=None, offset=None, mask=None, gwoff=None, ws_bytes=1 << 15, ok=None, modulated=True):
+    """(name, rc) of the three calls of one layer flavour with every pointer valid except those given, one call per
+    item, so that dcn_last_error() is that call's."""
     p = lambda v: ok if v is None else v
-    return [
-        ("offset_conv", lib.dcn_offset_conv_forward_modulated(ctypes.byref(s), p(x), ok, None, p(offset), p(mask), ok,
-                                                               ws_bytes, None)),
-        ("forward", lib.dcn_layer_forward_modulated(ctypes.byref(s), p(x), ok, None, ok, None, p(offset), p(mask), ok,
-                                                    ok, ws_bytes, None)),
-        ("backward", lib.dcn_layer_backward_modulated(ctypes.byref(s), p(x), p(offset), p(mask), ok, ok, ok, ok,
-                                                      p(gwoff), None, ok, None, ok, ws_bytes, None)),
-    ]
+    if modulated:
+        yield "offset_conv", lib.dcn_offset_conv_forward_modulated(ctypes.byref(s), p(x), ok, None, p(offset), p(mask),
+                                                                   ok, ws_bytes, None)
+        yield "forward", lib.dcn_layer_forward_modulated(ctypes.byref(s), p(x), ok, None, ok, None, p(offset), p(mask),
+                                                         ok, ok, ws_bytes, None)
+        yield "backward", lib.dcn_layer_backward_modulated(ctypes.byref(s), p(x), p(offset), p(mask), ok, ok, ok, ok,
+                                                           p(gwoff), None, ok, None, ok, ws_bytes, None)
+    else:
+        yield "offset_conv", lib.dcn_offset_conv_forward(ctypes.byref(s), p(x), ok, None, p(offset), ok, ws_bytes, None)
+        yield "forward", lib.dcn_layer_forward(ctypes.byref(s), p(x), ok, None, ok, None, p(offset), ok, ok, ws_bytes,
+                                               None)
+        yield "backward", lib.dcn_layer_backward(ctypes.byref(s), p(x), p(offset), ok, ok, ok, ok, p(gwoff), None, ok,
+                                                 None, ok, ws_bytes, None)
 
 
-@pytest.mark.parametrize("arg", ["x", "offset", "mask"])
-def test_layer_calls_reject_null_and_misaligned_pointers_by_name(arg):
+@pytest.mark.parametrize("modulated, arg", [(True, "x"), (True, "offset"), (True, "mask"), (False, "x"),
+                                             (False, "offset")], ids=["x", "offset", "mask", "plain-x", "plain-offset"])
+def test_layer_calls_reject_null_and_misaligned_pointers_by_name(modulated, arg):
     lib = dcn.load()
     buf, base, ok = _buffers()
     s = _shape()
     for ptr, code, text in ((ctypes.c_void_p(0), -2, f"{arg} is NULL"), (ctypes.c_void_p(base + 4), -3, arg)):
-        for name, rc in _calls(lib, s, ok=ok, **{arg: ptr}):
+        for name, rc in _calls(lib, s, ok=ok, modulated=modulated, **{arg: ptr}):
             assert rc == code, (name, rc)
             assert text.encode() in lib.dcn_last_error(), (name, lib.dcn_last_error())
     del buf
@@ -51,10 +60,11 @@ def test_layer_backward_rejects_a_bad_grad_offset_weight():
     lib = dcn.load()
     buf, base, ok = _buffers()
     s = _shape()
-    rc = dict(_calls(lib, s, ok=ok, gwoff=ctypes.c_void_p(0)))["backward"]
-    assert rc == -2 and b"grad_offset_weight is NULL" in lib.dcn_last_error()
-    rc = dict(_calls(lib, s, ok=ok, gwoff=ctypes.c_void_p(base + 8)))["backward"]
-    assert rc == -3 and b"grad_offset_weight" in lib.dcn_last_error()
+    for modulated in FLAVOURS:
+        rc = dict(_calls(lib, s, ok=ok, gwoff=ctypes.c_void_p(0), modulated=modulated))["backward"]
+        assert rc == -2 and b"grad_offset_weight is NULL" in lib.dcn_last_error(), modulated
+        rc = dict(_calls(lib, s, ok=ok, gwoff=ctypes.c_void_p(base + 8), modulated=modulated))["backward"]
+        assert rc == -3 and b"grad_offset_weight" in lib.dcn_last_error(), modulated
     del buf
 
 
@@ -86,9 +96,10 @@ def test_layer_calls_refuse_a_workspace_that_is_too_small():
     lib = dcn.load()
     buf, base, ok = _buffers()
     s = _shape()
-    for name, rc in _calls(lib, s, ok=ok, ws_bytes=16):
-        assert rc == -4, name
-        assert b"workspace" in lib.dcn_last_error(), name
+    for modulated in FLAVOURS:
+        for name, rc in _calls(lib, s, ok=ok, ws_bytes=16, modulated=modulated):
+            assert rc == -4, (name, modulated)
+            assert b"workspace" in lib.dcn_last_error(), (name, modulated)
     del buf
 
 
@@ -99,6 +110,10 @@ def test_force_simt_and_uncovered_shapes_answer_unsupported():
         assert [_lib.path_name(s, ph) for ph in (FWD, BWD)] == ["unsupported", "unsupported"]
         rc = lib.dcn_layer_forward_modulated(ctypes.byref(s), ok, ok, None, ok, None, ok, ok, ok, ok, 1 << 15, None)
         assert rc == -6 and b"DCN_PHASE_LAYER_FORWARD_MODULATED" in lib.dcn_last_error()
+        assert [_lib.path_name(s, ph) for ph in (_lib.PHASE_LAYER_FORWARD, _lib.PHASE_LAYER_BACKWARD)] == \
+            ["unsupported", "unsupported"]
+        rc = lib.dcn_layer_forward(ctypes.byref(s), ok, ok, None, ok, None, ok, ok, ok, 1 << 15, None)
+        assert rc == -6 and b"DCN_PHASE_LAYER_FORWARD)" in lib.dcn_last_error()
     del buf
 
 
