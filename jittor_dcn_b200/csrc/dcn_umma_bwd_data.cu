@@ -58,10 +58,13 @@ constexpr uint32_t kGImg = 128 * 64 * 2;                 // one bf16 image of a 
 struct __align__(16) ScatEntry {
   uint32_t base;  // BYTE offset (float image) of the top-left corner inside the framed image
   float fx, fy;
-  int gidx;       // index of the grad_offset element that receives g_iy (the channel moving the row);
-                  // g_ix goes ix_delta further (Params).  < 0: dead entry (padding column / row of
-                  // no instance / no corner inside the image): nothing to scatter, sample 0
+  uint32_t gidx;  // index of the grad_offset element that receives g_iy (the channel moving the row);
+                  // g_ix goes ix_delta further (Params).  kDeadEntry: dead entry (padding column / row of
+                  // no instance / no corner inside the image): nothing to scatter, sample 0.
+                  // Unsigned: grad_offset has B * 2N * HW elements, up to 2^32 - 2 under make_geo's bound
+                  // B * N * HW < 2^31, so a live index is at most 2^32 - 3 and never meets the sentinel
 };
+constexpr uint32_t kDeadEntry = 0xffffffffu;
 
 struct Params {
   Geo g;
@@ -125,7 +128,8 @@ __device__ __forceinline__ RowInfo decode(const Params& P, int inst) {
 
 struct PlanWork {
   float ox, oy;
-  int h, w, n, chan_base, gidx, valid;
+  int h, w, n, chan_base, valid;
+  uint32_t gidx;  // ScatEntry::gidx
   float mk;  // MOD: the mask value, loaded on the same prefetch as the offsets
 };
 
@@ -136,7 +140,7 @@ __device__ __forceinline__ void plan_prepare(const Params& P, int tile, int cb, 
   pw.valid = 0;
   pw.ox = pw.oy = 0.f;
   pw.h = pw.w = pw.n = pw.chan_base = 0;
-  pw.gidx = -1;
+  pw.gidx = kDeadEntry;
   uint32_t p, n, h, w;
   int b;
   if (VARIANT == DCN_VARIANT_TORCH) {
@@ -163,7 +167,10 @@ __device__ __forceinline__ void plan_prepare(const Params& P, int tile, int cb, 
   if (PLAIN) {
     pw.gidx = 0;  // live entry; a plain problem has no offsets and no coordinate gradient
   } else {
-    pw.gidx = (b * 2 * g.N + off_row_ch(g, (int)n)) * g.HW + (int)p;  // target of g_iy
+    // target of g_iy, formed in 64 bits: it passes 2^31 in the tail of a large batch
+    const size_t gi = ((size_t)b * 2 * g.N + off_row_ch(g, (int)n)) * g.HW + p;
+    DCN_DEV_ASSERT(gi < (size_t)g.B * 2 * g.N * g.HW);
+    pw.gidx = (uint32_t)gi;
     const float* ob = P.off + (size_t)b * 2 * g.N * g.HW;
     pw.ox = __ldg(ob + (size_t)off_row_ch(g, (int)n) * g.HW + p);
     pw.oy = __ldg(ob + (size_t)off_col_ch(g, (int)n) * g.HW + p);
@@ -181,7 +188,7 @@ __device__ __forceinline__ ScatEntry plan_finish_plain(const Geo& g, const PlanW
   ScatEntry e;
   int base = xt_null_base(g);
   e.fx = e.fy = 0.f;
-  e.gidx = -1;
+  e.gidx = kDeadEntry;
   if (pw.valid) {
     bool inside;
     base = plain_base(g, pw.h, pw.w, pw.n, inside);
@@ -195,7 +202,7 @@ __device__ __forceinline__ ScatEntry plan_finish(const Geo& g, const PlanWork& p
   ScatEntry e;
   int base = xt_null_base(g);
   e.fx = e.fy = 0.f;
-  e.gidx = -1;
+  e.gidx = kDeadEntry;
   if (pw.valid) {
     const Tap tp = tap_of(g, pw.h, pw.w, pw.n, pw.ox, pw.oy);
     bool inside;
@@ -391,8 +398,8 @@ __global__ void __launch_bounds__(threads_of(PW), 1) bwd_data_kernel(const __gri
           part_m[0] += __shfl_xor_sync(grp_mask, part_m[0], 1);
           if ((gl & 1) == 0 && (RW == 16 || lane < 16)) {
             const int col = cc + ((gl >> 1) & 7);
-            DCN_DEV_ASSERT(pl[col].gidx < 0 || (size_t)(mrow + col) < (size_t)g.B * g.N * g.HW);
-            if (pl[col].gidx >= 0 && part_m[0] != 0.f) atomicAdd(gmask + mrow + col, part_m[0]);
+            DCN_DEV_ASSERT(pl[col].gidx == kDeadEntry || (size_t)(mrow + col) < (size_t)g.B * g.N * g.HW);
+            if (pl[col].gidx != kDeadEntry && part_m[0] != 0.f) atomicAdd(gmask + mrow + col, part_m[0]);
           }
         };
         // one pass = 8 * NB columns whose accumulator values are already in registers
@@ -416,7 +423,7 @@ __global__ void __launch_bounds__(threads_of(PW), 1) bwd_data_kernel(const __gri
             const char* xp = ximg + (e4.x >> XS);
             const float v0 = (float)__ldg(reinterpret_cast<const XT*>(xp));
             if (PLAIN) {
-              if (gimg && (int)e4.w >= 0) atomicAdd(reinterpret_cast<float*>(gimg + e4.x), gs);
+              if (gimg && e4.w != kDeadEntry) atomicAdd(reinterpret_cast<float*>(gimg + e4.x), gs);
               part_g[8 * nb + u] = part_g[8 * NB + 8 * nb + u] = 0.f;
               if (FUSE) smp8[u] = v0;   // dead entries read the all-zero frame-only block
               continue;
@@ -428,7 +435,7 @@ __global__ void __launch_bounds__(threads_of(PW), 1) bwd_data_kernel(const __gri
             const float ex = __fsub_rn(1.0f, fx), sy = __fsub_rn(1.0f, fy);
             const float w0 = __fmul_rn(sy, ex), w1 = __fmul_rn(sy, fx), w2 = __fmul_rn(fy, ex),
                         w3 = __fmul_rn(fy, fx);
-            if (gimg && (int)e4.w >= 0) {
+            if (gimg && e4.w != kDeadEntry) {
               // coalesced red.global.add.f32 x4; a corner outside the image lands on the frame
               char* gp = gimg + e4.x;
               atomicAdd(reinterpret_cast<float*>(gp), gs * w0);
@@ -479,9 +486,10 @@ __global__ void __launch_bounds__(threads_of(PW), 1) bwd_data_kernel(const __gri
           }
           if (WIDE || (gl < 16 && (RW == 16 || lane < 16))) {
             const int vi = WIDE ? lane : (gl & 15), col = vi & (8 * NB - 1);
-            const int gidx = pl[cc + col].gidx;
+            const uint32_t gidx = pl[cc + col].gidx;
+            DCN_DEV_ASSERT(gidx == kDeadEntry || (size_t)gidx + (size_t)P.ix_delta < (size_t)g.B * 2 * g.N * g.HW);
             // lower half of the values: g_ix -> the column-moving offset channel; upper half: g_iy -> the row-moving one
-            if (gidx >= 0 && part_g[0] != 0.f)
+            if (gidx != kDeadEntry && part_g[0] != 0.f)
               atomicAdd(P.goff + (size_t)gidx + (vi < 8 * NB ? (size_t)P.ix_delta : 0),
                         part_g[0] * (vi < 8 * NB ? P.scale_ix : P.scale_iy));
           }
@@ -528,7 +536,7 @@ __global__ void __launch_bounds__(threads_of(PW), 1) bwd_data_kernel(const __gri
               } else {
                 v0 = __ldg(reinterpret_cast<const float2*>(xp));
               }
-              if (gpair && (int)e4.w >= 0) atomicAdd(reinterpret_cast<float2*>(gpair + e4.x), make_float2(ga[u], gb[u]));
+              if (gpair && e4.w != kDeadEntry) atomicAdd(reinterpret_cast<float2*>(gpair + e4.x), make_float2(ga[u], gb[u]));
               part_g[u] = part_g[4 + u] = 0.f;
               if (FUSE) {
                 sa[u] = v0.x;   // dead entries read the all-zero frame-only block
@@ -566,7 +574,7 @@ __global__ void __launch_bounds__(threads_of(PW), 1) bwd_data_kernel(const __gri
                 sb2[u] = mkv * bilb;
               }
             }
-            if (gpair && (int)e4.w >= 0) {
+            if (gpair && e4.w != kDeadEntry) {
               char* gp = gpair + e4.x;
               atomicAdd(reinterpret_cast<float2*>(gp), make_float2(ga[u] * w0, gb[u] * w0));
               atomicAdd(reinterpret_cast<float2*>(gp + dg1), make_float2(ga[u] * w1, gb[u] * w1));
@@ -615,9 +623,9 @@ __global__ void __launch_bounds__(threads_of(PW), 1) bwd_data_kernel(const __gri
           if (lane < 16) {
             // value index: lane bit 3 -> component (0 g_ix, 1 g_iy), bits 2..1 -> column inside the thread's four
             const int vi = (lane >> 1) & 7, col = cu0 + (vi & 3);
-            const int gidx = pl[col].gidx;
-            DCN_DEV_ASSERT(gidx < 0 || (size_t)gidx + (size_t)P.ix_delta < (size_t)g.B * 2 * g.N * g.HW);
-            if (gidx >= 0 && part_g[0] != 0.f)
+            const uint32_t gidx = pl[col].gidx;
+            DCN_DEV_ASSERT(gidx == kDeadEntry || (size_t)gidx + (size_t)P.ix_delta < (size_t)g.B * 2 * g.N * g.HW);
+            if (gidx != kDeadEntry && part_g[0] != 0.f)
               atomicAdd(P.goff + (size_t)gidx + (vi < 4 ? (size_t)P.ix_delta : 0),
                         part_g[0] * (vi < 4 ? P.scale_ix : P.scale_iy));
           }
@@ -639,8 +647,8 @@ __global__ void __launch_bounds__(threads_of(PW), 1) bwd_data_kernel(const __gri
             if (lane < 16 && (lane & 2) == 0) {
               // lane bits 3..2 -> column inside the thread's four
               const int col = cu0 + ((lane >> 2) & 3);
-              DCN_DEV_ASSERT(pl[col].gidx < 0 || (size_t)(mrow + col) < (size_t)g.B * g.N * g.HW);
-              if (pl[col].gidx >= 0 && part_m[0] != 0.f) atomicAdd(gmask + mrow + col, part_m[0]);
+              DCN_DEV_ASSERT(pl[col].gidx == kDeadEntry || (size_t)(mrow + col) < (size_t)g.B * g.N * g.HW);
+              if (pl[col].gidx != kDeadEntry && part_m[0] != 0.f) atomicAdd(gmask + mrow + col, part_m[0]);
             }
           }
         };
@@ -1196,7 +1204,9 @@ static bool bwd_data_tiling(const Geo& g, int operand, bd::Params* P) {
   P->gw = nullptr;
   P->nslices = P->nchunks = 1;
   P->cb_per_slice = 0;
-  if ((long long)g.B * 2 * g.N * g.HW > 0x7fffffffLL) return false;
+  // ScatEntry::gidx is an unsigned 32-bit grad_offset index with 0xffffffff reserved (make_geo's B*N*HW < 2^31 keeps
+  // every shape inside this bound; the check states the limit where the index is formed)
+  if ((long long)g.B * 2 * g.N * g.HW > 0xffffffffLL) return false;
   if ((long long)xt_image_stride(g) >= (1LL << 30)) return false;  // 32-bit byte offsets inside an image
   P->OB = (g.O + 63) / 64;
   if (P->OB > 4) return false;
