@@ -736,13 +736,6 @@ __global__ void __launch_bounds__(256) conv_weight_tiles_kernel(Params P, int dg
 }  // namespace cv
 
 // ---------------------------------------------------------------------------- host side
-static int conv_sms() {
-  int dev = 0, sms = 148;
-  cudaGetDevice(&dev);
-  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-  return sms;
-}
-
 static uint32_t conv_pow2_cols(int cols) {
   uint32_t c = 32;
   while ((int)c < cols) c <<= 1;
@@ -838,13 +831,13 @@ static bool conv_params(const Geo& g, int mode, cv::Params* Pp, int O) {
   const size_t all_w = (size_t)(mode == cv::MODE_DGRAD ? P.nchunks_n : P.nslab) * P.kh * P.kw * 2 * P.w_tile;
   P.w_res = 0;
   P.w_res_bytes = 0;
-  if (mode != cv::MODE_WGRAD && fixed + all_w + 2 * img_bytes <= 227 * 1024) {
+  if (mode != cv::MODE_WGRAD && fixed + all_w + 2 * img_bytes <= kSmemBudget) {
     P.w_res = 1;
     P.w_res_bytes = (uint32_t)all_w;
   }
   const bool wstream = mode != cv::MODE_WGRAD && !P.w_res;
   P.stage_bytes = (uint32_t)align_up(img_bytes + (wstream ? (size_t)P.kw * 2 * P.w_tile : 0), 1024);
-  int stages = (int)((227 * 1024 - fixed - P.w_res_bytes) / P.stage_bytes);
+  int stages = (int)((kSmemBudget - fixed - P.w_res_bytes) / P.stage_bytes);
   if (stages > cv::kMaxStages) stages = cv::kMaxStages;
   if (stages < 2) return false;
   P.stages = stages;
@@ -943,7 +936,7 @@ int conv_offset_forward(const Geo& g, const float* xt, const float* woff, const 
   P.bias = boff;
   P.out = offset_out;
   P.wtiles = wtiles;
-  const int sms = conv_sms();
+  const int sms = num_sms();
   if (mask_out)
     return conv_launch<cv::MODE_FWD, true>(P, P.num_tiles < sms ? P.num_tiles : sms, st, "conv_offset_mask_fwd_kernel",
                                            mask_out);
@@ -958,7 +951,7 @@ int conv_offset_backward(const Geo& g, int O, const float* xt, float* gxt, const
   int rc;
   if (!conv_bwd_shifted(g, O) && g.C < 64 && conv_small_supported(g, O))
     return conv_small_backward(g, O, xt, gxt, goff, woff, gwoff, wtiles, st);
-  const int sms = conv_sms();
+  const int sms = num_sms();
   if (gxt) {
     if (!conv_params(g, cv::MODE_DGRAD, &P, O)) {
       set_error("offset conv backward (shifted-view kernel): shape not supported");

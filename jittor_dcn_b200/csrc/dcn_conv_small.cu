@@ -436,13 +436,6 @@ static bool small_params(const Geo& g, cs::Params* Pp, int O) {
   return true;
 }
 
-static int small_sms() {
-  int dev = 0, sms = 148;
-  cudaGetDevice(&dev);
-  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-  return sms;
-}
-
 bool conv_small_supported(const Geo& g, int O) {
   cs::Params P;
   return small_params(g, &P, O);
@@ -483,7 +476,7 @@ int conv_small_forward(const Geo& g, int O, const float* xt, const float* woff, 
   P.chunks = (P.HoWo + 31) / 32;
   P.div_chunks = FastDiv::make(P.chunks);
   const long long units = (long long)P.B * P.chunks;
-  const int grid = (int)std::min<long long>((units + 7) / 8, (long long)small_sms() * 8);
+  const int grid = (int)std::min<long long>((units + 7) / 8, (long long)num_sms() * 8);
   if (mask_out) {
     KernelScope scope("conv_small_mask_fwd_kernel", st);
     if (NT == 4) cs::fwd_kernel<4, true><<<grid, cs::kThreads, 0, st>>>(P, mask_out);
@@ -513,7 +506,7 @@ int conv_small_backward(const Geo& g, int O, const float* xt, float* gxt, const 
     return DCN_ERR_UNSUPPORTED;
   }
   const int NT = (P.O + 7) / 8;
-  const int sms = small_sms();
+  const int sms = num_sms();
   int rc;
   P.xt = xt;
   P.goff = goff;

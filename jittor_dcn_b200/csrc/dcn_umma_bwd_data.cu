@@ -81,9 +81,13 @@ struct Params {
                          // V = 4 / 8: the forward-kernel order (channel / V, instance, channel % V) for MODE_WGRAD
   float* goff;           // grad_offset accumulators (zeroed)
   float scale_iy, scale_ix;  // chain-rule factors of the coordinate normalisation (1 for DCNv1)
-  int Gt, Rt, chunks, num_inst, num_tiles;  // backward tiling (rows = (instance, channel))
+  // Torch layout: t's row tiling, copied here by copy_row_tiling.  The kernels read it from these fields: their parameter
+  // offsets keep the scatter loop's schedule (read from t, ptxas pairs the constant loads differently and the fused
+  // Torch kernels spill more).
+  int Gt, Rt, chunks, num_inst;
+  int num_tiles;         // row tiles: t.num_tiles (Torch), or B * pix_blocks
   FastDiv divR, divChunks;
-  int pix_blocks;        // Jittor: ceil(HW / ncols) pixel blocks per image
+  int pix_blocks;        // pixel-row layouts: ceil(HW / ncols) pixel blocks per image
   int ix_delta;          // distance, in floats, from a tap's g_iy slot in grad_offset to its g_ix slot
   int ncols;             // TMEM columns per accumulator block: 128 or 64 (Torch: j's; Jittor: pixels)
   int cblocks;           // blocks per tile: Torch ceil(K / ncols) column blocks, Jittor ceil(K / 128) lane blocks
@@ -111,21 +115,6 @@ struct Params {
                          // next block then serialise with its MMAs, but both hide behind the previous scatter pass)
 };
 
-struct RowInfo {
-  int b, r0, chunk, valid;
-};
-__device__ __forceinline__ RowInfo decode(const Params& P, int inst) {
-  RowInfo ri;
-  ri.valid = inst < P.num_inst;
-  uint32_t bc, r0, b, ch;
-  P.divR.divmod((uint32_t)(ri.valid ? inst : 0), bc, r0);
-  P.divChunks.divmod(bc, b, ch);
-  ri.b = (int)b;
-  ri.r0 = (int)r0;
-  ri.chunk = (int)ch;
-  return ri;
-}
-
 struct PlanWork {
   float ox, oy;
   int h, w, n, chan_base, valid;
@@ -145,7 +134,7 @@ __device__ __forceinline__ void plan_prepare(const Params& P, int tile, int cb, 
   int b;
   if (VARIANT == DCN_VARIANT_TORCH) {
     const int il = e >> (P.ncols == 128 ? 7 : 6), cc = e & (P.ncols - 1), j = cb * P.ncols + cc;  // ncols = 64 | 128
-    const RowInfo ri = decode(P, tile * P.Rt + il);
+    const TileRowInfo ri = decode_inst(P, tile * P.Rt + il);
     if (!ri.valid || j >= g.K) return;
     uint32_t cbase, q;
     P.t.divP.divmod((uint32_t)(ri.r0 * g.K + j), cbase, q);
@@ -215,6 +204,23 @@ __device__ __forceinline__ ScatEntry plan_finish(const Geo& g, const PlanWork& p
   }
   e.base = 4u * (uint32_t)(base + pw.chan_base);
   return e;
+}
+
+// Butterfly reduce-scatter of NV values over the lanes that differ in lane bits S, S/2, ... (log2 NV bits): at the
+// step over bit s a lane keeps the half of its values that bit selects and adds the partner's copy of that half.
+// Afterwards v[0] is the sum over those lanes of value index (lane bit S, ..., lane bit 2S/NV) read as a binary number.
+template <int S, int NV>
+__device__ __forceinline__ void reduce_scatter(float (&v)[NV], unsigned mask, int lane) {
+#pragma unroll
+  for (int s = S, n = NV / 2; n >= 1; s >>= 1, n >>= 1) {
+    const bool up = (lane & s) != 0;
+#pragma unroll
+    for (int k = 0; k < n; ++k) {
+      const float send = up ? v[k] : v[k + n];
+      const float keep = up ? v[k + n] : v[k];
+      v[k] = keep + __shfl_xor_sync(mask, send, s);
+    }
+  }
 }
 
 // RW = lanes that share one sampling point (32, or 16 when only 16 channels do)
@@ -347,7 +353,7 @@ __global__ void __launch_bounds__(threads_of(PW), 1) bwd_data_kernel(const __gri
       if (VARIANT == DCN_VARIANT_TORCH) {
         slot = m / P.Gt;
         chan = m - slot * P.Gt;
-        bimg = decode(P, tile * P.Rt + slot).b;
+        bimg = decode_inst(P, tile * P.Rt + slot).b;
       } else {
         bimg = tile / P.pix_blocks;
       }
@@ -373,28 +379,14 @@ __global__ void __launch_bounds__(threads_of(PW), 1) bwd_data_kernel(const __gri
         const ScatEntry* pl = plan + pb * P.plan_cap + slot * ncols;
         const float* mkp = mplan + pb * P.plan_cap + slot * ncols;  // MOD only
         const uint32_t taddr = tmem_base + ((uint32_t)(quarter * 32) << 16) + (uint32_t)(acc * ncols);
-        // WIDE would reduce the coordinate gradient in batches of 16 columns (32 values over 32 lanes cost
-        // the same 31 shuffles as 16 values do).  Measured SLOWER on B200 (cfg2: 13.2 vs 11.7 ms): one
-        // long pass per block exposes more latency than the saved shuffles buy.  Kept for reference.
-        constexpr bool WIDE = false;
-        constexpr int NB = WIDE ? 2 : 1;  // 8-column sub-batches per reduction
-        static_assert(!MOD || !WIDE, "the grad_mask reduction assumes one 8-column batch");
+        // (reducing the coordinate gradient in batches of 16 columns was measured slower: DESIGN.md §5)
         // MOD: one grad_mask RED per column, after an 8-value reduce-scatter over the RW lanes of the sampling points
         auto mask_red = [&](const int cc, float (&part_m)[8]) {
           if (RW == 32) {
 #pragma unroll
             for (int k = 0; k < 8; ++k) part_m[k] += __shfl_xor_sync(0xffffffffu, part_m[k], 16);
           }
-#pragma unroll
-          for (int s = 8, n = 4; s >= 2; s >>= 1, n >>= 1) {
-            const bool up = (lane & s) != 0;
-#pragma unroll
-            for (int k = 0; k < n; ++k) {
-              const float send = up ? part_m[k] : part_m[k + n];
-              const float keep = up ? part_m[k + n] : part_m[k];
-              part_m[k] = keep + __shfl_xor_sync(grp_mask, send, s);
-            }
-          }
+          reduce_scatter<8>(part_m, grp_mask, lane);
           part_m[0] += __shfl_xor_sync(grp_mask, part_m[0], 1);
           if ((gl & 1) == 0 && (RW == 16 || lane < 16)) {
             const int col = cc + ((gl >> 1) & 7);
@@ -402,21 +394,17 @@ __global__ void __launch_bounds__(threads_of(PW), 1) bwd_data_kernel(const __gri
             if (pl[col].gidx != kDeadEntry && part_m[0] != 0.f) atomicAdd(gmask + mrow + col, part_m[0]);
           }
         };
-        // one pass = 8 * NB columns whose accumulator values are already in registers
-        auto pass = [&](const int cc, const uint32_t* rawv) {
-          float part_g[16 * NB];  // [0 .. 8*NB) g_ix of the batch's columns, [8*NB .. 16*NB) g_iy
-          float part_m[8];        // MOD: gA * sample of the batch's columns
-#pragma unroll
-          for (int nb = 0; nb < NB; ++nb) {
-          const int c0 = cc + 8 * nb;
-          const uint32_t* raw = rawv + 8 * nb;
+        // one pass = 8 columns whose accumulator values are already in registers
+        auto pass = [&](const int cc, const uint32_t* raw) {
+          float part_g[16];  // [0 .. 8) g_ix of the batch's columns, [8 .. 16) g_iy
+          float part_m[8];   // MOD: gA * sample of the batch's columns
           float smp8[8];     // fused: the 8 samples of this row
 #pragma unroll
           for (int u = 0; u < 8; ++u) {
             const float ga = __uint_as_float(raw[u]);
-            const float mkv = MOD ? mkp[c0 + u] : 1.f;
+            const float mkv = MOD ? mkp[cc + u] : 1.f;
             const float gs = MOD ? ga * mkv : ga;
-            const uint4 e4 = *reinterpret_cast<const uint4*>(pl + c0 + u);  // {base, fx, fy, gidx}
+            const uint4 e4 = *reinterpret_cast<const uint4*>(pl + cc + u);  // {base, fx, fy, gidx}
             const float fx = __uint_as_float(e4.y), fy = __uint_as_float(e4.z);
             // entry offsets are bytes of the float grad image; the bf16 x image is half as wide
             constexpr int XS = BF ? 1 : 0;
@@ -424,7 +412,7 @@ __global__ void __launch_bounds__(threads_of(PW), 1) bwd_data_kernel(const __gri
             const float v0 = (float)__ldg(reinterpret_cast<const XT*>(xp));
             if (PLAIN) {
               if (gimg && e4.w != kDeadEntry) atomicAdd(reinterpret_cast<float*>(gimg + e4.x), gs);
-              part_g[8 * nb + u] = part_g[8 * NB + 8 * nb + u] = 0.f;
+              part_g[u] = part_g[8 + u] = 0.f;
               if (FUSE) smp8[u] = v0;   // dead entries read the all-zero frame-only block
               continue;
             }
@@ -443,8 +431,8 @@ __global__ void __launch_bounds__(threads_of(PW), 1) bwd_data_kernel(const __gri
               atomicAdd(reinterpret_cast<float*>(gp + dg2), gs * w2);
               atomicAdd(reinterpret_cast<float*>(gp + dg2 + dg1), gs * w3);
             }
-            part_g[8 * nb + u] = gs * ((v1 - v0) * sy + (v3 - v2) * fy);
-            part_g[8 * NB + 8 * nb + u] = gs * ((v2 - v0) * ex + (v3 - v1) * fx);
+            part_g[u] = gs * ((v1 - v0) * sy + (v3 - v2) * fy);
+            part_g[8 + u] = gs * ((v2 - v0) * ex + (v3 - v1) * fx);
             // the sample itself (same blend order as the forward pass)
             if (MOD) {
               const float bil = fmaf(v3, w3, fmaf(v2, w2, fmaf(v1, w1, v0 * w0)));
@@ -455,43 +443,33 @@ __global__ void __launch_bounds__(threads_of(PW), 1) bwd_data_kernel(const __gri
             }
           }
           if (FUSE) {
-            // columns c0..c0+7 of row m: one 16-byte chunk of the MN-major operand, swizzled by m % 8
+            // columns cc..cc+7 of row m: one 16-byte chunk of the MN-major operand, swizzled by m % 8
             uint4 hi, lo;
             split_pair(smp8[0], smp8[1], hi.x, lo.x);
             split_pair(smp8[2], smp8[3], hi.y, lo.y);
             split_pair(smp8[4], smp8[5], hi.z, lo.z);
             split_pair(smp8[6], smp8[7], hi.w, lo.w);
-            const uint32_t so = (uint32_t)((((c0 >> 3) ^ m) & 7) << 4);
+            const uint32_t so = (uint32_t)((((cc >> 3) ^ m) & 7) << 4);
             *reinterpret_cast<uint4*>(s_row + so) = hi;
             if (!BF) *reinterpret_cast<uint4*>(s_row + s_img + so) = lo;
           }
-          }  // sub-batch
           if (PLAIN) return;
           if (MOD) mask_red(cc, part_m);
           // butterfly reduce-scatter over the RW lanes that share the sampling points:
-          // afterwards lane gl (< 16*NB) holds the total of value index gl
-          if (!WIDE && RW == 32) {
+          // afterwards lane gl (< 16) holds the total of value index gl
+          if (RW == 32) {
 #pragma unroll
             for (int k = 0; k < 16; ++k) part_g[k] += __shfl_xor_sync(0xffffffffu, part_g[k], 16);
           }
-#pragma unroll
-          for (int s = 8 * NB, n = 8 * NB; s >= 1; s >>= 1, n >>= 1) {
-            const bool up = (lane & s) != 0;
-#pragma unroll
-            for (int k = 0; k < n; ++k) {
-              const float send = up ? part_g[k] : part_g[k + n];
-              const float keep = up ? part_g[k + n] : part_g[k];
-              part_g[k] = keep + __shfl_xor_sync(grp_mask, send, s);
-            }
-          }
-          if (WIDE || (gl < 16 && (RW == 16 || lane < 16))) {
-            const int vi = WIDE ? lane : (gl & 15), col = vi & (8 * NB - 1);
+          reduce_scatter<8>(part_g, grp_mask, lane);
+          if (gl < 16 && (RW == 16 || lane < 16)) {
+            const int vi = gl & 15, col = vi & 7;
             const uint32_t gidx = pl[cc + col].gidx;
             DCN_DEV_ASSERT(gidx == kDeadEntry || (size_t)gidx + (size_t)P.ix_delta < (size_t)g.B * 2 * g.N * g.HW);
             // lower half of the values: g_ix -> the column-moving offset channel; upper half: g_iy -> the row-moving one
             if (gidx != kDeadEntry && part_g[0] != 0.f)
-              atomicAdd(P.goff + (size_t)gidx + (vi < 8 * NB ? (size_t)P.ix_delta : 0),
-                        part_g[0] * (vi < 8 * NB ? P.scale_ix : P.scale_iy));
+              atomicAdd(P.goff + (size_t)gidx + (vi < 8 ? (size_t)P.ix_delta : 0),
+                        part_g[0] * (vi < 8 ? P.scale_ix : P.scale_iy));
           }
         };
         // PAIR mode (all 32 lanes of the warp share the sampling points): lane pairs (2k, 2k+1) swap half of their
@@ -517,7 +495,7 @@ __global__ void __launch_bounds__(threads_of(PW), 1) bwd_data_kernel(const __gri
           char* gpair = gimg ? gimg - odd * 4 : nullptr;
           float part_g[8];  // [0..3] g_ix of this thread's 4 columns (both channels), [4..7] g_iy
           float sa[4], sb2[4];
-          float part_m[8];  // MOD: [0..3] gA * sample of this thread's 4 columns (both channels)
+          float part_m[4];  // MOD: gA * sample of this thread's 4 columns (both channels)
           float4 mk4 = make_float4(1.f, 1.f, 1.f, 1.f);
           if (MOD) mk4 = *reinterpret_cast<const float4*>(mkp + cu0);
 #pragma unroll
@@ -610,16 +588,7 @@ __global__ void __launch_bounds__(threads_of(PW), 1) bwd_data_kernel(const __gri
           // reduce-scatter of the 8 values over the 16 lanes of equal parity (lane bits 4..1)
 #pragma unroll
           for (int k = 0; k < 8; ++k) part_g[k] += __shfl_xor_sync(0xffffffffu, part_g[k], 16);
-#pragma unroll
-          for (int s2 = 8, n = 4; s2 >= 2; s2 >>= 1, n >>= 1) {
-            const bool up = (lane & s2) != 0;
-#pragma unroll
-            for (int k = 0; k < n; ++k) {
-              const float send = up ? part_g[k] : part_g[k + n];
-              const float keep = up ? part_g[k + n] : part_g[k];
-              part_g[k] = keep + __shfl_xor_sync(0xffffffffu, send, s2);
-            }
-          }
+          reduce_scatter<8>(part_g, 0xffffffffu, lane);
           if (lane < 16) {
             // value index: lane bit 3 -> component (0 g_ix, 1 g_iy), bits 2..1 -> column inside the thread's four
             const int vi = (lane >> 1) & 7, col = cu0 + (vi & 3);
@@ -633,16 +602,7 @@ __global__ void __launch_bounds__(threads_of(PW), 1) bwd_data_kernel(const __gri
             // grad_mask: the 4 values over the 16 lanes of equal parity, then one RED per column
 #pragma unroll
             for (int k = 0; k < 4; ++k) part_m[k] += __shfl_xor_sync(0xffffffffu, part_m[k], 16);
-#pragma unroll
-            for (int s2 = 8, n = 2; s2 >= 4; s2 >>= 1, n >>= 1) {
-              const bool up = (lane & s2) != 0;
-#pragma unroll
-              for (int k = 0; k < n; ++k) {
-                const float send = up ? part_m[k] : part_m[k + n];
-                const float keep = up ? part_m[k + n] : part_m[k];
-                part_m[k] = keep + __shfl_xor_sync(0xffffffffu, send, s2);
-              }
-            }
+            reduce_scatter<8>(part_m, 0xffffffffu, lane);
             part_m[0] += __shfl_xor_sync(0xffffffffu, part_m[0], 2);
             if (lane < 16 && (lane & 2) == 0) {
               // lane bits 3..2 -> column inside the thread's four
@@ -655,21 +615,16 @@ __global__ void __launch_bounds__(threads_of(PW), 1) bwd_data_kernel(const __gri
         constexpr bool PAIR = RW == 32;
         // (fetching both passes' accumulator values up front with one x16 load lets the compiler overlap the
         // second pass's loads with the first pass's shuffles, but measured slower: 11.85 vs 11.36 ms)
-        {
-          for (int cc = part * cols_per_part; cc < (part + 1) * cols_per_part; cc += 8 * NB) {
-            uint32_t raw[8 * NB];
-#pragma unroll
-            for (int nb = 0; nb < NB; ++nb) {
-              asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
-                           : "=r"(raw[8 * nb + 0]), "=r"(raw[8 * nb + 1]), "=r"(raw[8 * nb + 2]), "=r"(raw[8 * nb + 3]),
-                             "=r"(raw[8 * nb + 4]), "=r"(raw[8 * nb + 5]), "=r"(raw[8 * nb + 6]), "=r"(raw[8 * nb + 7])
-                           : "r"(taddr + cc + 8 * nb)
-                           : "memory");
-            }
-            asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-            if (PAIR) pass2(cc, raw);
-            else pass(cc, raw);
-          }
+        for (int cc = part * cols_per_part; cc < (part + 1) * cols_per_part; cc += 8) {
+          uint32_t raw[8];
+          asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
+                       : "=r"(raw[0]), "=r"(raw[1]), "=r"(raw[2]), "=r"(raw[3]), "=r"(raw[4]), "=r"(raw[5]),
+                         "=r"(raw[6]), "=r"(raw[7])
+                       : "r"(taddr + cc)
+                       : "memory");
+          asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+          if constexpr (PAIR) pass2(cc, raw);
+          else pass(cc, raw);
         }
         tc_fence_before();
         if (FUSE) fence_proxy_async_smem();
@@ -1026,7 +981,7 @@ __global__ void __launch_bounds__(256) gout_tiles_torch_kernel(const __grid_cons
   {
     // lanes: 16 instances (one 64-byte run) x 2 channels; the instance of a thread is fixed
     const int r = tid & 15;
-    const RowInfo ri = decode(P, blockIdx.x * kGtInst + r);
+    const TileRowInfo ri = decode_inst(P, blockIdx.x * kGtInst + r);
     const T* src = reinterpret_cast<const T*>(P.gout) + ((size_t)ri.b * g.Oimg + o0) * g.HW + ri.r0 +
                    ((size_t)ri.chunk * Gt + i0) * P.t.R;
     float* dst = gt_buf + r * kGtIS;
@@ -1162,7 +1117,6 @@ __global__ void __launch_bounds__(256) weight_tiles_bwd_kernel(Geo g, int ncols,
 //   real = bytes of one grad_out tile buffer, zero = shared zero images, other = everything but the grad_out
 //   buffers and the Wm^T stages
 static void choose_slices(bd::Params* P, int max_cb, size_t real, size_t zero, size_t other) {
-  const size_t cap = 227 * 1024;
   const int ns_min = (P->cblocks + max_cb - 1) / max_cb;
   double best = 1e30;
   for (int ns = ns_min; ns <= ns_min + 2 && ns <= P->cblocks; ++ns) {
@@ -1183,7 +1137,7 @@ static void choose_slices(bd::Params* P, int max_cb, size_t real, size_t zero, s
   for (const auto& pl : plans) {
     const size_t n_w = pl[1] ? n_res : (size_t)pl[2];
     const size_t need = pl[0] * real + zero + n_w * P->w_stage + other;
-    if (need <= cap || (pl[2] == 1 && need - 768 <= cap)) {
+    if (need <= kSmemBudget || (pl[2] == 1 && need - 768 <= kSmemBudget)) {
       P->g_nbuf = pl[0];
       P->w_resident = pl[1] ? (int)n_res : 0;
       P->w_ring = pl[2];
@@ -1193,11 +1147,24 @@ static void choose_slices(bd::Params* P, int max_cb, size_t real, size_t zero, s
 }
 
 // ---------------------------------------------------------------------------- host side
+static bool copy_row_tiling(const Geo& g, bd::Params* P) {
+  if (!make_tiling(g, &P->t)) return false;
+  P->Gt = P->t.Gt;
+  P->Rt = P->t.Rt;
+  P->chunks = P->t.chunks;
+  P->num_inst = P->t.num_inst;
+  P->num_tiles = P->t.num_tiles;
+  P->divR = P->t.divR;
+  P->divChunks = P->t.divChunks;
+  return true;
+}
+
 static bool bwd_data_tiling(const Geo& g, int operand, bd::Params* P) {
   const size_t nimg = operand == DCN_OPERAND_BF16 ? 1 : 2;
-  if (!make_tiling(g, &P->t)) return false;
+  if (!copy_row_tiling(g, P)) return false;
   P->fuse_w = 0;
   P->o_halves = 1;
+  P->o_cols = 0;
   P->w_resident = 0;
   P->w_ring = 2;
   P->g_nbuf = 1;
@@ -1209,107 +1176,50 @@ static bool bwd_data_tiling(const Geo& g, int operand, bd::Params* P) {
   if ((long long)g.B * 2 * g.N * g.HW > 0xffffffffLL) return false;
   if ((long long)xt_image_stride(g) >= (1LL << 30)) return false;  // 32-bit byte offsets inside an image
   P->OB = (g.O + 63) / 64;
-  if (P->OB > 4) return false;
-  P->Gt = P->Rt = P->chunks = P->num_inst = 1;
-  P->divR = FastDiv::make(1);
-  P->divChunks = FastDiv::make(1);
-  P->pix_blocks = 1;
-  if (g.variant == DCN_VARIANT_TORCH) {
-    const int G = P->t.G;
-    P->Gt = (G % 64 == 0) ? 64 : ((G % 32 == 0) ? 32 : 16);
-    P->Rt = 128 / P->Gt;
-    P->chunks = G / P->Gt;
-    const long long inst = (long long)g.B * P->chunks * P->t.R;
-    if (inst > 0x7fffffffLL) return false;
-    P->num_inst = (int)inst;
-    P->num_tiles = (int)((inst + P->Rt - 1) / P->Rt);
-    P->divR = FastDiv::make(P->t.R);
-    P->divChunks = FastDiv::make(P->chunks);
-    P->g_imgs = P->OB;
-    // fused weight gradient: 64-column blocks, <= 6 blocks of gW accumulators next to the 2 gA buffers
-    if (g.O <= 256) {
-      const int ncols = 64;
-      const int halves = g.O > 128 ? 2 : 1;  // the gW MMAs take 128 channels (two 64-o images) at a time
-      const size_t plan = 2 * (size_t)P->Rt * ncols * sizeof(bd::ScatEntry);
-      const size_t rest = 2 * (size_t)(nimg * ncols * 128) + 2 * nimg * (size_t)(128 * 128) + plan + 256 + 1024;
-      const size_t zero = (size_t)(2 * halves - P->OB) * nimg * bd::kGImg, real = (size_t)P->OB * nimg * bd::kGImg;
-      if (P->Rt * ncols <= bd::plan_max_of(4) && real + zero + rest <= 227 * 1024) {
-        P->fuse_w = 1;
-        P->o_halves = halves;
-        P->g_imgs = 2 * halves;
-        P->ncols = ncols;
-        P->cblocks = (g.K + ncols - 1) / ncols;
-        P->plan_cap = P->Rt * ncols;
-        P->g_img = bd::kGImg;
-        P->w_stage = (uint32_t)nimg * ncols * 128;
-        P->tmem_cols = 512;
-        const int max_cb = 6 / halves;  // 512 TMEM columns - 2 gA buffers, one accumulator set per half
-        choose_slices(P, max_cb, real, zero, rest - 2 * (size_t)P->w_stage);
-        return true;
-      }
-    }
-    // columns per accumulator block: 128 unless the plan ring / operand tiles would not fit
-    for (int ncols : {128, 64}) {
-      const size_t plan = 2 * (size_t)P->Rt * ncols * sizeof(bd::ScatEntry);
-      const size_t real = (size_t)P->OB * nimg * bd::kGImg;
-      const size_t rest = 2 * (size_t)(nimg * ncols * 128) + plan + 256 + 1024;
-      if (P->Rt * ncols <= bd::plan_max_of(4) && real + rest <= 227 * 1024) {
-        P->g_nbuf = (2 * real + rest <= 227 * 1024) ? 2 : 1;
-        P->ncols = ncols;
-        P->cblocks = (g.K + ncols - 1) / ncols;
-        P->plan_cap = P->Rt * ncols;
-        P->g_img = bd::kGImg;
-        P->w_stage = (uint32_t)nimg * ncols * 128;
-        P->tmem_cols = 2 * ncols;
-        return true;
-      }
-    }
-    return false;
-  }
-  P->g_imgs = P->OB;
-  // Jittor: a lane block of 128 columns must hold whole taps
-  if (!(g.C % 128 == 0 || g.C == 64 || g.C == 32 || g.C == 16)) return false;
-  const int taps = g.C >= 128 ? 1 : 128 / g.C;
-  P->o_cols = 0;
-  // fused weight gradient: 64-pixel tiles, gW^T accumulator blocks of O columns next to the 2 gA buffers
-  if (g.O <= 256) {
-    const int ncols = 64, o_cols = (g.O + 15) / 16 * 16;
-    const size_t plan = 2 * (size_t)taps * ncols * sizeof(bd::ScatEntry);
-    const size_t real = (size_t)P->OB * nimg * (ncols * 128);
-    const size_t rest = 2 * (size_t)(nimg * 128 * 128) + 2 * nimg * (size_t)(128 * 128) + plan + 256 + 1024;
-    int max_cb = (512 - 2 * ncols) / o_cols;
-    if (max_cb > 8) max_cb = 8;
-    if (taps * ncols <= bd::plan_max_of(4) && real + rest <= 227 * 1024 && max_cb >= 1) {
-      P->fuse_w = 1;
-      P->o_cols = o_cols;
-      P->ncols = ncols;
-      P->pix_blocks = (g.HW + ncols - 1) / ncols;
-      P->num_tiles = g.B * P->pix_blocks;
-      P->cblocks = (g.K + 127) / 128;
-      P->plan_cap = taps * ncols;
-      P->g_img = (uint32_t)ncols * 128;
-      P->w_stage = (uint32_t)nimg * 128 * 128;
-      P->tmem_cols = 512;
-      choose_slices(P, max_cb, real, 0, rest - 2 * (size_t)P->w_stage);
+  if (P->OB > 4) return false;  // so O <= 256, and the fused weight gradient is always a candidate
+  const bool torch = g.variant == DCN_VARIANT_TORCH;
+  // pixel-row layouts: a lane block of 128 columns must hold whole taps
+  if (!torch && !(g.C % 128 == 0 || g.C == 64 || g.C == 32 || g.C == 16)) return false;
+  // What the layouts differ in.  Plan entries per block column: Torch the Rt class instances of a tile, pixel-row
+  // the taps of a lane block.  Fused weight gradient: Torch one gW accumulator set per 128-channel half of the o axis
+  // (the gW MMAs take two 64-o images at a time, zero images complete the second one), <= 6 blocks next to the
+  // 2 gA buffers; pixel-row gW^T accumulator blocks of O columns rounded up to 16, <= 8 of them.
+  const int ent = torch ? P->t.Rt : (g.C >= 128 ? 1 : 128 / g.C);
+  const int halves = g.O > 128 ? 2 : 1;
+  const int o_cols = (g.O + 15) / 16 * 16;
+  const int max_cb = torch ? 6 / halves : min((512 - 2 * 64) / o_cols, 8);
+  const size_t zero = torch ? (size_t)(2 * halves - P->OB) * nimg * bd::kGImg : 0;
+  // candidates in order of preference: fused (64 columns), then unfused with 128 or 64 columns per accumulator block
+  // (Torch: columns j; pixel-row: pixels)
+  const struct { bool fuse; int ncols; } cands[3] = {{true, 64}, {false, 128}, {false, 64}};
+  for (const auto& c : cands) {
+    const int ncols = c.ncols;
+    const int w_rows = torch ? ncols : 128;  // Wm^T rows of a block: its columns j, or a lane block
+    const uint32_t g_img = torch ? bd::kGImg : (uint32_t)ncols * 128;  // grad_out image: 128 tile rows or ncols pixels
+    const uint32_t w_stage = (uint32_t)nimg * w_rows * 128;
+    const size_t real = (size_t)P->OB * nimg * g_img, z = c.fuse ? zero : 0;
+    // Wm^T ring, sample operand (fused), plan ring, barriers, alignment slack
+    const size_t rest = 2 * (size_t)w_stage + (c.fuse ? 2 * nimg * (size_t)(128 * 128) : 0) +
+                        2 * (size_t)ent * ncols * sizeof(bd::ScatEntry) + 256 + 1024;
+    if (ent * ncols > bd::plan_max_of(4) || real + z + rest > kSmemBudget) continue;
+    P->ncols = ncols;
+    P->cblocks = (g.K + w_rows - 1) / w_rows;
+    P->plan_cap = ent * ncols;
+    P->g_img = g_img;
+    P->w_stage = w_stage;
+    P->pix_blocks = torch ? 1 : (g.HW + ncols - 1) / ncols;
+    P->num_tiles = torch ? P->t.num_tiles : g.B * P->pix_blocks;
+    P->g_imgs = c.fuse && torch ? 2 * halves : P->OB;
+    P->tmem_cols = c.fuse ? 512 : 2 * ncols;
+    if (!c.fuse) {
+      P->g_nbuf = (2 * real + rest <= kSmemBudget) ? 2 : 1;
       return true;
     }
-  }
-  for (int ncols : {128, 64}) {
-    const size_t plan = 2 * (size_t)taps * ncols * sizeof(bd::ScatEntry);
-    const size_t real = (size_t)P->OB * nimg * (ncols * 128);
-    const size_t rest = 2 * (size_t)(nimg * 128 * 128) + plan + 256 + 1024;
-    if (taps * ncols <= bd::plan_max_of(4) && real + rest <= 227 * 1024) {
-      P->g_nbuf = (2 * real + rest <= 227 * 1024) ? 2 : 1;
-      P->ncols = ncols;
-      P->pix_blocks = (g.HW + ncols - 1) / ncols;
-      P->num_tiles = g.B * P->pix_blocks;
-      P->cblocks = (g.K + 127) / 128;
-      P->plan_cap = taps * ncols;
-      P->g_img = (uint32_t)ncols * 128;
-      P->w_stage = (uint32_t)nimg * 128 * 128;
-      P->tmem_cols = 2 * ncols;
-      return true;
-    }
+    P->fuse_w = 1;
+    if (torch) P->o_halves = halves;
+    else P->o_cols = o_cols;
+    choose_slices(P, max_cb, real, z, rest - 2 * (size_t)w_stage);
+    return true;
   }
   return false;
 }
@@ -1335,11 +1245,10 @@ size_t umma_bwd_data_wtile_bytes(const Geo& g, int operand) {
   return align_up((size_t)P.cblocks * P.OB * P.w_stage, 1024);
 }
 
-// the staging pass of the grad_out operand (Torch layout); P needs g, t, Gt, Rt, OB, num_inst, num_tiles,
-// divR, divChunks, gout, row_v
+// the staging pass of the grad_out operand (Torch layout); P needs g, copy_row_tiling, OB, gout, row_v
 static int launch_gout_tiles(const bd::Params& P, bool bf, uint8_t* gtiles, cudaStream_t st) {
-  const dim3 grid((unsigned)(((size_t)P.num_tiles * P.Rt + bd::kGtInst - 1) / bd::kGtInst),
-                  (unsigned)((P.OB * 64 / bd::kGtOsub) * (P.Gt / bd::kGtCh)));
+  const dim3 grid((unsigned)(((size_t)P.num_tiles * P.t.Rt + bd::kGtInst - 1) / bd::kGtInst),
+                  (unsigned)((P.OB * 64 / bd::kGtOsub) * (P.t.Gt / bd::kGtCh)));
   KernelScope scope("gout_tiles_kernel", st);
   if (bf)
     bd::gout_tiles_torch_kernel<__nv_bfloat16><<<grid, 256, 0, st>>>(P, gtiles);
@@ -1379,14 +1288,7 @@ int launch_gout_tiles_fwd_order(const Geo& g, int operand, const void* gout, uin
   bd::Params P;
   memset(&P, 0, sizeof(P));
   P.g = g;
-  if (!make_tiling(g, &P.t)) return DCN_ERR_UNSUPPORTED;
-  P.Gt = P.t.Gt;
-  P.Rt = P.t.Rt;
-  P.chunks = P.t.chunks;
-  P.num_inst = P.t.num_inst;
-  P.num_tiles = P.t.num_tiles;
-  P.divR = P.t.divR;
-  P.divChunks = P.t.divChunks;
+  if (!copy_row_tiling(g, &P)) return DCN_ERR_UNSUPPORTED;
   P.OB = (g.O + 63) / 64;
   P.gout = gout;
   P.row_v = operand == DCN_OPERAND_BF16 ? 8 : 4;
@@ -1400,6 +1302,46 @@ size_t umma_bwd_data_gtile_bytes(const Geo& g, int operand) {
   if (!bwd_data_tiling(g, operand, &P)) return 0;
   if (g.variant != DCN_VARIANT_TORCH) return gtile_pix_bytes(g, operand);
   return align_up((size_t)P.num_tiles * P.OB * (operand == DCN_OPERAND_BF16 ? 1 : 2) * bd::kGImg, 1024);
+}
+
+// what every launch of the data-gradient kernel takes besides its template arguments
+struct BdLaunch {
+  const bd::Params& P;
+  int grid;
+  size_t smem;
+  cudaStream_t st;
+  const float* mask;
+  float* gmask;
+};
+
+// one instantiation: opt in to its shared memory, launch it with its role layout, check the launch
+template <int VARIANT, int RW, bool FUSE, bool BF, int PW, bool PLAIN, bool MOD>
+static int launch_bd(const BdLaunch& L) {
+  DCN_CUDA_TRY(cudaFuncSetAttribute(bd::bwd_data_kernel<VARIANT, RW, FUSE, BF, PW, PLAIN, MOD>,
+                                    cudaFuncAttributeMaxDynamicSharedMemorySize, (int)L.smem));
+  bd::bwd_data_kernel<VARIANT, RW, FUSE, BF, PW, PLAIN, MOD>
+      <<<L.grid, bd::threads_of(PW), L.smem, L.st>>>(L.P, L.mask, L.gmask);
+  DCN_KERNEL_CHECK("umma_bwd_data_kernel");
+  return DCN_OK;
+}
+
+// lanes per sampling point and plan warps.  16 channels per point put 8 class instances / taps in a block column, so
+// such a plan has >= 512 entries; <= 128 entries (2 per plan thread) leave the plan to 2 warps: 20 warps, 96 registers
+// for the scatter loop.  Otherwise 4 plan warps keep up with the scatter.
+template <int VARIANT, bool FUSE, bool BF, bool PLAIN, bool MOD>
+static int launch_bd_split(const BdLaunch& L, bool narrow) {
+  if (narrow) return launch_bd<VARIANT, 16, FUSE, BF, 4, PLAIN, MOD>(L);
+  if (L.P.plan_cap <= 128) return launch_bd<VARIANT, 32, FUSE, BF, 2, PLAIN, MOD>(L);
+  return launch_bd<VARIANT, 32, FUSE, BF, 4, PLAIN, MOD>(L);
+}
+
+template <int VARIANT, bool MOD>
+static int launch_bd_operand(const BdLaunch& L, bool bf, bool narrow) {
+  if (bf)
+    return L.P.fuse_w ? launch_bd_split<VARIANT, true, true, false, MOD>(L, narrow)
+                      : launch_bd_split<VARIANT, false, true, false, MOD>(L, narrow);
+  return L.P.fuse_w ? launch_bd_split<VARIANT, true, false, false, MOD>(L, narrow)
+                    : launch_bd_split<VARIANT, false, false, false, MOD>(L, narrow);
 }
 
 // gxt (channels-last grad_x, may be null), goff and — when the shape fuses the weight gradient
@@ -1456,10 +1398,8 @@ int umma_bwd_data_any(const Geo& g, int operand, const void* xt, float* gxt, con
                 2 * (size_t)P.plan_cap * sizeof(bd::ScatEntry) + 256 + 1024;
   // modulated: the mask values beside the plan ring (float per entry; the kernel traps if the window is too small)
   if (mask) smem += 2 * (size_t)P.plan_cap * sizeof(float);
-  if (smem > 227 * 1024) smem = 227 * 1024;  // tight plan (choose_slices): less alignment slack, checked in the kernel
-  int dev = 0, sms = 148;
-  cudaGetDevice(&dev);
-  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+  if (smem > kSmemBudget) smem = kSmemBudget;  // tight plan (choose_slices): less alignment slack, checked in the kernel
+  const int sms = num_sms();
   int grid = P.num_tiles < sms ? P.num_tiles : sms;
   if (P.fuse_w) {
     P.nchunks = sms / P.nslices;
@@ -1467,102 +1407,28 @@ int umma_bwd_data_any(const Geo& g, int operand, const void* xt, float* gxt, con
     if (P.nchunks > P.num_tiles) P.nchunks = P.num_tiles;
     grid = P.nslices * P.nchunks;
   }
-  const bool narrow = g.variant == DCN_VARIANT_TORCH ? P.Gt == 16 : g.C == 16;  // 16 channels per sampling point
+  const BdLaunch L{P, grid, smem, st, mask, gmask};
+  // 16 channels per sampling point: RW = 16 lanes share one
+  const bool narrow = g.variant == DCN_VARIANT_TORCH ? P.t.Gt == 16 : g.C == 16;
   KernelScope scope(g.plain ? "umma_offset_conv_bwd_kernel" : "umma_bwd_data_kernel", st);
-#define DCN_LAUNCH_BD(V, RW, F, PW)                                                                       \
-  do {                                                                                                    \
-    if (bf) {                                                                                             \
-      DCN_CUDA_TRY(cudaFuncSetAttribute(bd::bwd_data_kernel<V, RW, F, true, PW>,                          \
-                                        cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));         \
-      bd::bwd_data_kernel<V, RW, F, true, PW><<<grid, bd::threads_of(PW), smem, st>>>(P, mask, gmask);              \
-    } else {                                                                                              \
-      DCN_CUDA_TRY(cudaFuncSetAttribute(bd::bwd_data_kernel<V, RW, F, false, PW>,                         \
-                                        cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));         \
-      bd::bwd_data_kernel<V, RW, F, false, PW><<<grid, bd::threads_of(PW), smem, st>>>(P, mask, gmask);             \
-    }                                                                                                     \
-  } while (0)
-  // <= 128 plan entries per block (2 per plan thread): 2 plan warps are enough (20 warps, 96 registers for
-  // the scatter loop); with more sampling points per block the plan would become the bottleneck: 4 warps
-  const bool slim = P.plan_cap <= 128;
   if (g.plain) {
     // regular convolution (the companion offset conv): pixel-row layout, fp32, weight gradient fused
     if (g.variant == DCN_VARIANT_TORCH || bf || !P.fuse_w) {
       set_error("plain (offset-conv) backward: pixel-row layout, fp32 operands, fused weight gradient only");
       return DCN_ERR_UNSUPPORTED;
     }
-#define DCN_LAUNCH_PLAIN(RW, PW)                                                                              \
-  do {                                                                                                        \
-    DCN_CUDA_TRY(cudaFuncSetAttribute(bd::bwd_data_kernel<DCN_VARIANT_JITTOR, RW, true, false, PW, true>,     \
-                                      cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));               \
-    bd::bwd_data_kernel<DCN_VARIANT_JITTOR, RW, true, false, PW, true><<<grid, bd::threads_of(PW), smem, st>>>(P, mask, gmask); \
-  } while (0)
-    if (narrow) {
-      if (slim) DCN_LAUNCH_PLAIN(16, 2);
-      else DCN_LAUNCH_PLAIN(16, 4);
-    } else {
-      if (slim) DCN_LAUNCH_PLAIN(32, 2);
-      else DCN_LAUNCH_PLAIN(32, 4);
-    }
-#undef DCN_LAUNCH_PLAIN
-    DCN_KERNEL_CHECK("umma_bwd_data_kernel");
-    return DCN_OK;
+    return launch_bd_split<DCN_VARIANT_JITTOR, true, false, true, false>(L, narrow);
   }
-#define DCN_LAUNCH_BD2(V, RW, F)                       \
-  do {                                                 \
-    if (slim) DCN_LAUNCH_BD(V, RW, F, 2);              \
-    else DCN_LAUNCH_BD(V, RW, F, 4);                   \
-  } while (0)
   if (mask) {
     // modulated DCNv1: the pixel-row instantiations with MOD
     if (g.variant != DCN_VARIANT_DCNV1 || !gmask) {
       set_error("umma bwd_data: a mask exists for the DCNv1 variant only, and needs grad_mask");
       return DCN_ERR_UNSUPPORTED;
     }
-#define DCN_LAUNCH_MOD(RW, F, PW)                                                                               \
-  do {                                                                                                          \
-    if (bf) {                                                                                                   \
-      DCN_CUDA_TRY(cudaFuncSetAttribute(bd::bwd_data_kernel<DCN_VARIANT_JITTOR, RW, F, true, PW, false, true>,  \
-                                        cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));               \
-      bd::bwd_data_kernel<DCN_VARIANT_JITTOR, RW, F, true, PW, false, true><<<grid, bd::threads_of(PW), smem, st>>>(P, mask, gmask); \
-    } else {                                                                                                    \
-      DCN_CUDA_TRY(cudaFuncSetAttribute(bd::bwd_data_kernel<DCN_VARIANT_JITTOR, RW, F, false, PW, false, true>, \
-                                        cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));               \
-      bd::bwd_data_kernel<DCN_VARIANT_JITTOR, RW, F, false, PW, false, true><<<grid, bd::threads_of(PW), smem, st>>>(P, mask, gmask); \
-    }                                                                                                           \
-  } while (0)
-#define DCN_LAUNCH_MOD2(RW, F)                         \
-  do {                                                 \
-    if (slim) DCN_LAUNCH_MOD(RW, F, 2);                \
-    else DCN_LAUNCH_MOD(RW, F, 4);                     \
-  } while (0)
-    if (P.fuse_w) {
-      if (narrow) DCN_LAUNCH_MOD2(16, true);
-      else DCN_LAUNCH_MOD2(32, true);
-    } else {
-      if (narrow) DCN_LAUNCH_MOD2(16, false);
-      else DCN_LAUNCH_MOD2(32, false);
-    }
-#undef DCN_LAUNCH_MOD2
-#undef DCN_LAUNCH_MOD
-  } else if (g.variant == DCN_VARIANT_TORCH) {
-    if (P.fuse_w) {
-      if (narrow) DCN_LAUNCH_BD(DCN_VARIANT_TORCH, 16, true, 4);
-      else DCN_LAUNCH_BD2(DCN_VARIANT_TORCH, 32, true);
-    } else {
-      if (narrow) DCN_LAUNCH_BD(DCN_VARIANT_TORCH, 16, false, 4);
-      else DCN_LAUNCH_BD2(DCN_VARIANT_TORCH, 32, false);
-    }
-  } else if (P.fuse_w) {
-    if (narrow) DCN_LAUNCH_BD2(DCN_VARIANT_JITTOR, 16, true);
-    else DCN_LAUNCH_BD2(DCN_VARIANT_JITTOR, 32, true);
-  } else {
-    if (narrow) DCN_LAUNCH_BD2(DCN_VARIANT_JITTOR, 16, false);
-    else DCN_LAUNCH_BD2(DCN_VARIANT_JITTOR, 32, false);
+    return launch_bd_operand<DCN_VARIANT_JITTOR, true>(L, bf, narrow);
   }
-#undef DCN_LAUNCH_BD2
-#undef DCN_LAUNCH_BD
-  DCN_KERNEL_CHECK("umma_bwd_data_kernel");
-  return DCN_OK;
+  if (g.variant == DCN_VARIANT_TORCH) return launch_bd_operand<DCN_VARIANT_TORCH, false>(L, bf, narrow);
+  return launch_bd_operand<DCN_VARIANT_JITTOR, false>(L, bf, narrow);
 }
 
 }  // namespace dcn

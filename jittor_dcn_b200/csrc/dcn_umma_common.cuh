@@ -7,6 +7,17 @@
 
 namespace dcn {
 
+// dynamic shared memory one block may opt in to on sm_100
+constexpr size_t kSmemBudget = 227 * 1024;
+
+// SMs of the current device (148 on a B200) for the grids of the persistent kernels
+__host__ inline int num_sms() {
+  int dev = 0, sms = 148;
+  cudaGetDevice(&dev);
+  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+  return sms;
+}
+
 // n / d for 0 <= n < 2^31 by multiply-high (d >= 1), exact.
 struct FastDiv {
   uint32_t d, mul, shr;
@@ -105,7 +116,9 @@ struct TileRowInfo {  // what a Torch-layout tile row needs
   int b, r0, chunk, valid;
 };
 
-__device__ __forceinline__ TileRowInfo decode_inst(const Tiling& t, int inst) {
+// T: Tiling, or a kernel parameter block that carries its num_inst, divR and divChunks
+template <class T>
+__device__ __forceinline__ TileRowInfo decode_inst(const T& t, int inst) {
   TileRowInfo ri;
   ri.valid = inst < t.num_inst;
   uint32_t bc, r0, b, ch;

@@ -34,12 +34,8 @@ namespace dcn {
 
 using namespace ptx;
 
-constexpr int kEpiWarps = 4, kPlanWarps = 4, kProdWarps = 16;
-constexpr int kPlanThreads = kPlanWarps * 32;
-constexpr int kProdThreads = kProdWarps * 32;
-constexpr int kFirstPlanWarp = kEpiWarps + 2, kFirstProdWarp = kFirstPlanWarp + kPlanWarps;
-constexpr int kFwdThreads = (kFirstProdWarp + kProdWarps) * 32;  // 832
-constexpr int kPlanPerThread = 4;                                // kPlanMax / kPlanThreads
+// the plan and gather roles follow the epilogue, MMA and loader warps; their sizes are template arguments
+constexpr int kEpiWarps = 4, kFirstPlanWarp = kEpiWarps + 2;
 constexpr int kPlanMax = 512;                                    // plan entries per K block (32 B each)
 constexpr uint32_t kATile = 128 * 64 * 2;                        // one bf16 A image (16 KB)
 constexpr uint32_t kAMnLbo = 1024, kAMnSbo = 2048;               // MN-major A: atom strides
@@ -217,11 +213,12 @@ __device__ __forceinline__ void split4(const float4& v, uint2& hi, uint2& lo) {
 template <int VARIANT, int MODE, bool BF, bool PLAIN = false, int PW = 4, int GW = 16, bool MOD = false>
 __global__ void __launch_bounds__((kFirstPlanWarp + PW + GW) * 32, 1)
     umma_gemm_kernel(const __grid_constant__ FwdParams P, const __grid_constant__ CUtensorMap tmap_out) {
-  // role layout of this instantiation (shadows the file-scope defaults)
+  // role layout of this instantiation
   constexpr int kPlanWarps = PW, kProdWarps = GW;
   constexpr int kPlanThreads = PW * 32, kProdThreads = GW * 32;
   constexpr int kFirstProdWarp = kFirstPlanWarp + PW;
   constexpr int kFwdThreads = (kFirstProdWarp + GW) * 32;
+  static_assert(kPlanMax % kPlanThreads == 0, "every plan thread owns the same number of plan slots");
   constexpr int kPlanPerThread = kPlanMax / kPlanThreads;
   constexpr int V = BF ? 8 : 4;
   constexpr int NIMG = BF ? 1 : 2;
@@ -938,18 +935,10 @@ static uint32_t pow2_cols(int cols) {
   return c;
 }
 
-static int num_sms() {
-  int dev = 0, sms = 148;
-  cudaGetDevice(&dev);
-  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-  return sms;
-}
-
 static bool tiling_ok(const Geo& g, Tiling* t) {
   if (!make_tiling(g, t)) return false;
   if (g.variant == DCN_VARIANT_TORCH && t->Rt * 64 > kPlanMax) return false;
   if (g.variant != DCN_VARIANT_TORCH && 128 * t->taps_per_kb > kPlanMax) return false;
-  static_assert(kPlanMax == kPlanPerThread * kPlanThreads, "plan slots");
   return true;
 }
 
@@ -1032,82 +1021,58 @@ static void common_params(const Geo& g, FwdParams& P) {
   P.mask = nullptr;
 }
 
+// one instantiation: opt in to its shared memory, launch it with its role layout, check the launch
+template <int VARIANT, int MODE, bool BF, bool PLAIN, int PW, int GW, bool MOD>
+static int launch_umma_gemm(const FwdParams& P, const CUtensorMap& tmap, int grid, size_t smem, cudaStream_t st) {
+  DCN_CUDA_TRY(cudaFuncSetAttribute(umma_gemm_kernel<VARIANT, MODE, BF, PLAIN, PW, GW, MOD>,
+                                    cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  umma_gemm_kernel<VARIANT, MODE, BF, PLAIN, PW, GW, MOD>
+      <<<grid, (kFirstPlanWarp + PW + GW) * 32, smem, st>>>(P, tmap);
+  DCN_KERNEL_CHECK(MODE == MODE_FWD ? "umma_fwd_kernel" : "umma_bwd_weight_kernel");
+  return DCN_OK;
+}
+
+// the plan / gather split: 8 + 8 warps when more than 256 coordinate chains per K block (16 channels per sampling
+// point), else 4 + 16
+template <int VARIANT, int MODE, bool MOD>
+static int launch_umma_gemm_split(bool bf, bool many_chains, const FwdParams& P, const CUtensorMap& tmap, int grid,
+                                  size_t smem, cudaStream_t st) {
+  if (many_chains)
+    return bf ? launch_umma_gemm<VARIANT, MODE, true, false, 8, 8, MOD>(P, tmap, grid, smem, st)
+              : launch_umma_gemm<VARIANT, MODE, false, false, 8, 8, MOD>(P, tmap, grid, smem, st);
+  return bf ? launch_umma_gemm<VARIANT, MODE, true, false, 4, 16, MOD>(P, tmap, grid, smem, st)
+            : launch_umma_gemm<VARIANT, MODE, false, false, 4, 16, MOD>(P, tmap, grid, smem, st);
+}
+
 template <int MODE>
 static int launch_gemm(const Geo& g, int operand, const FwdParams& P, const CUtensorMap& tmap, int grid,
                        size_t smem, cudaStream_t st) {
   if (g.plain) {
-    // regular convolution: pixel-row tiling, fp32 operands only
-    if (g.variant == DCN_VARIANT_TORCH || operand != DCN_OPERAND_FP32) {
-      set_error("plain (offset-conv) problems run in the pixel-row layout with fp32 operands");
-      return DCN_ERR_UNSUPPORTED;
+    // regular convolution: pixel-row tiling, fp32 operands, 4 + 16 warps; forward only (the weight gradient of the
+    // companion offset conv is fused into the data-gradient kernel)
+    if constexpr (MODE == MODE_FWD) {
+      if (g.variant != DCN_VARIANT_TORCH && operand == DCN_OPERAND_FP32)
+        return launch_umma_gemm<DCN_VARIANT_JITTOR, MODE, false, true, 4, 16, false>(P, tmap, grid, smem, st);
     }
-    DCN_CUDA_TRY(cudaFuncSetAttribute(umma_gemm_kernel<DCN_VARIANT_JITTOR, MODE, false, true>,
-                                      cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    umma_gemm_kernel<DCN_VARIANT_JITTOR, MODE, false, true><<<grid, kFwdThreads, smem, st>>>(P, tmap);
-    return DCN_OK;
+    set_error("plain (offset-conv) problems run forward only, in the pixel-row layout with fp32 operands");
+    return DCN_ERR_UNSUPPORTED;
   }
-#define DCN_GEMM_CASE(V, BFV)                                                                              \
-  do {                                                                                                     \
-    DCN_CUDA_TRY(cudaFuncSetAttribute(umma_gemm_kernel<V, MODE, BFV>,                                      \
-                                      cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));            \
-    umma_gemm_kernel<V, MODE, BFV><<<grid, kFwdThreads, smem, st>>>(P, tmap);                              \
-  } while (0)
   const bool bf = operand == DCN_OPERAND_BF16;
+  // more than 256 coordinate chains per K block: Torch layout with Rt = 8, pixel-row layouts with 4 taps per K block
+  // (measured at 256 and 128 chains per block — det3, c3, cfg2 — the 8 + 8 split is 18 - 43 % SLOWER: those are gather-bound)
+  const int n_ent = g.variant == DCN_VARIANT_TORCH ? P.t.Rt * 64 : 128 * P.t.taps_per_kb;
+  const bool many_chains = n_ent > 256;
   if (P.mask) {
     // modulated (DCNv1 only): the pixel-row instantiations with the mask folded into the plan entries
     if (g.variant != DCN_VARIANT_DCNV1) {
       set_error("umma: a mask exists for the DCNv1 variant only");
       return DCN_ERR_UNSUPPORTED;
     }
-    const int n_ent = 128 * P.t.taps_per_kb;
-#define DCN_GEMM_MOD(BFV, PWV, GWV)                                                                         \
-  do {                                                                                                     \
-    DCN_CUDA_TRY(cudaFuncSetAttribute(umma_gemm_kernel<DCN_VARIANT_JITTOR, MODE, BFV, false, PWV, GWV, true>, \
-                                      cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));            \
-    umma_gemm_kernel<DCN_VARIANT_JITTOR, MODE, BFV, false, PWV, GWV, true>                                 \
-        <<<grid, (kFirstPlanWarp + PWV + GWV) * 32, smem, st>>>(P, tmap);                                   \
-  } while (0)
-    if (n_ent > 256) {
-      if (bf) DCN_GEMM_MOD(true, 8, 8);
-      else DCN_GEMM_MOD(false, 8, 8);
-    } else {
-      if (bf) DCN_GEMM_MOD(true, 4, 16);
-      else DCN_GEMM_MOD(false, 4, 16);
-    }
-#undef DCN_GEMM_MOD
-    return DCN_OK;
+    return launch_umma_gemm_split<DCN_VARIANT_JITTOR, MODE, true>(bf, many_chains, P, tmap, grid, smem, st);
   }
-  // more than 256 coordinate chains per K block (16 channels per sampling point: Torch layout with Rt = 8, pixel-row
-  // layouts with 4 taps per K block): 8 plan + 8 gather warps
-  const int n_ent = g.variant == DCN_VARIANT_TORCH ? P.t.Rt * 64 : 128 * P.t.taps_per_kb;
-  // (measured at 256 and 128 chains per block — det3, c3, cfg2 — the 8 + 8 split is 18 - 43 % SLOWER: those are gather-bound)
-  if (n_ent > 256) {
-    constexpr int kThreads88 = (kFirstPlanWarp + 8 + 8) * 32;
-#define DCN_GEMM_CASE88(V, BFV)                                                                            \
-  do {                                                                                                     \
-    DCN_CUDA_TRY(cudaFuncSetAttribute(umma_gemm_kernel<V, MODE, BFV, false, 8, 8>,                         \
-                                      cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));            \
-    umma_gemm_kernel<V, MODE, BFV, false, 8, 8><<<grid, kThreads88, smem, st>>>(P, tmap);                  \
-  } while (0)
-    if (g.variant == DCN_VARIANT_TORCH) {
-      if (bf) DCN_GEMM_CASE88(DCN_VARIANT_TORCH, true);
-      else DCN_GEMM_CASE88(DCN_VARIANT_TORCH, false);
-    } else {
-      if (bf) DCN_GEMM_CASE88(DCN_VARIANT_JITTOR, true);
-      else DCN_GEMM_CASE88(DCN_VARIANT_JITTOR, false);
-    }
-#undef DCN_GEMM_CASE88
-    return DCN_OK;
-  }
-  if (g.variant == DCN_VARIANT_TORCH) {
-    if (bf) DCN_GEMM_CASE(DCN_VARIANT_TORCH, true);
-    else DCN_GEMM_CASE(DCN_VARIANT_TORCH, false);
-  } else {
-    if (bf) DCN_GEMM_CASE(DCN_VARIANT_JITTOR, true);
-    else DCN_GEMM_CASE(DCN_VARIANT_JITTOR, false);
-  }
-#undef DCN_GEMM_CASE
-  return DCN_OK;
+  if (g.variant == DCN_VARIANT_TORCH)
+    return launch_umma_gemm_split<DCN_VARIANT_TORCH, MODE, false>(bf, many_chains, P, tmap, grid, smem, st);
+  return launch_umma_gemm_split<DCN_VARIANT_JITTOR, MODE, false>(bf, many_chains, P, tmap, grid, smem, st);
 }
 
 // stage_x = false: the head of the workspace already holds the staged copy of x (an earlier
@@ -1147,17 +1112,17 @@ int umma_forward_any(const Geo& g, int operand, const void* x, const float* off,
     const int box_r = P.t.Rt < 4 ? 4 : P.t.Rt;
     const size_t bytes = sizeof(float) * (size_t)g.O * P.t.Gt * box_r;
     if (P.t.R % box_r == 0 && bytes <= 64 * 1024 && g.O <= 256 &&
-        (size_t)2 * P.stage_bytes + bytes + fixed <= 227 * 1024 && make_out_tensor_map(g, P.t, box_r, out, &tmap)) {
+        (size_t)2 * P.stage_bytes + bytes + fixed <= kSmemBudget && make_out_tensor_map(g, P.t, box_r, out, &tmap)) {
       P.tma_out = 1;
       P.box_r = box_r;
       P.tpg = box_r / P.t.Rt;
       P.stage_out_bytes = (uint32_t)align_up(bytes, 1024);
       // two staging buffers when three pipeline stages still fit next to them
-      P.n_ost = (size_t)3 * P.stage_bytes + 2 * P.stage_out_bytes + fixed <= 227 * 1024 ? 2 : 1;
+      P.n_ost = (size_t)3 * P.stage_bytes + 2 * P.stage_out_bytes + fixed <= kSmemBudget ? 2 : 1;
       fixed += (size_t)P.n_ost * P.stage_out_bytes;
     }
   }
-  const int stages = (int)((227 * 1024 - fixed) / P.stage_bytes);
+  const int stages = (int)((kSmemBudget - fixed) / P.stage_bytes);
   P.stages = stages > kFwdStages ? kFwdStages : stages;
   if (P.stages < 2) {
     set_error("umma forward: not enough shared memory for 2 stages");
@@ -1171,9 +1136,7 @@ int umma_forward_any(const Geo& g, int operand, const void* x, const float* off,
   const int groups = (P.t.num_tiles + P.tpg - 1) / P.tpg;  // CTAs walk groups of tpg tiles
   const int grid = groups < sms ? groups : sms;
   KernelScope scope(g.plain ? "umma_offset_conv_fwd_kernel" : "umma_fwd_kernel", st);
-  if ((rc = launch_gemm<MODE_FWD>(g, operand, P, tmap, grid, smem, st))) return rc;
-  DCN_KERNEL_CHECK("umma_fwd_kernel");
-  return DCN_OK;
+  return launch_gemm<MODE_FWD>(g, operand, P, tmap, grid, smem, st);
 }
 
 // ---- the companion offset convolution (deform_conv.py:16-21,58 / train.py:80-85,98) as a PLAIN problem -----------
@@ -1271,20 +1234,17 @@ int umma_wgrad_any(const Geo& g, int operand, const void* xt, const float* off, 
   P.tmem_cols = pow2_cols(P.o_blocks * P.kb_per_slice * 64);
   const size_t fixed = 2 * (size_t)P.plan_cap * sizeof(PlanEntry) + 256 + 1024;
   const size_t gbuf = 2 * (size_t)nimg * P.g_img;
-  P.n_gbuf = ((size_t)P.stages * P.stage_bytes + 2 * gbuf + fixed <= 227 * 1024) ? 2 : 1;
+  P.n_gbuf = ((size_t)P.stages * P.stage_bytes + 2 * gbuf + fixed <= kSmemBudget) ? 2 : 1;
   const size_t smem = (size_t)P.stages * P.stage_bytes + (size_t)P.n_gbuf * gbuf + fixed;
-  if (smem > 227 * 1024) {
+  if (smem > kSmemBudget) {
     set_error("umma wgrad: %zu bytes of shared memory needed", smem);
     return DCN_ERR_UNSUPPORTED;
   }
   const int grid = P.nslices * P.nchunks;
   KernelScope scope("umma_bwd_weight_kernel", st);
-  int rc;
   alignas(64) CUtensorMap tmap;
   memset(&tmap, 0, sizeof(tmap));
-  if ((rc = launch_gemm<MODE_WGRAD>(g, operand, P, tmap, grid, smem, st))) return rc;
-  DCN_KERNEL_CHECK("umma_bwd_weight_kernel");
-  return DCN_OK;
+  return launch_gemm<MODE_WGRAD>(g, operand, P, tmap, grid, smem, st);
 }
 
 }  // namespace dcn
