@@ -100,8 +100,12 @@ enum {
   DCN_FLAG_GRAD_X_FRAMED = 1 << 6, /* dcn_backward / dcn_layer_backward (tensor path): grad_x is NOT [B,C,H,W] but the framed
                                       channels-last accumulator itself — [B][(H+3) x (W+2)][C] floats in the layer's
                                       staging layout (dcn_staged_input_bytes) — overwritten; the post-op of the producer
-                                      layer reads it in that layout (dcn_bn_relu_backward_staged).  Excludes
-                                      DCN_FLAG_ACCUM_GRAD_X */
+                                      layer reads it in that layout (dcn_bn_relu_backward_staged).  dcn_backward,
+                                      dcn_backward_modulated and dcn_layer_backward* return DCN_ERR_UNSUPPORTED, before
+                                      any CUDA call, for this flag together with DCN_FLAG_ACCUM_GRAD_X, and for a
+                                      shape / operand / flags whose data gradient does not run on the tensor path
+                                      (dcn_path_name(s, DCN_PHASE_BACKWARD) other than "umma", or the generic fp32
+                                      data-gradient kernel inside it) */
   DCN_FLAG_XT_STAGED = 1 << 4      /* the workspace is the very buffer a preceding call of this library for the
                                       same shape / operand was given (dcn_offset_conv_forward, dcn_forward or
                                       dcn_layer_forward; sized for the largest phase used) and nothing has written

@@ -198,6 +198,21 @@ static int layer_refusal(const DcnShape* s, const Geo& g, int phase, const char*
   return DCN_ERR_UNSUPPORTED;
 }
 
+// DCN_FLAG_GRAD_X_FRAMED: grad_x is the consumer's framed channels-last accumulator.  Only the tensor-path data
+// gradient writes that layout, and it overwrites; any other data gradient, or an accumulating one, would leave NCHW
+// values (or a sum) in a buffer the caller reads as framed.  data_on_umma: the data gradient of this call runs there.
+static int grad_x_framed_refusal(const DcnShape* s, bool data_on_umma, const char* what) {
+  if (!(s->flags & DCN_FLAG_GRAD_X_FRAMED)) return DCN_OK;
+  if (s->flags & DCN_FLAG_ACCUM_GRAD_X)
+    set_error("%s: DCN_FLAG_GRAD_X_FRAMED excludes DCN_FLAG_ACCUM_GRAD_X (the framed grad_x is overwritten)", what);
+  else if (!data_on_umma)
+    set_error("%s: DCN_FLAG_GRAD_X_FRAMED needs the data gradient on the tensor path, which this shape / operand / "
+              "flags does not take", what);
+  else
+    return DCN_OK;
+  return DCN_ERR_UNSUPPORTED;
+}
+
 static int check_workspace(size_t have, size_t need, const char* what) {
   if (have >= need) return DCN_OK;
   set_error("%s workspace: have %zu bytes, need %zu", what, have, need);
@@ -395,6 +410,8 @@ static int backward_impl(const DcnShape* s, const void* x, const void* offset, c
       (rc = check_ptr(grad_x, "grad_x", want_gx)) || (rc = check_ptr(grad_offset, "grad_offset")) ||
       (rc = check_ptr(grad_weight, "grad_weight")) || (rc = check_ptr(grad_bias, "grad_bias", false)))
     return rc;
+  const bool data_on_umma = use_umma(s, g, DCN_PHASE_BACKWARD) && umma_bwd_data_on_tensor_path(g, s->operand);
+  if ((rc = grad_x_framed_refusal(s, data_on_umma, mask ? "modulated backward" : "backward"))) return rc;
   const size_t need = dcn_workspace_bytes(s, DCN_PHASE_BACKWARD);
   if (need && (rc = check_ptr(workspace, "workspace"))) return rc;
   if ((rc = check_workspace(workspace_bytes, need, "backward"))) return rc;
@@ -508,7 +525,8 @@ static int layer_backward_impl(const DcnShape* s, int phase, const char* what, c
       (rc = check_ptr(grad_x, "grad_x", want_gx)) || (rc = check_ptr(grad_offset_weight, "grad_offset_weight")) ||
       (rc = check_ptr(grad_offset_bias, "grad_offset_bias", false)) || (rc = check_ptr(grad_weight, "grad_weight")) ||
       (rc = check_ptr(grad_bias, "grad_bias", false)) || (rc = check_ptr(workspace, "workspace")) ||
-      (rc = layer_refusal(s, g, phase, what)))
+      (rc = layer_refusal(s, g, phase, what)) ||
+      (rc = grad_x_framed_refusal(s, umma_bwd_data_on_tensor_path(g, DCN_OPERAND_FP32), what)))
     return rc;
   const size_t need = layer_workspace(g, phase);
   if ((rc = check_workspace(workspace_bytes, need, what))) return rc;

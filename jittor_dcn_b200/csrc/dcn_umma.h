@@ -17,6 +17,9 @@ int umma_forward(const Geo& g, int operand, int flags, const void* x, const floa
 int umma_backward(const Geo& g, int operand, int flags, const void* x, const float* off,
                   const void* wt, const void* gout, float* gx, float* goff, float* gw, float* gb,
                   void* workspace, cudaStream_t st, const float* mask = nullptr, float* gmask = nullptr);
+// Does umma_backward run the data gradient of this problem on the tensor path (rather than the generic fp32 kernel)?
+// Only that kernel writes grad_x in the framed channels-last layout (DCN_FLAG_GRAD_X_FRAMED).
+bool umma_bwd_data_on_tensor_path(const Geo& g, int operand);
 
 // ---- whole layer (companion offset conv as a PLAIN problem + DCN span), fp32 operands.  n_out: the conv's output
 // channels, 2N, or 3N for the modulated layer (mmcv's ModulatedDeformConv2dPack: offsets, then one mask logit per tap)

@@ -58,6 +58,13 @@ static bool plain_bwd_ok(const Geo& g, int n_out) {
   return umma_bwd_data_supported(gp, DCN_OPERAND_FP32) && umma_bwd_data_fuses_wgrad(gp, DCN_OPERAND_FP32);
 }
 
+// decided on the largest output-channel group, which sizes every scratch region of umma_backward_any
+bool umma_bwd_data_on_tensor_path(const Geo& g, int operand) {
+  int gsize;
+  if (!o_groups(g, &gsize)) return false;
+  return operand != DCN_OPERAND_FP32 || umma_bwd_data_supported(o_group_geo(g, 0, gsize), operand);
+}
+
 // Whole-layer backward (DCN span + offset conv) on the tensor path: fp32 operands, one output-channel group or more,
 // data gradient on the tcgen05 kernel (so that the channels-last grad_x accumulator exists for both passes).
 bool umma_layer_bwd_supported(const Geo& g, int n_out) {
@@ -177,7 +184,8 @@ int umma_backward_any(const Geo& g, int operand, int flags, const void* xv, cons
   if (!(flags & DCN_FLAG_XT_STAGED) && (rc = launch_nchw_to_nhwc(g, t, x, xt, operand, st))) return rc;
   const bool want_gx = !(flags & DCN_FLAG_NO_GRAD_X) && gx != nullptr;
   bool all_fused = true;
-  if (operand != DCN_OPERAND_FP32 || umma_bwd_data_supported(g0, operand)) {
+  const bool data_on_umma = umma_bwd_data_on_tensor_path(g, operand);
+  if (data_on_umma) {
     // DCN_FLAG_GRAD_X_FRAMED: grad_x IS the framed channels-last accumulator (the producer-side post-op reads it in
     // that layout, dcn_bn_relu_backward_staged): scatter straight into the caller's buffer, no transposition at the end
     const bool gx_framed = (flags & DCN_FLAG_GRAD_X_FRAMED) != 0;
@@ -251,7 +259,6 @@ int umma_backward_any(const Geo& g, int operand, int flags, const void* xv, cons
   // pass of the remaining groups stages its grad_out tiles there
   for (int o0 = 0; o0 < g.O; o0 += gsize) {
     const Geo gc = o_group_geo(g, o0, gsize);
-    const bool data_on_umma = operand != DCN_OPERAND_FP32 || umma_bwd_data_supported(g0, operand);
     if (data_on_umma && umma_bwd_data_fuses_wgrad(gc, operand)) continue;
     if ((rc = umma_wgrad_any(gc, operand, xt, off, (const uint8_t*)goutv + (size_t)o0 * g.HW * esz,
                              gw + (size_t)o0 * g.K, rest, st, mask)))

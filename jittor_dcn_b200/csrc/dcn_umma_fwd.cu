@@ -404,6 +404,9 @@ __global__ void __launch_bounds__((kFirstPlanWarp + PW + GW) * 32, 1)
             }
           }
         }
+        tc_fence_before();
+        __syncwarp();
+        if (lane == 0) mbar_arrive(&tempty[acc]);
       } else {
         for (int c0 = 0; c0 < O; c0 += 16) {
           float v[16];

@@ -73,6 +73,61 @@ def test_null_and_misaligned_pointers_are_rejected_without_a_gpu():
     assert lib.dcn_status_string(-4) == b"workspace too small"
 
 
+def test_framed_grad_x_is_refused_where_no_kernel_writes_it_without_a_gpu():
+    """DCN_FLAG_GRAD_X_FRAMED asks for grad_x in the consumer's framed channels-last layout, which only the tensor-path
+    data gradient writes, and writes by overwriting.  Every backward entry point refuses the flag, before any CUDA call,
+    where another data gradient would run and for the pair with DCN_FLAG_ACCUM_GRAD_X.  (Otherwise NCHW values, or a
+    sum, would land in a buffer the caller reads as framed.)  A workspace of 0 bytes: the refusal comes before the
+    workspace check, so nothing could be launched."""
+    lib = dcn.load()
+    buf = ctypes.create_string_buffer(1 << 12)
+    ok = ctypes.c_void_p((ctypes.addressof(buf) + 255) // 256 * 256)
+    framed = _lib.FLAG_GRAD_X_FRAMED
+
+    def backward(s):
+        return lib.dcn_backward(ctypes.byref(s), ok, ok, ok, ok, ok, ok, ok, None, ok, 0, None)
+
+    def backward_modulated(s):
+        return lib.dcn_backward_modulated(ctypes.byref(s), ok, ok, ok, ok, ok, ok, ok, ok, ok, None, ok, 0, None)
+
+    def layer_backward(s):
+        return lib.dcn_layer_backward(ctypes.byref(s), ok, ok, ok, ok, ok, ok, ok, None, ok, None, ok, 0, None)
+
+    def layer_backward_modulated(s):
+        return lib.dcn_layer_backward_modulated(ctypes.byref(s), ok, ok, ok, ok, ok, ok, ok, ok, None, ok, None, ok, 0,
+                                                None)
+
+    def refused(call, s, why):
+        assert call(s) == -6, (call.__name__, lib.dcn_last_error())
+        msg = lib.dcn_last_error()
+        assert b"DCN_FLAG_GRAD_X_FRAMED" in msg and why in msg, (call.__name__, msg)
+
+    on_gemm = _lib.make_shape(2, 512, 512, 14, 14, 3, 1, 1, dcn.VARIANT_TORCH, dcn.OPERAND_FP32, framed)  # C5-like
+    assert _lib.path_name(on_gemm, 1) == "gemm"
+    on_simt = _lib.make_shape(2, 5, 8, 9, 13, 3, 1, 1, dcn.VARIANT_TORCH, dcn.OPERAND_FP32, framed)
+    assert _lib.path_name(on_simt, 1) == "simt"
+    # tensor-path backward whose fp32 data gradient still runs on the generic kernel (the fall-back inside it)
+    on_fallback = _lib.make_shape(2, 192, 16, 8, 8, 3, 1, 1, dcn.VARIANT_JITTOR, dcn.OPERAND_FP32, framed)
+    assert _lib.path_name(on_fallback, 1) == "umma"
+    forced = _lib.make_shape(2, 64, 64, 16, 16, 3, 1, 1, dcn.VARIANT_JITTOR, dcn.OPERAND_FP32,
+                             framed | _lib.FLAG_FORCE_SIMT)
+    for s in (on_gemm, on_simt, on_fallback, forced):
+        refused(backward, s, b"tensor path")
+    refused(backward_modulated, _lib.make_shape(2, 5, 8, 9, 13, 3, 1, 1, dcn.VARIANT_DCNV1, dcn.OPERAND_FP32, framed),
+            b"tensor path")
+    # the ACCUM pair, on a shape where every call runs on the tensor path
+    for variant, calls in ((dcn.VARIANT_JITTOR, (backward, layer_backward)),
+                           (dcn.VARIANT_DCNV1, (backward_modulated, layer_backward_modulated))):
+        s = _lib.make_shape(2, 64, 64, 16, 16, 3, 1, 1, variant, dcn.OPERAND_FP32, framed | _lib.FLAG_ACCUM_GRAD_X)
+        assert _lib.path_name(s, 1) == "umma" and _lib.path_name(s, 4 if variant == dcn.VARIANT_JITTOR else 6) == "umma"
+        for call in calls:
+            refused(call, s, b"DCN_FLAG_ACCUM_GRAD_X")
+        # without ACCUM the same calls pass the flag check and stop at the empty workspace
+        s.flags = framed
+        for call in calls:
+            assert call(s) == -4, (call.__name__, lib.dcn_last_error())
+
+
 def test_module_keeps_the_reference_interface():
     """ctor signature, attributes, parameter names/shapes and init of train.py:70-93."""
     m = dcn.TorchDeformConv2d(16, 32, 3, 2, 1)
