@@ -13,7 +13,7 @@
  *                                       (optimizer.backward)
  *
  * Beside it: multi-scale deformable attention (Deformable DETR's MSDeformAttn core), dcn_msda_forward /
- * dcn_msda_backward below.
+ * dcn_msda_backward, and DCNv3 (InternImage's core), dcn_v3_forward / dcn_v3_backward, below.
  *
  * The companion offset convolution (deform_conv.py:16-21,58 / train.py:80-85,98) stays a
  * framework convolution: its output is the `offset` argument here and `grad_offset` is
@@ -339,6 +339,44 @@ DCN_API int dcn_msda_backward(const DcnMsdaShape* s, const void* value, const in
                               const int64_t* level_start_index, const void* sampling_locations,
                               const void* attention_weights, const void* grad_out, void* grad_value,
                               void* grad_sampling_locations, void* grad_attention_weights, void* stream);
+
+/* ---- DCNv3 (InternImage's ops_dcnv3 core: DCNv3Function / dcnv3_core_pytorch), float32, channels-last ---------------
+ *   out[n, ho, wo, g*Gc + c] = sum_p m[n, ho, wo, g*P + p] * bilinear(input[n, :, :, g*Gc + c], y_p, x_p)
+ * P = kh*kw points in x-major order: p = i*kh + j with kernel column i < kw and kernel row j < kh (for a square kernel
+ * the transpose of torchvision's tap order).  Offsets are (dx, dy) per point: offset[n, ho, wo, 2*(g*P + p)] and
+ * [... + 1].  With hw = (dw*(kw-1)) / 2, hh = (dh*(kh-1)) / 2 (rounded down) and os = offset_scale, in unpadded pixel
+ * coordinates, evaluated in fp32 in this order:
+ *   x_p = (hw - pw + wo*sw) - hw*os + (i*dw + dx)*os        y_p = (hh - ph + ho*sh) - hh*os + (j*dh + dy)*os
+ * so os scales the dilation grid as well as the offsets.  Corners outside [0, H) x [0, W) read 0 (grid_sample, bilinear,
+ * zeros, align_corners=False on the zero-padded input); a NaN coordinate contributes 0.
+ *   Ho = (H + 2*ph - (dh*(kh-1) + 1)) / sh + 1 (rounded down), Wo likewise
+ *   input [N,H,W,G*Gc] f32   offset [N,Ho,Wo,G*P*2] f32   mask [N,Ho,Wo,G*P] f32   out [N,Ho,Wo,G*Gc] f32
+ * DCN_V3_FLAG_SOFTMAX_MASK: `mask` holds logits and m is their softmax over the P points of each (n, ho, wo, g)
+ * (InternImage's module applies that softmax right before the core); grad_mask is then the logits' gradient.
+ * Every pointer is 16-byte aligned.  No workspace and no host synchronisation: the calls can be captured in a CUDA graph.
+ * Checked before any CUDA call, in this order:
+ *   DCN_ERR_BAD_SHAPE     N, H, W, G, Gc, kh, kw < 1;  strides or dilations < 1;  paddings < 0;  Ho or Wo < 1;
+ *                         N*Ho*Wo*G or N*H*W above 2^31 - 1
+ *   DCN_ERR_NULL_POINTER / DCN_ERR_MISALIGNED   per pointer
+ *   DCN_ERR_UNSUPPORTED   Gc not in {16, 32, 64, 128, 256};  P > 32;  a flag other than DCN_V3_FLAG_SOFTMAX_MASK
+ * Backward: grad_input [N,H,W,G*Gc] is zeroed (cudaMemsetAsync) and accumulated with atomics (its summation order is not
+ * deterministic); grad_offset and grad_mask are each written by one plain store per element, bit-identical across runs.
+ * grad_offset = m*os*(sum_c g*dbil/dx, sum_c g*dbil/dy); grad_mask = sum_c g*bil, or with the softmax flag
+ * m_p*(gamma_p - sum_q m_q*gamma_q) with gamma = sum_c g*bil.  Each of the three may be NULL (not computed).
+ * InternImage's remove_center (the centre point dropped from the kernel) is not supported. */
+enum { DCN_V3_FLAG_SOFTMAX_MASK = 1 };
+
+typedef struct DcnV3Shape {
+  int32_t N, H, W, G, Gc;  /* batch, input extent, groups, channels per group (C = G*Gc) */
+  int32_t kh, kw, sh, sw, ph, pw, dh, dw; /* kernel, stride, padding, dilation */
+  int32_t flags;           /* DCN_V3_FLAG_* */
+} DcnV3Shape;
+
+DCN_API int dcn_v3_forward(const DcnV3Shape* s, float offset_scale, const void* input, const void* offset,
+                           const void* mask, void* out, void* stream);
+DCN_API int dcn_v3_backward(const DcnV3Shape* s, float offset_scale, const void* input, const void* offset,
+                            const void* mask, const void* grad_out, void* grad_input, void* grad_offset,
+                            void* grad_mask, void* stream);
 
 /* ---- producer of the first DCN layer's input (train.py:145,166 / 307,328: conv1 = Conv2d(1, 16, 3, 1, 1)) ------------
  * A 3 x 3, stride 1, padding 1 convolution with Cin <= 4 input channels and O in {16, 32} outputs, float32 NCHW,

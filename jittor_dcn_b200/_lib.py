@@ -40,7 +40,7 @@ EXPORTS = (
     "dcn_staged_input_bytes", "dcn_staged_input_clear", "dcn_layer_forward_chained",
     "dcn_bn_relu_forward_staged", "dcn_bn_relu_backward_staged", "dcn_stem_conv_forward", "dcn_stem_conv_backward",
     "dcn_offset_conv_forward_modulated", "dcn_layer_forward_modulated", "dcn_layer_backward_modulated",
-    "dcn_msda_forward", "dcn_msda_backward",
+    "dcn_msda_forward", "dcn_msda_backward", "dcn_v3_forward", "dcn_v3_backward",
 )
 
 
@@ -54,6 +54,15 @@ class DcnShape(ctypes.Structure):
 class DcnMsdaShape(ctypes.Structure):
     """Mirror of include/dcn_b200.h:DcnMsdaShape (multi-scale deformable attention)."""
     _fields_ = [(n, ctypes.c_int32) for n in ("B", "S", "Q", "M", "D", "L", "P", "flags")]
+
+
+class DcnV3Shape(ctypes.Structure):
+    """Mirror of include/dcn_b200.h:DcnV3Shape (DCNv3, InternImage's core)."""
+    _fields_ = [(n, ctypes.c_int32) for n in ("N", "H", "W", "G", "Gc", "kh", "kw", "sh", "sw", "ph", "pw", "dh", "dw",
+                                              "flags")]
+
+
+DCN_V3_FLAG_SOFTMAX_MASK = 1
 
 
 class DcnError(RuntimeError):
@@ -101,6 +110,9 @@ def load():
     msp = ctypes.POINTER(DcnMsdaShape)
     lib.dcn_msda_forward.argtypes = [msp, vp, vp, vp, vp, vp, vp, vp]
     lib.dcn_msda_backward.argtypes = [msp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp]
+    v3p, f32 = ctypes.POINTER(DcnV3Shape), ctypes.c_float
+    lib.dcn_v3_forward.argtypes = [v3p, f32, vp, vp, vp, vp, vp]
+    lib.dcn_v3_backward.argtypes = [v3p, f32, vp, vp, vp, vp, vp, vp, vp, vp]
     lib.dcn_comm_unique_id.argtypes = [vp]
     lib.dcn_comm_init.argtypes = [ctypes.c_int, ctypes.c_int, vp, ctypes.POINTER(vp)]
     lib.dcn_allreduce_sum_f32.argtypes = [vp, vp, sz, ctypes.c_float, vp]

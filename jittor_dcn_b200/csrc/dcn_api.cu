@@ -258,6 +258,68 @@ static int msda_shape_ok(const DcnMsdaShape* s, const char* what) {
   return DCN_OK;
 }
 
+// DCNv3 (dcn_dcnv3.cu)
+int dcnv3_forward(const DcnV3Shape& s, int Ho, int Wo, float offset_scale, const float* input, const float* offset,
+                  const float* mask, float* out, cudaStream_t st);
+int dcnv3_backward(const DcnV3Shape& s, int Ho, int Wo, float offset_scale, const float* input, const float* offset,
+                   const float* mask, const float* gout, float* ginput, float* goffset, float* gmask, cudaStream_t st);
+
+// floor((in + 2*pad - (dil*(k-1) + 1)) / stride) + 1, or 0 when the dilated kernel does not fit the padded input
+static long long dcnv3_out_extent(long long in, long long k, long long stride, long long pad, long long dil) {
+  const long long room = in + 2 * pad - (dil * (k - 1) + 1);
+  return room < 0 ? 0 : room / stride + 1;
+}
+
+// The shape checks of dcn_v3_forward / _backward: bad shapes (DCN_ERR_BAD_SHAPE) -> Ho, Wo.
+static int dcnv3_shape_ok(const DcnV3Shape* s, const char* what, int* Ho, int* Wo) {
+  if (!s) {
+    set_error("%s: DcnV3Shape is NULL", what);
+    return DCN_ERR_NULL_POINTER;
+  }
+  if (s->N <= 0 || s->H <= 0 || s->W <= 0 || s->G <= 0 || s->Gc <= 0 || s->kh <= 0 || s->kw <= 0 || s->sh <= 0 ||
+      s->sw <= 0 || s->dh <= 0 || s->dw <= 0 || s->ph < 0 || s->pw < 0) {
+    set_error("%s: bad shape N=%d H=%d W=%d G=%d Gc=%d k=(%d,%d) s=(%d,%d) p=(%d,%d) d=(%d,%d)", what, s->N, s->H, s->W,
+              s->G, s->Gc, s->kh, s->kw, s->sh, s->sw, s->ph, s->pw, s->dh, s->dw);
+    return DCN_ERR_BAD_SHAPE;
+  }
+  const long long ho = dcnv3_out_extent(s->H, s->kh, s->sh, s->ph, s->dh);
+  const long long wo = dcnv3_out_extent(s->W, s->kw, s->sw, s->pw, s->dw);
+  if (ho < 1 || wo < 1) {
+    set_error("%s: empty output Ho=%lld Wo=%lld (the dilated kernel does not fit the padded input)", what, ho, wo);
+    return DCN_ERR_BAD_SHAPE;
+  }
+  const long long items = (long long)s->N * ho * wo * s->G, pixels = (long long)s->N * s->H * s->W;
+  if (items > 0x7fffffffLL) {
+    set_error("%s: N*Ho*Wo*G = %lld exceeds the limit 2^31 - 1", what, items);
+    return DCN_ERR_BAD_SHAPE;
+  }
+  if (pixels > 0x7fffffffLL) {
+    set_error("%s: N*H*W = %lld exceeds the limit 2^31 - 1", what, pixels);
+    return DCN_ERR_BAD_SHAPE;
+  }
+  *Ho = (int)ho;
+  *Wo = (int)wo;
+  return DCN_OK;
+}
+
+// What the kernels cover (DCN_ERR_UNSUPPORTED), checked after the pointers.
+static int dcnv3_supported(const DcnV3Shape* s, const char* what) {
+  if (s->Gc != 16 && s->Gc != 32 && s->Gc != 64 && s->Gc != 128 && s->Gc != 256) {
+    set_error("%s: Gc = %d channels per group is not supported (Gc in {16, 32, 64, 128, 256})", what, s->Gc);
+    return DCN_ERR_UNSUPPORTED;
+  }
+  if ((long long)s->kh * s->kw > 32) {
+    set_error("%s: P = kh*kw = %lld points exceeds the limit P <= 32", what, (long long)s->kh * s->kw);
+    return DCN_ERR_UNSUPPORTED;
+  }
+  if (s->flags & ~DCN_V3_FLAG_SOFTMAX_MASK) {
+    set_error("%s: unknown flags 0x%x (only DCN_V3_FLAG_SOFTMAX_MASK = 1 is defined)", what,
+              (unsigned)s->flags & ~(unsigned)DCN_V3_FLAG_SOFTMAX_MASK);
+    return DCN_ERR_UNSUPPORTED;
+  }
+  return DCN_OK;
+}
+
 }  // namespace dcn
 
 using namespace dcn;
@@ -733,6 +795,30 @@ int dcn_msda_backward(const DcnMsdaShape* s, const void* value, const int64_t* s
   return msda_backward(*s, (const float*)value, spatial_shapes, level_start_index, (const float*)sampling_locations,
                        (const float*)attention_weights, (const float*)grad_out, (float*)grad_value,
                        (float*)grad_sampling_locations, (float*)grad_attention_weights, (cudaStream_t)stream);
+}
+
+int dcn_v3_forward(const DcnV3Shape* s, float offset_scale, const void* input, const void* offset, const void* mask,
+                   void* out, void* stream) {
+  int rc, Ho, Wo;
+  if ((rc = dcnv3_shape_ok(s, "dcn_v3_forward", &Ho, &Wo)) || (rc = check_ptr(input, "input")) ||
+      (rc = check_ptr(offset, "offset")) || (rc = check_ptr(mask, "mask")) || (rc = check_ptr(out, "out")) ||
+      (rc = dcnv3_supported(s, "dcn_v3_forward")))
+    return rc;
+  return dcnv3_forward(*s, Ho, Wo, offset_scale, (const float*)input, (const float*)offset, (const float*)mask,
+                       (float*)out, (cudaStream_t)stream);
+}
+
+int dcn_v3_backward(const DcnV3Shape* s, float offset_scale, const void* input, const void* offset, const void* mask,
+                    const void* grad_out, void* grad_input, void* grad_offset, void* grad_mask, void* stream) {
+  int rc, Ho, Wo;
+  if ((rc = dcnv3_shape_ok(s, "dcn_v3_backward", &Ho, &Wo)) || (rc = check_ptr(input, "input")) ||
+      (rc = check_ptr(offset, "offset")) || (rc = check_ptr(mask, "mask")) || (rc = check_ptr(grad_out, "grad_out")) ||
+      (rc = check_ptr(grad_input, "grad_input", false)) || (rc = check_ptr(grad_offset, "grad_offset", false)) ||
+      (rc = check_ptr(grad_mask, "grad_mask", false)) || (rc = dcnv3_supported(s, "dcn_v3_backward")))
+    return rc;
+  return dcnv3_backward(*s, Ho, Wo, offset_scale, (const float*)input, (const float*)offset, (const float*)mask,
+                        (const float*)grad_out, (float*)grad_input, (float*)grad_offset, (float*)grad_mask,
+                        (cudaStream_t)stream);
 }
 
 size_t dcn_bn_workspace_bytes(int32_t C) { return C > 0 ? bn_workspace_bytes(C) : 0; }

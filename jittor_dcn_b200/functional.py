@@ -919,3 +919,131 @@ def ms_deform_attn(value, spatial_shapes, level_start_index, sampling_locations,
     out[b, q, m*D + d] = sum_{l,p} a[b,q,m,l,p] * bilinear(value_l[b, :, :, m, d], x*W_l - 0.5, y*H_l - 0.5)."""
     return MSDeformAttnFunction.apply(value, spatial_shapes, level_start_index, sampling_locations, attention_weights,
                                       64)
+
+
+# ---- DCNv3 (InternImage's ops_dcnv3 core; csrc/dcn_dcnv3.cu) ------------------------------------------------------
+def _dcnv3_inputs(input, offset, mask, kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w, dilation_h, dilation_w,
+                  group, group_channels, softmax_mask):
+    """Checks shapes, dtypes and devices from tensor metadata only (no host synchronisation, so the call can be
+    captured in a CUDA graph) -> (DcnV3Shape, dense 16-byte aligned input, offset, mask)."""
+    floats = (("input", input), ("offset", offset), ("mask", mask))
+    for name, t in floats:
+        if not isinstance(t, torch.Tensor) or t.dtype != torch.float32:
+            raise ValueError(f"dcnv3: {name} must be a float32 tensor, got "
+                             f"{getattr(t, 'dtype', type(t).__name__)} (the kernels are float32 only)")
+    for name, t in floats:
+        if not t.is_cuda:
+            raise ValueError(f"dcnv3: {name} must be a CUDA tensor: there is no CPU path")
+    dev = input.device
+    for name, t in (("offset", offset), ("mask", mask)):
+        if t.device != dev:
+            raise ValueError(f"dcnv3: {name} is on {t.device}, input on {dev}")
+    geo = dict(kernel_h=kernel_h, kernel_w=kernel_w, stride_h=stride_h, stride_w=stride_w, pad_h=pad_h, pad_w=pad_w,
+               dilation_h=dilation_h, dilation_w=dilation_w, group=group, group_channels=group_channels)
+    for name, v in geo.items():
+        if isinstance(v, bool) or not isinstance(v, int):
+            raise ValueError(f"dcnv3: {name} must be an int, got {v!r}")
+        if v < (0 if name.startswith("pad") else 1):
+            raise ValueError(f"dcnv3: {name} = {v} is out of range (paddings >= 0, everything else >= 1)")
+    if input.dim() != 4:
+        raise ValueError(f"dcnv3: input must be [N, H, W, group*group_channels], got shape {tuple(input.shape)}")
+    N, H, W, C = (int(v) for v in input.shape)
+    if C != group * group_channels:
+        raise ValueError(f"dcnv3: input has {C} channels, group*group_channels = {group}*{group_channels} = "
+                         f"{group * group_channels}")
+    Ho = (H + 2 * pad_h - (dilation_h * (kernel_h - 1) + 1)) // stride_h + 1
+    Wo = (W + 2 * pad_w - (dilation_w * (kernel_w - 1) + 1)) // stride_w + 1
+    if Ho < 1 or Wo < 1:
+        raise ValueError(f"dcnv3: empty output {Ho} x {Wo}: the dilated kernel does not fit the padded {H} x {W} input")
+    P = kernel_h * kernel_w
+    if tuple(offset.shape) != (N, Ho, Wo, group * P * 2):
+        raise ValueError(f"dcnv3: offset shape {tuple(offset.shape)} != {(N, Ho, Wo, group * P * 2)} "
+                         f"(input {(N, H, W, C)}, {kernel_h}x{kernel_w} kernel, {group} groups)")
+    if tuple(mask.shape) != (N, Ho, Wo, group * P):
+        raise ValueError(f"dcnv3: mask shape {tuple(mask.shape)} != {(N, Ho, Wo, group * P)}")
+    if max(N, H, W, C) > 0x7fffffff:
+        raise ValueError(f"dcnv3: an extent of {(N, H, W, C)} exceeds 2^31 - 1")
+    shp = _lib.DcnV3Shape(N, H, W, group, group_channels, kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w,
+                          dilation_h, dilation_w, _lib.DCN_V3_FLAG_SOFTMAX_MASK if softmax_mask else 0)
+    return shp, _dev_ready(input), _dev_ready(offset), _dev_ready(mask)
+
+
+def dcn_v3_forward(input, offset, mask, kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w, dilation_h, dilation_w,
+                   group, group_channels, offset_scale, softmax_mask=False):
+    """out [N, Ho, Wo, group*group_channels] of the DCNv3 core on CUDA tensors (no autograd).  softmax_mask: `mask`
+    holds logits and the core applies InternImage's softmax over the kernel_h*kernel_w points of each group."""
+    lib = _lib.load()
+    shp, x, off, m = _dcnv3_inputs(input, offset, mask, kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w,
+                                   dilation_h, dilation_w, group, group_channels, softmax_mask)
+    out = torch.empty(tuple(off.shape[:3]) + (group * group_channels,), dtype=torch.float32, device=x.device)
+    with torch.cuda.device(x.device):
+        stream = torch.cuda.current_stream(x.device)
+        rc = lib.dcn_v3_forward(ctypes.byref(shp), float(offset_scale), _ptr(x), _ptr(off), _ptr(m), _ptr(out),
+                                ctypes.c_void_p(stream.cuda_stream))
+    _lib.check(rc, "dcn_v3_forward")
+    return out
+
+
+def dcn_v3_backward(input, offset, mask, grad_out, kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w, dilation_h,
+                    dilation_w, group, group_channels, offset_scale, softmax_mask=False, need=(True, True, True)):
+    """(grad_input, grad_offset, grad_mask); need[i] False -> None, not computed.  With softmax_mask, grad_mask is
+    the gradient of the logits."""
+    lib = _lib.load()
+    shp, x, off, m = _dcnv3_inputs(input, offset, mask, kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w,
+                                   dilation_h, dilation_w, group, group_channels, softmax_mask)
+    want = tuple(off.shape[:3]) + (group * group_channels,)
+    if not isinstance(grad_out, torch.Tensor) or tuple(grad_out.shape) != want:
+        raise ValueError(f"dcnv3: grad_out shape {tuple(getattr(grad_out, 'shape', ()))} != {want}")
+    go = _dev_ready(_to_device(grad_out, x.device))
+    gx, goff, gm = (torch.empty_like(t) if n else None for t, n in zip((x, off, m), need))
+    if gx is None and goff is None and gm is None:
+        return None, None, None
+    with torch.cuda.device(x.device):
+        stream = torch.cuda.current_stream(x.device)
+        rc = lib.dcn_v3_backward(ctypes.byref(shp), float(offset_scale), _ptr(x), _ptr(off), _ptr(m), _ptr(go),
+                                 _ptr(gx), _ptr(goff), _ptr(gm), ctypes.c_void_p(stream.cuda_stream))
+    _lib.check(rc, "dcn_v3_backward")
+    return gx, goff, gm
+
+
+class DCNv3Function(torch.autograd.Function):
+    """The DCNv3 core as one autograd node, with the positional interface of InternImage's ``DCNv3Function``:
+
+        DCNv3Function.apply(input, offset, mask, kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w,
+                            dilation_h, dilation_w, group, group_channels, offset_scale, im2col_step,
+                            remove_center=False) -> [N, Ho, Wo, group*group_channels]
+
+    input [N, H, W, group*group_channels], offset [N, Ho, Wo, group*P*2] ((dx, dy) per point, points x-major:
+    p = i*kernel_h + j for kernel column i and row j), mask [N, Ho, Wo, group*P], float32 on one CUDA device.
+    ``im2col_step`` is accepted and ignored: it exists only so that calls written for InternImage run unchanged.
+    ``remove_center=True`` is refused.  A trailing ``softmax_mask=True`` (not in InternImage's signature) makes `mask`
+    logits and applies InternImage's per-group softmax inside the node.  Differentiable in input, offset and mask;
+    only the gradients autograd asks for are computed, and the node never synchronises with the host."""
+
+    @staticmethod
+    def forward(ctx, input, offset, mask, kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w, dilation_h,
+                dilation_w, group, group_channels, offset_scale, im2col_step=256, remove_center=False,
+                softmax_mask=False):
+        if remove_center:
+            raise ValueError("dcnv3: remove_center=True is not supported")
+        ctx.geo = (kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w, dilation_h, dilation_w, group,
+                   group_channels, offset_scale, bool(softmax_mask))
+        out = dcn_v3_forward(input, offset, mask, *ctx.geo)
+        ctx.save_for_backward(input, offset, mask)
+        return out
+
+    @staticmethod
+    @torch.autograd.function.once_differentiable
+    def backward(ctx, grad_output):
+        need = tuple(ctx.needs_input_grad[:3])
+        gx, goff, gm = dcn_v3_backward(*ctx.saved_tensors, grad_output, *ctx.geo, need=need)
+        return (gx, goff, gm) + (None,) * 14
+
+
+def dcnv3_core(input, offset, mask, kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w, dilation_h, dilation_w,
+               group, group_channels, offset_scale, softmax_mask=False):
+    """Differentiable DCNv3 core (see DCNv3Function):
+    out[n, ho, wo, g*Gc + c] = sum_p m[n, ho, wo, g*P + p] * bilinear(input[n, :, :, g*Gc + c], y_p, x_p),
+    m = softmax over each group's P entries of `mask` if softmax_mask, else `mask` itself."""
+    return DCNv3Function.apply(input, offset, mask, kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w, dilation_h,
+                               dilation_w, group, group_channels, offset_scale, 256, False, softmax_mask)
