@@ -13,7 +13,8 @@
  *                                       (optimizer.backward)
  *
  * Beside it: multi-scale deformable attention (Deformable DETR's MSDeformAttn core), dcn_msda_forward /
- * dcn_msda_backward, and DCNv3 (InternImage's core), dcn_v3_forward / dcn_v3_backward, below.
+ * dcn_msda_backward, DCNv3 (InternImage's core), dcn_v3_forward / dcn_v3_backward, and DCNv4, dcn_v4_forward /
+ * dcn_v4_backward, below.
  *
  * The companion offset convolution (deform_conv.py:16-21,58 / train.py:80-85,98) stays a
  * framework convolution: its output is the `offset` argument here and `grad_offset` is
@@ -363,7 +364,7 @@ DCN_API int dcn_msda_backward(const DcnMsdaShape* s, const void* value, const in
  * deterministic); grad_offset and grad_mask are each written by one plain store per element, bit-identical across runs.
  * grad_offset = m*os*(sum_c g*dbil/dx, sum_c g*dbil/dy); grad_mask = sum_c g*bil, or with the softmax flag
  * m_p*(gamma_p - sum_q m_q*gamma_q) with gamma = sum_c g*bil.  Each of the three may be NULL (not computed).
- * InternImage's remove_center (the centre point dropped from the kernel) is not supported. */
+ * InternImage's remove_center (the centre point dropped from the kernel) is not supported here; DCNv4 below has it. */
 enum { DCN_V3_FLAG_SOFTMAX_MASK = 1 };
 
 typedef struct DcnV3Shape {
@@ -377,6 +378,34 @@ DCN_API int dcn_v3_forward(const DcnV3Shape* s, float offset_scale, const void* 
 DCN_API int dcn_v3_backward(const DcnV3Shape* s, float offset_scale, const void* input, const void* offset,
                             const void* mask, const void* grad_out, void* grad_input, void* grad_offset,
                             void* grad_mask, void* stream);
+
+/* ---- DCNv4 (the DCNv4 repository's DCNv4Function core), float32, channels-last --------------------------------------
+ * DCNv3's operator and coordinate chain (above) with three changes:
+ *   - no softmax: the mask is used as given;
+ *   - offsets and mask packed into one tensor offset_mask [N, Ho, Wo, Cm], Cm = ceil(3*G*K / 8)*8.  Group g owns
+ *     floats [g*3K, g*3K + 3K) of each pixel row: first 2K offsets as interleaved (dx, dy) per point, then K mask
+ *     values.  Columns [3*G*K, Cm) are padding: never read (NaN there reaches no output);
+ *   - DCN_V4_FLAG_REMOVE_CENTER drops the centre point of an odd kernel: K = kh*kw - 1 instead of kh*kw, and point
+ *     k < K of a group is grid point p = k + (k >= c), c = (kw/2)*kh + kh/2, i.e. kernel column i = p / kh, row
+ *     j = p % kh of DCNv3's x-major order (without the flag K = kh*kw and p = k).
+ *   x_p = (hw - pw + wo*sw) - hw*os + (i*dw + dx)*os        y_p = (hh - ph + ho*sh) - hh*os + (j*dh + dy)*os
+ *   input [N,H,W,G*Gc] f32   offset_mask [N,Ho,Wo,Cm] f32   out [N,Ho,Wo,G*Gc] f32
+ * Every pointer is 16-byte aligned.  No workspace and no host synchronisation: the calls can be captured in a CUDA graph.
+ * Checked before any CUDA call, in DCNv3's order and with its status codes, and in addition:
+ *   DCN_ERR_BAD_SHAPE     K = 0 (a 1 x 1 kernel with remove_center);  Cm above 2^31 - 1
+ *   DCN_ERR_UNSUPPORTED   Gc not in {16, 32, 64, 128, 256};  remove_center with an even kh or kw;  a flag other than
+ *                         DCN_V4_FLAG_REMOVE_CENTER (DCN_V3_FLAG_SOFTMAX_MASK included).  K has no upper limit.
+ * Backward: grad_input [N,H,W,G*Gc] is zeroed (cudaMemsetAsync) and accumulated with atomics (its summation order is not
+ * deterministic).  grad_offset_mask [N,Ho,Wo,Cm] has offset_mask's layout: each non-padding element is written by one
+ * plain store, bit-identical across runs, and the padding columns hold +0.0.  With g the incoming gradient and m the
+ * point's mask value, per point:  (d dx, d dy) = m*os*(sum_c g*dbil/dx, sum_c g*dbil/dy);  d m = sum_c g*bil.
+ * grad_input and grad_offset_mask may each be NULL (not computed). */
+enum { DCN_V4_FLAG_REMOVE_CENTER = 2 };
+
+DCN_API int dcn_v4_forward(const DcnV3Shape* s, float offset_scale, const void* input, const void* offset_mask,
+                           void* out, void* stream);
+DCN_API int dcn_v4_backward(const DcnV3Shape* s, float offset_scale, const void* input, const void* offset_mask,
+                            const void* grad_out, void* grad_input, void* grad_offset_mask, void* stream);
 
 /* ---- producer of the first DCN layer's input (train.py:145,166 / 307,328: conv1 = Conv2d(1, 16, 3, 1, 1)) ------------
  * A 3 x 3, stride 1, padding 1 convolution with Cin <= 4 input channels and O in {16, 32} outputs, float32 NCHW,

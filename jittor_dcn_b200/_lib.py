@@ -40,7 +40,7 @@ EXPORTS = (
     "dcn_staged_input_bytes", "dcn_staged_input_clear", "dcn_layer_forward_chained",
     "dcn_bn_relu_forward_staged", "dcn_bn_relu_backward_staged", "dcn_stem_conv_forward", "dcn_stem_conv_backward",
     "dcn_offset_conv_forward_modulated", "dcn_layer_forward_modulated", "dcn_layer_backward_modulated",
-    "dcn_msda_forward", "dcn_msda_backward", "dcn_v3_forward", "dcn_v3_backward",
+    "dcn_msda_forward", "dcn_msda_backward", "dcn_v3_forward", "dcn_v3_backward", "dcn_v4_forward", "dcn_v4_backward",
 )
 
 
@@ -63,6 +63,7 @@ class DcnV3Shape(ctypes.Structure):
 
 
 DCN_V3_FLAG_SOFTMAX_MASK = 1
+DCN_V4_FLAG_REMOVE_CENTER = 2
 
 
 class DcnError(RuntimeError):
@@ -113,6 +114,8 @@ def load():
     v3p, f32 = ctypes.POINTER(DcnV3Shape), ctypes.c_float
     lib.dcn_v3_forward.argtypes = [v3p, f32, vp, vp, vp, vp, vp]
     lib.dcn_v3_backward.argtypes = [v3p, f32, vp, vp, vp, vp, vp, vp, vp, vp]
+    lib.dcn_v4_forward.argtypes = [v3p, f32, vp, vp, vp, vp]
+    lib.dcn_v4_backward.argtypes = [v3p, f32, vp, vp, vp, vp, vp, vp]
     lib.dcn_comm_unique_id.argtypes = [vp]
     lib.dcn_comm_init.argtypes = [ctypes.c_int, ctypes.c_int, vp, ctypes.POINTER(vp)]
     lib.dcn_allreduce_sum_f32.argtypes = [vp, vp, sz, ctypes.c_float, vp]

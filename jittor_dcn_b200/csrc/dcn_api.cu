@@ -320,6 +320,47 @@ static int dcnv3_supported(const DcnV3Shape* s, const char* what) {
   return DCN_OK;
 }
 
+// DCNv4 (dcn_dcnv3.cu)
+long long dcnv4_row_floats(const DcnV3Shape& s);
+int dcnv4_forward(const DcnV3Shape& s, int Ho, int Wo, float offset_scale, const float* input, const float* offset_mask,
+                  float* out, cudaStream_t st);
+int dcnv4_backward(const DcnV3Shape& s, int Ho, int Wo, float offset_scale, const float* input, const float* offset_mask,
+                   const float* gout, float* ginput, float* goffset_mask, cudaStream_t st);
+
+// The shape checks of dcn_v4_forward / _backward: DCNv3's, then K >= 1 and the row width Cm.
+static int dcnv4_shape_ok(const DcnV3Shape* s, const char* what, int* Ho, int* Wo) {
+  int rc;
+  if ((rc = dcnv3_shape_ok(s, what, Ho, Wo))) return rc;
+  if ((long long)s->kh * s->kw == 1 && (s->flags & DCN_V4_FLAG_REMOVE_CENTER)) {
+    set_error("%s: K = 0 points: a 1 x 1 kernel with remove_center has none", what);
+    return DCN_ERR_BAD_SHAPE;
+  }
+  const long long cm = dcnv4_row_floats(*s);
+  if (cm > 0x7fffffffLL) {
+    set_error("%s: Cm = ceil(3*G*K / 8)*8 = %lld exceeds the limit 2^31 - 1", what, cm);
+    return DCN_ERR_BAD_SHAPE;
+  }
+  return DCN_OK;
+}
+
+// What the DCNv4 kernels cover (DCN_ERR_UNSUPPORTED), checked after the pointers.
+static int dcnv4_supported(const DcnV3Shape* s, const char* what) {
+  if (s->Gc != 16 && s->Gc != 32 && s->Gc != 64 && s->Gc != 128 && s->Gc != 256) {
+    set_error("%s: Gc = %d channels per group is not supported (Gc in {16, 32, 64, 128, 256})", what, s->Gc);
+    return DCN_ERR_UNSUPPORTED;
+  }
+  if (s->flags & ~DCN_V4_FLAG_REMOVE_CENTER) {
+    set_error("%s: unknown flags 0x%x (only DCN_V4_FLAG_REMOVE_CENTER = 2 is defined; DCNv4 has no softmax)", what,
+              (unsigned)s->flags & ~(unsigned)DCN_V4_FLAG_REMOVE_CENTER);
+    return DCN_ERR_UNSUPPORTED;
+  }
+  if ((s->flags & DCN_V4_FLAG_REMOVE_CENTER) && (s->kh % 2 == 0 || s->kw % 2 == 0)) {
+    set_error("%s: remove_center needs an odd kernel, got %d x %d (no centre point)", what, s->kh, s->kw);
+    return DCN_ERR_UNSUPPORTED;
+  }
+  return DCN_OK;
+}
+
 }  // namespace dcn
 
 using namespace dcn;
@@ -819,6 +860,29 @@ int dcn_v3_backward(const DcnV3Shape* s, float offset_scale, const void* input, 
   return dcnv3_backward(*s, Ho, Wo, offset_scale, (const float*)input, (const float*)offset, (const float*)mask,
                         (const float*)grad_out, (float*)grad_input, (float*)grad_offset, (float*)grad_mask,
                         (cudaStream_t)stream);
+}
+
+int dcn_v4_forward(const DcnV3Shape* s, float offset_scale, const void* input, const void* offset_mask, void* out,
+                   void* stream) {
+  int rc, Ho, Wo;
+  if ((rc = dcnv4_shape_ok(s, "dcn_v4_forward", &Ho, &Wo)) || (rc = check_ptr(input, "input")) ||
+      (rc = check_ptr(offset_mask, "offset_mask")) || (rc = check_ptr(out, "out")) ||
+      (rc = dcnv4_supported(s, "dcn_v4_forward")))
+    return rc;
+  return dcnv4_forward(*s, Ho, Wo, offset_scale, (const float*)input, (const float*)offset_mask, (float*)out,
+                       (cudaStream_t)stream);
+}
+
+int dcn_v4_backward(const DcnV3Shape* s, float offset_scale, const void* input, const void* offset_mask,
+                    const void* grad_out, void* grad_input, void* grad_offset_mask, void* stream) {
+  int rc, Ho, Wo;
+  if ((rc = dcnv4_shape_ok(s, "dcn_v4_backward", &Ho, &Wo)) || (rc = check_ptr(input, "input")) ||
+      (rc = check_ptr(offset_mask, "offset_mask")) || (rc = check_ptr(grad_out, "grad_out")) ||
+      (rc = check_ptr(grad_input, "grad_input", false)) ||
+      (rc = check_ptr(grad_offset_mask, "grad_offset_mask", false)) || (rc = dcnv4_supported(s, "dcn_v4_backward")))
+    return rc;
+  return dcnv4_backward(*s, Ho, Wo, offset_scale, (const float*)input, (const float*)offset_mask,
+                        (const float*)grad_out, (float*)grad_input, (float*)grad_offset_mask, (cudaStream_t)stream);
 }
 
 size_t dcn_bn_workspace_bytes(int32_t C) { return C > 0 ? bn_workspace_bytes(C) : 0; }

@@ -13,11 +13,26 @@
 // This is the gather core of dcn_gather.cuh with one level: item (n, ho, wo, g) <-> (b, q, m) of multi-scale
 // deformable attention with S = H*W tokens, Q = Ho*Wo queries, M = G heads of D = Gc channels; the location gradient
 // is scaled by m*os.
+//
+// DCNv4 (dcnv4_*_kernel) is the same chain with three changes: no softmax; offsets and mask packed into one tensor
+// offset_mask [N, Ho, Wo, Cm], Cm = ceil(3*G*K / 8)*8, where group g owns floats [g*3K, g*3K + 3K) of a pixel's row
+// (2K interleaved (dx, dy), then K mask values; columns [3*G*K, Cm) are padding, never read, written +0.0 in the
+// gradient); and remove_center, which drops the centre point c = (kw/2)*kh + kh/2 of an odd kernel, so that sample
+// s < K = kh*kw - 1 is grid point s + (s >= c).  A group's row starts only 4-byte aligned (3K floats per group), so
+// it is read and its gradient written with 4-byte accesses (PackedRows).
+#include <type_traits>
+
 #include <cuda_runtime.h>
 
 #include "dcn_gather.cuh"
 
 namespace dcn {
+
+// DCNv4: floats per pixel row of offset_mask, Cm = ceil(3*G*K / 8)*8 with K = kh*kw - remove_center
+long long dcnv4_row_floats(const DcnV3Shape& s) {
+  const long long K = (long long)s.kh * s.kw - ((s.flags & DCN_V4_FLAG_REMOVE_CENTER) ? 1 : 0);
+  return (3LL * s.G * K + 7) / 8 * 8;
+}
 
 namespace dcnv3 {
 
@@ -34,17 +49,51 @@ struct Args {
   float* gvalue;       // like input, or null        backward
   float* gloc;         // like offset, or null       backward
   float* gattn;        // like mask, or null         backward
-  int B, S, Q, M, D, L, P;  // N, H*W, Ho*Wo, G, Gc, 1, kh*kw
+  int B, S, Q, M, D, L, P;  // N, H*W, Ho*Wo, G, Gc, 1, kh*kw (DCNv4: K)
   // the coordinate generator
   int H, W, Wo, kh, sh, sw, dh, dw;
   int p0x, p0y;  // hw - pw, hh - ph: the unscaled part of the kernel centre at (ho, wo) = (0, 0)
   int hw, hh;
   float os;
+  // DCNv4 (PACKED): Cm = floats per pixel row of offset_mask; samples s >= center take grid point s + 1 (center = the
+  // centre point with remove_center, else P: none)
+  int Cm, center;
 };
 
-template <bool SOFTMAX>
+// Src::Rows of DCNv4's packed offset_mask (loc = offset_mask, gloc = gattn = grad_offset_mask): item (pixel, g) owns
+// the 3P floats at pixel*Cm + g*3P, (dx, dy) of sample s at 2s, 2s + 1 and its mask at 2P + s.
+struct PackedRows {
+  static __device__ __forceinline__ size_t at(const Args& a, int item) {
+    return (size_t)(item / a.M) * a.Cm + (size_t)(item % a.M) * 3 * a.P;
+  }
+  static __device__ __forceinline__ const float* loc_row(const Args& a, int item, int) { return a.loc + at(a, item); }
+  static __device__ __forceinline__ const float* attn_row(const Args& a, int item, int) {
+    return a.loc + at(a, item) + 2 * a.P;
+  }
+  static __device__ __forceinline__ size_t grad_slot(const Args& a, int item, int, int) { return at(a, item); }
+  static __device__ __forceinline__ void store_gattn(const Args& a, size_t row, int s, float v) {
+    a.gattn[row + 2 * a.P + s] = v;
+  }
+  static __device__ __forceinline__ void store_gloc(const Args& a, size_t row, int s, float2 v) {
+    float* p = a.gloc + row + 2 * s;
+    p[0] = v.x;
+    p[1] = v.y;
+  }
+  // the padding columns of a pixel's row: +0.0, written by the group of its last item
+  template <int G>
+  static __device__ __forceinline__ void end_grad(const Args& a, int item, int j, bool live) {
+    if (!a.gloc || !live || item % a.M != a.M - 1) return;
+    const int used = a.M * 3 * a.P;
+    float* p = a.gloc + (size_t)(item / a.M) * a.Cm + used;
+    for (int c = j; c < a.Cm - used; c += G) p[c] = 0.f;
+  }
+};
+
+template <bool SOFTMAX, bool PACKED = false>
 struct Source {
+  static_assert(!(SOFTMAX && PACKED), "DCNv4 has no softmax");
   using Args = dcnv3::Args;
+  using Rows = std::conditional_t<PACKED, PackedRows, gather::DenseRows>;
   struct Item {
     float x0, y0;   // (hw - pw + wo*sw) - hw*os, (hh - ph + ho*sh) - hh*os
     float mx, inv;  // softmax: max of the item's logits and 1 / sum exp(logit - max)
@@ -74,8 +123,15 @@ struct Source {
   }
 
   __device__ __forceinline__ Smp sample(const Item& it, const float* locp, const float* attnp, int s) const {
-    const float2 d = *reinterpret_cast<const float2*>(locp + 2 * s);  // (dx, dy)
-    const int i = s / a.kh, jr = s - i * a.kh;                        // kernel column, kernel row
+    float2 d;  // (dx, dy)
+    int p = s;  // grid point
+    if constexpr (PACKED) {
+      d = make_float2(locp[2 * s], locp[2 * s + 1]);
+      p += s >= a.center;
+    } else {
+      d = *reinterpret_cast<const float2*>(locp + 2 * s);
+    }
+    const int i = p / a.kh, jr = p - i * a.kh;  // kernel column, kernel row
     Smp r = gather::empty_sample();
     r.a = SOFTMAX ? expf(attnp[s] - it.mx) * it.inv : attnp[s];
     r.W = a.W;
@@ -100,36 +156,51 @@ __global__ void __launch_bounds__(kThreads) dcnv3_bwd_kernel(const Args a) {
   gather::bwd_body<G, V>(Source<SOFTMAX>{a});
 }
 
-template <int G, int V, bool SOFTMAX>
+template <int G, int V>
+__global__ void __launch_bounds__(kThreads) dcnv4_fwd_kernel(const Args a) {
+  gather::fwd_body<G, V>(Source<false, true>{a});
+}
+
+template <int G, int V>
+__global__ void __launch_bounds__(kThreads) dcnv4_bwd_kernel(const Args a) {
+  gather::bwd_body<G, V>(Source<false, true>{a});
+}
+
+enum class Op { v3, v3_softmax, v4 };
+
+template <int G, int V, Op OP>
 static int launch(const Args& a, bool backward, cudaStream_t st) {
+  constexpr bool SOFTMAX = OP == Op::v3_softmax;
   const long long threads = (long long)a.B * a.Q * a.M * G;
   const unsigned blocks = (unsigned)((threads + kThreads - 1) / kThreads);
-  if (!backward) {
-    KernelScope scope("dcnv3_fwd_kernel", st);
-    dcnv3_fwd_kernel<G, V, SOFTMAX><<<blocks, kThreads, 0, st>>>(a);
-    DCN_KERNEL_CHECK("dcnv3_fwd_kernel");
+  const char* name = OP == Op::v4 ? (backward ? "dcnv4_bwd_kernel" : "dcnv4_fwd_kernel")
+                                  : (backward ? "dcnv3_bwd_kernel" : "dcnv3_fwd_kernel");
+  KernelScope scope(name, st);
+  if constexpr (OP == Op::v4) {
+    if (!backward) dcnv4_fwd_kernel<G, V><<<blocks, kThreads, 0, st>>>(a);
+    else dcnv4_bwd_kernel<G, V><<<blocks, kThreads, 0, st>>>(a);
   } else {
-    KernelScope scope("dcnv3_bwd_kernel", st);
-    dcnv3_bwd_kernel<G, V, SOFTMAX><<<blocks, kThreads, 0, st>>>(a);
-    DCN_KERNEL_CHECK("dcnv3_bwd_kernel");
+    if (!backward) dcnv3_fwd_kernel<G, V, SOFTMAX><<<blocks, kThreads, 0, st>>>(a);
+    else dcnv3_bwd_kernel<G, V, SOFTMAX><<<blocks, kThreads, 0, st>>>(a);
   }
+  DCN_KERNEL_CHECK(name);
   return DCN_OK;
 }
 
-template <bool SOFTMAX>
+template <Op OP>
 static int dispatch_gc(const Args& a, bool backward, cudaStream_t st) {
   switch (a.D) {
-    case 16: return launch<4, 1, SOFTMAX>(a, backward, st);
-    case 32: return launch<8, 1, SOFTMAX>(a, backward, st);
-    case 64: return launch<16, 1, SOFTMAX>(a, backward, st);
-    case 128: return launch<32, 1, SOFTMAX>(a, backward, st);
-    case 256: return launch<32, 2, SOFTMAX>(a, backward, st);
+    case 16: return launch<4, 1, OP>(a, backward, st);
+    case 32: return launch<8, 1, OP>(a, backward, st);
+    case 64: return launch<16, 1, OP>(a, backward, st);
+    case 128: return launch<32, 1, OP>(a, backward, st);
+    case 256: return launch<32, 2, OP>(a, backward, st);
     default: set_error("dcnv3: Gc = %d is not supported", a.D); return DCN_ERR_UNSUPPORTED;
   }
 }
 
 static int dispatch(const Args& a, bool softmax, bool backward, cudaStream_t st) {
-  return softmax ? dispatch_gc<true>(a, backward, st) : dispatch_gc<false>(a, backward, st);
+  return softmax ? dispatch_gc<Op::v3_softmax>(a, backward, st) : dispatch_gc<Op::v3>(a, backward, st);
 }
 
 static Args make_args(const DcnV3Shape& s, int Ho, int Wo, float offset_scale, const float* input,
@@ -143,6 +214,18 @@ static Args make_args(const DcnV3Shape& s, int Ho, int Wo, float offset_scale, c
   a.p0x = a.hw - s.pw;
   a.p0y = a.hh - s.ph;
   a.os = offset_scale;
+  a.center = a.P;
+  return a;
+}
+
+// DCNv4: P = K points per group, loc = offset_mask
+static Args make_args_v4(const DcnV3Shape& s, int Ho, int Wo, float offset_scale, const float* input,
+                         const float* offset_mask) {
+  Args a = make_args(s, Ho, Wo, offset_scale, input, offset_mask, offset_mask);
+  const bool rc = s.flags & DCN_V4_FLAG_REMOVE_CENTER;
+  a.P -= rc;
+  a.center = rc ? (s.kw / 2) * s.kh + s.kh / 2 : a.P;
+  a.Cm = (int)dcnv4_row_floats(s);  // < 2^31 (dcn_api.cu)
   return a;
 }
 
@@ -164,6 +247,22 @@ int dcnv3_backward(const DcnV3Shape& s, int Ho, int Wo, float offset_scale, cons
   dcnv3::Args a = dcnv3::make_args(s, Ho, Wo, offset_scale, input, offset, mask);
   a.gout = gout; a.gvalue = ginput; a.gloc = goffset; a.gattn = gmask;
   return dcnv3::dispatch(a, s.flags & DCN_V3_FLAG_SOFTMAX_MASK, true, st);
+}
+
+int dcnv4_forward(const DcnV3Shape& s, int Ho, int Wo, float offset_scale, const float* input, const float* offset_mask,
+                  float* out, cudaStream_t st) {
+  dcnv3::Args a = dcnv3::make_args_v4(s, Ho, Wo, offset_scale, input, offset_mask);
+  a.out = out;
+  return dcnv3::dispatch_gc<dcnv3::Op::v4>(a, false, st);
+}
+
+int dcnv4_backward(const DcnV3Shape& s, int Ho, int Wo, float offset_scale, const float* input, const float* offset_mask,
+                   const float* gout, float* ginput, float* goffset_mask, cudaStream_t st) {
+  if (!ginput && !goffset_mask) return DCN_OK;
+  if (ginput) DCN_CUDA_TRY(cudaMemsetAsync(ginput, 0, sizeof(float) * (size_t)s.N * s.H * s.W * s.G * s.Gc, st));
+  dcnv3::Args a = dcnv3::make_args_v4(s, Ho, Wo, offset_scale, input, offset_mask);
+  a.gout = gout; a.gvalue = ginput; a.gloc = goffset_mask; a.gattn = goffset_mask;
+  return dcnv3::dispatch_gc<dcnv3::Op::v4>(a, true, st);
 }
 
 }  // namespace dcn

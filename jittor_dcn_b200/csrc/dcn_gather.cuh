@@ -1,10 +1,15 @@
-// dcn_gather.cuh — the depthwise bilinear gather core shared by multi-scale deformable attention (dcn_msda.cu) and
-// DCNv3 (dcn_dcnv3.cu).  Both compute, per item (batch, query, head) with its D contiguous channels of `value`,
+// dcn_gather.cuh — the depthwise bilinear gather core shared by multi-scale deformable attention (dcn_msda.cu),
+// DCNv3 and DCNv4 (dcn_dcnv3.cu).  All compute, per item (batch, query, head) with its D contiguous channels of `value`,
 //   out[item, d] = sum_s a_s * bilinear(value[b, :, m, d], y_s, x_s)
 // with corners outside the image reading 0.  Only where the samples come from differs; a sample source supplies it:
 //   Src::Args        tensors and extents.  Fields the core reads: value, loc, attn, gout, out, gvalue, gloc, gattn
 //                    and B, S, Q, M, D, L, P — value [B, S, M, D] (S tokens of M heads of D channels), items
 //                    B*Q*M, L*P samples per item, loc [items, L*P, 2], attn [items, L*P], out / gout [items, D].
+//   Src::Rows        where an item's per-sample data lives: loc_row / attn_row (the pointers handed to sample()),
+//                    grad_slot, store_gattn / store_gloc (where the three gradient elements of sample s go: the
+//                    slot is computed once, each store adds what it needs) and end_grad<G> (anything
+//                    else of the item's coordinate-side gradient).  DenseRows below is the layout just described;
+//                    DCNv4's packed offset_mask row is the other one (dcn_dcnv3.cu).
 //   Src::Item        per-item state, made once per item by begin<G>(item, j, attnp) with the whole group present.
 //   sample(it, locp, attnp, s)   the coordinate chain of sample s -> Smp (corner mask, NW token, fractions, weight).
 //   loc_scale(own, s)            (dx/dloc_x, dy/dloc_y) times the sample's weight: the factors of the two partials
@@ -41,6 +46,32 @@ struct Smp {
 };
 
 __device__ __forceinline__ Smp empty_sample() { return Smp{0, 0, 0u, 0.f, 0.f, 0.f}; }
+
+// Src::Rows of the dense layout: loc [items, L*P, 2] with one float2 per sample, attn [items, L*P], gradients alike.
+struct DenseRows {
+  template <class A>
+  static __device__ __forceinline__ const float* loc_row(const A& a, int item, int LP) {
+    return a.loc + (size_t)item * LP * 2;
+  }
+  template <class A>
+  static __device__ __forceinline__ const float* attn_row(const A& a, int item, int LP) {
+    return a.attn + (size_t)item * LP;
+  }
+  template <class A>
+  static __device__ __forceinline__ size_t grad_slot(const A&, int item, int LP, int s) {
+    return (size_t)item * LP + s;
+  }
+  template <class A>
+  static __device__ __forceinline__ void store_gattn(const A& a, size_t o, int, float v) {
+    a.gattn[o] = v;
+  }
+  template <class A>
+  static __device__ __forceinline__ void store_gloc(const A& a, size_t o, int, float2 v) {
+    *reinterpret_cast<float2*>(a.gloc + 2 * o) = v;
+  }
+  template <int G, class A>
+  static __device__ __forceinline__ void end_grad(const A&, int, int, bool) {}
+};
 
 // Corner mask, NW token and fractions of pixel coordinate (x, y) in an H x W image whose first token is `start`;
 // corners are also checked against [0, S).  A NaN coordinate saturates low (sat_int) and reads nothing.
@@ -109,8 +140,9 @@ __device__ __forceinline__ void fwd_body(const Src& src) {
   const int j = threadIdx.x & (G - 1);
   const int LP = a.L * a.P;
   const int m = item % a.M, b = item / (a.Q * a.M);
-  const float* locp = a.loc + (size_t)item * LP * 2;
-  const float* attnp = a.attn + (size_t)item * LP;
+  using Rows = typename Src::Rows;
+  const float* locp = Rows::loc_row(a, item, LP);
+  const float* attnp = Rows::attn_row(a, item, LP);
   const typename Src::Item it = src.template begin<G>(item, j, attnp);
   const size_t row = (size_t)a.M * a.D;  // floats per token
   const float* vb = a.value + ((size_t)b * a.S * a.M + m) * a.D + 4 * j;
@@ -161,8 +193,9 @@ __device__ __forceinline__ void bwd_body(const Src& src) {
   const int j = threadIdx.x & (G - 1);
   const int LP = a.L * a.P;
   const int m = item % a.M, b = item / (a.Q * a.M);
-  const float* locp = a.loc + (size_t)item * LP * 2;
-  const float* attnp = a.attn + (size_t)item * LP;
+  using Rows = typename Src::Rows;
+  const float* locp = Rows::loc_row(a, item, LP);
+  const float* attnp = Rows::attn_row(a, item, LP);
   const typename Src::Item it = src.template begin<G>(item, j, attnp);
   const size_t row = (size_t)a.M * a.D;
   const size_t vofs = ((size_t)b * a.S * a.M + m) * a.D + 4 * j;
@@ -249,20 +282,21 @@ __device__ __forceinline__ void bwd_body(const Src& src) {
     }
     const int s = s0 + j;
     if (live && j < K && s < LP) {  // the owner of sample s: one plain store per gradient element
-      const size_t o = (size_t)item * LP + s;
+      const size_t o = Rows::grad_slot(a, item, LP, s);
       if constexpr (Src::kSoftmax) {  // the logit gradient needs every gamma of the item: kept, written below
 #pragma unroll
         for (int r = 0; r < R; ++r)
           if (r * K == s0) keep_m[r] = own.a, keep_g[r] = pa[0];
       } else {
-        if (a.gattn) a.gattn[o] = pa[0];
+        if (a.gattn) Rows::store_gattn(a, o, s, pa[0]);
       }
       if (a.gloc) {
         const float2 sc = src.loc_scale(own, s);
-        *reinterpret_cast<float2*>(a.gloc + 2 * o) = make_float2(sc.x * px[0], sc.y * py[0]);
+        Rows::store_gloc(a, o, s, make_float2(sc.x * px[0], sc.y * py[0]));
       }
     }
   }
+  Rows::template end_grad<G>(a, item, j, live);
   if constexpr (Src::kSoftmax) {
     if (!a.gattn) return;
     // sum_q m_q*gamma_q over the item: each owner lane adds its samples in round order, then the group
@@ -273,7 +307,7 @@ __device__ __forceinline__ void bwd_body(const Src& src) {
 #pragma unroll
     for (int r = 0; r < R; ++r) {
       const int s = r * K + j;
-      if (live && j < K && s < LP) a.gattn[(size_t)item * LP + s] = keep_m[r] * (keep_g[r] - t);
+      if (live && j < K && s < LP) Rows::store_gattn(a, Rows::grad_slot(a, item, LP, s), s, keep_m[r] * (keep_g[r] - t));
     }
   }
 }

@@ -53,6 +53,7 @@ __device__ __forceinline__ void load_levels(const Args& a, Level* lv) {
 // The gather core's sample source (dcn_gather.cuh): normalised locations on the levels of the block's level table.
 struct Source {
   using Args = msda::Args;
+  using Rows = gather::DenseRows;
   struct Item {};
   static constexpr bool kSoftmax = false;
   const Args& a;

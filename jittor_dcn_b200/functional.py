@@ -922,39 +922,50 @@ def ms_deform_attn(value, spatial_shapes, level_start_index, sampling_locations,
 
 
 # ---- DCNv3 (InternImage's ops_dcnv3 core; csrc/dcn_dcnv3.cu) ------------------------------------------------------
-def _dcnv3_inputs(input, offset, mask, kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w, dilation_h, dilation_w,
-                  group, group_channels, softmax_mask):
-    """Checks shapes, dtypes and devices from tensor metadata only (no host synchronisation, so the call can be
-    captured in a CUDA graph) -> (DcnV3Shape, dense 16-byte aligned input, offset, mask)."""
-    floats = (("input", input), ("offset", offset), ("mask", mask))
+def _grid_inputs(what, floats, kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w, dilation_h, dilation_w, group,
+                 group_channels):
+    """The checks DCNv3 and DCNv4 share, on tensor metadata only: dtypes and devices of `floats` ((name, tensor), input
+    first), the geometry and the input's shape -> (N, H, W, C, Ho, Wo)."""
     for name, t in floats:
         if not isinstance(t, torch.Tensor) or t.dtype != torch.float32:
-            raise ValueError(f"dcnv3: {name} must be a float32 tensor, got "
+            raise ValueError(f"{what}: {name} must be a float32 tensor, got "
                              f"{getattr(t, 'dtype', type(t).__name__)} (the kernels are float32 only)")
     for name, t in floats:
         if not t.is_cuda:
-            raise ValueError(f"dcnv3: {name} must be a CUDA tensor: there is no CPU path")
+            raise ValueError(f"{what}: {name} must be a CUDA tensor: there is no CPU path")
+    input = floats[0][1]
     dev = input.device
-    for name, t in (("offset", offset), ("mask", mask)):
+    for name, t in floats[1:]:
         if t.device != dev:
-            raise ValueError(f"dcnv3: {name} is on {t.device}, input on {dev}")
+            raise ValueError(f"{what}: {name} is on {t.device}, input on {dev}")
     geo = dict(kernel_h=kernel_h, kernel_w=kernel_w, stride_h=stride_h, stride_w=stride_w, pad_h=pad_h, pad_w=pad_w,
                dilation_h=dilation_h, dilation_w=dilation_w, group=group, group_channels=group_channels)
     for name, v in geo.items():
         if isinstance(v, bool) or not isinstance(v, int):
-            raise ValueError(f"dcnv3: {name} must be an int, got {v!r}")
+            raise ValueError(f"{what}: {name} must be an int, got {v!r}")
         if v < (0 if name.startswith("pad") else 1):
-            raise ValueError(f"dcnv3: {name} = {v} is out of range (paddings >= 0, everything else >= 1)")
+            raise ValueError(f"{what}: {name} = {v} is out of range (paddings >= 0, everything else >= 1)")
     if input.dim() != 4:
-        raise ValueError(f"dcnv3: input must be [N, H, W, group*group_channels], got shape {tuple(input.shape)}")
+        raise ValueError(f"{what}: input must be [N, H, W, group*group_channels], got shape {tuple(input.shape)}")
     N, H, W, C = (int(v) for v in input.shape)
     if C != group * group_channels:
-        raise ValueError(f"dcnv3: input has {C} channels, group*group_channels = {group}*{group_channels} = "
+        raise ValueError(f"{what}: input has {C} channels, group*group_channels = {group}*{group_channels} = "
                          f"{group * group_channels}")
     Ho = (H + 2 * pad_h - (dilation_h * (kernel_h - 1) + 1)) // stride_h + 1
     Wo = (W + 2 * pad_w - (dilation_w * (kernel_w - 1) + 1)) // stride_w + 1
     if Ho < 1 or Wo < 1:
-        raise ValueError(f"dcnv3: empty output {Ho} x {Wo}: the dilated kernel does not fit the padded {H} x {W} input")
+        raise ValueError(f"{what}: empty output {Ho} x {Wo}: the dilated kernel does not fit the padded {H} x {W} "
+                         "input")
+    return N, H, W, C, Ho, Wo
+
+
+def _dcnv3_inputs(input, offset, mask, kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w, dilation_h, dilation_w,
+                  group, group_channels, softmax_mask):
+    """Checks shapes, dtypes and devices from tensor metadata only (no host synchronisation, so the call can be
+    captured in a CUDA graph) -> (DcnV3Shape, dense 16-byte aligned input, offset, mask)."""
+    N, H, W, C, Ho, Wo = _grid_inputs("dcnv3", (("input", input), ("offset", offset), ("mask", mask)), kernel_h,
+                                      kernel_w, stride_h, stride_w, pad_h, pad_w, dilation_h, dilation_w, group,
+                                      group_channels)
     P = kernel_h * kernel_w
     if tuple(offset.shape) != (N, Ho, Wo, group * P * 2):
         raise ValueError(f"dcnv3: offset shape {tuple(offset.shape)} != {(N, Ho, Wo, group * P * 2)} "
@@ -1047,3 +1058,114 @@ def dcnv3_core(input, offset, mask, kernel_h, kernel_w, stride_h, stride_w, pad_
     m = softmax over each group's P entries of `mask` if softmax_mask, else `mask` itself."""
     return DCNv3Function.apply(input, offset, mask, kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w, dilation_h,
                                dilation_w, group, group_channels, offset_scale, 256, False, softmax_mask)
+
+
+# ---- DCNv4 (the DCNv4 repository's DCNv4Function core; csrc/dcn_dcnv3.cu) ------------------------------------------
+def dcnv4_row_floats(kernel_h, kernel_w, group, remove_center=False):
+    """Cm, the floats per pixel of DCNv4's offset_mask: ceil(3*group*K / 8)*8 with K = kernel_h*kernel_w - remove_center
+    points per group."""
+    K = kernel_h * kernel_w - int(bool(remove_center))
+    return (3 * group * K + 7) // 8 * 8
+
+
+def _dcnv4_inputs(input, offset_mask, kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w, dilation_h, dilation_w,
+                  group, group_channels, remove_center):
+    """As _dcnv3_inputs, for the packed offset_mask -> (DcnV3Shape, dense 16-byte aligned input, offset_mask)."""
+    N, H, W, C, Ho, Wo = _grid_inputs("dcnv4", (("input", input), ("offset_mask", offset_mask)), kernel_h, kernel_w,
+                                      stride_h, stride_w, pad_h, pad_w, dilation_h, dilation_w, group, group_channels)
+    rc = bool(remove_center)
+    if rc and (kernel_h % 2 == 0 or kernel_w % 2 == 0):
+        raise ValueError(f"dcnv4: remove_center needs an odd kernel, got {kernel_h} x {kernel_w}")
+    K = kernel_h * kernel_w - rc
+    if K == 0:
+        raise ValueError("dcnv4: a 1 x 1 kernel with remove_center has no points (K = 0)")
+    Cm = dcnv4_row_floats(kernel_h, kernel_w, group, rc)
+    if offset_mask.dim() != 4 or tuple(offset_mask.shape[:3]) != (N, Ho, Wo):
+        raise ValueError(f"dcnv4: offset_mask shape {tuple(offset_mask.shape)} != {(N, Ho, Wo, Cm)} "
+                         f"(input {(N, H, W, C)}, {kernel_h}x{kernel_w} kernel)")
+    if int(offset_mask.shape[-1]) != Cm:
+        raise ValueError(f"dcnv4: offset_mask has {int(offset_mask.shape[-1])} floats per pixel, expected "
+                         f"Cm = ceil(3*group*K / 8)*8 = ceil(3*{group}*{K} / 8)*8 = {Cm} "
+                         f"(K = {kernel_h}*{kernel_w}{' - 1, remove_center' if rc else ''})")
+    if max(N, H, W, C) > 0x7fffffff:
+        raise ValueError(f"dcnv4: an extent of {(N, H, W, C)} exceeds 2^31 - 1")
+    shp = _lib.DcnV3Shape(N, H, W, group, group_channels, kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w,
+                          dilation_h, dilation_w, _lib.DCN_V4_FLAG_REMOVE_CENTER if rc else 0)
+    return shp, _dev_ready(input), _dev_ready(offset_mask)
+
+
+def dcn_v4_forward(input, offset_mask, kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w, dilation_h, dilation_w,
+                   group, group_channels, offset_scale, remove_center=False):
+    """out [N, Ho, Wo, group*group_channels] of the DCNv4 core on CUDA tensors (no autograd)."""
+    lib = _lib.load()
+    shp, x, om = _dcnv4_inputs(input, offset_mask, kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w, dilation_h,
+                               dilation_w, group, group_channels, remove_center)
+    out = torch.empty(tuple(om.shape[:3]) + (group * group_channels,), dtype=torch.float32, device=x.device)
+    with torch.cuda.device(x.device):
+        stream = torch.cuda.current_stream(x.device)
+        rc = lib.dcn_v4_forward(ctypes.byref(shp), float(offset_scale), _ptr(x), _ptr(om), _ptr(out),
+                                ctypes.c_void_p(stream.cuda_stream))
+    _lib.check(rc, "dcn_v4_forward")
+    return out
+
+
+def dcn_v4_backward(input, offset_mask, grad_out, kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w, dilation_h,
+                    dilation_w, group, group_channels, offset_scale, remove_center=False, need=(True, True)):
+    """(grad_input, grad_offset_mask); need[i] False -> None, not computed.  grad_offset_mask has offset_mask's packed
+    layout, with +0.0 in the padding columns."""
+    lib = _lib.load()
+    shp, x, om = _dcnv4_inputs(input, offset_mask, kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w, dilation_h,
+                               dilation_w, group, group_channels, remove_center)
+    want = tuple(om.shape[:3]) + (group * group_channels,)
+    if not isinstance(grad_out, torch.Tensor) or tuple(grad_out.shape) != want:
+        raise ValueError(f"dcnv4: grad_out shape {tuple(getattr(grad_out, 'shape', ()))} != {want}")
+    go = _dev_ready(_to_device(grad_out, x.device))
+    gx, gom = (torch.empty_like(t) if n else None for t, n in zip((x, om), need))
+    if gx is None and gom is None:
+        return None, None
+    with torch.cuda.device(x.device):
+        stream = torch.cuda.current_stream(x.device)
+        rc = lib.dcn_v4_backward(ctypes.byref(shp), float(offset_scale), _ptr(x), _ptr(om), _ptr(go), _ptr(gx),
+                                 _ptr(gom), ctypes.c_void_p(stream.cuda_stream))
+    _lib.check(rc, "dcn_v4_backward")
+    return gx, gom
+
+
+class DCNv4Function(torch.autograd.Function):
+    """The DCNv4 core as one autograd node, with the positional interface of the DCNv4 repository's ``DCNv4Function``:
+
+        DCNv4Function.apply(input, offset_mask, kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w,
+                            dilation_h, dilation_w, group, group_channels, offset_scale, im2col_step,
+                            remove_center) -> [N, Ho, Wo, group*group_channels]
+
+    input [N, H, W, group*group_channels], offset_mask [N, Ho, Wo, Cm] with Cm = ceil(3*group*K / 8)*8 and
+    K = kernel_h*kernel_w - remove_center: group g owns floats [g*3K, g*3K + 3K) of each pixel, first K interleaved
+    (dx, dy) offsets, then K mask values (used as given: no softmax); the remaining columns are padding and never read.
+    Points are DCNv3's, x-major (p = i*kernel_h + j for kernel column i and row j), with the centre point of an odd
+    kernel dropped when remove_center is set.  float32 on one CUDA device.  ``im2col_step`` is accepted and ignored.
+    Differentiable in input and offset_mask; only the gradients autograd asks for are computed, and the node never
+    synchronises with the host."""
+
+    @staticmethod
+    def forward(ctx, input, offset_mask, kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w, dilation_h, dilation_w,
+                group, group_channels, offset_scale, im2col_step=256, remove_center=False):
+        ctx.geo = (kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w, dilation_h, dilation_w, group, group_channels,
+                   offset_scale, bool(remove_center))
+        out = dcn_v4_forward(input, offset_mask, *ctx.geo)
+        ctx.save_for_backward(input, offset_mask)
+        return out
+
+    @staticmethod
+    @torch.autograd.function.once_differentiable
+    def backward(ctx, grad_output):
+        need = tuple(ctx.needs_input_grad[:2])
+        gx, gom = dcn_v4_backward(*ctx.saved_tensors, grad_output, *ctx.geo, need=need)
+        return (gx, gom) + (None,) * 13
+
+
+def dcnv4_core(input, offset_mask, kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w, dilation_h, dilation_w,
+               group, group_channels, offset_scale, remove_center=False):
+    """Differentiable DCNv4 core (see DCNv4Function): DCNv3's operator with the packed offset_mask, the mask used as
+    given, and optionally the kernel's centre point removed."""
+    return DCNv4Function.apply(input, offset_mask, kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w, dilation_h,
+                               dilation_w, group, group_channels, offset_scale, 256, remove_center)
