@@ -27,22 +27,6 @@ PHASE_LAYER_FORWARD, PHASE_LAYER_BACKWARD = 3, 4   # offset conv + DCN span (dcn
 PHASE_LAYER_FORWARD_MODULATED, PHASE_LAYER_BACKWARD_MODULATED = 5, 6
 ROI_POOL, PSROI_POOL = 0, 1                        # dcn_roi_pool_* kind (deform_conv.py:83 / :160)
 
-# every symbol include/dcn_b200.h declares (tests/test_abi.py checks the two lists agree)
-EXPORTS = (
-    "dcn_version", "dcn_last_error", "dcn_status_string", "dcn_output_hw", "dcn_workspace_bytes",
-    "dcn_path_name", "dcn_launch_count", "dcn_launch_count_reset", "dcn_profile_begin",
-    "dcn_profile_end", "dcn_forward", "dcn_backward", "dcn_forward_modulated", "dcn_backward_modulated",
-    "dcn_debug_corners", "dcn_comm_unique_id", "dcn_comm_init", "dcn_allreduce_sum_f32",
-    "dcn_comm_destroy", "dcn_bn_workspace_bytes", "dcn_bn_relu_forward", "dcn_bn_relu_backward",
-    "dcn_offset_conv_forward", "dcn_layer_forward", "dcn_layer_backward",
-    "dcn_p2p_handle_bytes", "dcn_p2p_create", "dcn_p2p_local_handle", "dcn_p2p_connect",
-    "dcn_p2p_allreduce_sum_f32", "dcn_p2p_destroy", "dcn_roi_pool_forward", "dcn_roi_pool_backward",
-    "dcn_staged_input_bytes", "dcn_staged_input_clear", "dcn_layer_forward_chained",
-    "dcn_bn_relu_forward_staged", "dcn_bn_relu_backward_staged", "dcn_stem_conv_forward", "dcn_stem_conv_backward",
-    "dcn_offset_conv_forward_modulated", "dcn_layer_forward_modulated", "dcn_layer_backward_modulated",
-    "dcn_msda_forward", "dcn_msda_backward", "dcn_v3_forward", "dcn_v3_backward", "dcn_v4_forward", "dcn_v4_backward",
-)
-
 
 class DcnShape(ctypes.Structure):
     """Mirror of include/dcn_b200.h:DcnShape."""
@@ -65,6 +49,67 @@ class DcnV3Shape(ctypes.Structure):
 DCN_V3_FLAG_SOFTMAX_MASK = 1
 DCN_V4_FLAG_REMOVE_CENTER = 2
 
+# export name -> (restype, argtypes) of every symbol include/dcn_b200.h declares; load() applies it, and
+# tests/test_binding_table.py checks it against the header's prototypes
+_i32, _f32, _sz, _vp, _str = ctypes.c_int32, ctypes.c_float, ctypes.c_size_t, ctypes.c_void_p, ctypes.c_char_p
+_i32p, _vpp = ctypes.POINTER(ctypes.c_int32), ctypes.POINTER(ctypes.c_void_p)
+_shp, _msp, _v3p = ctypes.POINTER(DcnShape), ctypes.POINTER(DcnMsdaShape), ctypes.POINTER(DcnV3Shape)
+BINDINGS = {
+    "dcn_version": (_i32, []),
+    "dcn_last_error": (_str, []),
+    "dcn_status_string": (_str, [_i32]),
+    "dcn_output_hw": (_i32, [_shp, _i32p, _i32p]),
+    "dcn_workspace_bytes": (_sz, [_shp, _i32]),
+    "dcn_path_name": (_str, [_shp, _i32]),
+    "dcn_launch_count": (ctypes.c_uint64, []),
+    "dcn_launch_count_reset": (None, []),
+    "dcn_profile_begin": (_i32, []),
+    "dcn_profile_end": (_i32, [_str, _sz]),
+    "dcn_forward": (_i32, [_shp, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "dcn_backward": (_i32, [_shp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "dcn_forward_modulated": (_i32, [_shp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "dcn_backward_modulated": (_i32, [_shp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "dcn_offset_conv_forward": (_i32, [_shp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "dcn_layer_forward": (_i32, [_shp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "dcn_layer_backward": (_i32, [_shp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "dcn_offset_conv_forward_modulated": (_i32, [_shp, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "dcn_layer_forward_modulated": (_i32, [_shp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "dcn_layer_backward_modulated": (_i32, [_shp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz,
+                                            _vp]),
+    "dcn_staged_input_bytes": (_sz, [_shp]),
+    "dcn_staged_input_clear": (_i32, [_shp, _vp, _vp]),
+    "dcn_layer_forward_chained": (_i32, [_shp, _shp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "dcn_bn_relu_forward_staged": (_i32, [_shp, _i32, _vp, _vp, _vp, _vp, _vp, _f32, _f32, _vp, _vp, _vp, _sz, _vp]),
+    "dcn_bn_relu_backward_staged": (_i32, [_shp, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "dcn_debug_corners": (_i32, [_shp, _vp, _vp, _vp, _vp, _vp]),
+    "dcn_roi_pool_forward": (_i32, [_i32, _i32, _i32, _i32, _i32, _i32, _vp, _vp, _vp, _f32, _f32, _i32, _vp, _vp]),
+    "dcn_roi_pool_backward": (_i32, [_i32, _i32, _i32, _i32, _i32, _i32, _vp, _vp, _vp, _f32, _f32, _i32, _vp, _vp,
+                                     _vp, _vp]),
+    "dcn_msda_forward": (_i32, [_msp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "dcn_msda_backward": (_i32, [_msp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "dcn_v3_forward": (_i32, [_v3p, _f32, _vp, _vp, _vp, _vp, _vp]),
+    "dcn_v3_backward": (_i32, [_v3p, _f32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "dcn_v4_forward": (_i32, [_v3p, _f32, _vp, _vp, _vp, _vp]),
+    "dcn_v4_backward": (_i32, [_v3p, _f32, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "dcn_stem_conv_forward": (_i32, [_i32, _i32, _i32, _i32, _i32, _vp, _vp, _vp, _vp, _vp]),
+    "dcn_stem_conv_backward": (_i32, [_i32, _i32, _i32, _i32, _i32, _vp, _vp, _vp, _vp, _vp]),
+    "dcn_bn_workspace_bytes": (_sz, [_i32]),
+    "dcn_bn_relu_forward": (_i32, [_i32, _i32, _i32, _i32, _vp, _vp, _vp, _vp, _vp, _f32, _f32, _vp, _vp, _vp, _sz,
+                                   _vp]),
+    "dcn_bn_relu_backward": (_i32, [_i32, _i32, _i32, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "dcn_comm_unique_id": (_i32, [_vp]),
+    "dcn_comm_init": (_i32, [_i32, _i32, _vp, _vpp]),
+    "dcn_allreduce_sum_f32": (_i32, [_vp, _vp, _sz, _f32, _vp]),
+    "dcn_comm_destroy": (_i32, [_vp]),
+    "dcn_p2p_handle_bytes": (_sz, []),
+    "dcn_p2p_create": (_i32, [_i32, _i32, _sz, _vpp]),
+    "dcn_p2p_local_handle": (_i32, [_vp, _vp]),
+    "dcn_p2p_connect": (_i32, [_vp, _vp]),
+    "dcn_p2p_allreduce_sum_f32": (_i32, [_vp, _vp, _sz, _f32, _vp]),
+    "dcn_p2p_destroy": (_i32, [_vp]),
+}
+EXPORTS = tuple(BINDINGS)
+
 
 class DcnError(RuntimeError):
     pass
@@ -83,64 +128,9 @@ def load():
             f"{LIB_PATH} is missing: the CUDA engine is not built and there is no CPU fallback. "
             "Run `python -m jittor_dcn_b200.build` (needs nvcc).")
     lib = ctypes.CDLL(LIB_PATH)
-    vp, sz, i32p = ctypes.c_void_p, ctypes.c_size_t, ctypes.POINTER(ctypes.c_int32)
-    shp = ctypes.POINTER(DcnShape)
-    lib.dcn_version.restype = ctypes.c_int
-    lib.dcn_last_error.restype = ctypes.c_char_p
-    lib.dcn_status_string.restype = ctypes.c_char_p
-    lib.dcn_status_string.argtypes = [ctypes.c_int]
-    lib.dcn_output_hw.argtypes = [shp, i32p, i32p]
-    lib.dcn_workspace_bytes.restype = sz
-    lib.dcn_workspace_bytes.argtypes = [shp, ctypes.c_int]
-    lib.dcn_path_name.restype = ctypes.c_char_p
-    lib.dcn_path_name.argtypes = [shp, ctypes.c_int]
-    lib.dcn_launch_count.restype = ctypes.c_uint64
-    lib.dcn_launch_count_reset.restype = None
-    lib.dcn_profile_end.argtypes = [ctypes.c_char_p, sz]
-    lib.dcn_forward.argtypes = [shp, vp, vp, vp, vp, vp, vp, sz, vp]
-    lib.dcn_backward.argtypes = [shp, vp, vp, vp, vp, vp, vp, vp, vp, vp, sz, vp]
-    lib.dcn_forward_modulated.argtypes = [shp, vp, vp, vp, vp, vp, vp, vp, sz, vp]
-    lib.dcn_backward_modulated.argtypes = [shp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, sz, vp]
-    lib.dcn_debug_corners.argtypes = [shp, vp, vp, vp, vp, vp]
-    lib.dcn_offset_conv_forward.argtypes = [shp, vp, vp, vp, vp, vp, sz, vp]
-    lib.dcn_layer_forward.argtypes = [shp, vp, vp, vp, vp, vp, vp, vp, vp, sz, vp]
-    lib.dcn_layer_backward.argtypes = [shp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, sz, vp]
-    lib.dcn_offset_conv_forward_modulated.argtypes = [shp, vp, vp, vp, vp, vp, vp, sz, vp]
-    lib.dcn_layer_forward_modulated.argtypes = [shp, vp, vp, vp, vp, vp, vp, vp, vp, vp, sz, vp]
-    lib.dcn_layer_backward_modulated.argtypes = [shp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, sz, vp]
-    msp = ctypes.POINTER(DcnMsdaShape)
-    lib.dcn_msda_forward.argtypes = [msp, vp, vp, vp, vp, vp, vp, vp]
-    lib.dcn_msda_backward.argtypes = [msp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp]
-    v3p, f32 = ctypes.POINTER(DcnV3Shape), ctypes.c_float
-    lib.dcn_v3_forward.argtypes = [v3p, f32, vp, vp, vp, vp, vp]
-    lib.dcn_v3_backward.argtypes = [v3p, f32, vp, vp, vp, vp, vp, vp, vp, vp]
-    lib.dcn_v4_forward.argtypes = [v3p, f32, vp, vp, vp, vp]
-    lib.dcn_v4_backward.argtypes = [v3p, f32, vp, vp, vp, vp, vp, vp]
-    lib.dcn_comm_unique_id.argtypes = [vp]
-    lib.dcn_comm_init.argtypes = [ctypes.c_int, ctypes.c_int, vp, ctypes.POINTER(vp)]
-    lib.dcn_allreduce_sum_f32.argtypes = [vp, vp, sz, ctypes.c_float, vp]
-    lib.dcn_comm_destroy.argtypes = [vp]
-    lib.dcn_p2p_handle_bytes.restype = sz
-    lib.dcn_p2p_create.argtypes = [ctypes.c_int, ctypes.c_int, sz, ctypes.POINTER(vp)]
-    lib.dcn_p2p_local_handle.argtypes = [vp, vp]
-    lib.dcn_p2p_connect.argtypes = [vp, vp]
-    lib.dcn_p2p_allreduce_sum_f32.argtypes = [vp, vp, sz, ctypes.c_float, vp]
-    lib.dcn_p2p_destroy.argtypes = [vp]
-    i32, f32 = ctypes.c_int32, ctypes.c_float
-    lib.dcn_bn_workspace_bytes.restype = sz
-    lib.dcn_bn_workspace_bytes.argtypes = [i32]
-    lib.dcn_bn_relu_forward.argtypes = [i32, i32, i32, i32, vp, vp, vp, vp, vp, f32, f32, vp, vp, vp, sz, vp]
-    lib.dcn_bn_relu_backward.argtypes = [i32, i32, i32, i32, vp, vp, vp, vp, vp, vp, vp, sz, vp]
-    lib.dcn_bn_relu_forward_staged.argtypes = [shp, i32, vp, vp, vp, vp, vp, f32, f32, vp, vp, vp, sz, vp]
-    lib.dcn_bn_relu_backward_staged.argtypes = [shp, i32, vp, vp, vp, vp, vp, vp, vp, sz, vp]
-    lib.dcn_staged_input_bytes.restype = sz
-    lib.dcn_staged_input_bytes.argtypes = [shp]
-    lib.dcn_staged_input_clear.argtypes = [shp, vp, vp]
-    lib.dcn_layer_forward_chained.argtypes = [shp, shp, vp, vp, vp, vp, vp, vp, vp, vp, sz, vp]
-    lib.dcn_roi_pool_forward.argtypes = [i32, i32, i32, i32, i32, i32, vp, vp, vp, f32, f32, i32, vp, vp]
-    lib.dcn_roi_pool_backward.argtypes = [i32, i32, i32, i32, i32, i32, vp, vp, vp, f32, f32, i32, vp, vp, vp, vp]
-    lib.dcn_stem_conv_forward.argtypes = [i32, i32, i32, i32, i32, vp, vp, vp, vp, vp]
-    lib.dcn_stem_conv_backward.argtypes = [i32, i32, i32, i32, i32, vp, vp, vp, vp, vp]
+    for name, (restype, argtypes) in BINDINGS.items():
+        fn = getattr(lib, name)
+        fn.restype, fn.argtypes = restype, argtypes
     _lib = lib
     return lib
 

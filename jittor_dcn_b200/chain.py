@@ -13,7 +13,7 @@ import torch
 import torch.nn as nn
 
 from . import _lib
-from .functional import _dev_ready, _ptr
+from .functional import _dev_ready, _run
 from .torch_module import fuse_eval_bn_relu
 
 
@@ -41,10 +41,8 @@ class ChainedDeformStages(nn.Module):
             off = torch.empty((B, 2 * layer.N, Ho, Wo), dtype=torch.float32, device=x.device)
             plan.append(dict(shape=shp, ws=ws, off=off, out_hw=(Ho, Wo)))
             C, H, W = layer.out_channels, Ho, Wo
-        stream = ctypes.c_void_p(torch.cuda.current_stream(x.device).cuda_stream)
         for st in plan[1:]:     # the frame of every chained input is zeroed once; the epilogues write interior pixels only
-            _lib.check(lib.dcn_staged_input_clear(ctypes.byref(st["shape"]), _ptr(st["ws"]), stream),
-                       "dcn_staged_input_clear")
+            _run("dcn_staged_input_clear", x.device, st["shape"], (st["ws"],))
         self._plan = (tuple(x.shape), x.device, plan)
         return plan
 
@@ -52,30 +50,23 @@ class ChainedDeformStages(nn.Module):
     def forward(self, x):
         if not x.is_cuda or x.dtype != torch.float32 or x.dim() != 4:
             raise ValueError("ChainedDeformStages expects a float32 NCHW CUDA tensor")
-        lib = _lib.load()
         x = _dev_ready(x)
         plan = self._plan[2] if self._plan and self._plan[0] == tuple(x.shape) and self._plan[1] == x.device \
             else self._build(x)
-        with torch.cuda.device(x.device):
-            stream = ctypes.c_void_p(torch.cuda.current_stream(x.device).cuda_stream)
-            last = len(plan) - 1
-            out = None
-            for i, (layer, st) in enumerate(zip(self.layers, plan)):
-                shp = st["shape"]
-                shp.flags = layer.engine_flags | _lib.FLAG_RELU_OUT | (_lib.FLAG_XT_STAGED if i > 0 else 0)
-                src = x if i == 0 else st["ws"]           # chained stages never read `x`: their input is staged
-                ow, ob = layer.offset_conv.weight, layer.offset_conv.bias
-                if i < last:
-                    rc = lib.dcn_layer_forward_chained(
-                        ctypes.byref(shp), ctypes.byref(plan[i + 1]["shape"]), _ptr(src), _ptr(ow), _ptr(ob),
-                        _ptr(layer.weight), _ptr(layer.bias), _ptr(st["off"]), _ptr(plan[i + 1]["ws"]), _ptr(st["ws"]),
-                        st["ws"].numel(), stream)
-                    _lib.check(rc, "dcn_layer_forward_chained")
-                else:
-                    Ho, Wo = st["out_hw"]
-                    out = torch.empty((shp.B, shp.O, Ho, Wo), dtype=torch.float32, device=x.device)
-                    rc = lib.dcn_layer_forward(ctypes.byref(shp), _ptr(src), _ptr(ow), _ptr(ob), _ptr(layer.weight),
-                                               _ptr(layer.bias), _ptr(st["off"]), _ptr(out), _ptr(st["ws"]),
-                                               st["ws"].numel(), stream)
-                    _lib.check(rc, "dcn_layer_forward")
+        last = len(plan) - 1
+        out = None
+        for i, (layer, st) in enumerate(zip(self.layers, plan)):
+            shp = st["shape"]
+            shp.flags = layer.engine_flags | _lib.FLAG_RELU_OUT | (_lib.FLAG_XT_STAGED if i > 0 else 0)
+            src = x if i == 0 else st["ws"]           # chained stages never read `x`: their input is staged
+            ow, ob = layer.offset_conv.weight, layer.offset_conv.bias
+            if i < last:
+                _run("dcn_layer_forward_chained", x.device, shp,
+                     (plan[i + 1]["shape"], src, ow, ob, layer.weight, layer.bias, st["off"], plan[i + 1]["ws"]),
+                     ws=st["ws"])
+            else:
+                Ho, Wo = st["out_hw"]
+                out = torch.empty((shp.B, shp.O, Ho, Wo), dtype=torch.float32, device=x.device)
+                _run("dcn_layer_forward", x.device, shp, (src, ow, ob, layer.weight, layer.bias, st["off"], out),
+                     ws=st["ws"])
         return out

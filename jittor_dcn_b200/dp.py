@@ -13,6 +13,7 @@ import torch
 import torch.distributed as dist
 
 from . import _lib
+from .functional import _run
 
 
 def shard_range(global_batch, rank, world):
@@ -81,11 +82,7 @@ class DcnComm:
 
     def allreduce_sum_(self, flat, scale=1.0):
         """flat <- scale * sum over ranks, in place, on the current stream (capturable in a CUDA graph)."""
-        stream = torch.cuda.current_stream(self.device)
-        _lib.check(self.lib.dcn_allreduce_sum_f32(self.handle, ctypes.c_void_p(flat.data_ptr()),
-                                                  flat.numel(), float(scale),
-                                                  ctypes.c_void_p(stream.cuda_stream)),
-                   "dcn_allreduce_sum_f32")
+        _run("dcn_allreduce_sum_f32", self.device, None, (self.handle, flat, flat.numel(), float(scale)))
         return flat
 
     def close(self):
@@ -122,10 +119,7 @@ class DcnP2P:
         return self.allreduce_sum_(flat, 1.0 / self.world)
 
     def allreduce_sum_(self, flat, scale=1.0):
-        stream = torch.cuda.current_stream(self.device)
-        _lib.check(self.lib.dcn_p2p_allreduce_sum_f32(self.handle, ctypes.c_void_p(flat.data_ptr()), flat.numel(),
-                                                      float(scale), ctypes.c_void_p(stream.cuda_stream)),
-                   "dcn_p2p_allreduce_sum_f32")
+        _run("dcn_p2p_allreduce_sum_f32", self.device, None, (self.handle, flat, flat.numel(), float(scale)))
         return flat
 
     def close(self):

@@ -53,10 +53,6 @@ def _dev_ready(t, dtype=torch.float32):
     return t
 
 
-def _ptr(t):
-    return None if t is None else ctypes.c_void_p(t.data_ptr())
-
-
 def _compute_device(x):
     if x.is_cuda:
         return x.device
@@ -101,18 +97,22 @@ def staged_workspace(x, weight, kernel_size=3, stride=1, padding=1, variant=VARI
     return torch.empty(need, dtype=torch.uint8, device=x.device)
 
 
-def _run(entry, dev, shp, tensors, phase=None, ws=None):
-    """lib.<entry>(shape, *tensors[, workspace, workspace_bytes], stream) on the current stream of `dev`, then its status
-    checked.  phase: the call takes a workspace, `ws` or else the cached scratch buffer sized for that phase."""
+def _run(entry, dev, shp, args, phase=None, ws=None):
+    """lib.<entry>(shp, *args[, workspace, workspace_bytes], stream) under the device guard of `dev` on its current
+    stream, then its status checked.  shp: the shape structure the entry point takes first, None for one that takes
+    none.  Tensors pass as their device pointers, ctypes structures by reference, None as NULL and everything else as
+    it is.  The call takes a workspace when `ws` or `phase` is given: `ws`, or else the cached scratch buffer that
+    `phase` needs for `shp`."""
     lib = _lib.load()
-    args = tuple(_ptr(t) for t in tensors)
+    args = [ctypes.c_void_p(a.data_ptr()) if isinstance(a, torch.Tensor) else
+            ctypes.byref(a) if isinstance(a, ctypes.Structure) else a for a in (args if shp is None else (shp, *args))]
     with torch.cuda.device(dev):
         stream = torch.cuda.current_stream(dev)
-        if phase is not None:
-            if ws is None:
-                ws = _workspace(dev, stream.cuda_stream, lib.dcn_workspace_bytes(ctypes.byref(shp), phase))
-            args += (_ptr(ws), ws.numel())
-        rc = getattr(lib, entry)(ctypes.byref(shp), *args, ctypes.c_void_p(stream.cuda_stream))
+        if ws is None and phase is not None:
+            ws = _workspace(dev, stream.cuda_stream, lib.dcn_workspace_bytes(args[0], phase))
+        if ws is not None:
+            args += [ctypes.c_void_p(ws.data_ptr()), ws.numel()]
+        rc = getattr(lib, entry)(*args, ctypes.c_void_p(stream.cuda_stream))
     _lib.check(rc, entry)
 
 
@@ -173,9 +173,9 @@ def _span_forward(x, offset, mask, weight, bias, kernel_size, stride, padding, v
     offset, mask, bias = _dev_ready(offset), _dev_ready(mask), _dev_ready(bias)
     out = torch.empty((shp.B, shp.O, Ho, Wo), dtype=torch.float32, device=x.device)
     if mask is None:
-        _run("dcn_forward", x.device, shp, (x, offset, weight, bias, out), PHASE_FORWARD, ws)
+        _run("dcn_forward", x.device, shp, (x, offset, weight, bias, out), phase=PHASE_FORWARD, ws=ws)
     else:
-        _run("dcn_forward_modulated", x.device, shp, (x, offset, mask, weight, bias, out), PHASE_FORWARD, ws)
+        _run("dcn_forward_modulated", x.device, shp, (x, offset, mask, weight, bias, out), phase=PHASE_FORWARD, ws=ws)
     return out
 
 
@@ -210,11 +210,11 @@ def _span_backward(x, offset, mask, weight, grad_out, has_bias, kernel_size, str
     gb = torch.empty((shp.O,), dtype=torch.float32, device=dev) if has_bias else None
     if mask is None:
         gmask = None
-        _run("dcn_backward", dev, shp, (x, offset, weight, grad_out, gx, goff, gw, gb), PHASE_BACKWARD, ws)
+        _run("dcn_backward", dev, shp, (x, offset, weight, grad_out, gx, goff, gw, gb), phase=PHASE_BACKWARD, ws=ws)
     else:
         gmask = torch.empty((shp.B, N, Ho, Wo), dtype=torch.float32, device=dev)
         _run("dcn_backward_modulated", dev, shp, (x, offset, mask, weight, grad_out, gx, goff, gmask, gw, gb),
-             PHASE_BACKWARD, ws)
+             phase=PHASE_BACKWARD, ws=ws)
     return gx, goff, gmask, gw, gb
 
 
@@ -322,10 +322,14 @@ def _layer_supported(x_shape, out_channels, kernel_size, stride, padding, varian
 
 
 def _layer_workspace(x, weight, kernel_size, stride, padding, variant, flags, modulated):
-    lib = _lib.load()
     shp = _shape_of(x, weight, kernel_size, stride, padding, variant, OPERAND_FP32, flags)
-    need = max(lib.dcn_workspace_bytes(ctypes.byref(shp), ph) for ph in _PHASES[modulated])
-    return torch.empty(need, dtype=torch.uint8, device=x.device)
+    return torch.empty(_layer_bytes(shp, modulated), dtype=torch.uint8, device=x.device)
+
+
+def _layer_bytes(shp, modulated=False):
+    """Bytes of one workspace for both calls of the layer; 0 when it does not run on the tensor path."""
+    lib = _lib.load()
+    return max(lib.dcn_workspace_bytes(ctypes.byref(shp), ph) for ph in _PHASES[modulated])
 
 
 def _check_offset_weight(offset_weight, shp, modulated):
@@ -349,11 +353,12 @@ def _offset_conv_forward(x, offset_weight, offset_bias, out_channels, kernel_siz
     x, offset_weight, offset_bias = _dev_ready(x), _dev_ready(offset_weight), _dev_ready(offset_bias)
     offset = torch.empty((B, 2 * N, Ho, Wo), dtype=torch.float32, device=x.device)
     if not modulated:
-        _run("dcn_offset_conv_forward", x.device, shp, (x, offset_weight, offset_bias, offset), PHASE_LAYER_FORWARD, ws)
+        _run("dcn_offset_conv_forward", x.device, shp, (x, offset_weight, offset_bias, offset),
+             phase=PHASE_LAYER_FORWARD, ws=ws)
         return offset, None
     mask = torch.empty((B, N, Ho, Wo), dtype=torch.float32, device=x.device)
     _run("dcn_offset_conv_forward_modulated", x.device, shp, (x, offset_weight, offset_bias, offset, mask),
-         PHASE_LAYER_FORWARD_MODULATED, ws)
+         phase=PHASE_LAYER_FORWARD_MODULATED, ws=ws)
     return offset, mask
 
 
@@ -361,20 +366,25 @@ def _layer_forward(x, offset_weight, offset_bias, weight, bias, kernel_size, str
                    modulated):
     """-> (offset, mask or None, out)"""
     shp = _shape_of(x, weight, kernel_size, stride, padding, variant, OPERAND_FP32, flags)
+    return _layer_forward_shaped(shp, _dev_ready(x), offset_weight, offset_bias, weight, bias, ws, modulated)
+
+
+def _layer_forward_shaped(shp, x, offset_weight, offset_bias, weight, bias, ws, modulated):
+    """_layer_forward once the shape is built; x is the dense input, or the workspace whose head holds it staged."""
     Ho, Wo = _lib.output_hw(shp)
     N = shp.kh * shp.kw
     _check_offset_weight(offset_weight, shp, modulated)
-    x, weight, bias = _dev_ready(x), _dev_ready(weight), _dev_ready(bias)
+    weight, bias = _dev_ready(weight), _dev_ready(bias)
     offset_weight, offset_bias = _dev_ready(offset_weight), _dev_ready(offset_bias)
     offset = torch.empty((shp.B, 2 * N, Ho, Wo), dtype=torch.float32, device=x.device)
     out = torch.empty((shp.B, shp.O, Ho, Wo), dtype=torch.float32, device=x.device)
     if not modulated:
         _run("dcn_layer_forward", x.device, shp, (x, offset_weight, offset_bias, weight, bias, offset, out),
-             PHASE_LAYER_FORWARD, ws)
+             phase=PHASE_LAYER_FORWARD, ws=ws)
         return offset, None, out
     mask = torch.empty((shp.B, N, Ho, Wo), dtype=torch.float32, device=x.device)
     _run("dcn_layer_forward_modulated", x.device, shp, (x, offset_weight, offset_bias, weight, bias, offset, mask, out),
-         PHASE_LAYER_FORWARD_MODULATED, ws)
+         phase=PHASE_LAYER_FORWARD_MODULATED, ws=ws)
     return offset, mask, out
 
 
@@ -386,22 +396,29 @@ def _layer_backward(x, offset, mask, offset_weight, weight, grad_out, has_offset
     if xt_staged and ws is not None:
         flags |= FLAG_XT_STAGED
     shp = _shape_of(x, weight, kernel_size, stride, padding, variant, OPERAND_FP32, flags)
+    x = _dev_ready(x)
+    gx = torch.empty(x.shape, dtype=torch.float32, device=x.device) if need_grad_x else None
+    return _layer_backward_shaped(shp, x, gx, offset, mask, offset_weight, weight, grad_out, has_offset_bias, has_bias,
+                                  ws)
+
+
+def _layer_backward_shaped(shp, x, gx, offset, mask, offset_weight, weight, grad_out, has_offset_bias, has_bias, ws):
+    """_layer_backward once the shape is built; x as in _layer_forward_shaped, gx its gradient buffer or None."""
     _check_offset_weight(offset_weight, shp, mask is not None)
-    x, weight, grad_out = _dev_ready(x), _dev_ready(weight), _dev_ready(grad_out)
+    weight, grad_out = _dev_ready(weight), _dev_ready(grad_out)
     offset, mask, offset_weight = _dev_ready(offset), _dev_ready(mask), _dev_ready(offset_weight)
     dev = x.device
-    gx = torch.empty(x.shape, dtype=torch.float32, device=dev) if need_grad_x else None
     gwoff = torch.empty(offset_weight.shape, dtype=torch.float32, device=dev)
     gboff = torch.empty((offset_weight.shape[0],), dtype=torch.float32, device=dev) if has_offset_bias else None
     gw = torch.empty(weight.shape, dtype=torch.float32, device=dev)
     gb = torch.empty((shp.O,), dtype=torch.float32, device=dev) if has_bias else None
     if mask is None:
         _run("dcn_layer_backward", dev, shp, (x, offset, offset_weight, weight, grad_out, gx, gwoff, gboff, gw, gb),
-             PHASE_LAYER_BACKWARD, ws)
+             phase=PHASE_LAYER_BACKWARD, ws=ws)
     else:
         _run("dcn_layer_backward_modulated", dev, shp,
-             (x, offset, mask, offset_weight, weight, grad_out, gx, gwoff, gboff, gw, gb), PHASE_LAYER_BACKWARD_MODULATED,
-             ws)
+             (x, offset, mask, offset_weight, weight, grad_out, gx, gwoff, gboff, gw, gb),
+             phase=PHASE_LAYER_BACKWARD_MODULATED, ws=ws)
     return gx, gwoff, gboff, gw, gb
 
 
@@ -559,7 +576,6 @@ class BatchNormReLUFunction(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, x, weight, bias, running_mean, running_var, training, momentum, eps):
-        lib = _lib.load()
         home = x.device
         dev = _compute_device(x)
         xd = _dev_ready(_to_device(x, dev))
@@ -569,14 +585,9 @@ class BatchNormReLUFunction(torch.autograd.Function):
         rm, rv = _to_device(running_mean, dev), _to_device(running_var, dev)
         y = torch.empty_like(xd)
         saved = torch.empty(4 * C, dtype=torch.float32, device=dev)
-        with torch.cuda.device(dev):
-            stream = torch.cuda.current_stream(dev)
-            need = lib.dcn_bn_workspace_bytes(C)
-            ws = torch.empty(need, dtype=torch.uint8, device=dev)
-            rc = lib.dcn_bn_relu_forward(B, C, HW, 1 if training else 0, _ptr(xd), _ptr(wd), _ptr(bd), _ptr(rm),
-                                         _ptr(rv), float(momentum), float(eps), _ptr(y), _ptr(saved), _ptr(ws),
-                                         ws.numel(), ctypes.c_void_p(stream.cuda_stream))
-        _lib.check(rc, "dcn_bn_relu_forward")
+        _run("dcn_bn_relu_forward", dev, None,
+             (B, C, HW, 1 if training else 0, xd, wd, bd, rm, rv, float(momentum), float(eps), y, saved),
+             ws=_bn_workspace(dev, C))
         if training and running_mean is not None and rm is not running_mean:
             running_mean.copy_(rm)       # host-resident module: write the updated statistics back
             running_var.copy_(rv)
@@ -587,28 +598,34 @@ class BatchNormReLUFunction(torch.autograd.Function):
 
     @staticmethod
     def backward(ctx, grad_y):
-        lib = _lib.load()
         xd, saved = ctx.saved_tensors
         dev = xd.device
         B, C = xd.shape[0], xd.shape[1]
         HW = xd.numel() // (B * C)
         gy = _dev_ready(_to_device(grad_y, dev))
-        gx = torch.empty_like(xd) if ctx.needs_input_grad[0] else None
-        gg = torch.empty(C, dtype=torch.float32, device=dev) if ctx.has_affine[0] else None
-        gb = torch.empty(C, dtype=torch.float32, device=dev) if ctx.has_affine[1] else None
-        with torch.cuda.device(dev):
-            stream = torch.cuda.current_stream(dev)
-            ws = torch.empty(lib.dcn_bn_workspace_bytes(C), dtype=torch.uint8, device=dev)
-            rc = lib.dcn_bn_relu_backward(B, C, HW, 1 if ctx.training else 0, _ptr(xd), _ptr(gy), _ptr(saved),
-                                          _ptr(gx), _ptr(gg), _ptr(gb), _ptr(ws), ws.numel(),
-                                          ctypes.c_void_p(stream.cuda_stream))
-        _lib.check(rc, "dcn_bn_relu_backward")
+        gx, gg, gb = _bn_grads(ctx, xd)
+        _run("dcn_bn_relu_backward", dev, None, (B, C, HW, 1 if ctx.training else 0, xd, gy, saved, gx, gg, gb),
+             ws=_bn_workspace(dev, C))
         home = ctx.home
 
         def back(t):
             return t if t is None or home == dev else t.to(home)
 
         return back(gx), back(gg), back(gb), None, None, None, None, None
+
+
+def _bn_workspace(dev, C):
+    """The scratch buffer the BatchNorm kernels take for C channels."""
+    return torch.empty(_lib.load().dcn_bn_workspace_bytes(C), dtype=torch.uint8, device=dev)
+
+
+def _bn_grads(ctx, x):
+    """The BatchNorm backward's outputs for input x: grad_x if autograd wants it, grad_gamma / grad_beta for the affine
+    parameters the node was given (None otherwise)."""
+    C = x.shape[1]
+    gx = torch.empty_like(x) if ctx.needs_input_grad[0] else None
+    gg, gb = (torch.empty(C, dtype=torch.float32, device=x.device) if has else None for has in ctx.has_affine)
+    return gx, gg, gb
 
 
 def batch_norm_relu(x, weight, bias, running_mean, running_var, training, momentum=0.1, eps=1e-5):
@@ -634,34 +651,24 @@ class StemConvFunction(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, x, weight, bias):
-        lib = _lib.load()
         xd, wd = _dev_ready(x), _dev_ready(weight)
         bd = _dev_ready(bias) if bias is not None else None
         B, Cin, H, W = xd.shape
         O = wd.shape[0]
         out = torch.empty(B, O, H, W, dtype=torch.float32, device=xd.device)
-        with torch.cuda.device(xd.device):
-            stream = torch.cuda.current_stream(xd.device)
-            rc = lib.dcn_stem_conv_forward(B, Cin, O, H, W, _ptr(xd), _ptr(wd), _ptr(bd), _ptr(out),
-                                           ctypes.c_void_p(stream.cuda_stream))
-        _lib.check(rc, "dcn_stem_conv_forward")
+        _run("dcn_stem_conv_forward", xd.device, None, (B, Cin, O, H, W, xd, wd, bd, out))
         ctx.save_for_backward(xd)
         ctx.O, ctx.has_bias = O, bias is not None
         return out
 
     @staticmethod
     def backward(ctx, grad_out):
-        lib = _lib.load()
         xd, = ctx.saved_tensors
         B, Cin, H, W = xd.shape
         go = _dev_ready(grad_out)
         gw = torch.empty(ctx.O, Cin, 3, 3, dtype=torch.float32, device=xd.device)
         gb = torch.empty(ctx.O, dtype=torch.float32, device=xd.device)
-        with torch.cuda.device(xd.device):
-            stream = torch.cuda.current_stream(xd.device)
-            rc = lib.dcn_stem_conv_backward(B, Cin, ctx.O, H, W, _ptr(xd), _ptr(go), _ptr(gw), _ptr(gb),
-                                            ctypes.c_void_p(stream.cuda_stream))
-        _lib.check(rc, "dcn_stem_conv_backward")
+        _run("dcn_stem_conv_backward", xd.device, None, (B, Cin, ctx.O, H, W, xd, go, gw, gb))
         return None, gw, gb if ctx.has_bias else None
 
 
@@ -692,48 +699,31 @@ class BatchNormReLUStagedFunction(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, x, weight, bias, running_mean, running_var, training, momentum, eps, consumer):
-        lib = _lib.load()
         x = _dev_ready(x)
         B, C, H, W = x.shape
         shp = _consumer_shape(x.shape, consumer)
-        need = max(lib.dcn_workspace_bytes(ctypes.byref(shp), PHASE_LAYER_FORWARD),
-                   lib.dcn_workspace_bytes(ctypes.byref(shp), PHASE_LAYER_BACKWARD))
+        need = _layer_bytes(shp)
         if need == 0:
             raise _lib.DcnError("staged post-op: the consumer layer does not run on the tensor path")
         dev = x.device
-        ws = torch.empty(need, dtype=torch.uint8, device=dev)
+        consumer_ws = torch.empty(need, dtype=torch.uint8, device=dev)
         saved = torch.empty(4 * C, dtype=torch.float32, device=dev)
-        with torch.cuda.device(dev):
-            stream = torch.cuda.current_stream(dev)
-            bws = torch.empty(lib.dcn_bn_workspace_bytes(C), dtype=torch.uint8, device=dev)
-            rc = lib.dcn_bn_relu_forward_staged(ctypes.byref(shp), 1 if training else 0, _ptr(x), _ptr(weight), _ptr(bias),
-                                                _ptr(running_mean), _ptr(running_var), float(momentum), float(eps),
-                                                _ptr(ws), _ptr(saved), _ptr(bws), bws.numel(),
-                                                ctypes.c_void_p(stream.cuda_stream))
-        _lib.check(rc, "dcn_bn_relu_forward_staged")
+        _run("dcn_bn_relu_forward_staged", dev, shp,
+             (1 if training else 0, x, weight, bias, running_mean, running_var, float(momentum), float(eps),
+              consumer_ws, saved), ws=_bn_workspace(dev, C))
         ctx.save_for_backward(x, saved)
         ctx.consumer, ctx.training = consumer, bool(training)
         ctx.has_affine = (weight is not None, bias is not None)
-        return _framed_view(ws, B, H, W, C)
+        return _framed_view(consumer_ws, B, H, W, C)
 
     @staticmethod
     def backward(ctx, grad_staged):
-        lib = _lib.load()
         x, saved = ctx.saved_tensors
-        C = x.shape[1]
-        dev = x.device
         shp = _consumer_shape(x.shape, ctx.consumer)
         g = _dev_ready(grad_staged)
-        gx = torch.empty_like(x) if ctx.needs_input_grad[0] else None
-        gg = torch.empty(C, dtype=torch.float32, device=dev) if ctx.has_affine[0] else None
-        gb = torch.empty(C, dtype=torch.float32, device=dev) if ctx.has_affine[1] else None
-        with torch.cuda.device(dev):
-            stream = torch.cuda.current_stream(dev)
-            bws = torch.empty(lib.dcn_bn_workspace_bytes(C), dtype=torch.uint8, device=dev)
-            rc = lib.dcn_bn_relu_backward_staged(ctypes.byref(shp), 1 if ctx.training else 0, _ptr(x), _ptr(g), _ptr(saved),
-                                                 _ptr(gx), _ptr(gg), _ptr(gb), _ptr(bws), bws.numel(),
-                                                 ctypes.c_void_p(stream.cuda_stream))
-        _lib.check(rc, "dcn_bn_relu_backward_staged")
+        gx, gg, gb = _bn_grads(ctx, x)
+        _run("dcn_bn_relu_backward_staged", x.device, shp, (1 if ctx.training else 0, x, g, saved, gx, gg, gb),
+             ws=_bn_workspace(x.device, x.shape[1]))
         return gx, gg, gb, None, None, None, None, None, None
 
 
@@ -748,7 +738,6 @@ class DeformLayerFramedFunction(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, xt, offset_weight, offset_bias, weight, bias, cfg):
-        lib = _lib.load()
         (C, H, W), kernel_size, stride, padding, variant, flags = cfg
         B = int(xt.shape[0])
         if tuple(xt.shape) != (B, H + 3, W + 2, C) or xt.dtype != torch.float32 or not xt.is_contiguous():
@@ -756,19 +745,10 @@ class DeformLayerFramedFunction(torch.autograd.Function):
         ws = _storage_tensor(xt)
         shp = _lib.make_shape(B, C, int(weight.shape[0]), H, W, kernel_size, stride, padding, variant, OPERAND_FP32,
                               flags | FLAG_XT_STAGED)
-        need = max(lib.dcn_workspace_bytes(ctypes.byref(shp), PHASE_LAYER_FORWARD),
-                   lib.dcn_workspace_bytes(ctypes.byref(shp), PHASE_LAYER_BACKWARD))
+        need = _layer_bytes(shp)
         if need == 0 or ws.numel() < need or xt.data_ptr() != ws.data_ptr():
             raise _lib.DcnError("staged input is not the head of a workspace of this layer")
-        Ho, Wo = _lib.output_hw(shp)
-        N = shp.kh * shp.kw
-        dev = xt.device
-        weight, bias = _dev_ready(weight), _dev_ready(bias)
-        offset_weight, offset_bias = _dev_ready(offset_weight), _dev_ready(offset_bias)
-        offset = torch.empty((B, 2 * N, Ho, Wo), dtype=torch.float32, device=dev)
-        out = torch.empty((B, shp.O, Ho, Wo), dtype=torch.float32, device=dev)
-        _run("dcn_layer_forward", dev, shp, (ws, offset_weight, offset_bias, weight, bias, offset, out),
-             PHASE_LAYER_FORWARD, ws)
+        offset, _, out = _layer_forward_shaped(shp, ws, offset_weight, offset_bias, weight, bias, ws, False)
         ctx.relu = bool(flags & FLAG_RELU_OUT)
         ctx.save_for_backward(xt, offset, offset_weight, weight, *((out,) if ctx.relu else ()))
         ctx.cfg = cfg
@@ -781,21 +761,14 @@ class DeformLayerFramedFunction(torch.autograd.Function):
         if ctx.relu:
             grad_out = grad_out * (ctx.saved_tensors[4] > 0)
         (C, H, W), kernel_size, stride, padding, variant, flags = ctx.cfg
-        B = int(xt.shape[0])
         ws = _storage_tensor(xt)
         need_gx = ctx.needs_input_grad[0]
         fl = (flags & ~FLAG_ACCUM_GRAD_X) | FLAG_XT_STAGED | _lib.FLAG_GRAD_X_FRAMED | (0 if need_gx else FLAG_NO_GRAD_X)
-        shp = _lib.make_shape(B, C, int(weight.shape[0]), H, W, kernel_size, stride, padding, variant, OPERAND_FP32, fl)
-        dev = xt.device
-        grad_out = _dev_ready(grad_out)
+        shp = _lib.make_shape(int(xt.shape[0]), C, int(weight.shape[0]), H, W, kernel_size, stride, padding, variant,
+                              OPERAND_FP32, fl)
         gxt = torch.empty_like(xt) if need_gx else None
-        gwoff = torch.empty(offset_weight.shape, dtype=torch.float32, device=dev)
-        gboff = torch.empty((offset_weight.shape[0],), dtype=torch.float32, device=dev) if ctx.has[0] else None
-        gw = torch.empty(weight.shape, dtype=torch.float32, device=dev)
-        gb = torch.empty((shp.O,), dtype=torch.float32, device=dev) if ctx.has[1] else None
-        _run("dcn_layer_backward", dev, shp, (ws, offset, offset_weight, weight, grad_out, gxt, gwoff, gboff, gw, gb),
-             PHASE_LAYER_BACKWARD, ws)
-        return gxt, gwoff, gboff, gw, gb, None
+        grads = _layer_backward_shaped(shp, ws, gxt, offset, None, offset_weight, weight, grad_out, *ctx.has, ws)
+        return grads + (None,)
 
 
 def deform_layer_framed(xt, in_chw, offset_weight, offset_bias, weight, bias=None, kernel_size=3, stride=1, padding=1,
@@ -852,22 +825,16 @@ def _msda_inputs(value, spatial_shapes, level_start_index, sampling_locations, a
 
 def dcn_msda_forward(value, spatial_shapes, level_start_index, sampling_locations, attention_weights):
     """out [B, Q, M*D] of multi-scale deformable attention on CUDA tensors (no autograd)."""
-    lib = _lib.load()
     shp, v, ss, ls, loc, aw = _msda_inputs(value, spatial_shapes, level_start_index, sampling_locations,
                                            attention_weights)
     out = torch.empty((shp.B, shp.Q, shp.M * shp.D), dtype=torch.float32, device=v.device)
-    with torch.cuda.device(v.device):
-        stream = torch.cuda.current_stream(v.device)
-        rc = lib.dcn_msda_forward(ctypes.byref(shp), _ptr(v), _ptr(ss), _ptr(ls), _ptr(loc), _ptr(aw), _ptr(out),
-                                  ctypes.c_void_p(stream.cuda_stream))
-    _lib.check(rc, "dcn_msda_forward")
+    _run("dcn_msda_forward", v.device, shp, (v, ss, ls, loc, aw, out))
     return out
 
 
 def dcn_msda_backward(value, spatial_shapes, level_start_index, sampling_locations, attention_weights, grad_out,
                       need=(True, True, True)):
     """(grad_value, grad_sampling_locations, grad_attention_weights); need[i] False -> None, not computed."""
-    lib = _lib.load()
     shp, v, ss, ls, loc, aw = _msda_inputs(value, spatial_shapes, level_start_index, sampling_locations,
                                            attention_weights)
     if tuple(grad_out.shape) != (shp.B, shp.Q, shp.M * shp.D):
@@ -876,11 +843,7 @@ def dcn_msda_backward(value, spatial_shapes, level_start_index, sampling_locatio
     gv, gl, ga = (torch.empty_like(t) if n else None for t, n in zip((v, loc, aw), need))
     if gv is None and gl is None and ga is None:
         return None, None, None
-    with torch.cuda.device(v.device):
-        stream = torch.cuda.current_stream(v.device)
-        rc = lib.dcn_msda_backward(ctypes.byref(shp), _ptr(v), _ptr(ss), _ptr(ls), _ptr(loc), _ptr(aw), _ptr(go),
-                                   _ptr(gv), _ptr(gl), _ptr(ga), ctypes.c_void_p(stream.cuda_stream))
-    _lib.check(rc, "dcn_msda_backward")
+    _run("dcn_msda_backward", v.device, shp, (v, ss, ls, loc, aw, go, gv, gl, ga))
     return gv, gl, ga
 
 
@@ -983,15 +946,10 @@ def dcn_v3_forward(input, offset, mask, kernel_h, kernel_w, stride_h, stride_w, 
                    group, group_channels, offset_scale, softmax_mask=False):
     """out [N, Ho, Wo, group*group_channels] of the DCNv3 core on CUDA tensors (no autograd).  softmax_mask: `mask`
     holds logits and the core applies InternImage's softmax over the kernel_h*kernel_w points of each group."""
-    lib = _lib.load()
     shp, x, off, m = _dcnv3_inputs(input, offset, mask, kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w,
                                    dilation_h, dilation_w, group, group_channels, softmax_mask)
     out = torch.empty(tuple(off.shape[:3]) + (group * group_channels,), dtype=torch.float32, device=x.device)
-    with torch.cuda.device(x.device):
-        stream = torch.cuda.current_stream(x.device)
-        rc = lib.dcn_v3_forward(ctypes.byref(shp), float(offset_scale), _ptr(x), _ptr(off), _ptr(m), _ptr(out),
-                                ctypes.c_void_p(stream.cuda_stream))
-    _lib.check(rc, "dcn_v3_forward")
+    _run("dcn_v3_forward", x.device, shp, (float(offset_scale), x, off, m, out))
     return out
 
 
@@ -999,7 +957,6 @@ def dcn_v3_backward(input, offset, mask, grad_out, kernel_h, kernel_w, stride_h,
                     dilation_w, group, group_channels, offset_scale, softmax_mask=False, need=(True, True, True)):
     """(grad_input, grad_offset, grad_mask); need[i] False -> None, not computed.  With softmax_mask, grad_mask is
     the gradient of the logits."""
-    lib = _lib.load()
     shp, x, off, m = _dcnv3_inputs(input, offset, mask, kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w,
                                    dilation_h, dilation_w, group, group_channels, softmax_mask)
     want = tuple(off.shape[:3]) + (group * group_channels,)
@@ -1009,11 +966,7 @@ def dcn_v3_backward(input, offset, mask, grad_out, kernel_h, kernel_w, stride_h,
     gx, goff, gm = (torch.empty_like(t) if n else None for t, n in zip((x, off, m), need))
     if gx is None and goff is None and gm is None:
         return None, None, None
-    with torch.cuda.device(x.device):
-        stream = torch.cuda.current_stream(x.device)
-        rc = lib.dcn_v3_backward(ctypes.byref(shp), float(offset_scale), _ptr(x), _ptr(off), _ptr(m), _ptr(go),
-                                 _ptr(gx), _ptr(goff), _ptr(gm), ctypes.c_void_p(stream.cuda_stream))
-    _lib.check(rc, "dcn_v3_backward")
+    _run("dcn_v3_backward", x.device, shp, (float(offset_scale), x, off, m, go, gx, goff, gm))
     return gx, goff, gm
 
 
@@ -1097,15 +1050,10 @@ def _dcnv4_inputs(input, offset_mask, kernel_h, kernel_w, stride_h, stride_w, pa
 def dcn_v4_forward(input, offset_mask, kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w, dilation_h, dilation_w,
                    group, group_channels, offset_scale, remove_center=False):
     """out [N, Ho, Wo, group*group_channels] of the DCNv4 core on CUDA tensors (no autograd)."""
-    lib = _lib.load()
     shp, x, om = _dcnv4_inputs(input, offset_mask, kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w, dilation_h,
                                dilation_w, group, group_channels, remove_center)
     out = torch.empty(tuple(om.shape[:3]) + (group * group_channels,), dtype=torch.float32, device=x.device)
-    with torch.cuda.device(x.device):
-        stream = torch.cuda.current_stream(x.device)
-        rc = lib.dcn_v4_forward(ctypes.byref(shp), float(offset_scale), _ptr(x), _ptr(om), _ptr(out),
-                                ctypes.c_void_p(stream.cuda_stream))
-    _lib.check(rc, "dcn_v4_forward")
+    _run("dcn_v4_forward", x.device, shp, (float(offset_scale), x, om, out))
     return out
 
 
@@ -1113,7 +1061,6 @@ def dcn_v4_backward(input, offset_mask, grad_out, kernel_h, kernel_w, stride_h, 
                     dilation_w, group, group_channels, offset_scale, remove_center=False, need=(True, True)):
     """(grad_input, grad_offset_mask); need[i] False -> None, not computed.  grad_offset_mask has offset_mask's packed
     layout, with +0.0 in the padding columns."""
-    lib = _lib.load()
     shp, x, om = _dcnv4_inputs(input, offset_mask, kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w, dilation_h,
                                dilation_w, group, group_channels, remove_center)
     want = tuple(om.shape[:3]) + (group * group_channels,)
@@ -1123,11 +1070,7 @@ def dcn_v4_backward(input, offset_mask, grad_out, kernel_h, kernel_w, stride_h, 
     gx, gom = (torch.empty_like(t) if n else None for t, n in zip((x, om), need))
     if gx is None and gom is None:
         return None, None
-    with torch.cuda.device(x.device):
-        stream = torch.cuda.current_stream(x.device)
-        rc = lib.dcn_v4_backward(ctypes.byref(shp), float(offset_scale), _ptr(x), _ptr(om), _ptr(go), _ptr(gx),
-                                 _ptr(gom), ctypes.c_void_p(stream.cuda_stream))
-    _lib.check(rc, "dcn_v4_backward")
+    _run("dcn_v4_backward", x.device, shp, (float(offset_scale), x, om, go, gx, gom))
     return gx, gom
 
 

@@ -6,19 +6,16 @@ Only `output_size == 1` is accepted: both reference modules sum the per-bin valu
 size — there is no behaviour to reproduce.  Constructor arguments, their defaults and the dead ones (`sampling_ratio`,
 `group_size`) are the reference's.
 """
-import ctypes
-
 import torch
 import torch.nn as nn
 
 from . import _lib
-from .functional import _dev_ready, _ptr
+from .functional import _dev_ready, _run
 
 
 class _RoIPoolFunction(torch.autograd.Function):
     @staticmethod
     def forward(ctx, features, rois, offsets, kind, spatial_scale, trans_std, no_trans):
-        lib = _lib.load()
         if not features.is_cuda:
             raise _lib.DcnError("jittor_dcn_b200 RoI pooling needs CUDA tensors: there is no CPU path")
         f, r = _dev_ready(features), _dev_ready(rois.to(features.device))
@@ -26,18 +23,14 @@ class _RoIPoolFunction(torch.autograd.Function):
         B, C, H, W = f.shape
         R = r.shape[0]
         out = torch.empty((R, C), dtype=torch.float32, device=f.device)
-        with torch.cuda.device(f.device):
-            st = torch.cuda.current_stream(f.device)
-            rc = lib.dcn_roi_pool_forward(kind, B, C, H, W, R, _ptr(f), _ptr(r), _ptr(o), float(spatial_scale),
-                                          float(trans_std), int(no_trans), _ptr(out), ctypes.c_void_p(st.cuda_stream))
-        _lib.check(rc, "dcn_roi_pool_forward")
+        _run("dcn_roi_pool_forward", f.device, None,
+             (kind, B, C, H, W, R, f, r, o, float(spatial_scale), float(trans_std), int(no_trans), out))
         ctx.save_for_backward(f, r, o if o is not None else torch.empty(0, device=f.device))
         ctx.cfg = (kind, spatial_scale, trans_std, no_trans, offsets is not None, None if offsets is None else offsets.shape)
         return out.view(R, C, 1, 1)
 
     @staticmethod
     def backward(ctx, grad_out):
-        lib = _lib.load()
         f, r, o = ctx.saved_tensors
         kind, spatial_scale, trans_std, no_trans, has_off, off_shape = ctx.cfg
         B, C, H, W = f.shape
@@ -45,12 +38,9 @@ class _RoIPoolFunction(torch.autograd.Function):
         g = _dev_ready(grad_out.reshape(R, C))
         gf = torch.empty_like(f) if ctx.needs_input_grad[0] else None
         go = torch.empty((R, 2), dtype=torch.float32, device=f.device) if (has_off and ctx.needs_input_grad[2]) else None
-        with torch.cuda.device(f.device):
-            st = torch.cuda.current_stream(f.device)
-            rc = lib.dcn_roi_pool_backward(kind, B, C, H, W, R, _ptr(f), _ptr(r), _ptr(o) if has_off else None,
-                                           float(spatial_scale), float(trans_std), int(no_trans), _ptr(g), _ptr(gf),
-                                           _ptr(go), ctypes.c_void_p(st.cuda_stream))
-        _lib.check(rc, "dcn_roi_pool_backward")
+        _run("dcn_roi_pool_backward", f.device, None,
+             (kind, B, C, H, W, R, f, r, o if has_off else None, float(spatial_scale), float(trans_std), int(no_trans),
+              g, gf, go))
         if go is not None:
             full = torch.zeros(off_shape, dtype=torch.float32, device=f.device).reshape(R, -1)
             full[:, :2] = go
