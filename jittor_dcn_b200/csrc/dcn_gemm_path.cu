@@ -255,6 +255,18 @@ __global__ void __launch_bounds__(256) bias_fill_kernel(int B, int O, int Oimg, 
   }
 }
 
+// DCN_FLAG_RELU_OUT: out[b, o, :] = max(out[b, o, :], 0) once the GEMMs have accumulated onto the bias
+__global__ void __launch_bounds__(256) relu_kernel(int B, int O, int Oimg, int HW, float* __restrict__ out) {
+  const size_t total = (size_t)B * O * HW;
+  for (size_t i = blockIdx.x * 256ull + threadIdx.x; i < total; i += (size_t)gridDim.x * 256) {
+    const int p = (int)(i % HW);
+    const size_t bo = i / HW;
+    const int o = (int)(bo % O), b = (int)(bo / O);
+    float* v = out + ((size_t)b * Oimg + o) * HW + p;
+    *v = fmaxf(*v, 0.f);
+  }
+}
+
 // goutT[o, b*HW + p] = gout[b, o, p]: rows of HW elements re-ordered (o, b)  (bf16 operands)
 __global__ void __launch_bounds__(256) gout_rows_kernel(int B, int O, int Oimg, int HW,
                                                         const __nv_bfloat16* __restrict__ gout,
@@ -399,22 +411,29 @@ int gemm_path_forward(const Geo& g, int operand, const void* x, const float* off
   std::lock_guard<std::mutex> use(gp::g_use_mu);   // a cuBLAS handle must not be driven by two host threads at once
   if ((cs = gp::g_api.SetStream(h, st)) != CUBLAS_STATUS_SUCCESS) return gp_cublas_fail(cs, "cublasSetStream");
   if (gp::g_api.SetWorkspace) gp::g_api.SetWorkspace(h, cws, gp::kCublasWs);
-  // row-major out_b[O, HW] += Wm[O, K] * A_b^T  <=>  column-major C'[HW, O] = op_T(A'[K, HW]) * B'[K, O]
-  KernelScope scope("cublas_gemm_fwd", st);
-  auto gemm = [&](const void* Sm, const void* Wm) {
-    count_launch();
-    return gp::g_api.GemmStridedBatchedEx(h, CUBLAS_OP_T, CUBLAS_OP_N, g.HW, g.O, g.K, &one, Sm, CUDA_R_16BF, g.K,
-                                          (long long)g.C * g.P, Wm, CUDA_R_16BF, g.K, 0, &one, out, CUDA_R_32F, g.HW,
-                                          (long long)g.Oimg * g.HW, g.B, CUBLAS_COMPUTE_32F, CUBLAS_GEMM_DEFAULT);
-  };
-  if (split) {
-    const __nv_bfloat16 *s_hi = (const __nv_bfloat16*)S, *s_lo = s_hi + nS;
-    if ((cs = gemm(s_lo, w_hi)) == CUBLAS_STATUS_SUCCESS && (cs = gemm(s_hi, w_lo)) == CUBLAS_STATUS_SUCCESS)
-      cs = gemm(s_hi, w_hi);
-  } else {
-    cs = gemm(S, wt);
+  {
+    // row-major out_b[O, HW] += Wm[O, K] * A_b^T  <=>  column-major C'[HW, O] = op_T(A'[K, HW]) * B'[K, O]
+    KernelScope scope("cublas_gemm_fwd", st);
+    auto gemm = [&](const void* Sm, const void* Wm) {
+      count_launch();
+      return gp::g_api.GemmStridedBatchedEx(h, CUBLAS_OP_T, CUBLAS_OP_N, g.HW, g.O, g.K, &one, Sm, CUDA_R_16BF, g.K,
+                                            (long long)g.C * g.P, Wm, CUDA_R_16BF, g.K, 0, &one, out, CUDA_R_32F, g.HW,
+                                            (long long)g.Oimg * g.HW, g.B, CUBLAS_COMPUTE_32F, CUBLAS_GEMM_DEFAULT);
+    };
+    if (split) {
+      const __nv_bfloat16 *s_hi = (const __nv_bfloat16*)S, *s_lo = s_hi + nS;
+      if ((cs = gemm(s_lo, w_hi)) == CUBLAS_STATUS_SUCCESS && (cs = gemm(s_hi, w_lo)) == CUBLAS_STATUS_SUCCESS)
+        cs = gemm(s_hi, w_hi);
+    } else {
+      cs = gemm(S, wt);
+    }
   }
   if (cs != CUBLAS_STATUS_SUCCESS) return gp_cublas_fail(cs, "cublasGemmStridedBatchedEx(forward)");
+  if (g.relu_out) {
+    KernelScope scope("gemm_relu_kernel", st);
+    gp::relu_kernel<<<1024, 256, 0, st>>>(g.B, g.O, g.Oimg, g.HW, out);
+    DCN_KERNEL_CHECK("gemm_relu_kernel");
+  }
   return DCN_OK;
 }
 
