@@ -82,7 +82,9 @@ enum {
    * (hi*hi + hi*lo + lo*hi, fp32 accumulate; |err| ~ 5e-6 relative). */
   DCN_OPERAND_FP32 = 0,
   /* x, weight, grad_out stored as bfloat16; out, all gradients float32; fp32 accumulate. */
-  DCN_OPERAND_BF16 = 1
+  DCN_OPERAND_BF16 = 1,
+  /* float16 operands: the DCNv3 / DCNv4 cores only (dcn_v3_*_typed, dcn_v4_*_typed); a DcnShape refuses it. */
+  DCN_OPERAND_FP16 = 2
 };
 
 /* DcnShape.flags */
@@ -341,7 +343,8 @@ DCN_API int dcn_msda_backward(const DcnMsdaShape* s, const void* value, const in
                               const void* attention_weights, const void* grad_out, void* grad_value,
                               void* grad_sampling_locations, void* grad_attention_weights, void* stream);
 
-/* ---- DCNv3 (InternImage's ops_dcnv3 core: DCNv3Function / dcnv3_core_pytorch), float32, channels-last ---------------
+/* ---- DCNv3 (InternImage's ops_dcnv3 core: DCNv3Function / dcnv3_core_pytorch), float32 (bf16 / fp16: the _typed
+ * calls below), channels-last ----------------------------------------------------------------------------------------
  *   out[n, ho, wo, g*Gc + c] = sum_p m[n, ho, wo, g*P + p] * bilinear(input[n, :, :, g*Gc + c], y_p, x_p)
  * P = kh*kw points in x-major order: p = i*kh + j with kernel column i < kw and kernel row j < kh (for a square kernel
  * the transpose of torchvision's tap order).  Offsets are (dx, dy) per point: offset[n, ho, wo, 2*(g*P + p)] and
@@ -379,7 +382,8 @@ DCN_API int dcn_v3_backward(const DcnV3Shape* s, float offset_scale, const void*
                             const void* mask, const void* grad_out, void* grad_input, void* grad_offset,
                             void* grad_mask, void* stream);
 
-/* ---- DCNv4 (the DCNv4 repository's DCNv4Function core), float32, channels-last --------------------------------------
+/* ---- DCNv4 (the DCNv4 repository's DCNv4Function core), float32 (bf16 / fp16: the _typed calls below),
+ * channels-last -------------------------------------------------------------------------------------------------------
  * DCNv3's operator and coordinate chain (above) with three changes:
  *   - no softmax: the mask is used as given;
  *   - offsets and mask packed into one tensor offset_mask [N, Ho, Wo, Cm], Cm = ceil(3*G*K / 8)*8.  Group g owns
@@ -406,6 +410,31 @@ DCN_API int dcn_v4_forward(const DcnV3Shape* s, float offset_scale, const void* 
                            void* out, void* stream);
 DCN_API int dcn_v4_backward(const DcnV3Shape* s, float offset_scale, const void* input, const void* offset_mask,
                             const void* grad_out, void* grad_input, void* grad_offset_mask, void* stream);
+
+/* ---- DCNv3 / DCNv4 on bfloat16 or float16 operands -----------------------------------------------------------------
+ * dcn_v{3,4}_{forward,backward}_typed take the operand right after the shape; every other argument, check and status
+ * is that of the call without the suffix, which is the typed call with DCN_OPERAND_FP32.  The operand is checked
+ * where the flags are, right after them: a value other than DCN_OPERAND_FP32, DCN_OPERAND_BF16 or DCN_OPERAND_FP16 is
+ * DCN_ERR_UNSUPPORTED.
+ *   DCN_OPERAND_FP32   every tensor float32, as above.
+ *   DCN_OPERAND_BF16   input, offset, mask / offset_mask, grad_out, out, grad_offset, grad_mask / grad_offset_mask
+ *   DCN_OPERAND_FP16   in bfloat16, resp. float16 (offset_mask's padding columns: +0.0 of that type).
+ * grad_input is float32 for every operand: it is accumulated with float atomics (red.global.add.v4.f32) over all the
+ * samples that touch a pixel, and rounding each partial sum to 16 bits would lose the small contributions.
+ * The kernels widen every half value to float32 exactly, run the float32 kernels' arithmetic in the same order and
+ * round each stored half value once, to nearest even.  So out, grad_offset, grad_mask and grad_offset_mask are bit for
+ * bit the float32 call's results on the widened operands, rounded to the operand type, and grad_input differs from it
+ * only by the order of the atomics. */
+DCN_API int dcn_v3_forward_typed(const DcnV3Shape* s, int32_t operand, float offset_scale, const void* input,
+                                 const void* offset, const void* mask, void* out, void* stream);
+DCN_API int dcn_v3_backward_typed(const DcnV3Shape* s, int32_t operand, float offset_scale, const void* input,
+                                  const void* offset, const void* mask, const void* grad_out, void* grad_input,
+                                  void* grad_offset, void* grad_mask, void* stream);
+DCN_API int dcn_v4_forward_typed(const DcnV3Shape* s, int32_t operand, float offset_scale, const void* input,
+                                 const void* offset_mask, void* out, void* stream);
+DCN_API int dcn_v4_backward_typed(const DcnV3Shape* s, int32_t operand, float offset_scale, const void* input,
+                                  const void* offset_mask, const void* grad_out, void* grad_input,
+                                  void* grad_offset_mask, void* stream);
 
 /* ---- producer of the first DCN layer's input (train.py:145,166 / 307,328: conv1 = Conv2d(1, 16, 3, 1, 1)) ------------
  * A 3 x 3, stride 1, padding 1 convolution with Cin <= 4 input channels and O in {16, 32} outputs, float32 NCHW,

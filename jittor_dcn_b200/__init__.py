@@ -5,7 +5,7 @@ binding and the two module classes that mirror the reference's operator interfac
 """
 from ._lib import (DCN_V3_FLAG_SOFTMAX_MASK, DCN_V4_FLAG_REMOVE_CENTER, DcnError, DcnMsdaShape, DcnShape, DcnV3Shape,
                    FLAG_ACCUM_GRAD_X, FLAG_FORCE_SIMT, FLAG_NO_GRAD_X, FLAG_RELU_OUT,
-                   OPERAND_BF16, OPERAND_FP32, VARIANT_DCNV1, VARIANT_JITTOR, VARIANT_TORCH, load, make_shape)
+                   OPERAND_BF16, OPERAND_FP16, OPERAND_FP32, VARIANT_DCNV1, VARIANT_JITTOR, VARIANT_TORCH, load, make_shape)
 from .deform_conv import DeformConv2d
 from .functional import (batch_norm_relu, clear_workspaces, dcn_backward, dcn_backward_modulated, dcn_corners,
                          dcn_forward, dcn_forward_modulated, dcn_layer_backward, dcn_layer_forward,
@@ -26,7 +26,7 @@ from .torch_module import (BatchNormReLU2d, ModulatedDeformConv2dPack, StemConv2
 __all__ = [
     "DeformConv2d", "TorchDeformConv2d", "BatchNormReLU2d", "batch_norm_relu", "TorchDeformConv2dJittorSemantics", "deform_conv2d",
     "dcn_forward", "dcn_backward", "dcn_corners", "deform_conv2d_v1", "VARIANT_DCNV1", "load", "make_shape", "DcnShape", "DcnError",
-    "VARIANT_JITTOR", "VARIANT_TORCH", "OPERAND_FP32", "OPERAND_BF16", "FLAG_ACCUM_GRAD_X",
+    "VARIANT_JITTOR", "VARIANT_TORCH", "OPERAND_FP32", "OPERAND_BF16", "OPERAND_FP16", "FLAG_ACCUM_GRAD_X",
     "FLAG_FORCE_SIMT", "FLAG_NO_GRAD_X", "FLAG_RELU_OUT", "clear_workspaces", "dcn_offset_conv_forward", "dcn_layer_forward", "dcn_layer_backward", "deform_layer",
     "layer_supported", "fuse_eval_bn_relu", "DeformRoIPool", "DeformPSRoIPool", "ChainedDeformStages", "StemConv2d",
     "dcn_forward_modulated", "dcn_backward_modulated", "deform_conv2d_modulated", "TorchvisionDeformConv2d",

@@ -15,6 +15,7 @@ VARIANT_TORCH = 1    # train.py:95-140
 VARIANT_DCNV1 = 2    # standard DCNv1 (torchvision.ops.deform_conv2d semantics), SURVEY 8f.3
 OPERAND_FP32 = 0
 OPERAND_BF16 = 1
+OPERAND_FP16 = 2     # DCNv3 / DCNv4 cores only (dcn_v3_*_typed, dcn_v4_*_typed)
 FLAG_ACCUM_GRAD_X = 1 << 0
 FLAG_FORCE_SIMT = 1 << 1
 FLAG_NO_GRAD_X = 1 << 2
@@ -91,6 +92,10 @@ BINDINGS = {
     "dcn_v3_backward": (_i32, [_v3p, _f32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "dcn_v4_forward": (_i32, [_v3p, _f32, _vp, _vp, _vp, _vp]),
     "dcn_v4_backward": (_i32, [_v3p, _f32, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "dcn_v3_forward_typed": (_i32, [_v3p, _i32, _f32, _vp, _vp, _vp, _vp, _vp]),
+    "dcn_v3_backward_typed": (_i32, [_v3p, _i32, _f32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "dcn_v4_forward_typed": (_i32, [_v3p, _i32, _f32, _vp, _vp, _vp, _vp]),
+    "dcn_v4_backward_typed": (_i32, [_v3p, _i32, _f32, _vp, _vp, _vp, _vp, _vp, _vp]),
     "dcn_stem_conv_forward": (_i32, [_i32, _i32, _i32, _i32, _i32, _vp, _vp, _vp, _vp, _vp]),
     "dcn_stem_conv_backward": (_i32, [_i32, _i32, _i32, _i32, _i32, _vp, _vp, _vp, _vp, _vp]),
     "dcn_bn_workspace_bytes": (_sz, [_i32]),

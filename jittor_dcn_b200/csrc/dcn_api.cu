@@ -79,7 +79,8 @@ static int geo_or_error(const DcnShape* s, Geo* g) {
     set_error("bad shape B=%d C=%d O=%d H=%d W=%d k=(%d,%d) s=(%d,%d) p=(%d,%d) variant=%d", s->B,
               s->C, s->O, s->H, s->W, s->kh, s->kw, s->sh, s->sw, s->ph, s->pw, s->variant);
   if (rc == DCN_OK && s->operand != DCN_OPERAND_FP32 && s->operand != DCN_OPERAND_BF16) {
-    set_error("unknown operand mode %d", s->operand);
+    set_error("unknown operand mode %d (DcnShape takes DCN_OPERAND_FP32 = 0 or DCN_OPERAND_BF16 = 1; "
+              "DCN_OPERAND_FP16 is for the DCNv3 / DCNv4 cores)", s->operand);
     rc = DCN_ERR_UNSUPPORTED;
   }
   return rc;
@@ -259,10 +260,11 @@ static int msda_shape_ok(const DcnMsdaShape* s, const char* what) {
 }
 
 // DCNv3 (dcn_dcnv3.cu)
-int dcnv3_forward(const DcnV3Shape& s, int Ho, int Wo, float offset_scale, const float* input, const float* offset,
-                  const float* mask, float* out, cudaStream_t st);
-int dcnv3_backward(const DcnV3Shape& s, int Ho, int Wo, float offset_scale, const float* input, const float* offset,
-                   const float* mask, const float* gout, float* ginput, float* goffset, float* gmask, cudaStream_t st);
+int dcnv3_forward(const DcnV3Shape& s, int operand, int Ho, int Wo, float offset_scale, const void* input,
+                  const void* offset, const void* mask, void* out, cudaStream_t st);
+int dcnv3_backward(const DcnV3Shape& s, int operand, int Ho, int Wo, float offset_scale, const void* input,
+                   const void* offset, const void* mask, const void* gout, float* ginput, void* goffset, void* gmask,
+                   cudaStream_t st);
 
 // floor((in + 2*pad - (dil*(k-1) + 1)) / stride) + 1, or 0 when the dilated kernel does not fit the padded input
 static long long dcnv3_out_extent(long long in, long long k, long long stride, long long pad, long long dil) {
@@ -302,8 +304,18 @@ static int dcnv3_shape_ok(const DcnV3Shape* s, const char* what, int* Ho, int* W
   return DCN_OK;
 }
 
+// The storage types of the DCNv3 / DCNv4 kernels: DCN_OPERAND_FP32, _BF16 or _FP16.
+static int dcnv34_operand_ok(int32_t operand, const char* what) {
+  if (operand != DCN_OPERAND_FP32 && operand != DCN_OPERAND_BF16 && operand != DCN_OPERAND_FP16) {
+    set_error("%s: unknown operand %d (DCN_OPERAND_FP32 = 0, DCN_OPERAND_BF16 = 1 or DCN_OPERAND_FP16 = 2)", what,
+              operand);
+    return DCN_ERR_UNSUPPORTED;
+  }
+  return DCN_OK;
+}
+
 // What the kernels cover (DCN_ERR_UNSUPPORTED), checked after the pointers.
-static int dcnv3_supported(const DcnV3Shape* s, const char* what) {
+static int dcnv3_supported(const DcnV3Shape* s, int32_t operand, const char* what) {
   if (s->Gc != 16 && s->Gc != 32 && s->Gc != 64 && s->Gc != 128 && s->Gc != 256) {
     set_error("%s: Gc = %d channels per group is not supported (Gc in {16, 32, 64, 128, 256})", what, s->Gc);
     return DCN_ERR_UNSUPPORTED;
@@ -317,15 +329,15 @@ static int dcnv3_supported(const DcnV3Shape* s, const char* what) {
               (unsigned)s->flags & ~(unsigned)DCN_V3_FLAG_SOFTMAX_MASK);
     return DCN_ERR_UNSUPPORTED;
   }
-  return DCN_OK;
+  return dcnv34_operand_ok(operand, what);
 }
 
 // DCNv4 (dcn_dcnv3.cu)
 long long dcnv4_row_floats(const DcnV3Shape& s);
-int dcnv4_forward(const DcnV3Shape& s, int Ho, int Wo, float offset_scale, const float* input, const float* offset_mask,
-                  float* out, cudaStream_t st);
-int dcnv4_backward(const DcnV3Shape& s, int Ho, int Wo, float offset_scale, const float* input, const float* offset_mask,
-                   const float* gout, float* ginput, float* goffset_mask, cudaStream_t st);
+int dcnv4_forward(const DcnV3Shape& s, int operand, int Ho, int Wo, float offset_scale, const void* input,
+                  const void* offset_mask, void* out, cudaStream_t st);
+int dcnv4_backward(const DcnV3Shape& s, int operand, int Ho, int Wo, float offset_scale, const void* input,
+                   const void* offset_mask, const void* gout, float* ginput, void* goffset_mask, cudaStream_t st);
 
 // The shape checks of dcn_v4_forward / _backward: DCNv3's, then K >= 1 and the row width Cm.
 static int dcnv4_shape_ok(const DcnV3Shape* s, const char* what, int* Ho, int* Wo) {
@@ -344,7 +356,8 @@ static int dcnv4_shape_ok(const DcnV3Shape* s, const char* what, int* Ho, int* W
 }
 
 // What the DCNv4 kernels cover (DCN_ERR_UNSUPPORTED), checked after the pointers.
-static int dcnv4_supported(const DcnV3Shape* s, const char* what) {
+static int dcnv4_supported(const DcnV3Shape* s, int32_t operand, const char* what) {
+  int rc;
   if (s->Gc != 16 && s->Gc != 32 && s->Gc != 64 && s->Gc != 128 && s->Gc != 256) {
     set_error("%s: Gc = %d channels per group is not supported (Gc in {16, 32, 64, 128, 256})", what, s->Gc);
     return DCN_ERR_UNSUPPORTED;
@@ -354,6 +367,7 @@ static int dcnv4_supported(const DcnV3Shape* s, const char* what) {
               (unsigned)s->flags & ~(unsigned)DCN_V4_FLAG_REMOVE_CENTER);
     return DCN_ERR_UNSUPPORTED;
   }
+  if ((rc = dcnv34_operand_ok(operand, what))) return rc;
   if ((s->flags & DCN_V4_FLAG_REMOVE_CENTER) && (s->kh % 2 == 0 || s->kw % 2 == 0)) {
     set_error("%s: remove_center needs an odd kernel, got %d x %d (no centre point)", what, s->kh, s->kw);
     return DCN_ERR_UNSUPPORTED;
@@ -838,51 +852,97 @@ int dcn_msda_backward(const DcnMsdaShape* s, const void* value, const int64_t* s
                        (float*)grad_sampling_locations, (float*)grad_attention_weights, (cudaStream_t)stream);
 }
 
+// One host body per DCNv3 / DCNv4 call: the untyped entry points are the typed ones on DCN_OPERAND_FP32.
+static int v3_forward(const char* what, const DcnV3Shape* s, int32_t operand, float offset_scale, const void* input,
+                      const void* offset, const void* mask, void* out, void* stream) {
+  int rc, Ho, Wo;
+  if ((rc = dcnv3_shape_ok(s, what, &Ho, &Wo)) || (rc = check_ptr(input, "input")) ||
+      (rc = check_ptr(offset, "offset")) || (rc = check_ptr(mask, "mask")) || (rc = check_ptr(out, "out")) ||
+      (rc = dcnv3_supported(s, operand, what)))
+    return rc;
+  return dcnv3_forward(*s, operand, Ho, Wo, offset_scale, input, offset, mask, out, (cudaStream_t)stream);
+}
+
+static int v3_backward(const char* what, const DcnV3Shape* s, int32_t operand, float offset_scale, const void* input,
+                       const void* offset, const void* mask, const void* grad_out, void* grad_input, void* grad_offset,
+                       void* grad_mask, void* stream) {
+  int rc, Ho, Wo;
+  if ((rc = dcnv3_shape_ok(s, what, &Ho, &Wo)) || (rc = check_ptr(input, "input")) ||
+      (rc = check_ptr(offset, "offset")) || (rc = check_ptr(mask, "mask")) || (rc = check_ptr(grad_out, "grad_out")) ||
+      (rc = check_ptr(grad_input, "grad_input", false)) || (rc = check_ptr(grad_offset, "grad_offset", false)) ||
+      (rc = check_ptr(grad_mask, "grad_mask", false)) || (rc = dcnv3_supported(s, operand, what)))
+    return rc;
+  return dcnv3_backward(*s, operand, Ho, Wo, offset_scale, input, offset, mask, grad_out, (float*)grad_input,
+                        grad_offset, grad_mask, (cudaStream_t)stream);
+}
+
+static int v4_forward(const char* what, const DcnV3Shape* s, int32_t operand, float offset_scale, const void* input,
+                      const void* offset_mask, void* out, void* stream) {
+  int rc, Ho, Wo;
+  if ((rc = dcnv4_shape_ok(s, what, &Ho, &Wo)) || (rc = check_ptr(input, "input")) ||
+      (rc = check_ptr(offset_mask, "offset_mask")) || (rc = check_ptr(out, "out")) ||
+      (rc = dcnv4_supported(s, operand, what)))
+    return rc;
+  return dcnv4_forward(*s, operand, Ho, Wo, offset_scale, input, offset_mask, out, (cudaStream_t)stream);
+}
+
+static int v4_backward(const char* what, const DcnV3Shape* s, int32_t operand, float offset_scale, const void* input,
+                       const void* offset_mask, const void* grad_out, void* grad_input, void* grad_offset_mask,
+                       void* stream) {
+  int rc, Ho, Wo;
+  if ((rc = dcnv4_shape_ok(s, what, &Ho, &Wo)) || (rc = check_ptr(input, "input")) ||
+      (rc = check_ptr(offset_mask, "offset_mask")) || (rc = check_ptr(grad_out, "grad_out")) ||
+      (rc = check_ptr(grad_input, "grad_input", false)) ||
+      (rc = check_ptr(grad_offset_mask, "grad_offset_mask", false)) || (rc = dcnv4_supported(s, operand, what)))
+    return rc;
+  return dcnv4_backward(*s, operand, Ho, Wo, offset_scale, input, offset_mask, grad_out, (float*)grad_input,
+                        grad_offset_mask, (cudaStream_t)stream);
+}
+
 int dcn_v3_forward(const DcnV3Shape* s, float offset_scale, const void* input, const void* offset, const void* mask,
                    void* out, void* stream) {
-  int rc, Ho, Wo;
-  if ((rc = dcnv3_shape_ok(s, "dcn_v3_forward", &Ho, &Wo)) || (rc = check_ptr(input, "input")) ||
-      (rc = check_ptr(offset, "offset")) || (rc = check_ptr(mask, "mask")) || (rc = check_ptr(out, "out")) ||
-      (rc = dcnv3_supported(s, "dcn_v3_forward")))
-    return rc;
-  return dcnv3_forward(*s, Ho, Wo, offset_scale, (const float*)input, (const float*)offset, (const float*)mask,
-                       (float*)out, (cudaStream_t)stream);
+  return v3_forward("dcn_v3_forward", s, DCN_OPERAND_FP32, offset_scale, input, offset, mask, out, stream);
 }
 
 int dcn_v3_backward(const DcnV3Shape* s, float offset_scale, const void* input, const void* offset, const void* mask,
                     const void* grad_out, void* grad_input, void* grad_offset, void* grad_mask, void* stream) {
-  int rc, Ho, Wo;
-  if ((rc = dcnv3_shape_ok(s, "dcn_v3_backward", &Ho, &Wo)) || (rc = check_ptr(input, "input")) ||
-      (rc = check_ptr(offset, "offset")) || (rc = check_ptr(mask, "mask")) || (rc = check_ptr(grad_out, "grad_out")) ||
-      (rc = check_ptr(grad_input, "grad_input", false)) || (rc = check_ptr(grad_offset, "grad_offset", false)) ||
-      (rc = check_ptr(grad_mask, "grad_mask", false)) || (rc = dcnv3_supported(s, "dcn_v3_backward")))
-    return rc;
-  return dcnv3_backward(*s, Ho, Wo, offset_scale, (const float*)input, (const float*)offset, (const float*)mask,
-                        (const float*)grad_out, (float*)grad_input, (float*)grad_offset, (float*)grad_mask,
-                        (cudaStream_t)stream);
+  return v3_backward("dcn_v3_backward", s, DCN_OPERAND_FP32, offset_scale, input, offset, mask, grad_out, grad_input,
+                     grad_offset, grad_mask, stream);
 }
 
 int dcn_v4_forward(const DcnV3Shape* s, float offset_scale, const void* input, const void* offset_mask, void* out,
                    void* stream) {
-  int rc, Ho, Wo;
-  if ((rc = dcnv4_shape_ok(s, "dcn_v4_forward", &Ho, &Wo)) || (rc = check_ptr(input, "input")) ||
-      (rc = check_ptr(offset_mask, "offset_mask")) || (rc = check_ptr(out, "out")) ||
-      (rc = dcnv4_supported(s, "dcn_v4_forward")))
-    return rc;
-  return dcnv4_forward(*s, Ho, Wo, offset_scale, (const float*)input, (const float*)offset_mask, (float*)out,
-                       (cudaStream_t)stream);
+  return v4_forward("dcn_v4_forward", s, DCN_OPERAND_FP32, offset_scale, input, offset_mask, out, stream);
 }
 
 int dcn_v4_backward(const DcnV3Shape* s, float offset_scale, const void* input, const void* offset_mask,
                     const void* grad_out, void* grad_input, void* grad_offset_mask, void* stream) {
-  int rc, Ho, Wo;
-  if ((rc = dcnv4_shape_ok(s, "dcn_v4_backward", &Ho, &Wo)) || (rc = check_ptr(input, "input")) ||
-      (rc = check_ptr(offset_mask, "offset_mask")) || (rc = check_ptr(grad_out, "grad_out")) ||
-      (rc = check_ptr(grad_input, "grad_input", false)) ||
-      (rc = check_ptr(grad_offset_mask, "grad_offset_mask", false)) || (rc = dcnv4_supported(s, "dcn_v4_backward")))
-    return rc;
-  return dcnv4_backward(*s, Ho, Wo, offset_scale, (const float*)input, (const float*)offset_mask,
-                        (const float*)grad_out, (float*)grad_input, (float*)grad_offset_mask, (cudaStream_t)stream);
+  return v4_backward("dcn_v4_backward", s, DCN_OPERAND_FP32, offset_scale, input, offset_mask, grad_out, grad_input,
+                     grad_offset_mask, stream);
+}
+
+int dcn_v3_forward_typed(const DcnV3Shape* s, int32_t operand, float offset_scale, const void* input,
+                         const void* offset, const void* mask, void* out, void* stream) {
+  return v3_forward("dcn_v3_forward_typed", s, operand, offset_scale, input, offset, mask, out, stream);
+}
+
+int dcn_v3_backward_typed(const DcnV3Shape* s, int32_t operand, float offset_scale, const void* input,
+                          const void* offset, const void* mask, const void* grad_out, void* grad_input,
+                          void* grad_offset, void* grad_mask, void* stream) {
+  return v3_backward("dcn_v3_backward_typed", s, operand, offset_scale, input, offset, mask, grad_out, grad_input,
+                     grad_offset, grad_mask, stream);
+}
+
+int dcn_v4_forward_typed(const DcnV3Shape* s, int32_t operand, float offset_scale, const void* input,
+                         const void* offset_mask, void* out, void* stream) {
+  return v4_forward("dcn_v4_forward_typed", s, operand, offset_scale, input, offset_mask, out, stream);
+}
+
+int dcn_v4_backward_typed(const DcnV3Shape* s, int32_t operand, float offset_scale, const void* input,
+                          const void* offset_mask, const void* grad_out, void* grad_input, void* grad_offset_mask,
+                          void* stream) {
+  return v4_backward("dcn_v4_backward_typed", s, operand, offset_scale, input, offset_mask, grad_out, grad_input,
+                     grad_offset_mask, stream);
 }
 
 size_t dcn_bn_workspace_bytes(int32_t C) { return C > 0 ? bn_workspace_bytes(C) : 0; }

@@ -16,8 +16,9 @@
 //                                sum g*dbil/dx, sum g*dbil/dy in the location gradient.
 //   kSoftmax         attn holds logits; the weight of sample s is softmax over the item's L*P logits.  The backward
 //                    then writes the logits' gradient m_s*(gamma_s - sum_q m_q*gamma_q), gamma = sum g*bil.
-// Mapping: a group of G = min(D/4, 32) lanes owns one item, V = D/(4G) float4 per lane; one corner of one head is 4*D
-// contiguous bytes, read in place with one float4 per lane; whether a corner is inside is the same for the group.
+// Mapping: a group of G = min(D/4, 32) lanes owns one item, V = D/(4G) runs of 4 channels per lane; one corner of one
+// head is D contiguous elements, read in place with one 4-channel load per lane; whether a corner is inside is the same
+// for the group.
 //   forward   the samples are cut into rounds of G: lane j runs the chain of sample s0 + j and hands the result to
 //             the group by shuffle.  `out` is written once, coalesced; no atomics.
 //   backward  rounds of K = min(G, 8) samples.  Per sample and lane: gvalue[corner] += a*w_k*g (red.global.add.v4.f32,
@@ -26,7 +27,15 @@
 //             of dcn_umma_bwd_data.cu, after which lane j holds the totals of sample s0 + j — the sample whose chain it
 //             computed — and writes its gradient elements with plain stores.  The two coordinate-side gradients are
 //             therefore deterministic; only gvalue depends on the order of the atomics.
+// Storage: value, loc, attn, gout, out, gloc and gattn are of one type T, taken from Src::Args's pointers: float, or
+// __nv_bfloat16 / __half (DCNv3 and DCNv4; MSDA is float only).  Every load widens T to float exactly (the ld*
+// helpers below; 4 channels of a half type are one 8-byte load), all arithmetic is the float32 arithmetic of the float
+// path in the same order, and every store of T rounds once to nearest even.  gvalue is float for every T: it is the
+// target of the float atomics.  So a kernel on half operands computes exactly what the float kernel computes on their
+// widened copies, rounded to T at the end.
 #pragma once
+#include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <cuda_runtime.h>
 
 #include "dcn_common.cuh"
@@ -36,6 +45,63 @@ namespace dcn {
 namespace gather {
 
 constexpr int kThreads = 256;
+
+__device__ __forceinline__ float widen(float v) { return v; }
+__device__ __forceinline__ float widen(__nv_bfloat16 v) { return __bfloat162float(v); }
+__device__ __forceinline__ float widen(__half v) { return __half2float(v); }
+
+// one element: loaded and widened, rounded and stored
+template <class T>
+__device__ __forceinline__ float ld1(const T* p) { return widen(*p); }
+__device__ __forceinline__ void st1(float* p, float v) { *p = v; }
+__device__ __forceinline__ void st1(__nv_bfloat16* p, float v) { *p = __float2bfloat16_rn(v); }
+__device__ __forceinline__ void st1(__half* p, float v) { *p = __float2half_rn(v); }
+
+// the 16 bits of a half type at bit 16*k of u, widened; v rounded to T, as bits
+template <class T>
+__device__ __forceinline__ float widen_bits(unsigned u, int k);
+template <>
+__device__ __forceinline__ float widen_bits<__nv_bfloat16>(unsigned u, int k) {
+  return __uint_as_float(k ? u & 0xffff0000u : u << 16);
+}
+template <>
+__device__ __forceinline__ float widen_bits<__half>(unsigned u, int k) {
+  return __half2float(__ushort_as_half((unsigned short)(k ? u >> 16 : u & 0xffffu)));
+}
+__device__ __forceinline__ unsigned narrow_bits(float v, __nv_bfloat16*) {
+  return __bfloat16_as_ushort(__float2bfloat16_rn(v));
+}
+__device__ __forceinline__ unsigned narrow_bits(float v, __half*) { return __half_as_ushort(__float2half_rn(v)); }
+template <class T>
+__device__ __forceinline__ unsigned narrow_pair(float lo, float hi) {
+  return narrow_bits(lo, (T*)nullptr) | narrow_bits(hi, (T*)nullptr) << 16;
+}
+
+// a pair, 8-byte (float) or 4-byte (half types) aligned
+__device__ __forceinline__ float2 ld2(const float* p) { return *reinterpret_cast<const float2*>(p); }
+template <class T>
+__device__ __forceinline__ float2 ld2(const T* p) {
+  const unsigned u = *reinterpret_cast<const unsigned*>(p);
+  return make_float2(widen_bits<T>(u, 0), widen_bits<T>(u, 1));
+}
+__device__ __forceinline__ void st2(float* p, float2 v) { *reinterpret_cast<float2*>(p) = v; }
+template <class T>
+__device__ __forceinline__ void st2(T* p, float2 v) {
+  *reinterpret_cast<unsigned*>(p) = narrow_pair<T>(v.x, v.y);
+}
+
+// 4 channels, read-only path: 16-byte (float) or 8-byte (half types) aligned
+__device__ __forceinline__ float4 ld4(const float* p) { return __ldg(reinterpret_cast<const float4*>(p)); }
+template <class T>
+__device__ __forceinline__ float4 ld4(const T* p) {
+  const uint2 u = __ldg(reinterpret_cast<const uint2*>(p));
+  return make_float4(widen_bits<T>(u.x, 0), widen_bits<T>(u.x, 1), widen_bits<T>(u.y, 0), widen_bits<T>(u.y, 1));
+}
+__device__ __forceinline__ void st4(float* p, float4 v) { *reinterpret_cast<float4*>(p) = v; }
+template <class T>
+__device__ __forceinline__ void st4(T* p, float4 v) {
+  *reinterpret_cast<uint2*>(p) = make_uint2(narrow_pair<T>(v.x, v.y), narrow_pair<T>(v.z, v.w));
+}
 
 // One sampling point after the coordinate chain.  mask bit k: corner k (NW, NE, SW, SE) lies inside the image and its
 // token index inside [0, S).  base = token of the NW corner (meaningful only when mask != 0).
@@ -47,14 +113,14 @@ struct Smp {
 
 __device__ __forceinline__ Smp empty_sample() { return Smp{0, 0, 0u, 0.f, 0.f, 0.f}; }
 
-// Src::Rows of the dense layout: loc [items, L*P, 2] with one float2 per sample, attn [items, L*P], gradients alike.
+// Src::Rows of the dense layout: loc [items, L*P, 2] with one pair per sample, attn [items, L*P], gradients alike.
 struct DenseRows {
   template <class A>
-  static __device__ __forceinline__ const float* loc_row(const A& a, int item, int LP) {
+  static __device__ __forceinline__ auto loc_row(const A& a, int item, int LP) {
     return a.loc + (size_t)item * LP * 2;
   }
   template <class A>
-  static __device__ __forceinline__ const float* attn_row(const A& a, int item, int LP) {
+  static __device__ __forceinline__ auto attn_row(const A& a, int item, int LP) {
     return a.attn + (size_t)item * LP;
   }
   template <class A>
@@ -63,11 +129,11 @@ struct DenseRows {
   }
   template <class A>
   static __device__ __forceinline__ void store_gattn(const A& a, size_t o, int, float v) {
-    a.gattn[o] = v;
+    st1(a.gattn + o, v);
   }
   template <class A>
   static __device__ __forceinline__ void store_gloc(const A& a, size_t o, int, float2 v) {
-    *reinterpret_cast<float2*>(a.gloc + 2 * o) = v;
+    st2(a.gloc + 2 * o, v);
   }
   template <int G, class A>
   static __device__ __forceinline__ void end_grad(const A&, int, int, bool) {}
@@ -141,11 +207,11 @@ __device__ __forceinline__ void fwd_body(const Src& src) {
   const int LP = a.L * a.P;
   const int m = item % a.M, b = item / (a.Q * a.M);
   using Rows = typename Src::Rows;
-  const float* locp = Rows::loc_row(a, item, LP);
-  const float* attnp = Rows::attn_row(a, item, LP);
+  const auto locp = Rows::loc_row(a, item, LP);
+  const auto attnp = Rows::attn_row(a, item, LP);
   const typename Src::Item it = src.template begin<G>(item, j, attnp);
-  const size_t row = (size_t)a.M * a.D;  // floats per token
-  const float* vb = a.value + ((size_t)b * a.S * a.M + m) * a.D + 4 * j;
+  const size_t row = (size_t)a.M * a.D;  // elements per token
+  const auto vb = a.value + ((size_t)b * a.S * a.M + m) * a.D + 4 * j;
   float4 acc[V];
 #pragma unroll
   for (int v = 0; v < V; ++v) acc[v] = make_float4(0.f, 0.f, 0.f, 0.f);
@@ -168,7 +234,7 @@ __device__ __forceinline__ void fwd_body(const Src& src) {
           if (!(sm.mask & (1u << c))) continue;
           const int t = sm.base + corner_delta(c, sm.W);
           DCN_DEV_ASSERT(t >= 0 && t < a.S && 4 * j + 4 * G * v < a.D);
-          val = axpy4(w[c], __ldg(reinterpret_cast<const float4*>(vb + (size_t)t * row + 4 * G * v)), val);
+          val = axpy4(w[c], ld4(vb + (size_t)t * row + 4 * G * v), val);
         }
         acc[v] = axpy4(sm.a, val, acc[v]);
       }
@@ -176,8 +242,7 @@ __device__ __forceinline__ void fwd_body(const Src& src) {
   }
   if (!live) return;
 #pragma unroll
-  for (int v = 0; v < V; ++v)
-    *reinterpret_cast<float4*>(a.out + (size_t)item * a.D + 4 * j + 4 * G * v) = acc[v];
+  for (int v = 0; v < V; ++v) st4(a.out + (size_t)item * a.D + 4 * j + 4 * G * v, acc[v]);
 }
 
 template <int G, int V, class Src>
@@ -194,12 +259,12 @@ __device__ __forceinline__ void bwd_body(const Src& src) {
   const int LP = a.L * a.P;
   const int m = item % a.M, b = item / (a.Q * a.M);
   using Rows = typename Src::Rows;
-  const float* locp = Rows::loc_row(a, item, LP);
-  const float* attnp = Rows::attn_row(a, item, LP);
+  const auto locp = Rows::loc_row(a, item, LP);
+  const auto attnp = Rows::attn_row(a, item, LP);
   const typename Src::Item it = src.template begin<G>(item, j, attnp);
   const size_t row = (size_t)a.M * a.D;
   const size_t vofs = ((size_t)b * a.S * a.M + m) * a.D + 4 * j;
-  const float* vb = a.value + vofs;
+  const auto vb = a.value + vofs;
   float* gvb = a.gvalue ? a.gvalue + vofs : nullptr;
   const bool coord = a.gloc || a.gattn;
   float keep_m[R], keep_g[R];
@@ -208,8 +273,7 @@ __device__ __forceinline__ void bwd_body(const Src& src) {
   float4 g[V];
 #pragma unroll
   for (int v = 0; v < V; ++v)
-    g[v] = live ? __ldg(reinterpret_cast<const float4*>(a.gout + (size_t)item * a.D + 4 * j + 4 * G * v))
-                : make_float4(0.f, 0.f, 0.f, 0.f);
+    g[v] = live ? ld4(a.gout + (size_t)item * a.D + 4 * j + 4 * G * v) : make_float4(0.f, 0.f, 0.f, 0.f);
   for (int s0 = 0; s0 < LP; s0 += K) {
     Smp own = empty_sample();
     if (live && j < K && s0 + j < LP) own = src.sample(it, locp, attnp, s0 + j);
@@ -235,7 +299,7 @@ __device__ __forceinline__ void bwd_body(const Src& src) {
             const float aw = sm.a * w[cn];
             atomicAdd(reinterpret_cast<float4*>(gvb + o), make_float4(aw * g[v].x, aw * g[v].y, aw * g[v].z, aw * g[v].w));
           }
-          if (coord) c[cn] = __ldg(reinterpret_cast<const float4*>(vb + o));
+          if (coord) c[cn] = ld4(vb + o);
         }
         if (coord) {
           float4 bil = make_float4(0.f, 0.f, 0.f, 0.f);

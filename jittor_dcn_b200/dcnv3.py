@@ -138,10 +138,12 @@ class DCNv3(nn.Module):
         offset = self.offset(x1)
         mask = self.mask(x1).reshape(N, H, W, -1)  # logits: the core applies the per-group softmax
 
-        # the core is float32: under autocast its operands are cast up and its output back to the layer's dtype
+        # all-bfloat16 or all-float16 operands (autocast, module.half()) go to the core as they are; any other mix runs
+        # on float32 copies, and the output comes back in x's dtype
+        half = x.dtype in (torch.bfloat16, torch.float16) and offset.dtype == mask.dtype == x.dtype
         with torch.autocast(device_type=input.device.type, enabled=False):
             x = DCNv3Function.apply(
-                x.float(), offset.float(), mask.float(),
+                *((x, offset, mask) if half else (x.float(), offset.float(), mask.float())),
                 self.kernel_size, self.kernel_size,
                 self.stride, self.stride,
                 self.pad, self.pad,

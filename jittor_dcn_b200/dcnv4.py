@@ -109,10 +109,12 @@ class DCNv4(nn.Module):
 
         x_proj = x
         dtype = x.dtype
-        # the core is float32: under autocast its operands are cast up and its output back to the layer's dtype
+        # bfloat16 or float16 x and offset_mask of one dtype (autocast, module.half()) go to the core as they are; any
+        # other mix (e.g. without_pointwise under autocast) runs on float32 copies, and the output comes back in x's dtype
+        half = x.dtype in (torch.bfloat16, torch.float16) and offset_mask.dtype == x.dtype
         with torch.autocast(device_type=input.device.type, enabled=False):
             x = DCNv4Function.apply(
-                x.float(), offset_mask.float(),
+                *((x, offset_mask) if half else (x.float(), offset_mask.float())),
                 self.kernel_size, self.kernel_size,
                 self.stride, self.stride,
                 self.pad, self.pad,

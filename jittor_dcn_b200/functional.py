@@ -8,9 +8,10 @@ import ctypes
 import torch
 
 from . import _lib
-from ._lib import (FLAG_ACCUM_GRAD_X, FLAG_FORCE_SIMT, FLAG_NO_GRAD_X, FLAG_RELU_OUT, FLAG_XT_STAGED, OPERAND_BF16, OPERAND_FP32,
-                   PHASE_BACKWARD, PHASE_FORWARD, PHASE_LAYER_BACKWARD, PHASE_LAYER_BACKWARD_MODULATED,
-                   PHASE_LAYER_FORWARD, PHASE_LAYER_FORWARD_MODULATED, VARIANT_DCNV1, VARIANT_JITTOR, VARIANT_TORCH)
+from ._lib import (FLAG_ACCUM_GRAD_X, FLAG_FORCE_SIMT, FLAG_NO_GRAD_X, FLAG_RELU_OUT, FLAG_XT_STAGED, OPERAND_BF16,
+                   OPERAND_FP16, OPERAND_FP32, PHASE_BACKWARD, PHASE_FORWARD, PHASE_LAYER_BACKWARD,
+                   PHASE_LAYER_BACKWARD_MODULATED, PHASE_LAYER_FORWARD, PHASE_LAYER_FORWARD_MODULATED, VARIANT_DCNV1,
+                   VARIANT_JITTOR, VARIANT_TORCH)
 
 _workspaces = {}
 _captured = []   # scratch buffers whose addresses are baked into CUDA graphs: alive until clear_workspaces()
@@ -885,14 +886,22 @@ def ms_deform_attn(value, spatial_shapes, level_start_index, sampling_locations,
 
 
 # ---- DCNv3 (InternImage's ops_dcnv3 core; csrc/dcn_dcnv3.cu) ------------------------------------------------------
+# the operand types of the DCNv3 / DCNv4 kernels: every tensor of a call but grad_input is of one of these
+_CORE_OPERANDS = {torch.float32: OPERAND_FP32, torch.bfloat16: OPERAND_BF16, torch.float16: OPERAND_FP16}
+
+
 def _grid_inputs(what, floats, kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w, dilation_h, dilation_w, group,
                  group_channels):
     """The checks DCNv3 and DCNv4 share, on tensor metadata only: dtypes and devices of `floats` ((name, tensor), input
     first), the geometry and the input's shape -> (N, H, W, C, Ho, Wo)."""
-    for name, t in floats:
-        if not isinstance(t, torch.Tensor) or t.dtype != torch.float32:
-            raise ValueError(f"{what}: {name} must be a float32 tensor, got "
-                             f"{getattr(t, 'dtype', type(t).__name__)} (the kernels are float32 only)")
+    # named: the first non-tensor, or else the first tensor that is not float32 (any refused mix of dtypes has one)
+    bad = [(n, t) for n, t in floats if not isinstance(t, torch.Tensor)]
+    if not bad and (len({t.dtype for _, t in floats}) != 1 or floats[0][1].dtype not in _CORE_OPERANDS):
+        bad = [(n, t) for n, t in floats if t.dtype != torch.float32]
+    if bad:
+        name, t = bad[0]
+        raise ValueError(f"{what}: {name} must be a float32 tensor, got {getattr(t, 'dtype', type(t).__name__)} "
+                         f"({', '.join(n for n, _ in floats)} must share one dtype: float32, bfloat16 or float16)")
     for name, t in floats:
         if not t.is_cuda:
             raise ValueError(f"{what}: {name} must be a CUDA tensor: there is no CPU path")
@@ -925,7 +934,7 @@ def _grid_inputs(what, floats, kernel_h, kernel_w, stride_h, stride_w, pad_h, pa
 def _dcnv3_inputs(input, offset, mask, kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w, dilation_h, dilation_w,
                   group, group_channels, softmax_mask):
     """Checks shapes, dtypes and devices from tensor metadata only (no host synchronisation, so the call can be
-    captured in a CUDA graph) -> (DcnV3Shape, dense 16-byte aligned input, offset, mask)."""
+    captured in a CUDA graph) -> (DcnV3Shape, dense 16-byte aligned input, offset, mask), all of input's dtype."""
     N, H, W, C, Ho, Wo = _grid_inputs("dcnv3", (("input", input), ("offset", offset), ("mask", mask)), kernel_h,
                                       kernel_w, stride_h, stride_w, pad_h, pad_w, dilation_h, dilation_w, group,
                                       group_channels)
@@ -939,7 +948,8 @@ def _dcnv3_inputs(input, offset, mask, kernel_h, kernel_w, stride_h, stride_w, p
         raise ValueError(f"dcnv3: an extent of {(N, H, W, C)} exceeds 2^31 - 1")
     shp = _lib.DcnV3Shape(N, H, W, group, group_channels, kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w,
                           dilation_h, dilation_w, _lib.DCN_V3_FLAG_SOFTMAX_MASK if softmax_mask else 0)
-    return shp, _dev_ready(input), _dev_ready(offset), _dev_ready(mask)
+    dt = input.dtype
+    return shp, _dev_ready(input, dt), _dev_ready(offset, dt), _dev_ready(mask, dt)
 
 
 def dcn_v3_forward(input, offset, mask, kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w, dilation_h, dilation_w,
@@ -948,8 +958,8 @@ def dcn_v3_forward(input, offset, mask, kernel_h, kernel_w, stride_h, stride_w, 
     holds logits and the core applies InternImage's softmax over the kernel_h*kernel_w points of each group."""
     shp, x, off, m = _dcnv3_inputs(input, offset, mask, kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w,
                                    dilation_h, dilation_w, group, group_channels, softmax_mask)
-    out = torch.empty(tuple(off.shape[:3]) + (group * group_channels,), dtype=torch.float32, device=x.device)
-    _run("dcn_v3_forward", x.device, shp, (float(offset_scale), x, off, m, out))
+    out = torch.empty(tuple(off.shape[:3]) + (group * group_channels,), dtype=x.dtype, device=x.device)
+    _run("dcn_v3_forward_typed", x.device, shp, (_CORE_OPERANDS[x.dtype], float(offset_scale), x, off, m, out))
     return out
 
 
@@ -962,12 +972,15 @@ def dcn_v3_backward(input, offset, mask, grad_out, kernel_h, kernel_w, stride_h,
     want = tuple(off.shape[:3]) + (group * group_channels,)
     if not isinstance(grad_out, torch.Tensor) or tuple(grad_out.shape) != want:
         raise ValueError(f"dcnv3: grad_out shape {tuple(getattr(grad_out, 'shape', ()))} != {want}")
-    go = _dev_ready(_to_device(grad_out, x.device))
-    gx, goff, gm = (torch.empty_like(t) if n else None for t, n in zip((x, off, m), need))
+    go = _dev_ready(_to_device(grad_out, x.device), x.dtype)
+    # grad_input accumulates in float32 (the kernels' atomics), then comes back in input's dtype
+    gx = torch.empty_like(x, dtype=torch.float32) if need[0] else None
+    goff, gm = (torch.empty_like(t) if n else None for t, n in zip((off, m), need[1:]))
     if gx is None and goff is None and gm is None:
         return None, None, None
-    _run("dcn_v3_backward", x.device, shp, (float(offset_scale), x, off, m, go, gx, goff, gm))
-    return gx, goff, gm
+    _run("dcn_v3_backward_typed", x.device, shp,
+         (_CORE_OPERANDS[x.dtype], float(offset_scale), x, off, m, go, gx, goff, gm))
+    return (None if gx is None else gx.to(x.dtype)), goff, gm
 
 
 class DCNv3Function(torch.autograd.Function):
@@ -978,7 +991,8 @@ class DCNv3Function(torch.autograd.Function):
                             remove_center=False) -> [N, Ho, Wo, group*group_channels]
 
     input [N, H, W, group*group_channels], offset [N, Ho, Wo, group*P*2] ((dx, dy) per point, points x-major:
-    p = i*kernel_h + j for kernel column i and row j), mask [N, Ho, Wo, group*P], float32 on one CUDA device.
+    p = i*kernel_h + j for kernel column i and row j), mask [N, Ho, Wo, group*P], on one CUDA device and all float32,
+    all bfloat16 or all float16; the output and the gradients come back in that dtype.
     ``im2col_step`` is accepted and ignored: it exists only so that calls written for InternImage run unchanged.
     ``remove_center=True`` is refused.  A trailing ``softmax_mask=True`` (not in InternImage's signature) makes `mask`
     logits and applies InternImage's per-group softmax inside the node.  Differentiable in input, offset and mask;
@@ -1044,7 +1058,8 @@ def _dcnv4_inputs(input, offset_mask, kernel_h, kernel_w, stride_h, stride_w, pa
         raise ValueError(f"dcnv4: an extent of {(N, H, W, C)} exceeds 2^31 - 1")
     shp = _lib.DcnV3Shape(N, H, W, group, group_channels, kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w,
                           dilation_h, dilation_w, _lib.DCN_V4_FLAG_REMOVE_CENTER if rc else 0)
-    return shp, _dev_ready(input), _dev_ready(offset_mask)
+    dt = input.dtype
+    return shp, _dev_ready(input, dt), _dev_ready(offset_mask, dt)
 
 
 def dcn_v4_forward(input, offset_mask, kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w, dilation_h, dilation_w,
@@ -1052,8 +1067,8 @@ def dcn_v4_forward(input, offset_mask, kernel_h, kernel_w, stride_h, stride_w, p
     """out [N, Ho, Wo, group*group_channels] of the DCNv4 core on CUDA tensors (no autograd)."""
     shp, x, om = _dcnv4_inputs(input, offset_mask, kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w, dilation_h,
                                dilation_w, group, group_channels, remove_center)
-    out = torch.empty(tuple(om.shape[:3]) + (group * group_channels,), dtype=torch.float32, device=x.device)
-    _run("dcn_v4_forward", x.device, shp, (float(offset_scale), x, om, out))
+    out = torch.empty(tuple(om.shape[:3]) + (group * group_channels,), dtype=x.dtype, device=x.device)
+    _run("dcn_v4_forward_typed", x.device, shp, (_CORE_OPERANDS[x.dtype], float(offset_scale), x, om, out))
     return out
 
 
@@ -1066,12 +1081,15 @@ def dcn_v4_backward(input, offset_mask, grad_out, kernel_h, kernel_w, stride_h, 
     want = tuple(om.shape[:3]) + (group * group_channels,)
     if not isinstance(grad_out, torch.Tensor) or tuple(grad_out.shape) != want:
         raise ValueError(f"dcnv4: grad_out shape {tuple(getattr(grad_out, 'shape', ()))} != {want}")
-    go = _dev_ready(_to_device(grad_out, x.device))
-    gx, gom = (torch.empty_like(t) if n else None for t, n in zip((x, om), need))
+    go = _dev_ready(_to_device(grad_out, x.device), x.dtype)
+    # grad_input accumulates in float32 (the kernels' atomics), then comes back in input's dtype
+    gx = torch.empty_like(x, dtype=torch.float32) if need[0] else None
+    gom = torch.empty_like(om) if need[1] else None
     if gx is None and gom is None:
         return None, None
-    _run("dcn_v4_backward", x.device, shp, (float(offset_scale), x, om, go, gx, gom))
-    return gx, gom
+    _run("dcn_v4_backward_typed", x.device, shp,
+         (_CORE_OPERANDS[x.dtype], float(offset_scale), x, om, go, gx, gom))
+    return (None if gx is None else gx.to(x.dtype)), gom
 
 
 class DCNv4Function(torch.autograd.Function):
@@ -1085,7 +1103,8 @@ class DCNv4Function(torch.autograd.Function):
     K = kernel_h*kernel_w - remove_center: group g owns floats [g*3K, g*3K + 3K) of each pixel, first K interleaved
     (dx, dy) offsets, then K mask values (used as given: no softmax); the remaining columns are padding and never read.
     Points are DCNv3's, x-major (p = i*kernel_h + j for kernel column i and row j), with the centre point of an odd
-    kernel dropped when remove_center is set.  float32 on one CUDA device.  ``im2col_step`` is accepted and ignored.
+    kernel dropped when remove_center is set.  input and offset_mask on one CUDA device, both float32, bfloat16 or
+    float16; the output and the gradients come back in that dtype.  ``im2col_step`` is accepted and ignored.
     Differentiable in input and offset_mask; only the gradients autograd asks for are computed, and the node never
     synchronises with the host."""
 
